@@ -1,12 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- log-density+gradient match-evaluations per second (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch: one `bplx_logdensity_fwdbwd` call for all the chains of
-this GPU.  The workload is the configuration the metric is quoted on, BASELINE.json configs[2]
-(NeutralDixonColesMatchPredictorWC, 220 teams, 40,000 weighted matches, 32,768 chains): at N GPUs the 32,768
-chains are partitioned over the ranks (STRONG scaling, chains are independent: no data-path collective).
+this GPU; the timed windows of `value` and of `e2e` are exactly K steps each.  The workload is the configuration
+the metric is quoted on, BASELINE.json configs[2] (NeutralDixonColesMatchPredictorWC, 220 teams, 40,000 weighted
+matches, 32,768 chains): at N GPUs the 32,768 chains are partitioned over the ranks (STRONG scaling, chains are independent: no data-path collective).
 `value` times the kernel with inputs resident in HBM (CUDA graph of K launches over rotating buffer sets larger
 than L2, CUDA events on the launch stream, max over ranks); `e2e` goes through the host-buffer C-ABI call with
 pinned host arrays, copies inside the timed region.  Two sub-records are timed on all ranks: the configs[4]
@@ -31,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree, which may be read-only
 
 L2_BYTES = 126e6
 FLOPS_PER_EVAL = {"dixon_coles": 26, "extended": 30, "neutral": 40, "neutral_wc": 46, "dynamic": 40}  # SURVEY.md 8(d)
@@ -159,8 +160,8 @@ def parity_sample(arr, theta_dc, lp, grad, cc, nsample=8, seed=0):
 
 
 def time_logdensity(problem, C, steps, warmup, radius, seed, use_graph=True, target_s=1.0, arr=None, pad_rows=False):
-    """Median device time of a K-step region (ms) over several repetitions; inputs rotate through buffer sets whose
-    total size exceeds the L2 whatever K is."""
+    """Device time of a K-step region (ms): of one region when target_s is 0, else the median over repetitions for
+    target_s seconds; inputs rotate through buffer sets whose total size exceeds the L2 whatever K is."""
     import torch
 
     from bpl_next_b200 import _abi
@@ -223,8 +224,28 @@ def time_logdensity(problem, C, steps, warmup, radius, seed, use_graph=True, tar
             if time.perf_counter() - t_start > target_s or len(times) >= 400:
                 break
     finite = bool(torch.isfinite(lps[0]).all().item())
+    last = (steps - 1) % nb  # the buffer set the last step of the region wrote
     return {"ms": float(np.median(times)), "reps": len(times), "nb": nb, "set_bytes": set_bytes, "finite": finite, "ld": ld,
-            "launches": launches, "parity": parity}
+            "launches": launches, "parity": parity, "last": (lps[last], grads[last], ccs[last])}
+
+
+DUMP_GRAD_BYTES = 48 << 20
+
+
+def dump_outputs(out_dir, lp, grad, corr_coef, suffix=""):
+    """The outputs of one log-density call as float32 .npy files: lp [C], corr_coef [C] and grad [D, C].  A gradient
+    larger than DUMP_GRAD_BYTES is written for a sample of chains only: the columns np.random.default_rng(0) draws
+    without replacement, in ascending order, so that runs with the same arguments write the same chains."""
+    import torch
+
+    D, C = grad.shape
+    n = min(C, DUMP_GRAD_BYTES // (4 * D))
+    if n < C:
+        cols = np.sort(np.random.default_rng(0).choice(C, n, replace=False))
+        grad = grad[:, torch.from_numpy(cols).to(grad.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("lp", lp), ("grad", grad), ("corr_coef", corr_coef)):
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), t.cpu().numpy().astype(np.float32))
 
 
 def time_e2e(problem, C, steps, warmup, radius, seed):
@@ -562,7 +583,13 @@ def main():
                          "before the mass matrix is adapted every transition of this 1,339-parameter posterior runs to the "
                          "cap, so the sub-record is a timing of the sharded fit path, not a converged posterior -- see rhat_max)")
     ap.add_argument("--fit-max-launches", type=int, default=0, help="cap on log-density launches of the fit sub-record (0: none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write lp, grad and corr_coef of the last one as DIR/<name>.npy (float32; "
+                         "grad [D, chains] for a fixed sample of chains when it is larger than 48 MiB; one set per rank, "
+                         "suffixed _rank<r>, when there are several)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -608,16 +635,19 @@ def main():
     barrier()
     with ClockSampler(local) as clk:
         r = time_logdensity(problem, C, args.steps, args.warmup, args.radius, args.seed + 1 + rank,
-                            use_graph=not args.no_graph, arr=arr if rank == 0 else None, pad_rows=args.pad_rows)
+                            use_graph=not args.no_graph, target_s=0, arr=arr if rank == 0 else None, pad_rows=args.pad_rows)
     barrier()
     ms = max_over_ranks(r["ms"])
     value = units_total * arr.num_matches * args.steps / (ms * 1e-3)
+    last = r.pop("last")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last, suffix=f"_rank{rank}" if world > 1 else "")
+    del last
 
     # ---- end to end (host buffers) ---------------------------------------------------------------------
     barrier()
-    e2e_steps = min(args.steps, 20) if C * problem.D * 4 > 64e6 else args.steps
-    dt, h2d, d2h = time_e2e(problem, C, e2e_steps, args.warmup, args.radius, args.seed + 7 + rank)
-    e2e_value = units_total * arr.num_matches * e2e_steps / max_over_ranks(dt)
+    dt, h2d, d2h = time_e2e(problem, C, args.steps, args.warmup, args.radius, args.seed + 7 + rank)
+    e2e_value = units_total * arr.num_matches * args.steps / max_over_ranks(dt)
     barrier()
 
     # ---- sub-records on all ranks -------------------------------------------------------------------------
@@ -678,8 +708,8 @@ def main():
                        "layout": f"chain-minor [D, C] resident in HBM, row pitch {r['ld']} floats",
                        "l2": f"inputs rotate through {r['nb']} buffer sets of {r['set_bytes'] / 1e6:.1f} MB each "
                              f"({r['nb'] * r['set_bytes'] / 1e6:.0f} MB > 126 MB L2)",
-                       "timing": f"{'CUDA graph of' if not args.no_graph else ''} {args.steps} launches, CUDA events on "
-                                 f"the launch stream, median of {r['reps']} repetitions, max over ranks",
+                       "timing": f"{'one replay of a CUDA graph of' if not args.no_graph else ''} {args.steps} launches, "
+                                 "CUDA events on the launch stream, max over ranks",
                        "waves": {"chain_groups_per_gpu": groups, "sms": 148, "waves": groups / 148.0,
                                  "quantisation_efficiency": groups / (148.0 * math.ceil(groups / 148.0)),
                                  "launches_per_step": r["launches"] / max(args.steps, 1),
@@ -688,7 +718,7 @@ def main():
                        "plan": st},
             "clocks": clk.summary(),
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "steps": e2e_steps,
+                    "steps": args.steps,
                     "api": "bplx_logdensity_fwdbwd_host (pinned numpy in/out, chain-major [C, D]; transposed on the device to "
                            "the native layout, copies and kernels pipelined in chunks)"},
             "gpu_launches": r["launches"],

@@ -4,6 +4,7 @@ here) and its three implementations called the way XLA's executor would: typed b
 result buffers, the stream.  The numbers must be those of the C ABI called directly."""
 import ctypes as C
 import os
+import shutil
 import subprocess
 
 import numpy as np
@@ -15,10 +16,17 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIBDIR = os.path.join(ROOT, "bpl_next_b200", "lib")
 
 
+def _cuda_include():
+    """include/ of the CUDA toolkit whose nvcc builds the library (NVCC, else nvcc on PATH)."""
+    nvcc = shutil.which(os.environ.get("NVCC", "nvcc"))
+    assert nvcc, "nvcc not found"
+    return os.path.join(os.path.dirname(os.path.dirname(os.path.realpath(nvcc))), "include")
+
+
 def _build(tmp_path):
     so = str(tmp_path / "libmockxla.so")
     cmd = ["g++", "-O1", "-std=c++17", "-shared", "-fPIC", "-Wall", "-Wno-comment", "-Werror",
-           "-I", os.path.join(ROOT, "tests", "xla_ffi_mock"), "-I", os.path.join(ROOT, "include"), "-I", "/usr/local/cuda/include",
+           "-I", os.path.join(ROOT, "tests", "xla_ffi_mock"), "-I", os.path.join(ROOT, "include"), "-I", _cuda_include(),
            os.path.join(ROOT, "tests", "xla_ffi_mock", "drive.cc"), "-L", LIBDIR, "-lbplx", f"-Wl,-rpath,{LIBDIR}", "-o", so]
     r = subprocess.run(cmd, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr

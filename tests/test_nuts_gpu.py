@@ -326,7 +326,8 @@ def test_chain_major_and_chain_minor_state_take_the_same_first_transitions():
     a, b = runs[0].samples[0], runs[1].samples[0]  # [D, C]
     same = ((a - b).abs().max(dim=0).values < 1e-3).float().mean().item()
     assert same > 0.95, same
-    assert torch.allclose(runs[0].lp[0], runs[1].lp[0], rtol=1e-3, atol=1e-2) or same > 0.95
+    close = (a - b).abs().max(dim=0).values < 1e-3  # the chains whose draws agree have the same log-density there
+    assert torch.allclose(runs[0].lp[0][close], runs[1].lp[0][close], rtol=1e-3, atol=1e-2)
     assert (runs[0].num_leapfrog == runs[1].num_leapfrog).mean() > 0.9
 
 

@@ -54,6 +54,13 @@ class Fixtures(C.Structure):
     ]
 
 
+class Observations(C.Structure):
+    _fields_ = [("fixtures", Fixtures), ("home_goals", C.c_void_p), ("away_goals", C.c_void_p)]
+
+
+PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
+
+
 class BplxError(RuntimeError):
     def __init__(self, status: int, message: str):
         super().__init__(f"bplx status {status}: {message}")
@@ -98,6 +105,12 @@ def declare(lib):
     lib.bplx_score_grid_ex.restype = i
     lib.bplx_score_grid_host.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), i, C.c_float, vp, vp]
     lib.bplx_score_grid_host.restype = i
+    lib.bplx_pointwise_loglik_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Observations)]
+    lib.bplx_pointwise_loglik_workspace_bytes.restype = sz
+    lib.bplx_pointwise_loglik.argtypes = [C.POINTER(Samples), C.POINTER(Observations), vp, sz, vp, vp, sz, vp]
+    lib.bplx_pointwise_loglik.restype = i
+    lib.bplx_psis_loo.argtypes = [vp, i, i, sz, C.c_double, vp, vp, vp, sz, vp]
+    lib.bplx_psis_loo.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

@@ -11,6 +11,7 @@
 #include "common.cuh"
 #include "plan.h"
 #include "problem.h"
+#include "loo.h"
 #include "score_grid.h"
 
 namespace bplx {
@@ -550,22 +551,29 @@ int bplx_logdensity_fwdbwd_host(bplx_problem* p, int C, const float* theta, floa
 }
 
 // ---- score grid ------------------------------------------------------------------------------------------
-static int check_grid_args(const bplx_samples* s, const bplx_fixtures* f, int max_goals) {
+// samples / fixtures checks shared by the score grid and the pointwise log-likelihood (`what` prefixes the message)
+static int check_sample_args(const bplx_samples* s, const bplx_fixtures* f, const char* what) {
   BPLX_REQUIRE(s && f, BPLX_E_INVALID, "samples / fixtures is NULL");
   BPLX_REQUIRE(s->model >= BPLX_DIXON_COLES && s->model <= BPLX_NEUTRAL_WC, BPLX_E_UNSUPPORTED,
-               "score grid: model %d unsupported (DYNAMIC predict is unusable in the reference)", s->model);
+               "%s: model %d unsupported (DYNAMIC predict is unusable in the reference)", what, s->model);
   BPLX_REQUIRE(s->num_samples > 0 && s->num_teams > 0 && f->num_fixtures > 0, BPLX_E_INVALID,
-               "score grid: num_samples, num_teams and num_fixtures must be positive");
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "max_goals must be in [1, 63] (got %d)", max_goals);
+               "%s: num_samples, num_teams and num_fixtures must be positive", what);
   BPLX_REQUIRE(s->attack && s->defence && s->corr_coef && f->home_team && f->away_team, BPLX_E_INVALID,
-               "score grid: attack, defence, corr_coef, home_team, away_team must not be NULL");
-  BPLX_REQUIRE(s->home_attack, BPLX_E_INVALID, "score grid: home_attack (home advantage) must not be NULL");
+               "%s: attack, defence, corr_coef, home_team, away_team must not be NULL", what);
+  BPLX_REQUIRE(s->home_attack, BPLX_E_INVALID, "%s: home_attack (home advantage) must not be NULL", what);
   if (s->model == BPLX_NEUTRAL || s->model == BPLX_NEUTRAL_WC)
     BPLX_REQUIRE(s->away_attack && s->home_defence && s->away_defence, BPLX_E_INVALID,
-                 "score grid: neutral models need away_attack, home_defence, away_defence");
+                 "%s: neutral models need away_attack, home_defence, away_defence", what);
   if (s->model == BPLX_NEUTRAL_WC)
     BPLX_REQUIRE(s->confederation_strength && s->num_conferences > 0 && f->home_conf && f->away_conf, BPLX_E_INVALID,
-                 "score grid: NEUTRAL_WC needs confederation_strength, home_conf, away_conf");
+                 "%s: NEUTRAL_WC needs confederation_strength, home_conf, away_conf", what);
+  return BPLX_OK;
+}
+
+static int check_grid_args(const bplx_samples* s, const bplx_fixtures* f, int max_goals) {
+  const int rc = check_sample_args(s, f, "score grid");
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "max_goals must be in [1, 63] (got %d)", max_goals);
   return BPLX_OK;
 }
 
@@ -706,6 +714,89 @@ int bplx_score_grid_host(const bplx_samples* s, const bplx_fixtures* f, int max_
   cleanup();
   cudaStreamDestroy(st);
   return rc;
+}
+
+// ---- pointwise log-likelihood and PSIS-LOO -----------------------------------------------------------------------
+static size_t pointwise_plan_for(const bplx_samples* s, const bplx_observations* o, PointwiseParams* pp, const char** err) {
+  pp->gp.model = s->model;
+  pp->gp.S = s->num_samples;
+  pp->gp.T = s->num_teams;
+  pp->gp.Cf = s->model == BPLX_NEUTRAL_WC ? s->num_conferences : 0;
+  pp->gp.F = o->fixtures.num_fixtures;
+  return pointwise_plan(pp, err);
+}
+
+size_t bplx_pointwise_loglik_workspace_bytes(const bplx_samples* s, const bplx_observations* obs) {
+  if (!s || !obs || s->num_samples <= 0 || s->num_teams <= 0 || obs->fixtures.num_fixtures <= 0) return 0;
+  PointwiseParams pp{};
+  return pointwise_plan_for(s, obs, &pp, nullptr);
+}
+
+int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, float* loglik, size_t ld, double* stats,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+  BPLX_REQUIRE(obs != nullptr, BPLX_E_INVALID, "observations is NULL");
+  int rc = check_sample_args(s, &obs->fixtures, "pointwise log-likelihood");
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID,
+               "pointwise log-likelihood: home_goals and away_goals must not be NULL");
+  BPLX_REQUIRE(stats != nullptr, BPLX_E_INVALID, "pointwise log-likelihood: stats is NULL");
+  BPLX_REQUIRE(!loglik || ld >= (size_t)s->num_samples, BPLX_E_INVALID,
+               "pointwise log-likelihood: ld (%zu) < num_samples (%d)", ld, s->num_samples);
+  PointwiseParams pp{};
+  const char* perr = nullptr;
+  const size_t need = pointwise_plan_for(s, obs, &pp, &perr);
+  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
+  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
+               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  GridParams& gp = pp.gp;
+  gp.attack = s->attack;
+  gp.defence = s->defence;
+  gp.ha = s->home_attack;
+  gp.aa = s->away_attack;
+  gp.hd = s->home_defence;
+  gp.ad = s->away_defence;
+  gp.conf = s->confederation_strength;
+  gp.corr = s->corr_coef;
+  gp.home = obs->fixtures.home_team;
+  gp.away = obs->fixtures.away_team;
+  gp.hconf = obs->fixtures.home_conf;
+  gp.aconf = obs->fixtures.away_conf;
+  gp.nv = obs->fixtures.neutral_venue;
+  gp.table = static_cast<float*>(workspace);
+  pp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) +
+                                         ((size_t)gp.S * gp.row_floats * 4 + 255) / 256 * 256);
+  pp.hg = obs->home_goals;
+  pp.ag = obs->away_goals;
+  pp.ll = loglik;
+  pp.ld = ld;
+  pp.stats = stats;
+  return launch_pointwise(pp, static_cast<cudaStream_t>(stream));
+}
+
+int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t ld, double r_eff, double* elpd_i,
+                  double* pareto_k, void* workspace, size_t workspace_bytes, void* stream) {
+  (void)workspace;
+  (void)workspace_bytes;
+  BPLX_REQUIRE(loglik && elpd_i && pareto_k, BPLX_E_INVALID, "psis loo: loglik, elpd_i and pareto_k must not be NULL");
+  BPLX_REQUIRE(num_matches > 0 && num_samples > 0, BPLX_E_INVALID,
+               "psis loo: num_matches and num_samples must be positive (got %d, %d)", num_matches, num_samples);
+  BPLX_REQUIRE(ld >= (size_t)num_samples, BPLX_E_INVALID, "psis loo: ld (%zu) < num_samples (%d)", ld, num_samples);
+  BPLX_REQUIRE(r_eff > 0.0 && r_eff <= 1e300, BPLX_E_INVALID, "psis loo: r_eff must be positive and finite (got %g)", r_eff);
+  PsisParams pp{};
+  pp.Mt = psis_tail_length(num_samples, r_eff);
+  BPLX_REQUIRE(pp.Mt <= kPsisTailMax, BPLX_E_UNSUPPORTED,
+               "psis loo: a tail of %d draws (ceil(min(0.2 S, 3 sqrt(S / r_eff)))) exceeds the kernel's limit of %d "
+               "(BPLX_PSIS_MAX_TAIL)", pp.Mt, kPsisTailMax);
+  pp.cap = 8;
+  while (pp.cap < pp.Mt) pp.cap <<= 1;
+  pp.ll = loglik;
+  pp.ld = ld;
+  pp.M = num_matches;
+  pp.S = num_samples;
+  pp.elpd = elpd_i;
+  pp.khat = pareto_k;
+  return launch_psis(pp, static_cast<cudaStream_t>(stream));
 }
 
 void bplx_reload_env(void) {

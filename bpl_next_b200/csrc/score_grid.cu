@@ -40,19 +40,6 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-struct RowLayout {
-  int P1, Q1, P0, EC, C;  // float offsets inside a sample row
-};
-__host__ __device__ inline RowLayout row_layout(int T, int Cf, int ntab) {
-  RowLayout L;
-  L.P1 = 0;
-  L.Q1 = 2 * T;
-  L.P0 = 4 * T;
-  L.EC = 2 * T * ntab;
-  L.C = L.EC + 2 * Cf;
-  return L;
-}
-
 }  // namespace
 
 // ---- pre-pass: the exponential tables ------------------------------------------------------------------------------
@@ -355,6 +342,14 @@ size_t score_grid_plan(GridParams* gp, const char** err) {
   return table_bytes + (size_t)gp->nsplit * gp->F * gp->g * gp->g * sizeof(float);
 }
 
+int launch_score_grid_tables(const GridParams& gp, cudaStream_t stream) {
+  const long long n = (long long)gp.S * (gp.T + gp.Cf + 1);
+  score_grid_tables<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(gp);
+  BPLX_CUDA(cudaGetLastError());
+  note_launch(1);
+  return BPLX_OK;
+}
+
 template <int R, int CC, bool SINGLE>
 static int launch_tile(const GridParams& gp, int ntiles, size_t smem, cudaStream_t stream) {
   auto* fn = &score_grid_kernel<R, CC, SINGLE>;
@@ -398,10 +393,8 @@ int launch_score_grid(const GridParams& gp, cudaStream_t stream) {
   BPLX_REQUIRE(smem <= 227 * 1024, BPLX_E_UNSUPPORTED, "score grid needs %zu bytes of shared memory per CTA (max %d)", smem,
                227 * 1024);
   if (!gp.reuse_tables) {
-    const long long n = (long long)gp.S * (gp.T + gp.Cf + 1);
-    score_grid_tables<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(gp);
-    BPLX_CUDA(cudaGetLastError());
-    note_launch(1);
+    rc = launch_score_grid_tables(gp, stream);
+    if (rc != BPLX_OK) return rc;
   }
   rc = gp.g <= 11 ? launch_tile<11, 11, true>(gp, ntiles, smem, stream) : launch_tile<8, 16, false>(gp, ntiles, smem, stream);
   if (rc != BPLX_OK) return rc;

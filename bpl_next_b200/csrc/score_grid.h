@@ -9,6 +9,20 @@ constexpr int kGridStageMax = 16;   // posterior samples per TMA stage (fewer wh
 constexpr int kGridStages = 2;      // stage buffers
 constexpr int kGridStageBytes = 100 * 1024;  // budget of one stage buffer
 
+// float offsets of the per-team tables inside a sample row of the exponential table (see score_grid_tables)
+struct RowLayout {
+  int P1, Q1, P0, EC, C;
+};
+__host__ __device__ inline RowLayout row_layout(int T, int Cf, int ntab) {
+  RowLayout L;
+  L.P1 = 0;
+  L.Q1 = 2 * T;
+  L.P0 = 4 * T;
+  L.EC = 2 * T * ntab;
+  L.C = L.EC + 2 * Cf;
+  return L;
+}
+
 struct GridParams {
   int model, S, T, Cf, F, g;
   int nsplit, samples_per_split;
@@ -31,5 +45,7 @@ struct GridParams {
 // workspace bytes (table + partial sums); 0 with *err set when a sample row does not fit a stage buffer
 size_t score_grid_plan(GridParams* gp, const char** err);
 int launch_score_grid(const GridParams& gp, cudaStream_t stream);
+// the pre-pass alone: fills gp.table ([S][row_floats]) from the sample arrays; reads model, S, T, Cf, ntab, row_floats
+int launch_score_grid_tables(const GridParams& gp, cudaStream_t stream);
 
 }  // namespace bplx

@@ -11,18 +11,22 @@ from __future__ import annotations
 
 from typing import Any, Dict, Iterable, Optional, Union
 
+import hashlib
 import warnings
 from datetime import datetime
 
 import numpy as np
 import torch
 
+from . import compare as bcompare
 from . import data as bdata
 from . import nuts as bnuts
 from . import parallel
-from .problem import Problem, score_grid_host
+from .problem import Problem, pointwise_loglik, psis_loo, score_grid_host
 
 MAX_GOALS = bdata.MAX_GOALS
+# device memory for the [matches, draws] log-likelihood matrix of loo(): larger match sets are processed in ranges
+LOO_MATRIX_BYTES = 4 << 30
 
 
 def _str_to_list(*args):
@@ -101,6 +105,7 @@ class _BplxPredictor:
         self.teams, self._teams_dict = meta["teams"], meta["teams_dict"]
         self._meta = meta
         self.problem = p = Problem(arr)
+        self._train_arrays = arr  # the matches log_likelihood() / waic() / loo() evaluate by default
         flat_dev, cc = _run_chains(p, num_chains, random_state, num_warmup, num_samples, thin, kw, self)
         s = constrain(flat_dev.cpu().numpy(), p.layout)
         s["corr_coef"] = cc.cpu().numpy()
@@ -200,6 +205,7 @@ class _BplxPredictor:
             s = constrain(flat_dev.cpu().numpy(), p.layout)
             s["corr_coef"] = cc.cpu().numpy()
             self._set_posterior(arr, s)
+            self._train_arrays = arr
         return out
 
     @staticmethod
@@ -270,6 +276,107 @@ class _BplxPredictor:
 
     def _extras_from_args(self, args, kw):
         return kw
+
+    # ---- model comparison: pointwise log-likelihood, WAIC, PSIS-LOO, held-out log score ------------------------
+    # ll[s, m] = log Pois(yh; lh) + log Pois(ya; la) + log tau(yh, ya; lh, la, corr_coef_s), with the rates of the predict
+    # path (neutral venues, confederations; Extended's fit-time clip of the rates at 15 is not applied), tau clamped at 0
+    # (a match can give -inf) and NO match weights: exp(ll) averaged over s is what predict_score_proba returns.
+    def _observations(self, data=None):
+        """Observed matches as index / goal arrays (the training data when ``data`` is None), and a key naming them."""
+        if data is None:
+            arr = getattr(self, "_train_arrays", None)
+            if arr is None:
+                raise ValueError("no training data recorded: fit the model first, or pass data")
+            obs = {"home_team": arr.home_team, "away_team": arr.away_team}
+            for k in ("neutral_venue", "home_conf", "away_conf"):
+                if getattr(arr, k) is not None:
+                    obs[k] = np.asarray(getattr(arr, k), dtype=np.uint8)
+            hg, ag = arr.home_goals, arr.away_goals
+        else:  # fixture arguments mapped as predict_* maps them
+            h, a = self._parse_fixture_args(data["home_team"], data["away_team"])
+            kw = {k: data[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in data}
+            obs = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw)}
+            hg, ag = bdata._goals(data["home_goals"]), bdata._goals(data["away_goals"])
+        obs["home_goals"], obs["away_goals"] = np.asarray(hg, dtype=np.uint8), np.asarray(ag, dtype=np.uint8)
+        names = np.asarray(self.teams).astype(str)
+        key = hashlib.sha1("|".join(names[obs["home_team"].astype(np.int64)]).encode())
+        key.update("|".join(names[obs["away_team"].astype(np.int64)]).encode())
+        key.update(obs["home_goals"].tobytes() + obs["away_goals"].tobytes())
+        return obs, key.hexdigest()
+
+    def _comparison_inputs(self, data):
+        import torch
+
+        obs, key = self._observations(data)
+        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
+              if v is not None}
+        do = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in obs.items()}
+        return ds, do, key
+
+    def log_likelihood(self, data=None) -> np.ndarray:
+        """Pointwise log-likelihood ``[S, M]`` float32 (numpyro's ``log_likelihood`` shape: draws x observations) of
+        the observed scores of ``data`` (reference ``training_data`` keys; default: the training data).
+
+        ``ll[s, m] = log Pois(yh; lh) + log Pois(ya; la) + log tau(yh, ya; lh, la, corr_coef_s)``: the rates are those of
+        ``predict_*`` (neutral venues and confederations included; Extended's fit-time clip of rates at 15 is not
+        applied), tau is clamped at 0 so a match can give -inf, and the value is UNWEIGHTED -- for a fit with time decay
+        or game weights it is the predictive density of the match, not the weighted pseudo-likelihood that was fitted.
+        ``exp(ll)`` averaged over the draws is what ``predict_score_proba`` returns for that match."""
+        ds, do, _ = self._comparison_inputs(data)
+        ll, _ = pointwise_loglik(self.model, ds, do)
+        return np.ascontiguousarray(ll.cpu().numpy().T)
+
+    def waic(self, data=None) -> Dict[str, Any]:
+        """WAIC of the fit on ``data`` (default: the training data), from the pointwise log-likelihood of
+        ``log_likelihood`` (unweighted; see there) without storing it:
+        ``lppd_m = logsumexp_s ll - log S``, ``p_waic_m = var_s ll`` with divisor S (ddof 0),
+        ``elpd_waic_m = lppd_m - p_waic_m``.  Returns ``elpd_waic`` (sum), ``se = sqrt(M var0(elpd_waic_m))``,
+        ``p_waic``, ``lppd``, the pointwise arrays and ``match_key`` (names the matches, for ``compare``)."""
+        ds, do, key = self._comparison_inputs(data)
+        _, st = pointwise_loglik(self.model, ds, do, want_matrix=False)
+        return bcompare.waic_from_stats(st.cpu().numpy(), int(ds["attack"].shape[0]), key)
+
+    def loo(self, r_eff: float = 1.0) -> Dict[str, Any]:
+        """Pareto-smoothed importance-sampling leave-one-out cross-validation on the training data (ArviZ's ``loo``;
+        Vehtari et al., JMLR 2024), every step on the GPU.  Per match m the log-ratios ``-ll[:, m]`` of
+        ``log_likelihood`` (unweighted: for a fit with time decay or game weights this evaluates predictive density, not
+        the weighted pseudo-likelihood that was fitted) get a generalised-Pareto-smoothed tail of
+        ``ceil(min(0.2 S, 3 sqrt(S / r_eff)))`` draws, and ``elpd_loo_m = logsumexp_s(lw + ll)``.
+
+        Returns ``elpd_loo = sum_m elpd_loo_m``, ``se = sqrt(M var0(elpd_loo_m))``, ``p_loo = sum_m lppd_m - elpd_loo``,
+        ``pointwise`` (``elpd_loo_m``), ``pareto_k`` (k-hat per match; +inf when the tail has at most 4 draws),
+        ``good_k = min(1 - 1/log10 S, 0.7)`` with ``n_k_above_good`` and ``n_k_above_0.7`` (the counts of unreliable
+        matches), ``r_eff`` (one scalar relative efficiency for every match) and ``match_key``.  A match whose
+        log-likelihood is not finite in some draw gets ``elpd_loo_m`` NaN and k-hat +inf.  The ``[M, S]`` matrix is
+        computed and smoothed in ranges of matches that keep it within ``LOO_MATRIX_BYTES`` of device memory; the
+        results do not depend on the range size.  To choose ``epsilon`` (time decay) use ``log_score`` on later
+        matches instead."""
+        import torch
+
+        ds, do, key = self._comparison_inputs(None)
+        S, M = int(ds["attack"].shape[0]), int(do["home_team"].shape[0])
+        rows = max(1, min(M, LOO_MATRIX_BYTES // (4 * S)))
+        buf = torch.empty((rows, S), dtype=torch.float32, device="cuda")
+        elpd, khat, lppd = [], [], []
+        for lo in range(0, M, rows):
+            hi = min(M, lo + rows)
+            ll, st = pointwise_loglik(self.model, ds, {k: v[lo:hi] for k, v in do.items()}, loglik=buf)
+            e, k = psis_loo(ll, r_eff)
+            elpd.append(e.cpu().numpy())
+            khat.append(k.cpu().numpy())
+            lppd.append(bcompare.lppd_from_stats(st.cpu().numpy(), S))
+        return bcompare.loo_from_pointwise(np.concatenate(elpd), np.concatenate(khat), np.concatenate(lppd), S, r_eff,
+                                           key)
+
+    def log_score(self, data) -> Dict[str, Any]:
+        """Held-out log score of the posterior predictive on ``data`` (matches not used in the fit, reference
+        ``training_data`` keys): ``log_score = sum_m lppd_m`` with ``lppd_m = log((1/S) sum_s exp(ll[s, m]))``, the log
+        of the probability ``predict_score_proba`` gives the observed score (``pointwise``).  The way to choose
+        ``epsilon`` / ``rescale_weights``: fit on earlier matches, score later ones."""
+        ds, do, _ = self._comparison_inputs(data)
+        _, st = pointwise_loglik(self.model, ds, do, want_matrix=False)
+        lppd = bcompare.lppd_from_stats(st.cpu().numpy(), int(ds["attack"].shape[0]))
+        return {"log_score": float(lppd.sum()), "pointwise": lppd, "num_matches": len(lppd)}
 
     # ---- simulation from the grid (bpl/base.py:150-246, bpl/_util.py:96-112) -----------------------------------
     @staticmethod
@@ -602,3 +709,7 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         self.attack = [att[:, j] for j in range(G)]  # the reference stores lists of [S, T] arrays (:308-309)
         self.defence = [dfn[:, j] for j in range(G)]
         return self
+
+    def _comparison_inputs(self, data):
+        raise NotImplementedError("model comparison needs the predictive distribution, and the dynamic model's predict "
+                                  "methods cannot run in the reference (SURVEY.md D3)")

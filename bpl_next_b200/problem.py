@@ -1,4 +1,5 @@
-"""Python handles over the C ABI: ``Problem`` (log-density + gradient) and ``score_grid``.
+"""Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik`` and
+``psis_loo``.
 
 torch is used only for device memory and streams; every number comes from ``libbplx.so``.
 """
@@ -236,3 +237,69 @@ def score_grid_host(model: str, samples: Dict[str, np.ndarray], fixtures: Dict[s
     _abi.check(lib.bplx_score_grid_host(C.byref(s), C.byref(f), max_goals, C.c_float(scale), grid.ctypes.data,
                                         None if outcome is None else outcome.ctypes.data))
     return grid, outcome
+
+
+def _device_ptr_fn(keep):
+    def ptr(t):
+        assert t.is_cuda and t.is_contiguous()
+        keep.append(t)
+        return int(t.data_ptr())
+    return ptr
+
+
+def pointwise_loglik(model: str, samples: Dict[str, torch.Tensor], observations: Dict[str, torch.Tensor],
+                     want_matrix: bool = True, loglik: Optional[torch.Tensor] = None, workspace=None, stream=None):
+    """Device path of ``bplx_pointwise_loglik``: posterior arrays ``[S, T]`` float32 and observed matches (the fixture
+    index tensors of ``score_grid`` plus ``home_goals`` / ``away_goals`` uint8) on the GPU.
+
+    ``ll[s, m] = log Pois(yh; lh) + log Pois(ya; la) + log tau(yh, ya; lh, la, corr_coef_s)`` with the rates of the
+    predict path (neutral venues and confederations included, no clip of the rates), tau clamped at 0 (a match can give
+    -inf) and no match weights.  Returns ``(loglik, stats)``: ``loglik`` is the match-major ``[M, S]`` float32 matrix
+    (a view of the ``[M, ld]`` buffer when one is passed in) or ``None`` when ``want_matrix`` is false; ``stats`` is
+    ``[M, 4]`` float64 = (max ll, sum exp(ll - max), sum ll, sum ll^2) over the draws (``compare.waic_from_stats``)."""
+    lib = _abi.lib()
+    keep = []
+    ptr = _device_ptr_fn(keep)
+    for k in _SAMPLE_KEYS + ("home_advantage",):
+        if samples.get(k) is not None:
+            assert samples[k].dtype == torch.float32
+    for k in ("home_goals", "away_goals"):
+        assert observations[k].dtype == torch.uint8, k
+    s = _samples_struct(model, samples, ptr)
+    o = _abi.Observations()
+    o.fixtures = _fixtures_struct(observations, ptr)
+    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    M, S = o.fixtures.num_fixtures, s.num_samples
+    dev = samples["attack"].device
+    need = int(lib.bplx_pointwise_loglik_workspace_bytes(C.byref(s), C.byref(o)))
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    ld = 0
+    if want_matrix:
+        if loglik is None:
+            loglik = torch.empty((M, S), dtype=torch.float32, device=dev)
+        assert loglik.dtype == torch.float32 and loglik.shape[0] >= M and loglik.stride(1) == 1
+        ld = int(loglik.stride(0)) if M > 1 else max(S, int(loglik.shape[1]))
+    stats = torch.empty((M, 4), dtype=torch.float64, device=dev)
+    _abi.check(lib.bplx_pointwise_loglik(C.byref(s), C.byref(o), _dptr(loglik) if want_matrix else None, ld,
+                                         _dptr(stats), _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    return (loglik[:M, :S] if want_matrix else None), stats
+
+
+def psis_loo(loglik: torch.Tensor, r_eff: float = 1.0, stream=None):
+    """Device path of ``bplx_psis_loo``: PSIS-LOO (ArviZ's ``_psislw`` / ``_gpdfit``) per row of the match-major
+    ``[M, S]`` float32 matrix (unit inner stride; the row pitch is passed as the leading dimension).  Returns
+    ``(elpd_i [M], pareto_k [M])`` float64 on the device: ``elpd_i[m] = logsumexp_s(lw + ll)`` with the Pareto-smoothed
+    normalised log-weights ``lw`` of the ratios ``-ll[m]``, ``pareto_k[m]`` the fitted shape (+inf when the tail has at
+    most 4 draws).  A row with a non-finite entry gives (NaN, +inf).  The tail, ``ceil(min(0.2 S, 3 sqrt(S / r_eff)))``
+    draws, must not exceed ``_abi.PSIS_MAX_TAIL``."""
+    assert loglik.is_cuda and loglik.dtype == torch.float32 and loglik.dim() == 2
+    assert loglik.stride(1) == 1 or loglik.shape[1] == 1
+    lib = _abi.lib()
+    M, S = int(loglik.shape[0]), int(loglik.shape[1])
+    ld = int(loglik.stride(0)) if M > 1 else S
+    elpd = torch.empty(M, dtype=torch.float64, device=loglik.device)
+    khat = torch.empty(M, dtype=torch.float64, device=loglik.device)
+    _abi.check(lib.bplx_psis_loo(_dptr(loglik), M, S, ld, C.c_double(r_eff), _dptr(elpd), _dptr(khat), None, 0,
+                                 _stream_ptr(stream)))
+    return elpd, khat

@@ -226,6 +226,45 @@ int bplx_score_grid_ex(const bplx_samples* s, const bplx_fixtures* f, int max_go
 int bplx_score_grid_host(const bplx_samples* s, const bplx_fixtures* f, int max_goals, float scale,
                          float* grid, float* outcome);
 
+/* ---- model comparison: pointwise log-likelihood of observed scores, PSIS-LOO ------------------ */
+/*
+ * Observed matches: the fixtures (device index arrays, as for the score grid) and their scores.
+ */
+typedef struct {
+  bplx_fixtures fixtures;        /* num_fixtures = M matches */
+  const uint8_t* home_goals;     /* device [M] */
+  const uint8_t* away_goals;     /* device [M] */
+} bplx_observations;
+
+size_t bplx_pointwise_loglik_workspace_bytes(const bplx_samples* s, const bplx_observations* obs);
+
+/*
+ * loglik[m * ld + s] = log Pois(yh; lh) + log Pois(ya; la) + log tau(yh, ya; lh, la, corr_coef[s])  (float32)
+ * with the rates of the predict path (bplx_score_grid: neutral venues and confederations included, no clip of the
+ * rates), tau clamped at 0 so that a match can give -inf, and no match weights: exp(loglik) averaged over s is the
+ * probability bplx_score_grid gives the observed cell.  Match-major [M, ld], ld >= S; loglik may be NULL (only the
+ * statistics are computed then, with no matrix traffic).
+ * stats[m * 4 + 0..3] (float64) = max_s ll, sum_s exp(ll - max), sum_s ll, sum_s ll^2: lppd_m = max + log(sum exp) -
+ * log S and var_s ll follow on the host.  Deterministic (sample splits are combined in a fixed order); the statistics do
+ * not depend on whether loglik is NULL.  DYNAMIC: BPLX_E_UNSUPPORTED.
+ */
+int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, float* loglik, size_t ld, double* stats,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Pareto-smoothed importance-sampling leave-one-out (Vehtari et al., JMLR 2024; ArviZ's _psislw / _gpdfit) per match
+ * over the rows of a match-major log-likelihood matrix loglik [M, ld] (device, float32, S draws per row):
+ *   elpd_i[m]   = log sum_s exp(lw[s] + ll[s])  with lw the smoothed, normalised log-weights of the ratios -ll
+ *   pareto_k[m] = the fitted shape k-hat; +inf when the tail has <= 4 draws
+ * Tail length Mt = ceil(min(0.2 S, 3 sqrt(S / r_eff))); Mt <= BPLX_PSIS_MAX_TAIL (16384, the shared-memory sort of one
+ * CTA), else BPLX_E_UNSUPPORTED.  S itself is not limited by shared memory.  A row with a non-finite entry gives
+ * elpd_i = NaN and pareto_k = +inf.  Outputs do not depend on how tied draws are ordered.  The current kernel needs no
+ * workspace: NULL, 0 is accepted.
+ */
+#define BPLX_PSIS_MAX_TAIL 16384
+int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t ld, double r_eff, double* elpd_i,
+                  double* pareto_k, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

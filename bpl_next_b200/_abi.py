@@ -58,7 +58,17 @@ class Observations(C.Structure):
     _fields_ = [("fixtures", Fixtures), ("home_goals", C.c_void_p), ("away_goals", C.c_void_p)]
 
 
+class Table(C.Structure):
+    _fields_ = [
+        ("num_slots", C.c_int32), ("num_positions", C.c_int32), ("num_points_bins", C.c_int32),
+        ("points_win", C.c_int32), ("points_draw", C.c_int32),
+        ("group", C.c_void_p), ("start_points", C.c_void_p), ("start_goals_for", C.c_void_p),
+        ("start_goals_against", C.c_void_p),
+    ]
+
+
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
+SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 
 
 class BplxError(RuntimeError):
@@ -111,6 +121,11 @@ def declare(lib):
     lib.bplx_pointwise_loglik.restype = i
     lib.bplx_psis_loo.argtypes = [vp, i, i, sz, C.c_double, vp, vp, vp, sz, vp]
     lib.bplx_psis_loo.restype = i
+    lib.bplx_simulate_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), C.POINTER(Table)]
+    lib.bplx_simulate_workspace_bytes.restype = sz
+    lib.bplx_simulate_table.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table), i, i,
+                                        C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.bplx_simulate_table.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

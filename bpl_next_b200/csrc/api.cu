@@ -1,4 +1,5 @@
 // api.cu -- the extern "C" surface declared in include/bplx.h.
+#include <limits.h>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -13,6 +14,7 @@
 #include "problem.h"
 #include "loo.h"
 #include "score_grid.h"
+#include "simulate.h"
 
 namespace bplx {
 
@@ -797,6 +799,97 @@ int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t 
   pp.elpd = elpd_i;
   pp.khat = pareto_k;
   return launch_psis(pp, static_cast<cudaStream_t>(stream));
+}
+
+// ---- season / group-stage simulation --------------------------------------------------------------------------
+static size_t simulate_plan_for(const bplx_samples* s, const bplx_fixtures* f, SimParams* sp) {
+  sp->gp.model = s->model;
+  sp->gp.S = s->num_samples;
+  sp->gp.T = s->num_teams;
+  sp->gp.Cf = s->model == BPLX_NEUTRAL_WC ? s->num_conferences : 0;
+  sp->gp.F = f->num_fixtures;
+  return simulate_plan(sp);
+}
+
+size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t) {
+  if (!s || !f || !t || s->num_samples <= 0 || s->num_teams <= 0 || f->num_fixtures <= 0) return 0;
+  SimParams sp{};
+  return simulate_plan_for(s, f, &sp);
+}
+
+int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
+                        const bplx_table* t, int max_goals, int sims_per_draw, unsigned long long seed,
+                        long long first_draw, unsigned long long* position_counts, unsigned long long* points_counts,
+                        uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  int rc = check_sample_args(s, f, "simulate");
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(t != nullptr, BPLX_E_INVALID, "simulate: table is NULL");
+  BPLX_REQUIRE(t->num_slots <= BPLX_SIM_MAX_TEAMS, BPLX_E_UNSUPPORTED,
+               "simulate: %d table slots exceed the kernel's limit of %d (BPLX_SIM_MAX_TEAMS)", t->num_slots,
+               BPLX_SIM_MAX_TEAMS);
+  BPLX_REQUIRE(t->num_slots >= 1, BPLX_E_INVALID, "simulate: the table needs at least one slot");
+  BPLX_REQUIRE(t->num_positions >= 1 && t->num_positions <= t->num_slots && t->num_points_bins >= 1, BPLX_E_INVALID,
+               "simulate: num_positions must be in [1, num_slots] and num_points_bins >= 1 (got %d, %d)",
+               t->num_positions, t->num_points_bins);
+  BPLX_REQUIRE(t->points_win >= 1 && t->points_draw >= 0 && t->points_draw <= t->points_win, BPLX_E_INVALID,
+               "simulate: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)",
+               t->points_win, t->points_draw);
+  BPLX_REQUIRE(t->start_points && t->start_goals_for && t->start_goals_against, BPLX_E_INVALID,
+               "simulate: start_points, start_goals_for and start_goals_against must not be NULL");
+  BPLX_REQUIRE(home_slot && away_slot, BPLX_E_INVALID, "simulate: home_slot and away_slot must not be NULL");
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "simulate: max_goals must be in [1, 63] (got %d)",
+               max_goals);
+  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "simulate: sims_per_draw must be >= 1 (got %d)", sims_per_draw);
+  BPLX_REQUIRE(first_draw >= 0 && first_draw + s->num_samples <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
+               "simulate: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits");
+  BPLX_REQUIRE((long long)s->num_samples * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
+               "simulate: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
+               (long long)s->num_samples * sims_per_draw);
+  BPLX_REQUIRE(position_counts && points_counts && invalid, BPLX_E_INVALID,
+               "simulate: position_counts, points_counts and invalid must not be NULL");
+  SimParams sp{};
+  const size_t need = simulate_plan_for(s, f, &sp);
+  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
+               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  GridParams& gp = sp.gp;
+  gp.attack = s->attack;
+  gp.defence = s->defence;
+  gp.ha = s->home_attack;
+  gp.aa = s->away_attack;
+  gp.hd = s->home_defence;
+  gp.ad = s->away_defence;
+  gp.conf = s->confederation_strength;
+  gp.corr = s->corr_coef;
+  gp.home = f->home_team;
+  gp.away = f->away_team;
+  gp.hconf = f->home_conf;
+  gp.aconf = f->away_conf;
+  gp.nv = f->neutral_venue;
+  gp.table = static_cast<float*>(workspace);
+  sp.hslot = home_slot;
+  sp.aslot = away_slot;
+  sp.group = t->group;
+  sp.start_pts = t->start_points;
+  sp.start_gf = t->start_goals_for;
+  sp.start_ga = t->start_goals_against;
+  sp.NT = t->num_slots;
+  sp.P = t->num_positions;
+  sp.B = t->num_points_bins;
+  sp.G = max_goals;
+  sp.R = sims_per_draw;
+  sp.pw = t->points_win;
+  sp.pd = t->points_draw;
+  sp.seed = seed;
+  sp.first_draw = first_draw;
+  sp.N = s->num_samples * sims_per_draw;
+  sp.pos_counts = position_counts;
+  sp.pts_counts = points_counts;
+  sp.invalid = invalid;
+  sp.positions = positions;
+  sp.scores = scores;
+  return launch_simulate(sp, static_cast<cudaStream_t>(stream));
 }
 
 void bplx_reload_env(void) {

@@ -46,9 +46,7 @@ __global__ void __launch_bounds__(kPwThreads, 3) pointwise_kernel(const __grid_c
   const int h = gp.home[f], a = gp.away[f];
   const bool wc = gp.model == BPLX_NEUTRAL_WC;
   const bool neutral = gp.ntab == 3 && gp.nv && gp.nv[f];
-  const int offH = (neutral ? L.P0 : L.P1) + 2 * h;
-  const int offA = (neutral ? L.P0 : L.Q1) + 2 * a;
-  const int offEh = wc ? L.EC + 2 * gp.hconf[f] : 0, offEa = wc ? L.EC + 2 * gp.aconf[f] : 0;
+  const FixtureOffsets off = fixture_offsets(L, h, a, neutral, wc, wc ? gp.hconf[f] : 0, wc ? gp.aconf[f] : 0);
   const int offC = L.C;
   const int yh = pp.hg[f], ya = pp.ag[f];
   const float fyh = (float)yh, fya = (float)ya;
@@ -78,15 +76,8 @@ __global__ void __launch_bounds__(kPwThreads, 3) pointwise_kernel(const __grid_c
   __syncthreads();
 
   auto loglik = [&](const float* row) -> float {
-    const float2 rh = *reinterpret_cast<const float2*>(row + offH);
-    const float2 ra = *reinterpret_cast<const float2*>(row + offA);
-    float lh = rh.x * (neutral ? ra.y : ra.x), la = rh.y * (neutral ? ra.x : ra.y);
-    if (wc) {
-      const float2 eh = *reinterpret_cast<const float2*>(row + offEh);
-      const float2 ea = *reinterpret_cast<const float2*>(row + offEa);
-      lh *= eh.x * ea.y;
-      la *= ea.x * eh.y;
-    }
+    const float2 lam = fixture_rates(row, off, neutral, wc);
+    const float lh = lam.x, la = lam.y;
     float ll = fmaf(fyh, logf(lh), fmaf(fya, logf(la), cst - lh - la));
     if (cell) {
       const float c = row[offC];

@@ -23,6 +23,35 @@ __host__ __device__ inline RowLayout row_layout(int T, int Cf, int ntab) {
   return L;
 }
 
+// float offsets, inside a sample row, of the table entries the rates of one fixture read (see score_grid_tables)
+struct FixtureOffsets {
+  int h, a, eh, ea;
+};
+__host__ __device__ inline FixtureOffsets fixture_offsets(const RowLayout& L, int home, int away, bool neutral, bool wc,
+                                                          int home_conf, int away_conf) {
+  FixtureOffsets o;
+  o.h = (neutral ? L.P0 : L.P1) + 2 * home;
+  o.a = (neutral ? L.P0 : L.Q1) + 2 * away;
+  o.eh = wc ? L.EC + 2 * home_conf : 0;
+  o.ea = wc ? L.EC + 2 * away_conf : 0;
+  return o;
+}
+
+// the predict path's rates (lambda_h, lambda_a) of one fixture from one sample row: neutral venues and confederations
+// included, no clip
+__device__ __forceinline__ float2 fixture_rates(const float* row, const FixtureOffsets& o, bool neutral, bool wc) {
+  const float2 rh = *reinterpret_cast<const float2*>(row + o.h);
+  const float2 ra = *reinterpret_cast<const float2*>(row + o.a);
+  float lh = rh.x * (neutral ? ra.y : ra.x), la = rh.y * (neutral ? ra.x : ra.y);
+  if (wc) {
+    const float2 eh = *reinterpret_cast<const float2*>(row + o.eh);
+    const float2 ea = *reinterpret_cast<const float2*>(row + o.ea);
+    lh *= eh.x * ea.y;
+    la *= ea.x * eh.y;
+  }
+  return make_float2(lh, la);
+}
+
 struct GridParams {
   int model, S, T, Cf, F, g;
   int nsplit, samples_per_split;

@@ -22,11 +22,16 @@ from . import compare as bcompare
 from . import data as bdata
 from . import nuts as bnuts
 from . import parallel
+from . import season as bseason
 from .problem import Problem, pointwise_loglik, psis_loo, score_grid_host
+from .problem import simulate_table as _simulate_table
 
 MAX_GOALS = bdata.MAX_GOALS
 # device memory for the [matches, draws] log-likelihood matrix of loo(): larger match sets are processed in ranges
 LOO_MATRIX_BYTES = 4 << 30
+# device memory for the raw outputs of simulate_table(return_simulations=True) (positions and scores): larger runs are
+# processed in ranges of posterior draws
+SIM_OUTPUT_BYTES = 1 << 30
 
 
 def _str_to_list(*args):
@@ -418,6 +423,89 @@ class _BplxPredictor:
         """``[fixtures, num_samples]`` names of the winning team, or ``"Draw"`` (``bpl/base.py:197-246``)."""
         return self._sample_outcome(home_team, away_team, num_samples, random_state, max_goals)
 
+    # ---- season / group-stage simulation -------------------------------------------------------------------------
+    def simulate_table(self, fixtures, played=None, teams=None, groups=None, num_sims_per_draw: int = 1,
+                       random_state: Optional[int] = None, max_goals: int = MAX_GOALS, points=(3, 1),
+                       return_simulations: bool = False) -> Dict[str, Any]:
+        """Finishing-position and points probabilities of a league table or of group tables, simulated on the GPU.
+
+        Every simulated season takes ONE posterior draw and plays every remaining fixture with that draw's rates, so a
+        team that is stronger in a draw is stronger in all of its matches of that season (sampling fixtures one by one,
+        as ``sample_score`` does, loses that correlation and makes the spread of final points too narrow).  Each of the
+        S draws gives ``num_sims_per_draw`` seasons: ``num_simulations = S * num_sims_per_draw``.
+
+        ``fixtures``: the remaining matches with reference ``training_data`` keys (``home_team``, ``away_team``, and
+        ``neutral_venue`` / ``home_conf`` / ``away_conf`` where the model has them, mapped as ``predict_*`` maps them).
+        ``played``: results so far (``home_team``, ``away_team``, ``home_goals``, ``away_goals``) that make the starting
+        table.  ``teams``: the table (default: the sorted union of the teams in ``fixtures`` and ``played``); every team
+        in a fixture must be known to the model and in the table, and at most 64 teams are supported.  ``groups``: a
+        mapping team -> group label, or labels aligned with ``teams``; teams are then ranked within their group.
+        ``points``: (win, draw).
+
+        A fixture's score is drawn from the draw's own score grid up to ``max_goals`` (tau clamped at 0, normalised by
+        its sum); averaged over draws this is ``predict_score_grid_proba``.  Teams are ranked by points, goal
+        difference, goals for, then a random key: head-to-head and fair-play rules are NOT modelled, ties left after
+        goals for are decided by lot.
+
+        Returns ``teams``, ``groups`` (each team's label, or None), ``position_proba [T, P]`` (P = the largest group;
+        position 0 = first), ``points_proba [T, B]`` (points GAINED in ``fixtures``), ``start_points``,
+        ``expected_points`` (final), ``num_simulations``, ``sims_per_draw`` and ``seed`` (from the clock when
+        ``random_state`` is None; pass it back to repeat the run).  With ``return_simulations`` also ``positions [N, T]``
+        and ``home_score`` / ``away_score`` ``[F, N]`` (``sample_score``'s shape); the draws are then processed in
+        ranges that keep these within ``SIM_OUTPUT_BYTES`` of device memory, and the results do not depend on the range
+        size.  Raises if any simulation met a non-finite rate."""
+        import torch
+
+        home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"])
+        tteams = bseason.table_teams(home, away, played, teams)
+        table = bseason.build_table(tteams, played, groups, points)
+        hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
+        h, a = self._parse_fixture_args(home, away)
+        kw = {k: fixtures[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in fixtures}
+        fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw), "home_slot": hs, "away_slot": as_}
+        seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
+        R = int(num_sims_per_draw)
+        if R < 1:
+            raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
+        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
+              if v is not None}
+        dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
+        dtab = {k: None if table[k] is None else torch.from_numpy(table[k]).cuda()
+                for k in ("start_points", "start_goals_for", "start_goals_against", "group")}
+        dtab.update({k: table[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
+        S, T, F = int(ds["attack"].shape[0]), len(tteams), len(h)
+        step = (2 ** 31 - 1) // R  # simulations per call stay below 2^31
+        if return_simulations:
+            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F))))
+        if step < 1:
+            raise ValueError(f"num_sims_per_draw={R} is too large for one draw per call")
+        pos_c = pts_c = None
+        invalid = 0
+        raw = []
+        for lo in range(0, S, step):
+            hi = min(S, lo + step)
+            out = _simulate_table(self.model, {k: v[lo:hi] for k, v in ds.items()}, dfx, dtab, max_goals, R, seed,
+                                  first_draw=lo, want_positions=return_simulations, want_scores=return_simulations)
+            pos_c = out["position_counts"] if pos_c is None else pos_c + out["position_counts"]
+            pts_c = out["points_counts"] if pts_c is None else pts_c + out["points_counts"]
+            invalid += int(out["invalid"].item())
+            if return_simulations:
+                raw.append((out["positions"].cpu().numpy(), out["scores"].cpu().numpy()))
+        N = S * R
+        if invalid:
+            raise ValueError(f"{invalid} of {N} simulations met a non-finite scoring rate or score-grid normaliser: "
+                             "check the posterior draws")
+        res = {"teams": tteams,
+               "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
+               **bseason.probabilities(table, pos_c.cpu().numpy(), pts_c.cpu().numpy(), N),
+               "start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
+               "seed": seed}
+        if return_simulations:
+            sc = np.concatenate([r[1] for r in raw])
+            res.update(positions=np.concatenate([r[0] for r in raw]), home_score=np.ascontiguousarray(sc[:, :, 0].T),
+                       away_score=np.ascontiguousarray(sc[:, :, 1].T))
+        return res
+
     # ---- a team the model has not seen (extended_dixon_coles.py:401-462 and the neutral siblings) ---------------
     def _new_team_pair(self, team_name, team_covariates):
         """Draws of (attack, defence) for a new team from the fitted hierarchical prior, one per posterior sample."""
@@ -709,6 +797,10 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         self.attack = [att[:, j] for j in range(G)]  # the reference stores lists of [S, T] arrays (:308-309)
         self.defence = [dfn[:, j] for j in range(G)]
         return self
+
+    def simulate_table(self, *args, **kwargs):
+        raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
+                                  "cannot run in the reference (SURVEY.md D3)")
 
     def _comparison_inputs(self, data):
         raise NotImplementedError("model comparison needs the predictive distribution, and the dynamic model's predict "

@@ -1,5 +1,5 @@
-"""Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik`` and
-``psis_loo``.
+"""Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik``,
+``psis_loo`` and ``simulate_table``.
 
 torch is used only for device memory and streams; every number comes from ``libbplx.so``.
 """
@@ -303,3 +303,71 @@ def psis_loo(loglik: torch.Tensor, r_eff: float = 1.0, stream=None):
     _abi.check(lib.bplx_psis_loo(_dptr(loglik), M, S, ld, C.c_double(r_eff), _dptr(elpd), _dptr(khat), None, 0,
                                  _stream_ptr(stream)))
     return elpd, khat
+
+
+_TABLE_ARRAYS = ("start_points", "start_goals_for", "start_goals_against")
+
+
+def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor], table: dict,
+                   max_goals: int, sims_per_draw: int, seed: int, first_draw: int = 0, want_positions: bool = False,
+                   want_scores: bool = False, workspace=None, stream=None) -> Dict[str, Optional[torch.Tensor]]:
+    """Device path of ``bplx_simulate_table``: season / group-stage simulation, one posterior draw per simulated season.
+
+    ``samples``: posterior arrays ``[S, T]`` on the GPU (the draws of this call; ``first_draw`` is the global index of
+    the first one).  ``fixtures``: the index tensors of ``score_grid`` plus ``home_slot`` / ``away_slot`` (uint8 table
+    slots).  ``table``: ``start_points``, ``start_goals_for``, ``start_goals_against`` (int32 ``[T_tab]``), ``group``
+    (uint8 ``[T_tab]`` or None) on the GPU, and the ints ``num_positions`` (largest group), ``num_points_bins``,
+    ``points_win``, ``points_draw`` (``season.build_table`` / ``season.fixture_slots`` make them).
+
+    Simulation ``n = (first_draw + s) R + r`` uses draw s and the Philox words of ``curand_init(seed, n, 0)``: words 2f,
+    2f+1 sample fixture f's score from the draw's own grid (tau clamped at 0, normalised by its sum), word 2F + t is slot
+    t's tie-break key.  Teams are ranked within their group by points, goal difference, goals for, then the key;
+    head-to-head and fair-play rules are not modelled, so ties left after goals for are decided by lot.  Returns
+    ``position_counts [T_tab, P]`` and ``points_counts [T_tab, B]`` (points gained; int64), ``invalid`` (int64 ``[1]``:
+    simulations with a non-finite rate or normaliser, left out of the counts), and when asked ``positions [N, T_tab]``
+    and ``scores [N, F, 2]`` (uint8; 255 marks an invalid simulation / fixture), N = S R."""
+    lib = _abi.lib()
+    keep = []
+    ptr = _device_ptr_fn(keep)
+    for k in _SAMPLE_KEYS + ("home_advantage",):
+        if samples.get(k) is not None:
+            assert samples[k].dtype == torch.float32
+    for k, dt in _FIXTURE_KEYS:
+        if fixtures.get(k) is not None:
+            assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
+    for k in ("home_slot", "away_slot"):
+        assert fixtures[k].dtype == torch.uint8, k
+    for k in _TABLE_ARRAYS:
+        assert table[k].dtype == torch.int32, k
+    T_tab = int(table["start_points"].shape[0])
+    if T_tab > _abi.SIM_MAX_TEAMS:
+        raise ValueError(f"the table has {T_tab} slots; at most {_abi.SIM_MAX_TEAMS} are supported")
+    top = int(torch.maximum(fixtures["home_slot"].max(), fixtures["away_slot"].max()))
+    if top >= T_tab:
+        raise ValueError(f"a fixture names table slot {top}, but the table has {T_tab} slots")
+    s = _samples_struct(model, samples, ptr)
+    f = _fixtures_struct(fixtures, ptr)
+    t = _abi.Table()
+    t.num_slots = T_tab
+    t.num_positions, t.num_points_bins = int(table["num_positions"]), int(table["num_points_bins"])
+    t.points_win, t.points_draw = int(table["points_win"]), int(table["points_draw"])
+    t.group = None if table.get("group") is None else ptr(table["group"])
+    for k in _TABLE_ARRAYS:
+        setattr(t, k, ptr(table[k]))
+    dev = samples["attack"].device
+    need = int(lib.bplx_simulate_workspace_bytes(C.byref(s), C.byref(f), C.byref(t)))
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    N, F = s.num_samples * int(sims_per_draw), f.num_fixtures
+    pos_counts = torch.empty((T_tab, t.num_positions), dtype=torch.int64, device=dev)
+    pts_counts = torch.empty((T_tab, t.num_points_bins), dtype=torch.int64, device=dev)
+    invalid = torch.empty(1, dtype=torch.int64, device=dev)
+    positions = torch.empty((N, T_tab), dtype=torch.uint8, device=dev) if want_positions else None
+    scores = torch.empty((N, F, 2), dtype=torch.uint8, device=dev) if want_scores else None
+    _abi.check(lib.bplx_simulate_table(C.byref(s), C.byref(f), ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"]),
+                                       C.byref(t), int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                       int(first_draw), _dptr(pos_counts), _dptr(pts_counts), _dptr(positions),
+                                       _dptr(scores), _dptr(invalid), _dptr(workspace), workspace.numel(),
+                                       _stream_ptr(stream)))
+    return {"position_counts": pos_counts, "points_counts": pts_counts, "invalid": invalid, "positions": positions,
+            "scores": scores}

@@ -265,6 +265,66 @@ int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, f
 int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t ld, double r_eff, double* elpd_i,
                   double* pareto_k, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- season / group-stage simulation: finishing positions and points per posterior draw ------------------------ */
+/*
+ * A table of T_tab slots (T_tab <= BPLX_SIM_MAX_TEAMS), their starting points / goals for / goals against, an optional
+ * group id per slot, and F remaining fixtures: `fixtures` gives the model team indices, neutral-venue flags and
+ * confederations the predict path needs, home_slot / away_slot (device uint8 [F]) the table slots that play them.
+ *
+ * Simulation n = (first_draw + s) * R + r (R = sims_per_draw) uses draw s of `samples`.  Its random numbers are the
+ * outputs of curand_init(seed, n, 0) followed by curand() (Philox4_32_10): words 2f and 2f+1 become u_h and u_a of
+ * fixture f through curand_uniform (in (0, 1]), word 2F + t is the tie-break key of slot t.  Every word has a fixed
+ * address, so a rounding difference in one fixture cannot shift the random numbers of any other fixture.
+ *
+ * Fixture f in draw s: lambda_h, lambda_a are the predict path's rates (bplx_score_grid: neutral venues and confederations
+ * included, Extended's clip not applied); G = max_goals (1..63);
+ *   w(i, j) = tau+(i, j) Pois(i; lambda_h) Pois(j; lambda_a),  0 <= i, j <= G,
+ * tau+ = tau clamped at 0 on the four low-score cells and 1 elsewhere; Z = sum w, m(i) = sum_j w(i, j).  Home goals are
+ * the smallest i with sum_{i' <= i} m(i') >= u_h Z, away goals the smallest j with sum_{j' <= j} w(i, j') >= u_a m(i);
+ * when rounding leaves a target unmet, the last index with positive mass.  A cell of zero probability is never returned.
+ * Per draw this is the draw's own grid normalised by its sum; averaged over draws it converges to bplx_score_grid.
+ *
+ * Table: points_win for a win, points_draw for a draw (0 <= points_draw <= points_win, points_win >= 1); goal
+ * difference and goals for accumulate on top of the start.  Teams are ranked WITHIN THEIR GROUP by points, then goal
+ * difference, then goals for, then the tie-break key, all descending; if even the keys are equal the lower slot ranks
+ * first.  Position k (0-based) of slot t = the number of teams of its group ranked ahead of t.  Head-to-head and
+ * fair-play rules are not modelled: ties left after goals for are decided by lot (the tie-break key).
+ *
+ * Outputs (device; integer counts, so they are the same bits whatever order the atomics run in; overwritten):
+ *   position_counts [T_tab, P]  P = num_positions, the largest group size
+ *   points_counts   [T_tab, B]  points GAINED in the remaining fixtures, B = num_points_bins
+ *                               = points_win * max_t(remaining fixtures of t) + 1
+ *   invalid [1]                 simulations in which some fixture had a non-finite rate, a normaliser that is not
+ *                               positive and finite, or a slot >= T_tab (and simulations whose group is larger than P
+ *                               or whose gained points do not fit B: the bins are never overrun).  They are left out of
+ *                               the histograms; their positions row is 0xFF and the offending fixture's scores 0xFF.
+ *   positions [N, T_tab] uint8, scores [N, F, 2] uint8 (home, away): optional, NULL to skip; N = num_samples * R, row
+ *                               (s * R + r) of this call.
+ * Draw ranges: calls on draws [0, k) and [k, S) (samples cut to the range, first_draw = 0 and k) give counts that sum to
+ * the single call's counts and raw rows that concatenate to its rows.  The workspace holds the [S, row] exponential
+ * table of bplx_score_grid's pre-pass.  DYNAMIC: BPLX_E_UNSUPPORTED; T_tab > 64 or N >= 2^31 in one call: BPLX_E_UNSUPPORTED;
+ * G outside [1, 63], R < 1 or bad point values: BPLX_E_INVALID.
+ */
+#define BPLX_SIM_MAX_TEAMS 64
+typedef struct {
+  int32_t num_slots;              /* T_tab */
+  int32_t num_positions;          /* P: the largest group size */
+  int32_t num_points_bins;        /* B */
+  int32_t points_win;
+  int32_t points_draw;
+  const uint8_t* group;           /* device [T_tab] group id per slot, or NULL: one group */
+  const int32_t* start_points;    /* device [T_tab] */
+  const int32_t* start_goals_for;
+  const int32_t* start_goals_against;
+} bplx_table;
+
+size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t);
+int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
+                        const bplx_table* t, int max_goals, int sims_per_draw, unsigned long long seed,
+                        long long first_draw, unsigned long long* position_counts, unsigned long long* points_counts,
+                        uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
+                        size_t workspace_bytes, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

@@ -1,0 +1,173 @@
+"""Times season / group-stage simulation (bplx_simulate_table) on one GPU.
+
+    python scripts/simulate_time.py [--samples 16384] [--reps 20] [--out FILE.json]
+
+Workloads (synthetic posterior draws, fixed seeds):
+  league     20-team DixonColes league, F = 380 (a double round robin) and F = 190 (half a season), R = 64 and R = 1
+  world cup  48-team group stage, 12 groups of four, 72 fixtures at neutral venues, NeutralWC draws of configs[5]'s shape
+             (T = 220 model teams, Cf = 6), R = 64 and R = 1
+CUDA events around `--reps` calls after warm-up; a call is the whole entry point (count reset, exponential-table
+pre-pass, simulation kernel), issued straight through the C ABI so that no host synchronisation sits in the timed
+window.  Reports simulations/s and sampled scores/s, the GPU name and power limit read in the same run, and the float64
+oracle's CPU time on a few simulations of the league.
+"""
+from __future__ import annotations
+
+import argparse
+import ctypes as C
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
+
+
+def gpu_info():
+    try:
+        r = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30)
+        return r.stdout.strip().splitlines()[0]
+    except Exception as e:  # noqa: BLE001
+        import torch
+        return f"{torch.cuda.get_device_name()} (power limit not read: {e})"
+
+
+def league(S, F):
+    """20 teams, DixonColes draws; F = 380: every ordered pair once, F = 190: the first half of that list."""
+    rng = np.random.default_rng(7)
+    T = 20
+    s = {"attack": rng.normal(0, 0.3, (S, T)).astype(np.float32), "defence": rng.normal(0, 0.3, (S, T)).astype(np.float32),
+         "home_advantage": rng.normal(0.25, 0.05, S).astype(np.float32),
+         "corr_coef": rng.uniform(-0.1, 0.1, S).astype(np.float32)}
+    pairs = [(i, j) for i in range(T) for j in range(T) if i != j][:F]
+    h, a = np.array([p[0] for p in pairs]), np.array([p[1] for p in pairs])
+    fx = {"home_team": h.astype(np.uint16), "away_team": a.astype(np.uint16)}
+    return "dixon_coles", s, fx, h.astype(np.uint8), a.astype(np.uint8), T, None
+
+
+def world_cup(S):
+    """48 of configs[5]'s 220 teams in 12 groups of four, each group a round robin at neutral venues."""
+    from oracle import datasets
+
+    s, _ = datasets.config_5(S=S, F=1)
+    rng = np.random.default_rng(11)
+    teams = rng.choice(220, 48, replace=False)
+    group = np.repeat(np.arange(12), 4)
+    hs, as_ = [], []
+    for g in range(12):
+        m = np.arange(4 * g, 4 * g + 4)
+        for i in range(4):
+            for j in range(i + 1, 4):
+                hs.append(m[i])
+                as_.append(m[j])
+    hs, as_ = np.array(hs), np.array(as_)
+    fx = {"home_team": teams[hs].astype(np.uint16), "away_team": teams[as_].astype(np.uint16),
+          "home_conf": (teams[hs] % 6).astype(np.uint8), "away_conf": (teams[as_] % 6).astype(np.uint8),
+          "neutral_venue": np.ones(len(hs), np.uint8)}
+    return "neutral_wc", s, fx, hs.astype(np.uint8), as_.astype(np.uint8), 48, group.astype(np.uint8)
+
+
+def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
+    """The bplx_simulate_table call with every argument built once; returns (call, outputs, keep-alive)."""
+    import torch
+
+    from bpl_next_b200 import _abi, problem
+
+    lib = _abi.lib()
+    keep = []
+    ptr = problem._device_ptr_fn(keep)
+    dev = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in s.items()}
+    dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
+    st = problem._samples_struct(model, dev, ptr)
+    ft = problem._fixtures_struct(dfx, ptr)
+    rem = np.bincount(hs, minlength=T_tab) + np.bincount(as_, minlength=T_tab)
+    t = _abi.Table()
+    t.num_slots, t.points_win, t.points_draw = T_tab, 3, 1
+    t.num_positions = T_tab if group is None else int(np.bincount(group).max())
+    t.num_points_bins = int(3 * rem.max() + 1)
+    zeros = torch.zeros(T_tab, dtype=torch.int32, device="cuda")
+    t.start_points = t.start_goals_for = t.start_goals_against = ptr(zeros)
+    t.group = None if group is None else ptr(torch.from_numpy(group).cuda())
+    d_hs, d_as = ptr(torch.from_numpy(hs).cuda()), ptr(torch.from_numpy(as_).cuda())
+    pc = torch.empty((T_tab, t.num_positions), dtype=torch.int64, device="cuda")
+    bc = torch.empty((T_tab, t.num_points_bins), dtype=torch.int64, device="cuda")
+    inv = torch.empty(1, dtype=torch.int64, device="cuda")
+    need = int(lib.bplx_simulate_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t)))
+    ws = torch.empty(need, dtype=torch.uint8, device="cuda")
+    stream = torch.cuda.current_stream().cuda_stream
+    args = (C.byref(st), C.byref(ft), d_hs, d_as, C.byref(t), 15, R, seed, 0, ptr(pc), ptr(bc), None, None, ptr(inv),
+            ptr(ws), ws.numel(), stream)
+
+    def call():
+        _abi.check(lib.bplx_simulate_table(*args))
+
+    return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, zeros, ws)
+
+
+def time_ms(fn, reps):
+    import torch
+    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    start.record()
+    for _ in range(reps):
+        fn()
+    end.record()
+    torch.cuda.synchronize()
+    return start.elapsed_time(end) / reps
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--samples", type=int, default=16384)
+    ap.add_argument("--reps", type=int, default=20)
+    ap.add_argument("--out", default=None)
+    a = ap.parse_args()
+
+    import torch
+
+    from oracle import simulate as osim
+
+    if not torch.cuda.is_available():
+        raise SystemExit("simulate_time.py measures the GPU kernel and needs a CUDA device")
+    S = a.samples
+    rows = []
+    for name, make in (("league F=380", lambda: league(S, 380)), ("league F=190", lambda: league(S, 190)),
+                       ("world cup groups", lambda: world_cup(S))):
+        model, s, fx, hs, as_, T_tab, group = make()
+        for R in (64, 1):
+            call, out, _keep = prepared_call(model, s, fx, hs, as_, T_tab, group, R)
+            for _ in range(3):
+                call()
+            torch.cuda.synchronize()
+            assert int(out["invalid"].item()) == 0
+            ms = time_ms(call, a.reps)
+            N, F = S * R, len(hs)
+            rows.append({"workload": name, "model": model, "S": S, "R": R, "N": N, "F": F, "T_tab": T_tab,
+                         "ms": ms, "sims_per_s": N / (ms * 1e-3), "scores_per_s": N * F / (ms * 1e-3)})
+            print(json.dumps(rows[-1]), flush=True)
+
+    # the float64 oracle on the CPU: 2 draws x 64 simulations of the F = 380 league
+    model, s, fx, hs, as_, T_tab, _ = league(2, 380)
+    tab = {"start_points": np.zeros(T_tab, np.int32), "start_goals_for": np.zeros(T_tab, np.int32),
+           "start_goals_against": np.zeros(T_tab, np.int32), "group": None, "points_win": 3, "points_draw": 1,
+           "num_positions": T_tab, "num_points_bins": 3 * 38 + 1}
+    t0 = time.perf_counter()
+    osim.simulate(model, s, fx, hs, as_, tab, 15, 64, seed=1)
+    t_or = time.perf_counter() - t0
+    res = {"gpu": gpu_info(), "reps": a.reps, "workloads": rows,
+           "oracle_cpu": {"sims": 128, "F": 380, "s": t_or, "sims_per_s": 128 / t_or}}
+    txt = json.dumps(res, indent=1)
+    print(txt)
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        with open(a.out, "w") as f:
+            f.write(txt + "\n")
+
+
+if __name__ == "__main__":
+    main()

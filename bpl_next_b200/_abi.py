@@ -67,8 +67,20 @@ class Table(C.Structure):
     ]
 
 
+class Bracket(C.Structure):
+    _fields_ = [
+        ("num_ties", C.c_int32), ("num_rounds", C.c_int32), ("num_groups", C.c_int32), ("best_position", C.c_int32),
+        ("best_count", C.c_int32),
+        ("kind", C.c_void_p), ("arg0", C.c_void_p), ("arg1", C.c_void_p), ("round", C.c_void_p),
+        ("neutral_venue", C.c_void_p), ("slot_team", C.c_void_p), ("slot_conf", C.c_void_p), ("best_alloc", C.c_void_p),
+    ]
+
+
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
+KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
+# BPLX_ENTRANT_*
+ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0, 1, 2, 3, 4
 
 
 class BplxError(RuntimeError):
@@ -126,6 +138,13 @@ def declare(lib):
     lib.bplx_simulate_table.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table), i, i,
                                         C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.bplx_simulate_table.restype = i
+    lib.bplx_simulate_tournament_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), C.POINTER(Table),
+                                                             C.POINTER(Bracket)]
+    lib.bplx_simulate_tournament_workspace_bytes.restype = sz
+    lib.bplx_simulate_tournament.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                             C.POINTER(Bracket), i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp,
+                                             vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.bplx_simulate_tournament.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

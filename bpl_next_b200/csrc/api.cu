@@ -554,21 +554,25 @@ int bplx_logdensity_fwdbwd_host(bplx_problem* p, int C, const float* theta, floa
 
 // ---- score grid ------------------------------------------------------------------------------------------
 // samples / fixtures checks shared by the score grid and the pointwise log-likelihood (`what` prefixes the message)
-static int check_sample_args(const bplx_samples* s, const bplx_fixtures* f, const char* what) {
+// allow_no_fixtures: F = 0 is accepted (a tournament whose group stage is already played), the fixture arrays may then
+// be NULL
+static int check_sample_args(const bplx_samples* s, const bplx_fixtures* f, const char* what,
+                             bool allow_no_fixtures = false) {
   BPLX_REQUIRE(s && f, BPLX_E_INVALID, "samples / fixtures is NULL");
   BPLX_REQUIRE(s->model >= BPLX_DIXON_COLES && s->model <= BPLX_NEUTRAL_WC, BPLX_E_UNSUPPORTED,
                "%s: model %d unsupported (DYNAMIC predict is unusable in the reference)", what, s->model);
-  BPLX_REQUIRE(s->num_samples > 0 && s->num_teams > 0 && f->num_fixtures > 0, BPLX_E_INVALID,
+  const bool fixtures = !(allow_no_fixtures && f->num_fixtures == 0);
+  BPLX_REQUIRE(s->num_samples > 0 && s->num_teams > 0 && (f->num_fixtures > 0 || !fixtures), BPLX_E_INVALID,
                "%s: num_samples, num_teams and num_fixtures must be positive", what);
-  BPLX_REQUIRE(s->attack && s->defence && s->corr_coef && f->home_team && f->away_team, BPLX_E_INVALID,
+  BPLX_REQUIRE(s->attack && s->defence && s->corr_coef && (!fixtures || (f->home_team && f->away_team)), BPLX_E_INVALID,
                "%s: attack, defence, corr_coef, home_team, away_team must not be NULL", what);
   BPLX_REQUIRE(s->home_attack, BPLX_E_INVALID, "%s: home_attack (home advantage) must not be NULL", what);
   if (s->model == BPLX_NEUTRAL || s->model == BPLX_NEUTRAL_WC)
     BPLX_REQUIRE(s->away_attack && s->home_defence && s->away_defence, BPLX_E_INVALID,
                  "%s: neutral models need away_attack, home_defence, away_defence", what);
   if (s->model == BPLX_NEUTRAL_WC)
-    BPLX_REQUIRE(s->confederation_strength && s->num_conferences > 0 && f->home_conf && f->away_conf, BPLX_E_INVALID,
-                 "%s: NEUTRAL_WC needs confederation_strength, home_conf, away_conf", what);
+    BPLX_REQUIRE(s->confederation_strength && s->num_conferences > 0 && (!fixtures || (f->home_conf && f->away_conf)),
+                 BPLX_E_INVALID, "%s: NEUTRAL_WC needs confederation_strength, home_conf, away_conf", what);
   return BPLX_OK;
 }
 
@@ -817,42 +821,40 @@ size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures*
   return simulate_plan_for(s, f, &sp);
 }
 
-int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
-                        const bplx_table* t, int max_goals, int sims_per_draw, unsigned long long seed,
-                        long long first_draw, unsigned long long* position_counts, unsigned long long* points_counts,
-                        uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
-                        size_t workspace_bytes, void* stream) {
-  int rc = check_sample_args(s, f, "simulate");
+// validates the arguments bplx_simulate_table and bplx_simulate_tournament share and fills *sp (its workspace aside)
+static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                          const uint8_t* away_slot, const bplx_table* t, int max_goals, int sims_per_draw,
+                          unsigned long long seed, long long first_draw, unsigned long long* position_counts,
+                          unsigned long long* points_counts, uint8_t* positions, uint8_t* scores,
+                          unsigned long long* invalid, const char* what, bool allow_no_fixtures, SimParams* out) {
+  int rc = check_sample_args(s, f, what, allow_no_fixtures);
   if (rc != BPLX_OK) return rc;
-  BPLX_REQUIRE(t != nullptr, BPLX_E_INVALID, "simulate: table is NULL");
+  BPLX_REQUIRE(t != nullptr, BPLX_E_INVALID, "%s: table is NULL", what);
   BPLX_REQUIRE(t->num_slots <= BPLX_SIM_MAX_TEAMS, BPLX_E_UNSUPPORTED,
-               "simulate: %d table slots exceed the kernel's limit of %d (BPLX_SIM_MAX_TEAMS)", t->num_slots,
+               "%s: %d table slots exceed the kernel's limit of %d (BPLX_SIM_MAX_TEAMS)", what, t->num_slots,
                BPLX_SIM_MAX_TEAMS);
-  BPLX_REQUIRE(t->num_slots >= 1, BPLX_E_INVALID, "simulate: the table needs at least one slot");
+  BPLX_REQUIRE(t->num_slots >= 1, BPLX_E_INVALID, "%s: the table needs at least one slot", what);
   BPLX_REQUIRE(t->num_positions >= 1 && t->num_positions <= t->num_slots && t->num_points_bins >= 1, BPLX_E_INVALID,
-               "simulate: num_positions must be in [1, num_slots] and num_points_bins >= 1 (got %d, %d)",
+               "%s: num_positions must be in [1, num_slots] and num_points_bins >= 1 (got %d, %d)", what,
                t->num_positions, t->num_points_bins);
   BPLX_REQUIRE(t->points_win >= 1 && t->points_draw >= 0 && t->points_draw <= t->points_win, BPLX_E_INVALID,
-               "simulate: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)",
+               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
                t->points_win, t->points_draw);
   BPLX_REQUIRE(t->start_points && t->start_goals_for && t->start_goals_against, BPLX_E_INVALID,
-               "simulate: start_points, start_goals_for and start_goals_against must not be NULL");
-  BPLX_REQUIRE(home_slot && away_slot, BPLX_E_INVALID, "simulate: home_slot and away_slot must not be NULL");
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "simulate: max_goals must be in [1, 63] (got %d)",
+               "%s: start_points, start_goals_for and start_goals_against must not be NULL", what);
+  BPLX_REQUIRE((home_slot && away_slot) || f->num_fixtures == 0, BPLX_E_INVALID,
+               "%s: home_slot and away_slot must not be NULL", what);
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
                max_goals);
-  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "simulate: sims_per_draw must be >= 1 (got %d)", sims_per_draw);
+  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
   BPLX_REQUIRE(first_draw >= 0 && first_draw + s->num_samples <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
-               "simulate: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits");
+               "%s: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits", what);
   BPLX_REQUIRE((long long)s->num_samples * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
-               "simulate: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
-               (long long)s->num_samples * sims_per_draw);
+               "%s: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
+               what, (long long)s->num_samples * sims_per_draw);
   BPLX_REQUIRE(position_counts && points_counts && invalid, BPLX_E_INVALID,
-               "simulate: position_counts, points_counts and invalid must not be NULL");
-  SimParams sp{};
-  const size_t need = simulate_plan_for(s, f, &sp);
-  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
-               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
-  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+               "%s: position_counts, points_counts and invalid must not be NULL", what);
+  SimParams& sp = *out;
   GridParams& gp = sp.gp;
   gp.attack = s->attack;
   gp.defence = s->defence;
@@ -867,7 +869,6 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
   gp.hconf = f->home_conf;
   gp.aconf = f->away_conf;
   gp.nv = f->neutral_venue;
-  gp.table = static_cast<float*>(workspace);
   sp.hslot = home_slot;
   sp.aslot = away_slot;
   sp.group = t->group;
@@ -889,7 +890,164 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
   sp.invalid = invalid;
   sp.positions = positions;
   sp.scores = scores;
+  return BPLX_OK;
+}
+
+int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
+                        const bplx_table* t, int max_goals, int sims_per_draw, unsigned long long seed,
+                        long long first_draw, unsigned long long* position_counts, unsigned long long* points_counts,
+                        uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  SimParams sp{};
+  int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
+                          points_counts, positions, scores, invalid, "simulate", false, &sp);
+  if (rc != BPLX_OK) return rc;
+  const size_t need = simulate_plan_for(s, f, &sp);
+  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
+               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  sp.gp.table = static_cast<float*>(workspace);
   return launch_simulate(sp, static_cast<cudaStream_t>(stream));
+}
+
+// ---- tournament simulation -----------------------------------------------------------------------------------
+static size_t alloc_bytes(const bplx_bracket* b) {
+  return b->best_alloc ? ((size_t)b->best_count << b->num_groups) : 0;
+}
+
+size_t bplx_simulate_tournament_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
+                                                const bplx_bracket* b) {
+  if (!s || !f || !t || !b || s->num_samples <= 0 || s->num_teams <= 0 || f->num_fixtures < 0) return 0;
+  if (b->num_groups < 0 || b->num_groups > BPLX_SIM_MAX_TEAMS || b->best_count < 0) return 0;
+  if (b->best_alloc && b->num_groups > BPLX_KO_MAX_ALLOC_GROUPS) return 0;
+  SimParams sp{};
+  return simulate_plan_for(s, f, &sp) + (alloc_bytes(b) + 255) / 256 * 256;
+}
+
+// the bracket checks the kernel relies on; fills sp->ko
+static int check_bracket(const bplx_bracket* b, const bplx_samples* s, int NT, int P, KoParams* ko) {
+  BPLX_REQUIRE(b != nullptr, BPLX_E_INVALID, "tournament: bracket is NULL");
+  const int K = b->num_ties;
+  BPLX_REQUIRE(K >= 1, BPLX_E_INVALID, "tournament: the bracket needs at least one tie (got %d)", K);
+  BPLX_REQUIRE(K <= BPLX_KO_MAX_TIES, BPLX_E_UNSUPPORTED,
+               "tournament: %d ties exceed the kernel's limit of %d (BPLX_KO_MAX_TIES)", K, BPLX_KO_MAX_TIES);
+  BPLX_REQUIRE(b->num_rounds >= 1 && b->num_rounds <= BPLX_KO_MAX_ROUNDS, BPLX_E_UNSUPPORTED,
+               "tournament: num_rounds must be in [1, %d] (got %d)", BPLX_KO_MAX_ROUNDS, b->num_rounds);
+  BPLX_REQUIRE(b->num_groups >= 0 && b->num_groups <= NT, BPLX_E_INVALID,
+               "tournament: num_groups must be in [0, num_slots] (got %d)", b->num_groups);
+  BPLX_REQUIRE(b->best_count >= 0 && b->best_count <= BPLX_KO_MAX_BEST, BPLX_E_UNSUPPORTED,
+               "tournament: best_count must be in [0, %d] (got %d)", BPLX_KO_MAX_BEST, b->best_count);
+  BPLX_REQUIRE(b->best_count <= b->num_groups, BPLX_E_INVALID,
+               "tournament: best_count (%d) exceeds num_groups (%d)", b->best_count, b->num_groups);
+  BPLX_REQUIRE(b->best_count == 0 || (b->best_position >= 0 && b->best_position < P), BPLX_E_INVALID,
+               "tournament: best_position must be in [0, num_positions) (got %d)", b->best_position);
+  BPLX_REQUIRE(b->kind && b->arg0 && b->arg1 && b->round && b->slot_team, BPLX_E_INVALID,
+               "tournament: kind, arg0, arg1, round and slot_team must not be NULL");
+  BPLX_REQUIRE(s->model != BPLX_NEUTRAL_WC || b->slot_conf, BPLX_E_INVALID, "tournament: NEUTRAL_WC needs slot_conf");
+  for (int t = 0; t < NT; t++) {
+    BPLX_REQUIRE(b->slot_team[t] < s->num_teams, BPLX_E_INVALID,
+                 "tournament: slot_team[%d] = %d is not a model team (T = %d)", t, b->slot_team[t], s->num_teams);
+    if (s->model == BPLX_NEUTRAL_WC)
+      BPLX_REQUIRE(b->slot_conf[t] < s->num_conferences, BPLX_E_INVALID,
+                   "tournament: slot_conf[%d] = %d is not a confederation (Cf = %d)", t, b->slot_conf[t],
+                   s->num_conferences);
+  }
+  for (int k = 0; k < K; k++) {
+    BPLX_REQUIRE(b->round[k] < b->num_rounds, BPLX_E_INVALID, "tournament: tie %d: round %d >= num_rounds (%d)", k,
+                 b->round[k], b->num_rounds);
+    for (int side = 0; side < 2; side++) {
+      const int kind = b->kind[2 * k + side], a0 = b->arg0[2 * k + side], a1 = b->arg1[2 * k + side];
+      const char* sd = side ? "away" : "home";
+      switch (kind) {
+        case BPLX_ENTRANT_SLOT:
+          BPLX_REQUIRE(a0 < NT, BPLX_E_INVALID, "tournament: tie %d %s: slot %d outside the table (%d slots)", k, sd,
+                       a0, NT);
+          break;
+        case BPLX_ENTRANT_GROUP_POS:
+          BPLX_REQUIRE(a0 < b->num_groups && a1 < P, BPLX_E_INVALID,
+                       "tournament: tie %d %s: group %d position %d out of range (%d groups, %d positions)", k, sd, a0,
+                       a1, b->num_groups, P);
+          break;
+        case BPLX_ENTRANT_BEST:
+          BPLX_REQUIRE(a0 < b->best_count, BPLX_E_INVALID, "tournament: tie %d %s: BEST %d >= best_count (%d)", k, sd,
+                       a0, b->best_count);
+          break;
+        case BPLX_ENTRANT_WINNER:
+        case BPLX_ENTRANT_LOSER:
+          BPLX_REQUIRE(a0 < k, BPLX_E_INVALID, "tournament: tie %d %s: refers to tie %d, which is not earlier", k, sd,
+                       a0);
+          break;
+        default:
+          BPLX_REQUIRE(false, BPLX_E_INVALID, "tournament: tie %d %s: unknown entrant kind %d", k, sd, kind);
+      }
+      ko->kind[side][k] = (uint8_t)kind;
+      ko->arg0[side][k] = (uint8_t)a0;
+      ko->arg1[side][k] = (uint8_t)a1;
+    }
+    ko->round[k] = b->round[k];
+    ko->neutral[k] = b->neutral_venue ? (b->neutral_venue[k] != 0) : 0;
+  }
+  if (b->best_alloc) {
+    BPLX_REQUIRE(b->best_count >= 1, BPLX_E_INVALID, "tournament: an allocation table needs best_count >= 1");
+    BPLX_REQUIRE(b->num_groups <= BPLX_KO_MAX_ALLOC_GROUPS, BPLX_E_UNSUPPORTED,
+                 "tournament: an allocation table supports at most %d groups (got %d)", BPLX_KO_MAX_ALLOC_GROUPS,
+                 b->num_groups);
+    for (unsigned mask = 0; mask < (1u << b->num_groups); mask++) {
+      unsigned seen = 0;
+      for (int j = 0; j < b->best_count; j++) {
+        const int g = b->best_alloc[(size_t)mask * b->best_count + j];
+        if (g == 0xFF) continue;
+        BPLX_REQUIRE(g < b->num_groups && ((mask >> g) & 1u) && !((seen >> g) & 1u), BPLX_E_INVALID,
+                     "tournament: allocation row 0x%x entry %d: group %d is not a distinct group of the row's set", mask,
+                     j, g);
+        seen |= 1u << g;
+      }
+    }
+  }
+  for (int t = 0; t < NT; t++) {
+    ko->slot_team[t] = b->slot_team[t];
+    ko->slot_conf[t] = b->slot_conf ? b->slot_conf[t] : 0;
+  }
+  ko->K = K;
+  ko->nr = b->num_rounds;
+  ko->ng = b->num_groups;
+  ko->bp = b->best_position;
+  ko->bc = b->best_count;
+  return BPLX_OK;
+}
+
+int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                             const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b, int max_goals,
+                             int sims_per_draw, unsigned long long seed, long long first_draw,
+                             unsigned long long* position_counts, unsigned long long* points_counts,
+                             unsigned long long* reach_counts, unsigned long long* win_counts, uint8_t* positions,
+                             uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
+                             unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream) {
+  SimParams sp{};
+  int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
+                          points_counts, positions, scores, invalid, "tournament", true, &sp);
+  if (rc != BPLX_OK) return rc;
+  rc = check_bracket(b, s, t->num_slots, t->num_positions, &sp.ko);
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
+  const size_t table = simulate_plan_for(s, f, &sp);
+  const size_t need = table + (alloc_bytes(b) + 255) / 256 * 256;
+  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
+               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  sp.gp.table = static_cast<float*>(workspace);
+  sp.ko.reach = reach_counts;
+  sp.ko.win = win_counts;
+  sp.ko.entrants = ko_entrants;
+  sp.ko.scores = ko_scores;
+  sp.ko.winners = ko_winners;
+  if (b->best_alloc) {
+    uint8_t* const dst = static_cast<uint8_t*>(workspace) + table;
+    BPLX_CUDA(cudaMemcpyAsync(dst, b->best_alloc, alloc_bytes(b), cudaMemcpyHostToDevice,
+                              static_cast<cudaStream_t>(stream)));
+    sp.ko.alloc = dst;
+  }
+  return launch_simulate_tournament(sp, static_cast<cudaStream_t>(stream));
 }
 
 void bplx_reload_env(void) {

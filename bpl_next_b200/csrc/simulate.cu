@@ -126,11 +126,40 @@ __device__ __forceinline__ bool sample_score(float lh, float la, float c, float 
   return true;
 }
 
+// the draw's un-normalised win masses on the same clamped, truncated grid as sample_score: hw = sum_{i > j} w(i, j),
+// aw = sum_{i < j} w(i, j), with running prefixes of the pmfs (O(G)); tau+ enters through the cells (1, 0) and (0, 1)
+__device__ __forceinline__ void win_masses(float lh, float la, float c, int G, float& hw, float& aw) {
+  float p = lh, q = la, Pc = 1.0f + lh, Qc = 1.0f + la;  // p_1, q_1, sum_{i <= 1} p_i, sum_{j <= 1} q_j
+  hw = lh * fmaxf(fmaf(c, la, 1.0f), 0.0f);               // w(1, 0) = tau+(1, 0) p_1 q_0
+  aw = la * fmaxf(fmaf(c, lh, 1.0f), 0.0f);               // w(0, 1)
+  for (int k = 2; k <= G; k++) {
+    p *= lh * c_sim_inv_k[k];
+    q *= la * c_sim_inv_k[k];
+    hw = fmaf(p, Qc, hw);
+    aw = fmaf(q, Pc, aw);
+    Qc += q;
+    Pc += p;
+  }
+}
+
+// word w of the Philox sequence of simulation n (curand_init(seed, n, 0) followed by w + 1 curand()) without a state:
+// the tournament kernel reads the slot tie-break keys only when points, goal difference and goals for are level
+__device__ __forceinline__ uint32_t philox_word(unsigned long long seed, unsigned long long n, unsigned w) {
+  const uint4 o = curand_Philox4x32_10(make_uint4(w >> 2, 0u, (unsigned)n, (unsigned)(n >> 32)),
+                                       make_uint2((unsigned)seed, (unsigned)(seed >> 32)));
+  const unsigned r = w & 3u;
+  return r == 0 ? o.x : r == 1 ? o.y : r == 2 ? o.z : o.w;
+}
+
 }  // namespace
 
+// KO = false: season / group stage (bplx_simulate_table).  KO = true: the same group stage, then the knockout bracket
+// (bplx_simulate_tournament; see simulate_tournament_phase below).
+template <bool KO>
 __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_constant__ SimParams sp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const GridParams& gp = sp.gp;
+  const KoParams& ko = sp.ko;
   const int NT = sp.NT, tid = threadIdx.x;
   // [slot][thread] accumulators, then the histograms, then the group member lists
   int* const s_pts = reinterpret_cast<int*>(smem_raw);
@@ -139,12 +168,26 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   uint32_t* const s_key = reinterpret_cast<uint32_t*>(s_gd + NT * kSimThreads);
   unsigned* const h_pos = s_key + NT * kSimThreads;
   unsigned* const h_pts = h_pos + NT * sp.P;
-  int* const s_members = reinterpret_cast<int*>(h_pts + (sp.points_in_smem ? NT * sp.B : 0));
+  unsigned* const h_reach = h_pts + (sp.points_in_smem ? NT * sp.B : 0);  // tournament: [NT][nr] each
+  unsigned* const h_win = h_reach + (KO ? NT * ko.nr : 0);
+  int* const s_members = reinterpret_cast<int*>(h_win + (KO ? NT * ko.nr : 0));
   int* const s_gbeg = s_members + NT;
   int* const s_gcnt = s_gbeg + NT;
+  // Tournament: the keys are not stored (philox_word reads one when it is needed), so the s_key words hold bytes:
+  // k_q [NT][thread] = the slot ranked p-th in its group at member index gbeg + p, k_best [bc][thread] = the slot of
+  // BEST j, k_gtab = per CTA, first member index [ng] and size [ng] of each group id.  The per-tie winner / loser bytes
+  // go into the thread's OWN s_gf / s_gd words once its ranking and best-placed selection are done (byte b in byte
+  // b % 4 of word [b / 4][thread], so a thread that reaches its ties early never touches the words another thread is
+  // still ranking), or after the member lists when 2K bytes exceed those 2 T_tab words.
+  uint8_t* const k_q = reinterpret_cast<uint8_t*>(s_key);
+  uint8_t* const k_best = k_q + NT * kSimThreads;
+  uint8_t* const k_gtab = k_best + (KO ? ko.bc : 0) * kSimThreads;
+  uint8_t* const k_wl = KO && !ko.wl_overlay ? reinterpret_cast<uint8_t*>(s_gcnt + NT) : reinterpret_cast<uint8_t*>(s_gf);
   __shared__ unsigned s_invalid;
   __shared__ int s_groups_fit;
 #define ACC(arr, t) arr[(t) * kSimThreads + tid]
+#define BYTE(arr, k) arr[(k) * kSimThreads + tid]
+#define WL(b) k_wl[(((b) >> 2) * kSimThreads + tid) * 4 + ((b) & 3)]
 
   if (tid == 0) {
     s_invalid = 0;
@@ -153,6 +196,19 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   for (int k = tid; k < NT * sp.P; k += kSimThreads) h_pos[k] = 0;
   if (sp.points_in_smem)
     for (int k = tid; k < NT * sp.B; k += kSimThreads) h_pts[k] = 0;
+  if constexpr (KO) {
+    for (int k = tid; k < 2 * NT * ko.nr; k += kSimThreads) h_reach[k] = 0;  // h_win follows h_reach
+    for (int g = tid; g < ko.ng; g += kSimThreads) {
+      int beg = 0, cnt = 0;
+      for (int u = 0; u < NT; u++) {
+        const int gu = sp.group ? sp.group[u] : 0;
+        beg += gu < g;
+        cnt += gu == g;
+      }
+      k_gtab[g] = (uint8_t)beg;
+      k_gtab[ko.ng + g] = (uint8_t)cnt;
+    }
+  }
   __syncthreads();
   // group member lists: slots sorted by (group, slot); s_gbeg / s_gcnt = where a slot's group starts and its size
   for (int t = tid; t < NT; t += kSimThreads) {
@@ -213,45 +269,186 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
       }
       if (sc) *reinterpret_cast<uchar2*>(sc + 2 * f) = make_uchar2((unsigned char)hg, (unsigned char)ag);
     }
-    for (int t = 0; t < NT; t++) {
-      ACC(s_key, t) = curand(&rng);
-      ACC(s_gd, t) = ACC(s_gf, t) - ACC(s_gd, t);
-      const int gained = ACC(s_pts, t) - sp.start_pts[t];
-      ok = ok && gained >= 0 && gained < sp.B;  // (bins sized by the caller: a short one is refused, never overrun)
-    }
-    ok = ok && s_groups_fit;
-    uint8_t* const prow = sp.positions ? sp.positions + (size_t)i * NT : nullptr;
-    if (!ok) {
-      atomicAdd(&s_invalid, 1u);
-      if (prow)
-        for (int t = 0; t < NT; t++) prow[t] = 0xFF;
+    if constexpr (!KO) {
+      for (int t = 0; t < NT; t++) {
+        ACC(s_key, t) = curand(&rng);
+        ACC(s_gd, t) = ACC(s_gf, t) - ACC(s_gd, t);
+        const int gained = ACC(s_pts, t) - sp.start_pts[t];
+        ok = ok && gained >= 0 && gained < sp.B;  // (bins sized by the caller: a short one is refused, never overrun)
+      }
+      ok = ok && s_groups_fit;
+      uint8_t* const prow = sp.positions ? sp.positions + (size_t)i * NT : nullptr;
+      if (!ok) {
+        atomicAdd(&s_invalid, 1u);
+        if (prow)
+          for (int t = 0; t < NT; t++) prow[t] = 0xFF;
+      } else {
+        for (int t = 0; t < NT; t++) {
+          const int pt = ACC(s_pts, t), dt = ACC(s_gd, t), ft = ACC(s_gf, t);
+          const uint32_t kt = ACC(s_key, t);
+          const int g0 = s_gbeg[t], gc = s_gcnt[t];
+          int pos = 0;
+          for (int m = 0; m < gc; m++) {
+            const int u = s_members[g0 + m];
+            const int pu = ACC(s_pts, u), du = ACC(s_gd, u), fu = ACC(s_gf, u);
+            const uint32_t ku = ACC(s_key, u);
+            pos += pu != pt ? pu > pt : du != dt ? du > dt : fu != ft ? fu > ft : ku != kt ? ku > kt : u < t;
+          }
+          if (prow) prow[t] = (uint8_t)pos;
+          atomicAdd(&h_pos[t * sp.P + pos], 1u);
+          const int gained = pt - sp.start_pts[t];
+          if (sp.points_in_smem) atomicAdd(&h_pts[t * sp.B + gained], 1u);
+          else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
+        }
+      }
     } else {
       for (int t = 0; t < NT; t++) {
-        const int pt = ACC(s_pts, t), dt = ACC(s_gd, t), ft = ACC(s_gf, t);
-        const uint32_t kt = ACC(s_key, t);
-        const int g0 = s_gbeg[t], gc = s_gcnt[t];
-        int pos = 0;
-        for (int m = 0; m < gc; m++) {
-          const int u = s_members[g0 + m];
-          const int pu = ACC(s_pts, u), du = ACC(s_gd, u), fu = ACC(s_gf, u);
-          const uint32_t ku = ACC(s_key, u);
-          pos += pu != pt ? pu > pt : du != dt ? du > dt : fu != ft ? fu > ft : ku != kt ? ku > kt : u < t;
+        ACC(s_gd, t) = ACC(s_gf, t) - ACC(s_gd, t);
+        const int gained = ACC(s_pts, t) - sp.start_pts[t];
+        ok = ok && gained >= 0 && gained < sp.B;
+      }
+      ok = ok && s_groups_fit;
+      const unsigned wkey = 2u * (unsigned)gp.F;  // word of slot 0's tie-break key
+      // a slot u ranked ahead of slot t (u != t): points, goal difference, goals for, the key, then the lower slot
+      auto ahead = [&](int u, int t) -> bool {
+        const int pu = ACC(s_pts, u), pt = ACC(s_pts, t);
+        if (pu != pt) return pu > pt;
+        const int du = ACC(s_gd, u), dt = ACC(s_gd, t);
+        if (du != dt) return du > dt;
+        const int fu = ACC(s_gf, u), ft = ACC(s_gf, t);
+        if (fu != ft) return fu > ft;
+        const uint32_t ku = philox_word(sp.seed, n, wkey + u), kt = philox_word(sp.seed, n, wkey + t);
+        return ku != kt ? ku > kt : u < t;
+      };
+      if (ok) {
+        // ranking within the groups: k_q[gbeg + position] = slot
+        for (int t = 0; t < NT; t++) {
+          const int g0 = s_gbeg[t], gc = s_gcnt[t];
+          int pos = 0;
+          for (int m = 0; m < gc; m++) {
+            const int u = s_members[g0 + m];
+            if (u != t) pos += ahead(u, t);
+          }
+          BYTE(k_q, g0 + pos) = (uint8_t)t;
         }
-        if (prow) prow[t] = (uint8_t)pos;
-        atomicAdd(&h_pos[t * sp.P + pos], 1u);
-        const int gained = pt - sp.start_pts[t];
-        if (sp.points_in_smem) atomicAdd(&h_pts[t * sp.B + gained], 1u);
-        else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
+        // best-placed qualifiers: the slot at best_position of every group, ranked across groups
+        if (ko.bc > 0) {
+          unsigned mask = 0;
+          int nq = 0;
+          for (int g = 0; g < ko.ng; g++) {
+            if (k_gtab[ko.ng + g] <= ko.bp) continue;
+            const int t = BYTE(k_q, k_gtab[g] + ko.bp);
+            int rk = 0;
+            for (int h = 0; h < ko.ng; h++)
+              if (h != g && k_gtab[ko.ng + h] > ko.bp) rk += ahead(BYTE(k_q, k_gtab[h] + ko.bp), t);
+            if (rk < ko.bc) {
+              nq++;
+              if (ko.alloc) mask |= 1u << g;
+              else BYTE(k_best, rk) = (uint8_t)t;
+            }
+          }
+          ok = nq == ko.bc;
+          if (ok && ko.alloc) {
+            const uint8_t* const arow = ko.alloc + (size_t)mask * ko.bc;
+            for (int j = 0; j < ko.bc; j++) {
+              const int g = arow[j];
+              if (g < ko.ng && ((mask >> g) & 1u)) BYTE(k_best, j) = BYTE(k_q, k_gtab[g] + ko.bp);
+              else ok = false;  // an allocation row of 0xFF
+            }
+          }
+        }
+      }
+      // the ties in play order; words 2F + T_tab + 3k, + 1 (the score) and + 2 (the decider) of tie k
+      skipahead((unsigned long long)NT, &rng);
+      uint8_t* const ent = ko.entrants ? ko.entrants + (size_t)i * ko.K * 2 : nullptr;
+      uint8_t* const ksc = ko.scores ? ko.scores + (size_t)i * ko.K * 2 : nullptr;
+      uint8_t* const kwn = ko.winners ? ko.winners + (size_t)i * ko.K : nullptr;
+#pragma unroll 1
+      for (int k = 0; k < ko.K && ok; k++) {
+        int e[2];
+#pragma unroll
+        for (int side = 0; side < 2; side++) {
+          const int a0 = ko.arg0[side][k];
+          switch (ko.kind[side][k]) {
+            case BPLX_ENTRANT_SLOT: e[side] = a0; break;
+            case BPLX_ENTRANT_GROUP_POS: {
+              const int p = ko.arg1[side][k];
+              ok = ok && p < k_gtab[ko.ng + a0];
+              e[side] = ok ? BYTE(k_q, k_gtab[a0] + p) : 0;
+              break;
+            }
+            case BPLX_ENTRANT_BEST: e[side] = BYTE(k_best, a0); break;
+            case BPLX_ENTRANT_WINNER: e[side] = WL(2 * a0); break;
+            default: e[side] = WL(2 * a0 + 1); break;
+          }
+        }
+        const float uh = curand_uniform(&rng), ua = curand_uniform(&rng), ud = curand_uniform(&rng);
+        if (!ok) break;
+        const int hs = e[0], as = e[1];
+        const bool neutral = gp.ntab == 3 && ko.neutral[k];
+        const FixtureOffsets off = fixture_offsets(L, ko.slot_team[hs], ko.slot_team[as], neutral, wc,
+                                                   wc ? ko.slot_conf[hs] : 0, wc ? ko.slot_conf[as] : 0);
+        const float2 lam = fixture_rates(row, off, neutral, wc);
+        int hg = 0, ag = 0;
+        ok = sample_score(lam.x, lam.y, c, uh, ua, sp.G, hg, ag);
+        bool home_through = hg > ag;
+        if (ok && hg == ag) {  // a drawn tie: the home entrant goes through iff u_d (hw + aw) <= hw
+          float hw, aw;
+          win_masses(lam.x, lam.y, c, sp.G, hw, aw);
+          const float tot = hw + aw;
+          ok = tot > 0.0f;
+          home_through = ud * tot <= hw;
+        }
+        if (!ok) break;
+        const int w = home_through ? hs : as;
+        WL(2 * k) = (uint8_t)w;
+        WL(2 * k + 1) = (uint8_t)(home_through ? as : hs);
+        if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2((unsigned char)hs, (unsigned char)as);
+        if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2((unsigned char)hg, (unsigned char)ag);
+        if (kwn) kwn[k] = (uint8_t)w;
+      }
+      uint8_t* const prow = sp.positions ? sp.positions + (size_t)i * NT : nullptr;
+      if (!ok) {
+        atomicAdd(&s_invalid, 1u);
+        if (prow)
+          for (int t = 0; t < NT; t++) prow[t] = 0xFF;
+        for (int k = 0; k < ko.K; k++) {
+          if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2(0xFF, 0xFF);
+          if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2(0xFF, 0xFF);
+          if (kwn) kwn[k] = 0xFF;
+        }
+      } else {
+        for (int m = 0; m < NT; m++) {
+          const int t = BYTE(k_q, m), pos = m - s_gbeg[t];
+          if (prow) prow[t] = (uint8_t)pos;
+          atomicAdd(&h_pos[t * sp.P + pos], 1u);
+          const int gained = ACC(s_pts, t) - sp.start_pts[t];
+          if (sp.points_in_smem) atomicAdd(&h_pts[t * sp.B + gained], 1u);
+          else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
+        }
+        for (int k = 0; k < ko.K; k++) {
+          const int r = ko.round[k], w = WL(2 * k), l = WL(2 * k + 1);
+          atomicAdd(&h_reach[w * ko.nr + r], 1u);
+          atomicAdd(&h_reach[l * ko.nr + r], 1u);
+          atomicAdd(&h_win[w * ko.nr + r], 1u);
+        }
       }
     }
   }
 #undef ACC
+#undef BYTE
+#undef WL
   __syncthreads();
   for (int k = tid; k < NT * sp.P; k += kSimThreads)
     if (h_pos[k]) atomicAdd(&sp.pos_counts[k], (unsigned long long)h_pos[k]);
   if (sp.points_in_smem)
     for (int k = tid; k < NT * sp.B; k += kSimThreads)
       if (h_pts[k]) atomicAdd(&sp.pts_counts[k], (unsigned long long)h_pts[k]);
+  if constexpr (KO)
+    for (int k = tid; k < NT * ko.nr; k += kSimThreads) {
+      if (h_reach[k]) atomicAdd(&ko.reach[k], (unsigned long long)h_reach[k]);
+      if (h_win[k]) atomicAdd(&ko.win[k], (unsigned long long)h_win[k]);
+    }
   if (tid == 0 && s_invalid) atomicAdd(sp.invalid, (unsigned long long)s_invalid);
 }
 
@@ -265,7 +462,13 @@ size_t simulate_plan(SimParams* sp) {
 }
 
 size_t simulate_smem_bytes(SimParams* sp) {
-  const size_t base = (size_t)sp->NT * kSimThreads * 16 + (size_t)sp->NT * sp->P * 4 + (size_t)sp->NT * 12;
+  size_t base = (size_t)sp->NT * kSimThreads * 16 + (size_t)sp->NT * sp->P * 4 + (size_t)sp->NT * 12;
+  if (sp->ko.K > 0) {
+    // the reach / win histograms; the winner / loser bytes overlay s_gf and s_gd when they fit there (K <= 4 T_tab)
+    base += (size_t)sp->NT * sp->ko.nr * 8;
+    sp->ko.wl_overlay = sp->ko.K <= 4 * sp->NT;
+    if (!sp->ko.wl_overlay) base += (size_t)(2 * sp->ko.K + 3) / 4 * 4 * kSimThreads;
+  }
   const size_t pts = (size_t)sp->NT * sp->B * 4;
   sp->points_in_smem = base + pts <= (size_t)kSimSmemMax;
   return base + (sp->points_in_smem ? pts : 0);
@@ -281,26 +484,36 @@ static int upload_sim_constants() {
   return BPLX_OK;
 }
 
-int launch_simulate(SimParams& sp, cudaStream_t stream) {
+template <bool KO>
+static int launch_simulate_impl(SimParams& sp, cudaStream_t stream) {
   int rc = upload_sim_constants();
   if (rc != BPLX_OK) return rc;
+  if (!KO) sp.ko.K = 0;
   const size_t smem = simulate_smem_bytes(&sp);
   BPLX_REQUIRE(smem <= (size_t)kSimSmemMax, BPLX_E_UNSUPPORTED,
                "simulate: %zu bytes of shared memory per CTA needed (max %d)", smem, kSimSmemMax);
   static size_t smem_set = 48 * 1024;
   if (smem > smem_set) {
-    BPLX_CUDA(cudaFuncSetAttribute(simulate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BPLX_CUDA(cudaFuncSetAttribute(simulate_kernel<KO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set = smem;
   }
   BPLX_CUDA(cudaMemsetAsync(sp.pos_counts, 0, (size_t)sp.NT * sp.P * 8, stream));
   BPLX_CUDA(cudaMemsetAsync(sp.pts_counts, 0, (size_t)sp.NT * sp.B * 8, stream));
   BPLX_CUDA(cudaMemsetAsync(sp.invalid, 0, 8, stream));
+  if (KO) {
+    BPLX_CUDA(cudaMemsetAsync(sp.ko.reach, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
+    BPLX_CUDA(cudaMemsetAsync(sp.ko.win, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
+  }
   rc = launch_score_grid_tables(sp.gp, stream);
   if (rc != BPLX_OK) return rc;
-  simulate_kernel<<<(unsigned)((sp.N + kSimThreads - 1) / kSimThreads), kSimThreads, smem, stream>>>(sp);
+  simulate_kernel<KO><<<(unsigned)((sp.N + kSimThreads - 1) / kSimThreads), kSimThreads, smem, stream>>>(sp);
   BPLX_CUDA(cudaGetLastError());
   note_launch(1);
   return BPLX_OK;
 }
+
+int launch_simulate(SimParams& sp, cudaStream_t stream) { return launch_simulate_impl<false>(sp, stream); }
+
+int launch_simulate_tournament(SimParams& sp, cudaStream_t stream) { return launch_simulate_impl<true>(sp, stream); }
 
 }  // namespace bplx

@@ -7,6 +7,26 @@ namespace bplx {
 constexpr int kSimThreads = 128;    // simulations per CTA (one thread per simulation)
 constexpr int kSimMaxTeams = 64;    // BPLX_SIM_MAX_TEAMS
 constexpr int kSimSmemMax = 227 * 1024;
+constexpr int kKoMaxTies = 64;      // BPLX_KO_MAX_TIES
+constexpr int kKoMaxRounds = 16;    // BPLX_KO_MAX_ROUNDS
+constexpr int kKoMaxBest = 16;      // BPLX_KO_MAX_BEST
+
+// the knockout bracket of a tournament simulation (K = 0: group stage only, the bplx_simulate_table kernel).  The per-tie
+// arrays travel by value in the kernel parameters (read warp-uniformly from the constant bank).
+struct KoParams {
+  int K, nr, ng, bp, bc;          // ties, rounds, groups, best_position, best_count (0: no best-placed pool)
+  int wl_overlay;                 // the per-tie winner / loser bytes live in the dead s_gf / s_gd accumulators
+  const uint8_t* alloc;           // device [2^ng][bc] allocation table or NULL (in the workspace)
+  unsigned long long *reach, *win;  // [NT][nr]
+  uint8_t *entrants, *scores, *winners;  // [N][K][2], [N][K][2], [N][K] or NULL
+  uint8_t kind[2][kKoMaxTies];    // (home, away) entrant kinds: BPLX_ENTRANT_*
+  uint8_t arg0[2][kKoMaxTies];    // slot / group / j / earlier tie
+  uint8_t arg1[2][kKoMaxTies];    // position of GROUP_POS
+  uint8_t round[kKoMaxTies];
+  uint8_t neutral[kKoMaxTies];
+  uint16_t slot_team[kSimMaxTeams];
+  uint8_t slot_conf[kSimMaxTeams];
+};
 
 struct SimParams {
   GridParams gp;                  // samples (S = draws of this call), fixtures (F), table layout; gp.table = workspace
@@ -22,12 +42,16 @@ struct SimParams {
   int points_in_smem;             // the gained-points histogram is kept per CTA in shared memory
   unsigned long long *pos_counts, *pts_counts, *invalid;  // [NT][P], [NT][B], [1]
   uint8_t *positions, *scores;    // [N][NT], [N][F][2] or NULL
+  KoParams ko;                    // the tournament kernel only
 };
 
 // fills sp->gp's plan fields (model, S, T, Cf, F set) and returns the workspace bytes (the [S][row_floats] table)
 size_t simulate_plan(SimParams* sp);
-// shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem)
+// shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
+// the tournament kernel (sets sp->ko.wl_overlay)
 size_t simulate_smem_bytes(SimParams* sp);
 int launch_simulate(SimParams& sp, cudaStream_t stream);
+// the tournament kernel: group stage as launch_simulate, then the bracket of sp.ko (ko.K >= 1)
+int launch_simulate_tournament(SimParams& sp, cudaStream_t stream);
 
 }  // namespace bplx

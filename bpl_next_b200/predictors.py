@@ -25,12 +25,13 @@ from . import parallel
 from . import season as bseason
 from .problem import Problem, pointwise_loglik, psis_loo, score_grid_host
 from .problem import simulate_table as _simulate_table
+from .problem import simulate_tournament as _simulate_tournament
 
 MAX_GOALS = bdata.MAX_GOALS
 # device memory for the [matches, draws] log-likelihood matrix of loo(): larger match sets are processed in ranges
 LOO_MATRIX_BYTES = 4 << 30
-# device memory for the raw outputs of simulate_table(return_simulations=True) (positions and scores): larger runs are
-# processed in ranges of posterior draws
+# device memory for the raw outputs of simulate_table / simulate_tournament(return_simulations=True) (positions, scores,
+# knockout entrants, scores and winners): larger runs are processed in ranges of posterior draws
 SIM_OUTPUT_BYTES = 1 << 30
 
 
@@ -506,6 +507,129 @@ class _BplxPredictor:
                        away_score=np.ascontiguousarray(sc[:, :, 1].T))
         return res
 
+    def _slot_confs(self, tteams, fixtures, team_conf):
+        """Confederation index of every table team (NeutralWC): ``team_conf`` (team -> name or index), else inferred
+        from the group fixtures, which must then give each team one confederation."""
+        conf = {}
+        if team_conf is None and fixtures is not None and "home_conf" in fixtures:
+            for side in ("home", "away"):
+                for t, c in zip(_str_to_list(fixtures[side + "_team"])[0], _str_to_list(fixtures[side + "_conf"])[0]):
+                    if conf.setdefault(t, c) != c:
+                        raise ValueError(f"team {t!r} plays for confederations {conf[t]!r} and {c!r} in the fixtures: "
+                                         "pass team_conf")
+        elif team_conf is not None:
+            conf = dict(team_conf)
+        missing = [t for t in tteams if t not in conf]
+        if missing:
+            raise ValueError(f"the confederation of {missing[:3]!r} is unknown: pass team_conf")
+        return np.asarray([self._conferences_dict[conf[t]] if isinstance(conf[t], str) else int(conf[t])
+                           for t in tteams], np.uint8)
+
+    def simulate_tournament(self, fixtures, bracket, played=None, teams=None, groups=None, best=None, team_conf=None,
+                            num_sims_per_draw: int = 1, random_state: Optional[int] = None, max_goals: int = MAX_GOALS,
+                            points=(3, 1), return_simulations: bool = False) -> Dict[str, Any]:
+        """A tournament simulated on the GPU: the group stage of ``simulate_table``, then a knockout bracket, with ONE
+        posterior draw per simulated tournament, so a team that is stronger in a draw is stronger in every match of its
+        path.  (Chaining ``predict_outcome_proba`` calls cannot give this: the opponent of a round depends on earlier
+        results, and the same uncertain strengths run through all of a team's matches.)
+
+        ``fixtures``, ``played``, ``teams``, ``groups``, ``points``, ``num_sims_per_draw``, ``random_state``,
+        ``max_goals``: as ``simulate_table``; ``fixtures`` may be None or empty (a cup whose draw is made: the entrants
+        are ``("team", name)``).  ``bracket``: the ties in play order, ``{"id", "round", "home", "away",
+        "neutral_venue"}``, entrants ``("group", label, position)``, ``("best", j)``, ``("winner", id)``,
+        ``("loser", id)`` or ``("team", name)``; ``best``: the best-placed qualifiers, ``{"position", "count",
+        "allocation"}`` (``season.build_bracket``).  ``team_conf`` (NeutralWC): team -> confederation, needed for the
+        ties; inferred from the fixtures' confederations when they are consistent.
+
+        A tie is played like a group fixture from the draw's own grid.  A drawn tie goes to the home entrant with
+        probability ``hw_s / (hw_s + aw_s)``, the draw's own home and away win masses: the per-draw form of the
+        knockout renormalisation, which differs from ``predict_outcome_proba(knockout=True)`` (that renormalises after
+        averaging over the draws).  Extra time and penalties are not modelled; best-placed teams are ranked by points,
+        goal difference, goals for, then lot.
+
+        Returns everything ``simulate_table`` returns, plus ``rounds`` (labels by first appearance), ``reach_proba`` /
+        ``win_proba [T, rounds]`` (the team plays / wins a tie of the round) and ``champion_proba [T]``.  With
+        ``return_simulations`` also ``positions [N, T]``, ``home_score`` / ``away_score [F, N]``, ``ko_entrants [N, K,
+        2]`` (table slots), ``ko_scores [N, K, 2]`` and ``ko_winners [N, K]``; the draws are then processed in ranges
+        within ``SIM_OUTPUT_BYTES`` and the results do not depend on the range size.  Raises if a simulation was invalid
+        (a non-finite rate, or an allocation row the bracket does not cover)."""
+        import torch
+
+        fixtures = fixtures if fixtures is not None and len(_str_to_list(fixtures["home_team"])[0]) else None
+        home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"]) if fixtures else ([], [])
+        named = [e[1] for tie in bracket for e in (tuple(tie["home"]), tuple(tie["away"])) if e[0] == "team"]
+        if teams is None:
+            tteams = bseason.table_teams(home + named, away, played) if (home or named or played) else []
+        else:
+            tteams = bseason.table_teams(home, away, played, teams)
+        table = bseason.build_table(tteams, played, groups, points)
+        br = bseason.build_bracket(table, bracket, best)
+        known = set(np.asarray(self.teams).tolist())
+        unknown = [t for t in tteams if t not in known]
+        if unknown:
+            raise ValueError(f"team {unknown[0]!r} is not known to the model")
+        br["slot_team"] = np.asarray([self._teams_dict[t] for t in tteams], np.uint16)
+        if self.model == "neutral_wc":
+            br["slot_conf"] = self._slot_confs(tteams, fixtures, team_conf)
+        if fixtures:
+            hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
+            h, a = self._parse_fixture_args(home, away)
+            kw = {k: fixtures[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in fixtures}
+            fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw), "home_slot": hs,
+                  "away_slot": as_}
+        else:
+            fx = {}
+            table["num_points_bins"] = 1
+            table["num_positions"] = len(tteams) if table["group"] is None else int(np.bincount(table["group"]).max())
+        seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
+        R = int(num_sims_per_draw)
+        if R < 1:
+            raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
+        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
+              if v is not None}
+        dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
+        dtab = {k: None if table[k] is None else torch.from_numpy(table[k]).cuda()
+                for k in ("start_points", "start_goals_for", "start_goals_against", "group")}
+        dtab.update({k: table[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
+        S, T, F, K = int(ds["attack"].shape[0]), len(tteams), len(home), len(bracket)
+        step = (2 ** 31 - 1) // R
+        if return_simulations:
+            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F + 5 * K))))
+        if step < 1:
+            raise ValueError(f"num_sims_per_draw={R} is too large for one draw per call")
+        acc, invalid, raw = {}, 0, []
+        keys = ("position_counts", "points_counts", "reach_counts", "win_counts")
+        for lo in range(0, S, step):
+            hi = min(S, lo + step)
+            out = _simulate_tournament(self.model, {k: v[lo:hi] for k, v in ds.items()}, dfx, dtab, br, max_goals, R,
+                                       seed, first_draw=lo, want_positions=return_simulations,
+                                       want_scores=return_simulations, want_knockout=return_simulations)
+            for k in keys:
+                acc[k] = out[k] if k not in acc else acc[k] + out[k]
+            invalid += int(out["invalid"].item())
+            if return_simulations:
+                raw.append({k: out[k].cpu().numpy() for k in ("positions", "scores", "ko_entrants", "ko_scores",
+                                                              "ko_winners")})
+        N = S * R
+        if invalid:
+            raise ValueError(f"{invalid} of {N} simulations were invalid: a non-finite scoring rate or score-grid "
+                             "normaliser (check the posterior draws), or best-placed qualifiers the bracket does not "
+                             "place")
+        cnt = {k: v.cpu().numpy() for k, v in acc.items()}
+        res = {"teams": tteams,
+               "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
+               **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N),
+               **bseason.bracket_probabilities(br, cnt["reach_counts"], cnt["win_counts"], N),
+               "start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
+               "seed": seed}
+        if return_simulations:
+            cat = {k: np.concatenate([r[k] for r in raw]) for k in raw[0]}
+            sc = cat["scores"]
+            res.update(positions=cat["positions"], home_score=np.ascontiguousarray(sc[:, :, 0].T),
+                       away_score=np.ascontiguousarray(sc[:, :, 1].T), ko_entrants=cat["ko_entrants"],
+                       ko_scores=cat["ko_scores"], ko_winners=cat["ko_winners"])
+        return res
+
     # ---- a team the model has not seen (extended_dixon_coles.py:401-462 and the neutral siblings) ---------------
     def _new_team_pair(self, team_name, team_covariates):
         """Draws of (attack, defence) for a new team from the fitted hierarchical prior, one per posterior sample."""
@@ -799,6 +923,10 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         return self
 
     def simulate_table(self, *args, **kwargs):
+        raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
+                                  "cannot run in the reference (SURVEY.md D3)")
+
+    def simulate_tournament(self, *args, **kwargs):
         raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
                                   "cannot run in the reference (SURVEY.md D3)")
 

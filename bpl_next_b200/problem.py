@@ -371,3 +371,101 @@ def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[
                                        _stream_ptr(stream)))
     return {"position_counts": pos_counts, "points_counts": pts_counts, "invalid": invalid, "positions": positions,
             "scores": scores}
+
+
+def _bracket_struct(bracket: dict, keep: list):
+    """``_abi.Bracket`` over host copies of the arrays of ``bracket`` (kept alive in ``keep``)."""
+    def host(k, dt):
+        v = bracket.get(k)
+        if v is None:
+            return None
+        a = np.ascontiguousarray(v, dtype=dt)
+        keep.append(a)
+        return a.ctypes.data
+
+    b = _abi.Bracket()
+    b.num_ties, b.num_rounds = int(len(bracket["round"])), int(bracket["num_rounds"])
+    b.num_groups, b.best_position, b.best_count = (int(bracket[k]) for k in ("num_groups", "best_position", "best_count"))
+    for k in ("kind", "arg0", "arg1", "round", "neutral_venue", "slot_conf", "best_alloc"):
+        setattr(b, k, host(k, np.uint8))
+    b.slot_team = host("slot_team", np.uint16)
+    return b
+
+
+def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor], table: dict,
+                        bracket: dict, max_goals: int, sims_per_draw: int, seed: int, first_draw: int = 0,
+                        want_positions: bool = False, want_scores: bool = False, want_knockout: bool = False,
+                        workspace=None, stream=None) -> Dict[str, Optional[torch.Tensor]]:
+    """Device path of ``bplx_simulate_tournament``: the group stage of ``simulate_table`` (same Philox words, same
+    ranking: with the same seed its outputs are bit-identical), then a knockout bracket, one posterior draw per
+    simulated tournament.
+
+    ``samples``, ``fixtures``, ``table``: as ``simulate_table`` (``fixtures`` may have no fixtures: a bracket whose
+    entrants are all known).  ``bracket``: host arrays ``kind``, ``arg0``, ``arg1`` (uint8 ``[K, 2]``, home and away
+    entrant: ``_abi.ENTRANT_*`` and their arguments), ``round`` (``[K]``), ``neutral_venue`` (``[K]`` or None),
+    ``slot_team`` (uint16 ``[T_tab]``), ``slot_conf`` (``[T_tab]``, NeutralWC), ``best_alloc`` (``[2^num_groups,
+    best_count]`` or None) and the ints ``num_rounds``, ``num_groups``, ``best_position``, ``best_count``
+    (``season.build_bracket`` makes them).
+
+    Tie k uses words 2F + T_tab + 3k and + 1 for its score, from the draw's own grid like a group fixture, and + 2 for
+    the decider of a drawn tie: the home entrant goes through iff ``u_d (hw_s + aw_s) <= hw_s`` with ``hw_s`` / ``aw_s``
+    the draw's own home / away win masses, i.e. with probability ``hw_s / (hw_s + aw_s)`` per draw (the per-draw form of
+    ``predict_outcome_proba(knockout=True)``, which renormalises after averaging over the draws).  Extra time and
+    penalties are not modelled.  Returns ``simulate_table``'s outputs plus ``reach_counts`` / ``win_counts`` (int64
+    ``[T_tab, num_rounds]``: ties of round r the slot played / won), and when ``want_knockout`` ``ko_entrants``,
+    ``ko_scores`` (uint8 ``[N, K, 2]``) and ``ko_winners`` (``[N, K]``); 255 marks an invalid simulation."""
+    lib = _abi.lib()
+    keep = []
+    ptr = _device_ptr_fn(keep)
+    for k in _SAMPLE_KEYS + ("home_advantage",):
+        if samples.get(k) is not None:
+            assert samples[k].dtype == torch.float32
+    F = int(len(fixtures["home_team"])) if fixtures.get("home_team") is not None else 0
+    if F:
+        for k, dt in _FIXTURE_KEYS:
+            if fixtures.get(k) is not None:
+                assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
+        for k in ("home_slot", "away_slot"):
+            assert fixtures[k].dtype == torch.uint8, k
+    for k in _TABLE_ARRAYS:
+        assert table[k].dtype == torch.int32, k
+    T_tab = int(table["start_points"].shape[0])
+    if T_tab > _abi.SIM_MAX_TEAMS:
+        raise ValueError(f"the table has {T_tab} slots; at most {_abi.SIM_MAX_TEAMS} are supported")
+    if F:
+        top = int(torch.maximum(fixtures["home_slot"].max(), fixtures["away_slot"].max()))
+        if top >= T_tab:
+            raise ValueError(f"a fixture names table slot {top}, but the table has {T_tab} slots")
+    s = _samples_struct(model, samples, ptr)
+    f = _fixtures_struct(fixtures, ptr) if F else _abi.Fixtures()
+    t = _abi.Table()
+    t.num_slots = T_tab
+    t.num_positions, t.num_points_bins = int(table["num_positions"]), int(table["num_points_bins"])
+    t.points_win, t.points_draw = int(table["points_win"]), int(table["points_draw"])
+    t.group = None if table.get("group") is None else ptr(table["group"])
+    for k in _TABLE_ARRAYS:
+        setattr(t, k, ptr(table[k]))
+    b = _bracket_struct(bracket, keep)
+    dev = samples["attack"].device
+    need = int(lib.bplx_simulate_tournament_workspace_bytes(C.byref(s), C.byref(f), C.byref(t), C.byref(b)))
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    N, K, nr = s.num_samples * int(sims_per_draw), b.num_ties, b.num_rounds
+    i64 = dict(dtype=torch.int64, device=dev)
+    u8 = dict(dtype=torch.uint8, device=dev)
+    out = {"position_counts": torch.empty((T_tab, t.num_positions), **i64),
+           "points_counts": torch.empty((T_tab, t.num_points_bins), **i64),
+           "reach_counts": torch.empty((T_tab, nr), **i64), "win_counts": torch.empty((T_tab, nr), **i64),
+           "invalid": torch.empty(1, **i64),
+           "positions": torch.empty((N, T_tab), **u8) if want_positions else None,
+           "scores": torch.empty((N, F, 2), **u8) if want_scores else None,
+           "ko_entrants": torch.empty((N, K, 2), **u8) if want_knockout else None,
+           "ko_scores": torch.empty((N, K, 2), **u8) if want_knockout else None,
+           "ko_winners": torch.empty((N, K), **u8) if want_knockout else None}
+    _abi.check(lib.bplx_simulate_tournament(
+        C.byref(s), C.byref(f), ptr(fixtures["home_slot"]) if F else None, ptr(fixtures["away_slot"]) if F else None,
+        C.byref(t), C.byref(b), int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
+        *(_dptr(out[k]) for k in ("position_counts", "points_counts", "reach_counts", "win_counts", "positions",
+                                  "scores", "ko_entrants", "ko_scores", "ko_winners", "invalid")),
+        _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    return out

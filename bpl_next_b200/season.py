@@ -5,15 +5,19 @@ inputs from team names and played results and turns its integer counts into prob
 full text is in ``include/bplx.h``): every simulated season takes ONE posterior draw and plays every remaining fixture
 with that draw's rates, so a team that is stronger in a draw is stronger in all of its matches of that season.  Teams
 are ranked within their group by points, goal difference, goals for, then a random tie-break key; head-to-head and
-fair-play rules are not modelled, so ties left after goals for are decided by lot.
+fair-play rules are not modelled, so ties left after goals for are decided by lot.  ``build_bracket`` and
+``bracket_probabilities`` do the same for a knockout bracket played after the group stage (``problem.simulate_tournament``).
 """
 from __future__ import annotations
 
+import itertools
 from typing import Any, Dict, Optional, Sequence, Tuple
 
 import numpy as np
 
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
+KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
+ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0, 1, 2, 3, 4  # BPLX_ENTRANT_*
 
 
 def _names(x) -> list:
@@ -129,3 +133,127 @@ def probabilities(table: Dict[str, Any], position_counts: np.ndarray, points_cou
     start = np.asarray(table["start_points"], np.int64)
     return {"position_proba": pos, "points_proba": pts,
             "expected_points": start + pts @ np.arange(pts.shape[1], dtype=np.float64)}
+
+
+# ---- tournament: a knockout bracket after the group stage ---------------------------------------------------------
+def _group_sizes(table: Dict[str, Any]) -> Tuple[list, np.ndarray]:
+    """Group labels (``[None]`` for a table without groups) and the size of each group."""
+    T = len(table["teams"])
+    if table.get("group") is None:
+        return [None], np.asarray([T])
+    return list(table["group_labels"]), np.bincount(table["group"], minlength=len(table["group_labels"]))
+
+
+def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: Optional[Dict[str, Any]] = None
+                  ) -> Dict[str, Any]:
+    """The knockout bracket ``problem.simulate_tournament`` takes, from ties in play order.
+
+    Each tie is ``{"id", "round", "home", "away", "neutral_venue"}`` (``neutral_venue`` optional, default 0); an entrant
+    is ``("group", label, position)`` (0-based position in the group; label None for a table without groups),
+    ``("best", j)`` (the j-th best-placed qualifier), ``("winner", id)`` / ``("loser", id)`` of an earlier tie, or
+    ``("team", name)`` (a table team already through).  Round labels are ordered by first appearance; the last tie is
+    the final and must be alone in its round.  ``best``: ``{"position": p, "count": c, "allocation": None or
+    {frozenset(group labels): [group label of BEST j for j < c]}}`` -- the best c of the teams placed p in their
+    groups qualify, ranked across groups by points, goal difference, goals for, then lot; with an allocation every
+    c-subset of the groups must have a row, and each row is a permutation of its subset.  ``slot_team`` / ``slot_conf``
+    are left to the caller (they need the model's team and confederation indices)."""
+    teams = list(table["teams"])
+    slot = {t: i for i, t in enumerate(teams)}
+    labels, sizes = _group_sizes(table)
+    gid = {g: k for k, g in enumerate(labels)}
+    ties = list(ties)
+    K = len(ties)
+    if not 1 <= K <= KO_MAX_TIES:
+        raise ValueError(f"a bracket has 1 to {KO_MAX_TIES} ties, got {K}")
+    bp, bc, alloc = 0, 0, None
+    if best is not None:
+        bp, bc, alloc = int(best["position"]), int(best["count"]), best.get("allocation")
+        if not 1 <= bc <= min(KO_MAX_BEST, len(labels)):
+            raise ValueError(f"best count must be in [1, {min(KO_MAX_BEST, len(labels))}], got {bc}")
+        if not 0 <= bp < int(sizes.max()):
+            raise ValueError(f"best position {bp} is outside every group")
+    index, rounds, used = {}, [], set()
+    kind = np.zeros((K, 2), np.uint8)
+    arg0 = np.zeros((K, 2), np.uint8)
+    arg1 = np.zeros((K, 2), np.uint8)
+    rnd = np.zeros(K, np.uint8)
+    nv = np.zeros(K, np.uint8)
+    for k, tie in enumerate(ties):
+        tid = tie["id"]
+        if tid in index:
+            raise ValueError(f"tie id {tid!r} is used twice")
+        if tie["round"] not in rounds:
+            rounds.append(tie["round"])
+        rnd[k] = rounds.index(tie["round"])
+        nv[k] = 1 if tie.get("neutral_venue", 0) else 0
+        for side, key in enumerate(("home", "away")):
+            e = tuple(tie[key])
+            src = e
+            if e[0] == "group":
+                _, g, p = e
+                if g not in gid:
+                    raise ValueError(f"tie {tid!r}: unknown group {g!r}")
+                if not 0 <= int(p) < sizes[gid[g]]:
+                    raise ValueError(f"tie {tid!r}: group {g!r} has no position {p}")
+                kind[k, side], arg0[k, side], arg1[k, side] = ENTRANT_GROUP_POS, gid[g], int(p)
+                src = ("group", g, int(p))
+            elif e[0] == "best":
+                j = int(e[1])
+                if not 0 <= j < bc:
+                    raise ValueError(f"tie {tid!r}: best {j} is not one of the {bc} best-placed qualifiers")
+                kind[k, side], arg0[k, side] = ENTRANT_BEST, j
+                src = ("best", j)
+            elif e[0] in ("winner", "loser"):
+                ref = e[1]
+                if ref not in index:
+                    if any(t["id"] == ref for t in ties[k:]):
+                        raise ValueError(f"tie {tid!r} refers to tie {ref!r}, which is not played before it")
+                    raise ValueError(f"tie {tid!r} refers to an unknown tie id {ref!r}")
+                kind[k, side] = ENTRANT_WINNER if e[0] == "winner" else ENTRANT_LOSER
+                arg0[k, side] = index[ref]
+            elif e[0] == "team":
+                if e[1] not in slot:
+                    raise ValueError(f"tie {tid!r}: team {e[1]!r} is not in the table")
+                kind[k, side], arg0[k, side] = ENTRANT_SLOT, slot[e[1]]
+            else:
+                raise ValueError(f"tie {tid!r}: unknown entrant {e!r}")
+            if src in used:
+                raise ValueError(f"tie {tid!r}: entrant {src!r} is used twice")
+            used.add(src)
+        index[tid] = k
+    if len(rounds) > KO_MAX_ROUNDS:
+        raise ValueError(f"a bracket has at most {KO_MAX_ROUNDS} rounds, got {len(rounds)}")
+    if (rnd == rnd[-1]).sum() != 1:
+        raise ValueError(f"the last tie is the final and must be alone in its round {rounds[rnd[-1]]!r}")
+    best_alloc = None
+    if alloc is not None:
+        ng = len(labels)
+        if ng > KO_MAX_ALLOC_GROUPS:
+            raise ValueError(f"an allocation table supports at most {KO_MAX_ALLOC_GROUPS} groups, got {ng}")
+        best_alloc = np.full((1 << ng, bc), 0xFF, np.uint8)
+        rows = {frozenset(k): list(v) for k, v in alloc.items()}
+        for sub in itertools.combinations(range(ng), bc):
+            key = frozenset(labels[g] for g in sub)
+            if key not in rows:
+                raise ValueError(f"the allocation misses the qualifying groups {sorted(key, key=str)}")
+            row = rows[key]
+            if len(row) != bc or set(row) != key:
+                raise ValueError(f"allocation row {sorted(key, key=str)}: {row!r} is not a permutation of its groups")
+            best_alloc[sum(1 << g for g in sub)] = [gid[g] for g in row]
+        extra = [k for k in rows if len(k) != bc or not k <= set(labels)]
+        if extra:
+            raise ValueError(f"the allocation has a row for {sorted(extra[0], key=str)}, not {bc} of the table's groups")
+    return {"ids": [t["id"] for t in ties], "rounds": rounds, "num_rounds": len(rounds), "kind": kind, "arg0": arg0,
+            "arg1": arg1, "round": rnd, "neutral_venue": nv, "num_groups": len(labels), "best_position": bp,
+            "best_count": bc, "best_alloc": best_alloc}
+
+
+def bracket_probabilities(bracket: Dict[str, Any], reach_counts: np.ndarray, win_counts: np.ndarray,
+                          num_simulations: int) -> Dict[str, np.ndarray]:
+    """Counts -> ``reach_proba`` / ``win_proba [T, rounds]`` (a team reaches / wins a tie of the round) and
+    ``champion_proba [T]`` (it wins the last tie)."""
+    n = float(num_simulations)
+    reach = np.asarray(reach_counts, np.float64) / n
+    win = np.asarray(win_counts, np.float64) / n
+    return {"rounds": list(bracket["rounds"]), "reach_proba": reach, "win_proba": win,
+            "champion_proba": win[:, int(bracket["round"][-1])].copy()}

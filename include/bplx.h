@@ -325,6 +325,85 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
                         uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
                         size_t workspace_bytes, void* stream);
 
+/* ---- tournament simulation: a knockout bracket after the group stage, one posterior draw per tournament --------- */
+/*
+ * Group stage: exactly bplx_simulate_table's definition (same simulation index n, same Philox words 2f, 2f+1 and
+ * 2F + t, same ranking); with the same seed its outputs are bit-identical to a bplx_simulate_table call, except that a
+ * simulation made invalid by its bracket is left out here.  F = 0 is allowed (a cup whose draw is already made).
+ *
+ * Bracket: K ties in play order.  Each tie has a home and an away entrant, a round id and (neutral models) a
+ * neutral-venue flag; for DIXON_COLES and EXTENDED the home entrant is at home.  An entrant is
+ *   BPLX_ENTRANT_SLOT t            a fixed table slot (a team already through)
+ *   BPLX_ENTRANT_GROUP_POS (g, p)  the slot ranked p (0-based) in group g
+ *   BPLX_ENTRANT_BEST j            the j-th best-placed qualifier (below)
+ *   BPLX_ENTRANT_WINNER k'         the winner of the earlier tie k' < k
+ *   BPLX_ENTRANT_LOSER k'          its loser (third-place matches)
+ * Best-placed qualifiers: one pool, the slots at position best_position of every group, ranked across groups by
+ * points, goal difference, goals for, then the slot tie-break key (word 2F + t), then the lower slot; the first
+ * best_count qualify.  Without an allocation table BEST j is the j-th best; with one (dense [2^num_groups][best_count]
+ * group ids, indexed by the bit set of the groups whose team qualified: the form of FIFA's and UEFA's third-place
+ * tables) BEST j is the position-best_position slot of group alloc[mask][j].  Fair play, rankings and head-to-head are
+ * not modelled: ties left after goals for are decided by lot.
+ * A tie is played like a group fixture, from the draw's own clamped, truncated grid, with the rates of its entrants'
+ * model teams (slot_team) and, for NEUTRAL_WC, their confederations (slot_conf).  Words 2F + T_tab + 3k and + 1 sample
+ * its score, word + 2 is the decider u_d (curand_uniform); every word has a fixed address, used or not.  A drawn tie goes
+ * to the home entrant iff u_d (hw_s + aw_s) <= hw_s, hw_s = sum_{i > j} w(i, j) and aw_s = sum_{i < j} w(i, j) the
+ * draw's own win masses on the same grid: P(home advances | draw s) = hw_s / (hw_s + aw_s), the per-draw form of the
+ * knockout renormalisation of predict_outcome_proba(knockout=True), which renormalises AFTER averaging over the draws.
+ * Extra time and penalties are not modelled (the model knows 90-minute scores only); two-legged ties are out of scope.
+ *
+ * Invalid simulations (bplx_simulate_table's, and a tie with a non-finite rate or a bad normaliser, hw + aw not positive
+ * on a drawn tie, a GROUP_POS beyond its group, fewer than best_count groups with a slot at best_position, or an
+ * allocation entry of 0xFF) are counted in `invalid` and left out of every histogram; their positions, ko_entrants,
+ * ko_scores and ko_winners rows are 0xFF.
+ *
+ * Outputs (device; integer counts, additive over draw ranges; overwritten): position_counts, points_counts and invalid
+ * as bplx_simulate_table; reach_counts [T_tab, num_rounds]: ties of round r the slot played; win_counts [T_tab,
+ * num_rounds]: ties of round r it won (the winner of the last tie is the champion).  Optional raw rows (NULL to skip):
+ * positions [N, T_tab], scores [N, F, 2], ko_entrants [N, K, 2] (slots), ko_scores [N, K, 2], ko_winners [N, K].
+ * Limits: K <= 64 ties, <= 16 rounds, best_count <= 16, num_groups <= 16 with an allocation table; T_tab <= 64 and
+ * N < 2^31 per call as bplx_simulate_table; DYNAMIC: BPLX_E_UNSUPPORTED.
+ *
+ * The bracket's arrays are HOST arrays: the call validates them (entrants reference earlier ties only, groups and
+ * positions in range, BEST j < best_count, allocation entries are 0xFF or distinct groups of their mask) and passes
+ * them to the kernel; the allocation table is copied into the workspace (cudaMemcpyAsync from the caller's array, so a
+ * pageable array makes the call wait for the stream).
+ */
+#define BPLX_KO_MAX_TIES 64
+#define BPLX_KO_MAX_ROUNDS 16
+#define BPLX_KO_MAX_BEST 16
+#define BPLX_KO_MAX_ALLOC_GROUPS 16
+#define BPLX_ENTRANT_SLOT 0
+#define BPLX_ENTRANT_GROUP_POS 1
+#define BPLX_ENTRANT_BEST 2
+#define BPLX_ENTRANT_WINNER 3
+#define BPLX_ENTRANT_LOSER 4
+typedef struct {
+  int32_t num_ties;               /* K, 1..64 */
+  int32_t num_rounds;             /* 1..16 */
+  int32_t num_groups;             /* group ids 0 .. num_groups-1 that GROUP_POS and the pool refer to (<= T_tab) */
+  int32_t best_position;          /* position of the best-placed pool (0-based) */
+  int32_t best_count;             /* 0..16 qualifiers from the pool (0: no pool) */
+  const uint8_t* kind;            /* host [K, 2] (home, away) BPLX_ENTRANT_* */
+  const uint8_t* arg0;            /* host [K, 2] slot / group / j / earlier tie */
+  const uint8_t* arg1;            /* host [K, 2] position of GROUP_POS, else ignored */
+  const uint8_t* round;           /* host [K] round id < num_rounds */
+  const uint8_t* neutral_venue;   /* host [K] 1 = neutral, or NULL (all 0) */
+  const uint16_t* slot_team;      /* host [T_tab] model team of each table slot */
+  const uint8_t* slot_conf;       /* host [T_tab] confederation of each slot (NEUTRAL_WC), else NULL */
+  const uint8_t* best_alloc;      /* host [2^num_groups, best_count] group ids or 0xFF, or NULL */
+} bplx_bracket;
+
+size_t bplx_simulate_tournament_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
+                                                const bplx_bracket* b);
+int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                             const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b, int max_goals,
+                             int sims_per_draw, unsigned long long seed, long long first_draw,
+                             unsigned long long* position_counts, unsigned long long* points_counts,
+                             unsigned long long* reach_counts, unsigned long long* win_counts, uint8_t* positions,
+                             uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
+                             unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

@@ -583,12 +583,37 @@ static int check_grid_args(const bplx_samples* s, const bplx_fixtures* f, int ma
   return BPLX_OK;
 }
 
-static size_t grid_plan(const bplx_samples* s, const bplx_fixtures* f, int max_goals, GridParams* gp, const char** err) {
+// the shape (model, S, T, Cf, F) and the sample / fixture arrays of gp; with F = 0 the fixture arrays may be NULL
+static void bind_samples(const bplx_samples* s, const bplx_fixtures* f, GridParams* gp) {
   gp->model = s->model;
   gp->S = s->num_samples;
   gp->T = s->num_teams;
   gp->Cf = s->model == BPLX_NEUTRAL_WC ? s->num_conferences : 0;
   gp->F = f->num_fixtures;
+  gp->attack = s->attack;
+  gp->defence = s->defence;
+  gp->ha = s->home_attack;
+  gp->aa = s->away_attack;
+  gp->hd = s->home_defence;
+  gp->ad = s->away_defence;
+  gp->conf = s->confederation_strength;
+  gp->corr = s->corr_coef;
+  gp->home = f->home_team;
+  gp->away = f->away_team;
+  gp->hconf = f->home_conf;
+  gp->aconf = f->away_conf;
+  gp->nv = f->neutral_venue;
+}
+
+static int check_workspace(const void* workspace, size_t workspace_bytes, size_t need) {
+  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
+               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  return BPLX_OK;
+}
+
+static size_t grid_plan(const bplx_samples* s, const bplx_fixtures* f, int max_goals, GridParams* gp, const char** err) {
+  bind_samples(s, f, gp);
   gp->g = max_goals + 1;
   return score_grid_plan(gp, err);
 }
@@ -614,25 +639,10 @@ int bplx_score_grid_ex(const bplx_samples* s, const bplx_fixtures* f, int max_go
   const size_t need = grid_plan(s, f, max_goals, &gp, &perr);
   BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "score grid: unsupported shape");
   gp.scale = scale;
-  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
-               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
-  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
-  gp.attack = s->attack;
-  gp.defence = s->defence;
-  gp.ha = s->home_attack;
-  gp.aa = s->away_attack;
-  gp.hd = s->home_defence;
-  gp.ad = s->away_defence;
-  gp.conf = s->confederation_strength;
-  gp.corr = s->corr_coef;
-  gp.home = f->home_team;
-  gp.away = f->away_team;
-  gp.hconf = f->home_conf;
-  gp.aconf = f->away_conf;
-  gp.nv = f->neutral_venue;
+  rc = check_workspace(workspace, workspace_bytes, need);
+  if (rc != BPLX_OK) return rc;
   gp.table = static_cast<float*>(workspace);
-  gp.partial = reinterpret_cast<float*>(static_cast<unsigned char*>(workspace) +
-                                        ((size_t)gp.S * gp.row_floats * 4 + 255) / 256 * 256);
+  gp.partial = reinterpret_cast<float*>(static_cast<unsigned char*>(workspace) + table_layout(&gp));
   gp.grid = grid;
   gp.outcome = outcome;
   gp.reuse_tables = (flags & BPLX_GRID_REUSE_TABLES) ? 1 : 0;
@@ -724,11 +734,7 @@ int bplx_score_grid_host(const bplx_samples* s, const bplx_fixtures* f, int max_
 
 // ---- pointwise log-likelihood and PSIS-LOO -----------------------------------------------------------------------
 static size_t pointwise_plan_for(const bplx_samples* s, const bplx_observations* o, PointwiseParams* pp, const char** err) {
-  pp->gp.model = s->model;
-  pp->gp.S = s->num_samples;
-  pp->gp.T = s->num_teams;
-  pp->gp.Cf = s->model == BPLX_NEUTRAL_WC ? s->num_conferences : 0;
-  pp->gp.F = o->fixtures.num_fixtures;
+  bind_samples(s, &o->fixtures, &pp->gp);
   return pointwise_plan(pp, err);
 }
 
@@ -752,26 +758,10 @@ int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, f
   const char* perr = nullptr;
   const size_t need = pointwise_plan_for(s, obs, &pp, &perr);
   BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
-  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
-               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
-  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
-  GridParams& gp = pp.gp;
-  gp.attack = s->attack;
-  gp.defence = s->defence;
-  gp.ha = s->home_attack;
-  gp.aa = s->away_attack;
-  gp.hd = s->home_defence;
-  gp.ad = s->away_defence;
-  gp.conf = s->confederation_strength;
-  gp.corr = s->corr_coef;
-  gp.home = obs->fixtures.home_team;
-  gp.away = obs->fixtures.away_team;
-  gp.hconf = obs->fixtures.home_conf;
-  gp.aconf = obs->fixtures.away_conf;
-  gp.nv = obs->fixtures.neutral_venue;
-  gp.table = static_cast<float*>(workspace);
-  pp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) +
-                                         ((size_t)gp.S * gp.row_floats * 4 + 255) / 256 * 256);
+  rc = check_workspace(workspace, workspace_bytes, need);
+  if (rc != BPLX_OK) return rc;
+  pp.gp.table = static_cast<float*>(workspace);
+  pp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + table_layout(&pp.gp));
   pp.hg = obs->home_goals;
   pp.ag = obs->away_goals;
   pp.ll = loglik;
@@ -806,13 +796,10 @@ int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t 
 }
 
 // ---- season / group-stage simulation --------------------------------------------------------------------------
+// the workspace of a simulation is the [S][row_floats] exponential table
 static size_t simulate_plan_for(const bplx_samples* s, const bplx_fixtures* f, SimParams* sp) {
-  sp->gp.model = s->model;
-  sp->gp.S = s->num_samples;
-  sp->gp.T = s->num_teams;
-  sp->gp.Cf = s->model == BPLX_NEUTRAL_WC ? s->num_conferences : 0;
-  sp->gp.F = f->num_fixtures;
-  return simulate_plan(sp);
+  bind_samples(s, f, &sp->gp);
+  return table_layout(&sp->gp);
 }
 
 size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t) {
@@ -821,7 +808,8 @@ size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures*
   return simulate_plan_for(s, f, &sp);
 }
 
-// validates the arguments bplx_simulate_table and bplx_simulate_tournament share and fills *sp (its workspace aside)
+// validates the arguments bplx_simulate_table and bplx_simulate_tournament share and fills *sp (its samples, fixtures
+// and workspace aside: simulate_plan_for binds those)
 static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
                           const uint8_t* away_slot, const bplx_table* t, int max_goals, int sims_per_draw,
                           unsigned long long seed, long long first_draw, unsigned long long* position_counts,
@@ -855,20 +843,6 @@ static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const u
   BPLX_REQUIRE(position_counts && points_counts && invalid, BPLX_E_INVALID,
                "%s: position_counts, points_counts and invalid must not be NULL", what);
   SimParams& sp = *out;
-  GridParams& gp = sp.gp;
-  gp.attack = s->attack;
-  gp.defence = s->defence;
-  gp.ha = s->home_attack;
-  gp.aa = s->away_attack;
-  gp.hd = s->home_defence;
-  gp.ad = s->away_defence;
-  gp.conf = s->confederation_strength;
-  gp.corr = s->corr_coef;
-  gp.home = f->home_team;
-  gp.away = f->away_team;
-  gp.hconf = f->home_conf;
-  gp.aconf = f->away_conf;
-  gp.nv = f->neutral_venue;
   sp.hslot = home_slot;
   sp.aslot = away_slot;
   sp.group = t->group;
@@ -902,10 +876,8 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "simulate", false, &sp);
   if (rc != BPLX_OK) return rc;
-  const size_t need = simulate_plan_for(s, f, &sp);
-  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
-               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
-  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  rc = check_workspace(workspace, workspace_bytes, simulate_plan_for(s, f, &sp));
+  if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
   return launch_simulate(sp, static_cast<cudaStream_t>(stream));
 }
@@ -1031,10 +1003,8 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
   if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
   const size_t table = simulate_plan_for(s, f, &sp);
-  const size_t need = table + (alloc_bytes(b) + 255) / 256 * 256;
-  BPLX_REQUIRE(workspace && workspace_bytes >= need, BPLX_E_WORKSPACE,
-               "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
-  BPLX_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15u) == 0, BPLX_E_INVALID, "workspace must be 16-byte aligned");
+  rc = check_workspace(workspace, workspace_bytes, table + (alloc_bytes(b) + 255) / 256 * 256);
+  if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
   sp.ko.reach = reach_counts;
   sp.ko.win = win_counts;

@@ -162,10 +162,7 @@ __global__ void pointwise_finalize(const __grid_constant__ PointwiseParams pp) {
 
 size_t pointwise_plan(PointwiseParams* pp, const char** err) {
   GridParams* gp = &pp->gp;
-  const bool neu = gp->model == BPLX_NEUTRAL || gp->model == BPLX_NEUTRAL_WC;
-  gp->ntab = neu ? 3 : 2;
-  const RowLayout L = row_layout(gp->T, gp->Cf, gp->ntab);
-  gp->row_floats = (L.C + 1 + 3) / 4 * 4;
+  const size_t table_bytes = table_layout(gp);
   const size_t row_bytes = (size_t)gp->row_floats * 4;
   if (row_bytes > (size_t)kPwStageBytes) {
     if (err) *err = "pointwise log-likelihood: a sample row (teams x tables) does not fit one stage buffer: too many teams";
@@ -183,7 +180,6 @@ size_t pointwise_plan(PointwiseParams* pp, const char** err) {
   sps = (sps + gp->ns_stage - 1) / gp->ns_stage * gp->ns_stage;
   gp->nsplit = (gp->S + sps - 1) / sps;
   gp->samples_per_split = sps;
-  const size_t table_bytes = ((size_t)gp->S * row_bytes + 255) / 256 * 256;
   return table_bytes + (size_t)gp->nsplit * gp->F * 4 * sizeof(double);
 }
 

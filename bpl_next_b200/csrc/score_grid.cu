@@ -301,6 +301,14 @@ static void tile_shape(int g, int* R, int* CC, int* ntiles) {
   }
 }
 
+size_t table_layout(GridParams* gp) {
+  const bool neu = gp->model == BPLX_NEUTRAL || gp->model == BPLX_NEUTRAL_WC;
+  gp->ntab = neu ? 3 : 2;
+  const RowLayout L = row_layout(gp->T, gp->Cf, gp->ntab);
+  gp->row_floats = (L.C + 1 + 3) / 4 * 4;
+  return ((size_t)gp->S * gp->row_floats * 4 + 255) / 256 * 256;
+}
+
 size_t score_grid_plan(GridParams* gp, const char** err) {
   static int sms = 0;
   if (sms == 0) {
@@ -309,10 +317,7 @@ size_t score_grid_plan(GridParams* gp, const char** err) {
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0)
       sms = 148;
   }
-  const bool neu = gp->model == BPLX_NEUTRAL || gp->model == BPLX_NEUTRAL_WC;
-  gp->ntab = neu ? 3 : 2;
-  const RowLayout L = row_layout(gp->T, gp->Cf, gp->ntab);
-  gp->row_floats = (L.C + 1 + 3) / 4 * 4;
+  const size_t table_bytes = table_layout(gp);
   const size_t row_bytes = (size_t)gp->row_floats * 4;
   if (row_bytes > (size_t)kGridStageBytes) {
     if (err) *err = "score grid: a sample row (teams x tables) does not fit one stage buffer: too many teams";
@@ -338,7 +343,6 @@ size_t score_grid_plan(GridParams* gp, const char** err) {
   sps = (sps + gp->ns_stage - 1) / gp->ns_stage * gp->ns_stage;
   gp->nsplit = (gp->S + sps - 1) / sps;
   gp->samples_per_split = sps;
-  const size_t table_bytes = ((size_t)gp->S * row_bytes + 255) / 256 * 256;
   return table_bytes + (size_t)gp->nsplit * gp->F * gp->g * gp->g * sizeof(float);
 }
 

@@ -70,6 +70,9 @@ struct GridParams {
   float* outcome;  // [F][3] or NULL
 };
 
+// fills ntab / row_floats of `gp` (model, S, T, Cf set) and returns the bytes of the [S][row_floats] exponential table,
+// rounded up to 256: what follows the table in a workspace starts there
+size_t table_layout(GridParams* gp);
 // fills nsplit / samples_per_split / ns_stage / ntab / row_floats of `gp` (S, T, Cf, F, g, model set) and returns the
 // workspace bytes (table + partial sums); 0 with *err set when a sample row does not fit a stage buffer
 size_t score_grid_plan(GridParams* gp, const char** err);

@@ -452,15 +452,6 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   if (tid == 0 && s_invalid) atomicAdd(sp.invalid, (unsigned long long)s_invalid);
 }
 
-size_t simulate_plan(SimParams* sp) {
-  GridParams* gp = &sp->gp;
-  const bool neu = gp->model == BPLX_NEUTRAL || gp->model == BPLX_NEUTRAL_WC;
-  gp->ntab = neu ? 3 : 2;
-  const RowLayout L = row_layout(gp->T, gp->Cf, gp->ntab);
-  gp->row_floats = (L.C + 1 + 3) / 4 * 4;
-  return ((size_t)gp->S * gp->row_floats * 4 + 255) / 256 * 256;
-}
-
 size_t simulate_smem_bytes(SimParams* sp) {
   size_t base = (size_t)sp->NT * kSimThreads * 16 + (size_t)sp->NT * sp->P * 4 + (size_t)sp->NT * 12;
   if (sp->ko.K > 0) {

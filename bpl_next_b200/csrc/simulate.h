@@ -45,8 +45,6 @@ struct SimParams {
   KoParams ko;                    // the tournament kernel only
 };
 
-// fills sp->gp's plan fields (model, S, T, Cf, F set) and returns the workspace bytes (the [S][row_floats] table)
-size_t simulate_plan(SimParams* sp);
 // shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
 // the tournament kernel (sets sp->ko.wl_overlay)
 size_t simulate_smem_bytes(SimParams* sp);

@@ -237,6 +237,18 @@ class _BplxPredictor:
     def _fixture_extras(self, n, **kw) -> Dict[str, np.ndarray]:
         return {}
 
+    def _fixture_arrays(self, home_team, away_team, fixtures) -> Dict[str, np.ndarray]:
+        """Index arrays of fixtures, mapped as ``predict_*`` maps them; the model's ``neutral_venue`` / ``home_conf`` /
+        ``away_conf`` come from ``fixtures``."""
+        h, a = self._parse_fixture_args(home_team, away_team)
+        kw = {k: fixtures[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in fixtures}
+        return {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw)}
+
+    def _device_samples(self) -> Dict[str, torch.Tensor]:
+        """The posterior draws as float32 device tensors."""
+        return {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
+                if v is not None}
+
     def _grid(self, home_team, away_team, max_goals, **kw):
         h, a = self._parse_fixture_args(home_team, away_team)
         fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw)}
@@ -298,10 +310,8 @@ class _BplxPredictor:
                 if getattr(arr, k) is not None:
                     obs[k] = np.asarray(getattr(arr, k), dtype=np.uint8)
             hg, ag = arr.home_goals, arr.away_goals
-        else:  # fixture arguments mapped as predict_* maps them
-            h, a = self._parse_fixture_args(data["home_team"], data["away_team"])
-            kw = {k: data[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in data}
-            obs = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw)}
+        else:
+            obs = self._fixture_arrays(data["home_team"], data["away_team"], data)
             hg, ag = bdata._goals(data["home_goals"]), bdata._goals(data["away_goals"])
         obs["home_goals"], obs["away_goals"] = np.asarray(hg, dtype=np.uint8), np.asarray(ag, dtype=np.uint8)
         names = np.asarray(self.teams).astype(str)
@@ -311,11 +321,8 @@ class _BplxPredictor:
         return obs, key.hexdigest()
 
     def _comparison_inputs(self, data):
-        import torch
-
         obs, key = self._observations(data)
-        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
-              if v is not None}
+        ds = self._device_samples()
         do = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in obs.items()}
         return ds, do, key
 
@@ -455,56 +462,67 @@ class _BplxPredictor:
         and ``home_score`` / ``away_score`` ``[F, N]`` (``sample_score``'s shape); the draws are then processed in
         ranges that keep these within ``SIM_OUTPUT_BYTES`` of device memory, and the results do not depend on the range
         size.  Raises if any simulation met a non-finite rate."""
-        import torch
-
         home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"])
         tteams = bseason.table_teams(home, away, played, teams)
         table = bseason.build_table(tteams, played, groups, points)
         hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
-        h, a = self._parse_fixture_args(home, away)
-        kw = {k: fixtures[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in fixtures}
-        fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw), "home_slot": hs, "away_slot": as_}
+        fx = {**self._fixture_arrays(home, away, fixtures), "home_slot": hs, "away_slot": as_}
+        return self._simulate(table, fx, None, num_sims_per_draw, random_state, max_goals, return_simulations,
+                              "met a non-finite scoring rate or score-grid normaliser: check the posterior draws")
+
+    def _simulate(self, table, fx, bracket, num_sims_per_draw, random_state, max_goals, return_simulations,
+                  invalid_reason) -> Dict[str, Any]:
+        """``simulate_table`` (``bracket`` None) and ``simulate_tournament`` from the host table, fixture arrays (with
+        their slots; ``{}`` for none) and bracket: the draws in ranges, counts summed over the ranges, probabilities."""
         seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
         R = int(num_sims_per_draw)
         if R < 1:
             raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
-        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
-              if v is not None}
+        ds = self._device_samples()
         dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
         dtab = {k: None if table[k] is None else torch.from_numpy(table[k]).cuda()
                 for k in ("start_points", "start_goals_for", "start_goals_against", "group")}
         dtab.update({k: table[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
-        S, T, F = int(ds["attack"].shape[0]), len(tteams), len(h)
+        S, T, F = int(ds["attack"].shape[0]), len(table["teams"]), len(fx.get("home_team", ()))
+        K = 0 if bracket is None else len(bracket["round"])
         step = (2 ** 31 - 1) // R  # simulations per call stay below 2^31
-        if return_simulations:
-            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F))))
+        if return_simulations:  # bytes per simulation: positions, scores and the knockout entrants, scores, winners
+            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F + 5 * K))))
         if step < 1:
             raise ValueError(f"num_sims_per_draw={R} is too large for one draw per call")
-        pos_c = pts_c = None
-        invalid = 0
-        raw = []
+        acc, invalid, raw = {}, 0, []
         for lo in range(0, S, step):
             hi = min(S, lo + step)
-            out = _simulate_table(self.model, {k: v[lo:hi] for k, v in ds.items()}, dfx, dtab, max_goals, R, seed,
-                                  first_draw=lo, want_positions=return_simulations, want_scores=return_simulations)
-            pos_c = out["position_counts"] if pos_c is None else pos_c + out["position_counts"]
-            pts_c = out["points_counts"] if pts_c is None else pts_c + out["points_counts"]
-            invalid += int(out["invalid"].item())
+            draws = {k: v[lo:hi] for k, v in ds.items()}
+            if bracket is None:
+                out = _simulate_table(self.model, draws, dfx, dtab, max_goals, R, seed, first_draw=lo,
+                                      want_positions=return_simulations, want_scores=return_simulations)
+            else:
+                out = _simulate_tournament(self.model, draws, dfx, dtab, bracket, max_goals, R, seed, first_draw=lo,
+                                           want_positions=return_simulations, want_scores=return_simulations,
+                                           want_knockout=return_simulations)
+            invalid += int(out.pop("invalid").item())
+            for k, v in out.items():
+                if k.endswith("_counts"):
+                    acc[k] = v if k not in acc else acc[k] + v
             if return_simulations:
-                raw.append((out["positions"].cpu().numpy(), out["scores"].cpu().numpy()))
+                raw.append({k: v.cpu().numpy() for k, v in out.items() if not k.endswith("_counts")})
         N = S * R
         if invalid:
-            raise ValueError(f"{invalid} of {N} simulations met a non-finite scoring rate or score-grid normaliser: "
-                             "check the posterior draws")
-        res = {"teams": tteams,
+            raise ValueError(f"{invalid} of {N} simulations {invalid_reason}")
+        cnt = {k: v.cpu().numpy() for k, v in acc.items()}
+        res = {"teams": table["teams"],
                "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
-               **bseason.probabilities(table, pos_c.cpu().numpy(), pts_c.cpu().numpy(), N),
-               "start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
-               "seed": seed}
+               **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N)}
+        if bracket is not None:
+            res.update(bseason.bracket_probabilities(bracket, cnt["reach_counts"], cnt["win_counts"], N))
+        res.update({"start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
+                    "seed": seed})
         if return_simulations:
-            sc = np.concatenate([r[1] for r in raw])
-            res.update(positions=np.concatenate([r[0] for r in raw]), home_score=np.ascontiguousarray(sc[:, :, 0].T),
-                       away_score=np.ascontiguousarray(sc[:, :, 1].T))
+            cat = {k: np.concatenate([r[k] for r in raw]) for k in raw[0]}
+            sc = cat.pop("scores")
+            res.update(positions=cat.pop("positions"), home_score=np.ascontiguousarray(sc[:, :, 0].T),
+                       away_score=np.ascontiguousarray(sc[:, :, 1].T), **cat)
         return res
 
     def _slot_confs(self, tteams, fixtures, team_conf):
@@ -553,8 +571,6 @@ class _BplxPredictor:
         2]`` (table slots), ``ko_scores [N, K, 2]`` and ``ko_winners [N, K]``; the draws are then processed in ranges
         within ``SIM_OUTPUT_BYTES`` and the results do not depend on the range size.  Raises if a simulation was invalid
         (a non-finite rate, or an allocation row the bracket does not cover)."""
-        import torch
-
         fixtures = fixtures if fixtures is not None and len(_str_to_list(fixtures["home_team"])[0]) else None
         home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"]) if fixtures else ([], [])
         named = [e[1] for tie in bracket for e in (tuple(tie["home"]), tuple(tie["away"])) if e[0] == "team"]
@@ -573,62 +589,13 @@ class _BplxPredictor:
             br["slot_conf"] = self._slot_confs(tteams, fixtures, team_conf)
         if fixtures:
             hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
-            h, a = self._parse_fixture_args(home, away)
-            kw = {k: fixtures[k] for k in ("neutral_venue", "home_conf", "away_conf") if k in fixtures}
-            fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw), "home_slot": hs,
-                  "away_slot": as_}
+            fx = {**self._fixture_arrays(home, away, fixtures), "home_slot": hs, "away_slot": as_}
         else:
             fx = {}
-            table["num_points_bins"] = 1
-            table["num_positions"] = len(tteams) if table["group"] is None else int(np.bincount(table["group"]).max())
-        seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
-        R = int(num_sims_per_draw)
-        if R < 1:
-            raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
-        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in self._samples().items()
-              if v is not None}
-        dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
-        dtab = {k: None if table[k] is None else torch.from_numpy(table[k]).cuda()
-                for k in ("start_points", "start_goals_for", "start_goals_against", "group")}
-        dtab.update({k: table[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
-        S, T, F, K = int(ds["attack"].shape[0]), len(tteams), len(home), len(bracket)
-        step = (2 ** 31 - 1) // R
-        if return_simulations:
-            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F + 5 * K))))
-        if step < 1:
-            raise ValueError(f"num_sims_per_draw={R} is too large for one draw per call")
-        acc, invalid, raw = {}, 0, []
-        keys = ("position_counts", "points_counts", "reach_counts", "win_counts")
-        for lo in range(0, S, step):
-            hi = min(S, lo + step)
-            out = _simulate_tournament(self.model, {k: v[lo:hi] for k, v in ds.items()}, dfx, dtab, br, max_goals, R,
-                                       seed, first_draw=lo, want_positions=return_simulations,
-                                       want_scores=return_simulations, want_knockout=return_simulations)
-            for k in keys:
-                acc[k] = out[k] if k not in acc else acc[k] + out[k]
-            invalid += int(out["invalid"].item())
-            if return_simulations:
-                raw.append({k: out[k].cpu().numpy() for k in ("positions", "scores", "ko_entrants", "ko_scores",
-                                                              "ko_winners")})
-        N = S * R
-        if invalid:
-            raise ValueError(f"{invalid} of {N} simulations were invalid: a non-finite scoring rate or score-grid "
-                             "normaliser (check the posterior draws), or best-placed qualifiers the bracket does not "
-                             "place")
-        cnt = {k: v.cpu().numpy() for k, v in acc.items()}
-        res = {"teams": tteams,
-               "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
-               **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N),
-               **bseason.bracket_probabilities(br, cnt["reach_counts"], cnt["win_counts"], N),
-               "start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
-               "seed": seed}
-        if return_simulations:
-            cat = {k: np.concatenate([r[k] for r in raw]) for k in raw[0]}
-            sc = cat["scores"]
-            res.update(positions=cat["positions"], home_score=np.ascontiguousarray(sc[:, :, 0].T),
-                       away_score=np.ascontiguousarray(sc[:, :, 1].T), ko_entrants=cat["ko_entrants"],
-                       ko_scores=cat["ko_scores"], ko_winners=cat["ko_winners"])
-        return res
+            bseason._size_histograms(table)
+        return self._simulate(table, fx, br, num_sims_per_draw, random_state, max_goals, return_simulations,
+                              "were invalid: a non-finite scoring rate or score-grid normaliser (check the posterior "
+                              "draws), or best-placed qualifiers the bracket does not place")
 
     # ---- a team the model has not seen (extended_dixon_coles.py:401-462 and the neutral siblings) ---------------
     def _new_team_pair(self, team_name, team_covariates):

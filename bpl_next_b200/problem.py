@@ -170,6 +170,34 @@ def _fixtures_struct(fixtures: dict, ptr):
     return f
 
 
+def _device_ptr_fn(keep):
+    def ptr(t):
+        assert t.is_cuda and t.is_contiguous()
+        keep.append(t)
+        return int(t.data_ptr())
+    return ptr
+
+
+def _check_inputs(samples: dict, fixtures: dict, uint8_keys=()):
+    """dtypes of device inputs: float32 samples, uint16 / uint8 fixture indices, and ``fixtures[k]`` uint8 for every k
+    of ``uint8_keys``."""
+    for k in _SAMPLE_KEYS + ("home_advantage",):
+        if samples.get(k) is not None:
+            assert samples[k].dtype == torch.float32
+    for k, dt in _FIXTURE_KEYS:
+        if fixtures.get(k) is not None:
+            assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
+    for k in uint8_keys:
+        assert fixtures[k].dtype == torch.uint8, k
+
+
+def _workspace(workspace, need: int, device):
+    """``workspace`` when it holds ``need`` bytes, else a new device buffer."""
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=device)
+    return workspace
+
+
 def score_grid_workspace_bytes(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor],
                                max_goals: int) -> int:
     """Bytes of device workspace ``score_grid`` needs for these shapes (``bplx_score_grid_workspace_bytes``)."""
@@ -187,25 +215,13 @@ def score_grid(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str,
     ``workspace`` passed in still holds the exponential tables a previous call built from these very samples."""
     lib = _abi.lib()
     keep = []
-
-    def ptr(t):
-        assert t.is_cuda and t.is_contiguous()
-        keep.append(t)
-        return int(t.data_ptr())
-
-    for k in _SAMPLE_KEYS + ("home_advantage",):
-        if samples.get(k) is not None:
-            assert samples[k].dtype == torch.float32
-    for k, dt in _FIXTURE_KEYS:
-        if fixtures.get(k) is not None:
-            assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
+    ptr = _device_ptr_fn(keep)
+    _check_inputs(samples, fixtures)
     s = _samples_struct(model, samples, ptr)
     f = _fixtures_struct(fixtures, ptr)
     g = max_goals + 1
     dev = samples["attack"].device
-    need = int(lib.bplx_score_grid_workspace_bytes(C.byref(s), C.byref(f), max_goals))
-    if workspace is None or workspace.numel() < need:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    workspace = _workspace(workspace, int(lib.bplx_score_grid_workspace_bytes(C.byref(s), C.byref(f), max_goals)), dev)
     grid = torch.empty((f.num_fixtures, g, g), dtype=torch.float32, device=dev) if grid is None else grid
     if want_outcome and outcome is None:
         outcome = torch.empty((f.num_fixtures, 3), dtype=torch.float32, device=dev)
@@ -239,14 +255,6 @@ def score_grid_host(model: str, samples: Dict[str, np.ndarray], fixtures: Dict[s
     return grid, outcome
 
 
-def _device_ptr_fn(keep):
-    def ptr(t):
-        assert t.is_cuda and t.is_contiguous()
-        keep.append(t)
-        return int(t.data_ptr())
-    return ptr
-
-
 def pointwise_loglik(model: str, samples: Dict[str, torch.Tensor], observations: Dict[str, torch.Tensor],
                      want_matrix: bool = True, loglik: Optional[torch.Tensor] = None, workspace=None, stream=None):
     """Device path of ``bplx_pointwise_loglik``: posterior arrays ``[S, T]`` float32 and observed matches (the fixture
@@ -260,20 +268,14 @@ def pointwise_loglik(model: str, samples: Dict[str, torch.Tensor], observations:
     lib = _abi.lib()
     keep = []
     ptr = _device_ptr_fn(keep)
-    for k in _SAMPLE_KEYS + ("home_advantage",):
-        if samples.get(k) is not None:
-            assert samples[k].dtype == torch.float32
-    for k in ("home_goals", "away_goals"):
-        assert observations[k].dtype == torch.uint8, k
+    _check_inputs(samples, observations, ("home_goals", "away_goals"))
     s = _samples_struct(model, samples, ptr)
     o = _abi.Observations()
     o.fixtures = _fixtures_struct(observations, ptr)
     o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
     M, S = o.fixtures.num_fixtures, s.num_samples
     dev = samples["attack"].device
-    need = int(lib.bplx_pointwise_loglik_workspace_bytes(C.byref(s), C.byref(o)))
-    if workspace is None or workspace.numel() < need:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    workspace = _workspace(workspace, int(lib.bplx_pointwise_loglik_workspace_bytes(C.byref(s), C.byref(o))), dev)
     ld = 0
     if want_matrix:
         if loglik is None:
@@ -326,51 +328,20 @@ def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[
     ``position_counts [T_tab, P]`` and ``points_counts [T_tab, B]`` (points gained; int64), ``invalid`` (int64 ``[1]``:
     simulations with a non-finite rate or normaliser, left out of the counts), and when asked ``positions [N, T_tab]``
     and ``scores [N, F, 2]`` (uint8; 255 marks an invalid simulation / fixture), N = S R."""
-    lib = _abi.lib()
-    keep = []
-    ptr = _device_ptr_fn(keep)
-    for k in _SAMPLE_KEYS + ("home_advantage",):
-        if samples.get(k) is not None:
-            assert samples[k].dtype == torch.float32
-    for k, dt in _FIXTURE_KEYS:
-        if fixtures.get(k) is not None:
-            assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
-    for k in ("home_slot", "away_slot"):
-        assert fixtures[k].dtype == torch.uint8, k
-    for k in _TABLE_ARRAYS:
-        assert table[k].dtype == torch.int32, k
-    T_tab = int(table["start_points"].shape[0])
-    if T_tab > _abi.SIM_MAX_TEAMS:
-        raise ValueError(f"the table has {T_tab} slots; at most {_abi.SIM_MAX_TEAMS} are supported")
-    top = int(torch.maximum(fixtures["home_slot"].max(), fixtures["away_slot"].max()))
-    if top >= T_tab:
-        raise ValueError(f"a fixture names table slot {top}, but the table has {T_tab} slots")
-    s = _samples_struct(model, samples, ptr)
-    f = _fixtures_struct(fixtures, ptr)
+    return _simulate(model, samples, fixtures, table, None, max_goals, sims_per_draw, seed, first_draw, want_positions,
+                     want_scores, False, workspace, stream)
+
+
+def _table_struct(table: dict, ptr):
+    """``_abi.Table`` over the device arrays of ``table``: one slot per entry of ``start_points``."""
     t = _abi.Table()
-    t.num_slots = T_tab
+    t.num_slots = int(table["start_points"].shape[0])
     t.num_positions, t.num_points_bins = int(table["num_positions"]), int(table["num_points_bins"])
     t.points_win, t.points_draw = int(table["points_win"]), int(table["points_draw"])
     t.group = None if table.get("group") is None else ptr(table["group"])
     for k in _TABLE_ARRAYS:
         setattr(t, k, ptr(table[k]))
-    dev = samples["attack"].device
-    need = int(lib.bplx_simulate_workspace_bytes(C.byref(s), C.byref(f), C.byref(t)))
-    if workspace is None or workspace.numel() < need:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
-    N, F = s.num_samples * int(sims_per_draw), f.num_fixtures
-    pos_counts = torch.empty((T_tab, t.num_positions), dtype=torch.int64, device=dev)
-    pts_counts = torch.empty((T_tab, t.num_points_bins), dtype=torch.int64, device=dev)
-    invalid = torch.empty(1, dtype=torch.int64, device=dev)
-    positions = torch.empty((N, T_tab), dtype=torch.uint8, device=dev) if want_positions else None
-    scores = torch.empty((N, F, 2), dtype=torch.uint8, device=dev) if want_scores else None
-    _abi.check(lib.bplx_simulate_table(C.byref(s), C.byref(f), ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"]),
-                                       C.byref(t), int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF,
-                                       int(first_draw), _dptr(pos_counts), _dptr(pts_counts), _dptr(positions),
-                                       _dptr(scores), _dptr(invalid), _dptr(workspace), workspace.numel(),
-                                       _stream_ptr(stream)))
-    return {"position_counts": pos_counts, "points_counts": pts_counts, "invalid": invalid, "positions": positions,
-            "scores": scores}
+    return t
 
 
 def _bracket_struct(bracket: dict, keep: list):
@@ -414,19 +385,19 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
     penalties are not modelled.  Returns ``simulate_table``'s outputs plus ``reach_counts`` / ``win_counts`` (int64
     ``[T_tab, num_rounds]``: ties of round r the slot played / won), and when ``want_knockout`` ``ko_entrants``,
     ``ko_scores`` (uint8 ``[N, K, 2]``) and ``ko_winners`` (``[N, K]``); 255 marks an invalid simulation."""
+    return _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw,
+                     want_positions, want_scores, want_knockout, workspace, stream)
+
+
+def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw, want_positions,
+              want_scores, want_knockout, workspace, stream):
+    """``simulate_tournament``, and ``simulate_table`` when ``bracket`` is None (``bplx_simulate_table``: the group
+    stage kernel)."""
     lib = _abi.lib()
     keep = []
     ptr = _device_ptr_fn(keep)
-    for k in _SAMPLE_KEYS + ("home_advantage",):
-        if samples.get(k) is not None:
-            assert samples[k].dtype == torch.float32
     F = int(len(fixtures["home_team"])) if fixtures.get("home_team") is not None else 0
-    if F:
-        for k, dt in _FIXTURE_KEYS:
-            if fixtures.get(k) is not None:
-                assert fixtures[k].dtype == (torch.uint16 if dt == np.uint16 else torch.uint8), k
-        for k in ("home_slot", "away_slot"):
-            assert fixtures[k].dtype == torch.uint8, k
+    _check_inputs(samples, fixtures, ("home_slot", "away_slot") if F else ())
     for k in _TABLE_ARRAYS:
         assert table[k].dtype == torch.int32, k
     T_tab = int(table["start_points"].shape[0])
@@ -438,34 +409,32 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
             raise ValueError(f"a fixture names table slot {top}, but the table has {T_tab} slots")
     s = _samples_struct(model, samples, ptr)
     f = _fixtures_struct(fixtures, ptr) if F else _abi.Fixtures()
-    t = _abi.Table()
-    t.num_slots = T_tab
-    t.num_positions, t.num_points_bins = int(table["num_positions"]), int(table["num_points_bins"])
-    t.points_win, t.points_draw = int(table["points_win"]), int(table["points_draw"])
-    t.group = None if table.get("group") is None else ptr(table["group"])
-    for k in _TABLE_ARRAYS:
-        setattr(t, k, ptr(table[k]))
-    b = _bracket_struct(bracket, keep)
+    t = _table_struct(table, ptr)
+    b = None if bracket is None else _bracket_struct(bracket, keep)
+    structs = (C.byref(s), C.byref(f), C.byref(t)) + (() if b is None else (C.byref(b),))
+    ws_bytes = lib.bplx_simulate_workspace_bytes if b is None else lib.bplx_simulate_tournament_workspace_bytes
     dev = samples["attack"].device
-    need = int(lib.bplx_simulate_tournament_workspace_bytes(C.byref(s), C.byref(f), C.byref(t), C.byref(b)))
-    if workspace is None or workspace.numel() < need:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
-    N, K, nr = s.num_samples * int(sims_per_draw), b.num_ties, b.num_rounds
+    workspace = _workspace(workspace, int(ws_bytes(*structs)), dev)
+    N = s.num_samples * int(sims_per_draw)
     i64 = dict(dtype=torch.int64, device=dev)
     u8 = dict(dtype=torch.uint8, device=dev)
     out = {"position_counts": torch.empty((T_tab, t.num_positions), **i64),
-           "points_counts": torch.empty((T_tab, t.num_points_bins), **i64),
-           "reach_counts": torch.empty((T_tab, nr), **i64), "win_counts": torch.empty((T_tab, nr), **i64),
-           "invalid": torch.empty(1, **i64),
-           "positions": torch.empty((N, T_tab), **u8) if want_positions else None,
-           "scores": torch.empty((N, F, 2), **u8) if want_scores else None,
-           "ko_entrants": torch.empty((N, K, 2), **u8) if want_knockout else None,
-           "ko_scores": torch.empty((N, K, 2), **u8) if want_knockout else None,
-           "ko_winners": torch.empty((N, K), **u8) if want_knockout else None}
-    _abi.check(lib.bplx_simulate_tournament(
-        C.byref(s), C.byref(f), ptr(fixtures["home_slot"]) if F else None, ptr(fixtures["away_slot"]) if F else None,
-        C.byref(t), C.byref(b), int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
-        *(_dptr(out[k]) for k in ("position_counts", "points_counts", "reach_counts", "win_counts", "positions",
-                                  "scores", "ko_entrants", "ko_scores", "ko_winners", "invalid")),
-        _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+           "points_counts": torch.empty((T_tab, t.num_points_bins), **i64)}
+    if b is not None:
+        out.update(reach_counts=torch.empty((T_tab, b.num_rounds), **i64),
+                   win_counts=torch.empty((T_tab, b.num_rounds), **i64))
+    out.update(invalid=torch.empty(1, **i64), positions=torch.empty((N, T_tab), **u8) if want_positions else None,
+               scores=torch.empty((N, F, 2), **u8) if want_scores else None)
+    if b is not None:
+        K = b.num_ties
+        out.update(ko_entrants=torch.empty((N, K, 2), **u8) if want_knockout else None,
+                   ko_scores=torch.empty((N, K, 2), **u8) if want_knockout else None,
+                   ko_winners=torch.empty((N, K), **u8) if want_knockout else None)
+    # the C functions take the outputs in the order of `out`, with `invalid` last
+    outputs = [_dptr(v) for k, v in out.items() if k != "invalid"] + [_dptr(out["invalid"])]
+    slots = (ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"])) if F else (None, None)
+    run = lib.bplx_simulate_table if b is None else lib.bplx_simulate_tournament
+    _abi.check(run(*structs[:2], *slots, *structs[2:], int(max_goals), int(sims_per_draw),
+                   int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw), *outputs, _dptr(workspace), workspace.numel(),
+                   _stream_ptr(stream)))
     return out

@@ -15,9 +15,8 @@ from typing import Any, Dict, Optional, Sequence, Tuple
 
 import numpy as np
 
-SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
-KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
-ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0, 1, 2, 3, 4  # BPLX_ENTRANT_*
+from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_SLOT, ENTRANT_WINNER, KO_MAX_ALLOC_GROUPS,
+                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, SIM_MAX_TEAMS)
 
 
 def _names(x) -> list:
@@ -116,11 +115,17 @@ def fixture_slots(table: Dict[str, Any], home, away, known_teams=None) -> Tuple[
             raise ValueError(f"team {h!r} plays itself")
     hs = np.asarray([slot[t] for t in home], np.uint8)
     as_ = np.asarray([slot[t] for t in away], np.uint8)
+    _size_histograms(table, hs, as_)
+    return hs, as_
+
+
+def _size_histograms(table: Dict[str, Any], home_slot=(), away_slot=()) -> None:
+    """Sets ``num_positions`` (the largest group) and ``num_points_bins`` (``points_win * max_t(remaining fixtures of
+    t) + 1``: 1 when there are no fixtures) in ``table`` for the fixtures between these slots."""
     T = len(table["teams"])
-    rem = np.bincount(hs, minlength=T) + np.bincount(as_, minlength=T)
+    rem = np.bincount(np.concatenate([home_slot, away_slot]).astype(np.int64), minlength=T)
     table["num_points_bins"] = int(table["points_win"] * rem.max() + 1)
     table["num_positions"] = T if table["group"] is None else int(np.bincount(table["group"]).max())
-    return hs, as_
 
 
 def probabilities(table: Dict[str, Any], position_counts: np.ndarray, points_counts: np.ndarray,

@@ -73,6 +73,21 @@ def world_cup(S):
     return "neutral_wc", s, fx, hs.astype(np.uint8), as_.astype(np.uint8), 48, group.astype(np.uint8)
 
 
+def device_table(T_tab, group, hs, as_):
+    """A table of T_tab slots on the GPU, every team on zero, 3 points a win and 1 a draw, its histograms sized for the
+    fixtures between slots hs and as_."""
+    import torch
+
+    from bpl_next_b200 import season
+
+    zeros = torch.zeros(T_tab, dtype=torch.int32, device="cuda")
+    tab = {"teams": range(T_tab), "group": group, "points_win": 3, "points_draw": 1}
+    season._size_histograms(tab, hs, as_)
+    tab.update(start_points=zeros, start_goals_for=zeros, start_goals_against=zeros,
+               group=None if group is None else torch.from_numpy(group).cuda())
+    return tab
+
+
 def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
     """The bplx_simulate_table call with every argument built once; returns (call, outputs, keep-alive)."""
     import torch
@@ -86,14 +101,8 @@ def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
     dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
     st = problem._samples_struct(model, dev, ptr)
     ft = problem._fixtures_struct(dfx, ptr)
-    rem = np.bincount(hs, minlength=T_tab) + np.bincount(as_, minlength=T_tab)
-    t = _abi.Table()
-    t.num_slots, t.points_win, t.points_draw = T_tab, 3, 1
-    t.num_positions = T_tab if group is None else int(np.bincount(group).max())
-    t.num_points_bins = int(3 * rem.max() + 1)
-    zeros = torch.zeros(T_tab, dtype=torch.int32, device="cuda")
-    t.start_points = t.start_goals_for = t.start_goals_against = ptr(zeros)
-    t.group = None if group is None else ptr(torch.from_numpy(group).cuda())
+    tab = device_table(T_tab, group, hs, as_)
+    t = problem._table_struct(tab, ptr)
     d_hs, d_as = ptr(torch.from_numpy(hs).cuda()), ptr(torch.from_numpy(as_).cuda())
     pc = torch.empty((T_tab, t.num_positions), dtype=torch.int64, device="cuda")
     bc = torch.empty((T_tab, t.num_points_bins), dtype=torch.int64, device="cuda")
@@ -107,7 +116,7 @@ def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
     def call():
         _abi.check(lib.bplx_simulate_table(*args))
 
-    return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, zeros, ws)
+    return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, tab, ws)
 
 
 def time_ms(fn, reps):

@@ -30,7 +30,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
 sys.dont_write_bytecode = True
 
-from simulate_time import gpu_info, prepared_call, time_ms, world_cup  # noqa: E402
+from simulate_time import device_table, gpu_info, prepared_call, time_ms, world_cup  # noqa: E402
 
 
 def _knockout(entrants):
@@ -86,14 +86,8 @@ def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1):
         d_hs, d_as = ptr(torch.from_numpy(hs).cuda()), ptr(torch.from_numpy(as_).cuda())
     else:
         ft, d_hs, d_as = _abi.Fixtures(), None, None
-    rem = np.bincount(hs, minlength=T_tab) + np.bincount(as_, minlength=T_tab)
-    t = _abi.Table()
-    t.num_slots, t.points_win, t.points_draw = T_tab, 3, 1
-    t.num_positions = T_tab if group is None else int(np.bincount(group).max())
-    t.num_points_bins = int(3 * rem.max() + 1)
-    zeros = torch.zeros(T_tab, dtype=torch.int32, device="cuda")
-    t.start_points = t.start_goals_for = t.start_goals_against = ptr(zeros)
-    t.group = None if group is None else ptr(torch.from_numpy(group).cuda())
+    tab = device_table(T_tab, group, hs, as_)
+    t = problem._table_struct(tab, ptr)
     b = problem._bracket_struct(br, keep)
     cnt = {k: torch.empty(n, dtype=torch.int64, device="cuda") for k, n in
            (("pos", T_tab * t.num_positions), ("pts", T_tab * t.num_points_bins), ("reach", T_tab * b.num_rounds),
@@ -108,7 +102,7 @@ def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1):
     def call():
         _abi.check(lib.bplx_simulate_tournament(*args))
 
-    return call, cnt, (keep, st, ft, t, b, dev, zeros, ws)
+    return call, cnt, (keep, st, ft, t, b, dev, tab, ws)
 
 
 def smem_bytes(T_tab, P, B, nr=0, K=0):

@@ -153,22 +153,17 @@ def test_expected_points_against_the_outcome_probabilities():
     assert (np.abs(pr["expected_points"] - want) <= 5 * se).all(), (pr["expected_points"] - want) / se
 
 
-def _raw_call(model, s, fx, hs, as_, tab, G, R, num_slots=None):
-    """bplx_simulate_table called directly (no Python-side checks); returns (status, invalid count)."""
+def _raw_call(model, s, fx, hs, as_, tab, G, R):
+    """bplx_simulate_table called directly (no Python-side checks) on one table without groups; returns (status,
+    invalid count)."""
     from bpl_next_b200 import problem
 
     lib = _abi.lib()
     keep = []
     ptr = problem._device_ptr_fn(keep)
-    ds, dfx, dt = _dev(s), _dev(fx), _dev_table(tab)
-    st = problem._samples_struct(model, ds, ptr)
-    ft = problem._fixtures_struct(dfx, ptr)
-    t = _abi.Table()
-    t.num_slots = len(tab["start_points"]) if num_slots is None else num_slots
-    t.num_positions, t.num_points_bins = tab["num_positions"], tab["num_points_bins"]
-    t.points_win, t.points_draw = tab["points_win"], tab["points_draw"]
-    t.group = None
-    t.start_points, t.start_goals_for, t.start_goals_against = (ptr(dt[k]) for k in problem._TABLE_ARRAYS)
+    st = problem._samples_struct(model, _dev(s), ptr)
+    ft = problem._fixtures_struct(_dev(fx), ptr)
+    t = problem._table_struct(dict(_dev_table(tab), group=None), ptr)
     slots = _dev({"h": hs, "a": as_})
     pc = torch.empty((t.num_slots, t.num_positions), dtype=torch.int64, device="cuda")
     bc = torch.empty((t.num_slots, t.num_points_bins), dtype=torch.int64, device="cuda")

@@ -13,18 +13,9 @@ from bpl_next_b200 import _abi, season
 from oracle import predict as op
 from tests import tournament_oracle as otour
 from tests.test_score_grid_gpu import make_samples
+from tests.test_simulate_gpu import _dev, _dev_table
 
 pytestmark = pytest.mark.gpu
-
-
-def _dev(d):
-    return {k: (None if v is None else torch.from_numpy(np.ascontiguousarray(v)).cuda()) for k, v in d.items()}
-
-
-def _dev_table(tab):
-    d = _dev({k: tab[k] for k in ("start_points", "start_goals_for", "start_goals_against", "group")})
-    d.update({k: tab[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
-    return d
 
 
 def _alloc(labels, count):
@@ -80,8 +71,7 @@ def _case(model, S, T_tab, grouped, F, seed, Cf=4, best=False):
             fx["home_conf"] = rng.integers(0, Cf, F).astype(np.uint8)
             fx["away_conf"] = rng.integers(0, Cf, F).astype(np.uint8)
     else:
-        tab["num_points_bins"] = 1
-        tab["num_positions"] = T_tab if tab["group"] is None else int(np.bincount(tab["group"]).max())
+        season._size_histograms(tab)
     bspec = None
     if grouped:
         L = tab["group_labels"]
@@ -300,12 +290,7 @@ def _raw_call(model, s, tab, br, R=2, slot_team=None):
     ptr = problem._device_ptr_fn(keep)
     st = problem._samples_struct(model, _dev(s), ptr)
     ft = _abi.Fixtures()
-    dt = _dev_table(tab)
-    t = _abi.Table()
-    t.num_slots = len(tab["start_points"])
-    t.num_positions, t.num_points_bins, t.points_win, t.points_draw = tab["num_positions"], 1, 3, 1
-    t.start_points, t.start_goals_for, t.start_goals_against = (ptr(dt[k]) for k in problem._TABLE_ARRAYS)
-    t.group = None if dt["group"] is None else ptr(dt["group"])
+    t = problem._table_struct(dict(_dev_table(tab), num_points_bins=1, points_win=3, points_draw=1), ptr)
     b = problem._bracket_struct(dict(br, slot_team=br["slot_team"] if slot_team is None else slot_team), keep)
     K, nr = b.num_ties, max(b.num_rounds, 1)
     cnt = [torch.empty(64 * 64, dtype=torch.int64, device="cuda") for _ in range(5)]

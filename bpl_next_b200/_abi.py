@@ -81,6 +81,9 @@ SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
 # BPLX_ENTRANT_*
 ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0, 1, 2, 3, 4
+# BPLX_TIE_*, BPLX_EXTRA_TIME_FRACTION
+TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS = 0, 1, 2
+EXTRA_TIME_FRACTION = 1.0 / 3.0
 
 
 class BplxError(RuntimeError):
@@ -145,6 +148,10 @@ def declare(lib):
                                              C.POINTER(Bracket), i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp,
                                              vp, vp, vp, vp, vp, vp, sz, vp]
     lib.bplx_simulate_tournament.restype = i
+    lib.bplx_simulate_tournament_ex.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                                C.POINTER(Bracket), vp, i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp,
+                                                vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.bplx_simulate_tournament_ex.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

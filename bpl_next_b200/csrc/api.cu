@@ -897,7 +897,8 @@ size_t bplx_simulate_tournament_workspace_bytes(const bplx_samples* s, const bpl
 }
 
 // the bracket checks the kernel relies on; fills sp->ko
-static int check_bracket(const bplx_bracket* b, const bplx_samples* s, int NT, int P, KoParams* ko) {
+static int check_bracket(const bplx_bracket* b, const uint8_t* tie_format, const bplx_samples* s, int NT, int P,
+                         KoParams* ko) {
   BPLX_REQUIRE(b != nullptr, BPLX_E_INVALID, "tournament: bracket is NULL");
   const int K = b->num_ties;
   BPLX_REQUIRE(K >= 1, BPLX_E_INVALID, "tournament: the bracket needs at least one tie (got %d)", K);
@@ -958,6 +959,11 @@ static int check_bracket(const bplx_bracket* b, const bplx_samples* s, int NT, i
     }
     ko->round[k] = b->round[k];
     ko->neutral[k] = b->neutral_venue ? (b->neutral_venue[k] != 0) : 0;
+    ko->format[k] = tie_format ? tie_format[k] : BPLX_TIE_ONE_MATCH;
+    BPLX_REQUIRE(ko->format[k] <= BPLX_TIE_TWO_LEGS, BPLX_E_INVALID,
+                 "tournament: tie %d: format %d is not a BPLX_TIE_* value", k, ko->format[k]);
+    BPLX_REQUIRE(ko->format[k] != BPLX_TIE_TWO_LEGS || !ko->neutral[k], BPLX_E_INVALID,
+                 "tournament: tie %d: a two-legged tie cannot be at a neutral venue", k);
   }
   if (b->best_alloc) {
     BPLX_REQUIRE(b->best_count >= 1, BPLX_E_INVALID, "tournament: an allocation table needs best_count >= 1");
@@ -988,18 +994,20 @@ static int check_bracket(const bplx_bracket* b, const bplx_samples* s, int NT, i
   return BPLX_OK;
 }
 
-int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
-                             const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b, int max_goals,
-                             int sims_per_draw, unsigned long long seed, long long first_draw,
-                             unsigned long long* position_counts, unsigned long long* points_counts,
-                             unsigned long long* reach_counts, unsigned long long* win_counts, uint8_t* positions,
-                             uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
-                             unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream) {
+int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                const uint8_t* tie_format, int max_goals, int sims_per_draw, unsigned long long seed,
+                                long long first_draw, unsigned long long* position_counts,
+                                unsigned long long* points_counts, unsigned long long* reach_counts,
+                                unsigned long long* win_counts, unsigned long long* decided_counts, uint8_t* positions,
+                                uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
+                                uint8_t* ko_extra, unsigned long long* invalid, void* workspace,
+                                size_t workspace_bytes, void* stream) {
   SimParams sp{};
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "tournament", true, &sp);
   if (rc != BPLX_OK) return rc;
-  rc = check_bracket(b, s, t->num_slots, t->num_positions, &sp.ko);
+  rc = check_bracket(b, tie_format, s, t->num_slots, t->num_positions, &sp.ko);
   if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
   const size_t table = simulate_plan_for(s, f, &sp);
@@ -1008,9 +1016,11 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
   sp.gp.table = static_cast<float*>(workspace);
   sp.ko.reach = reach_counts;
   sp.ko.win = win_counts;
+  sp.ko.decided = decided_counts;
   sp.ko.entrants = ko_entrants;
   sp.ko.scores = ko_scores;
   sp.ko.winners = ko_winners;
+  sp.ko.extra = ko_extra;
   if (b->best_alloc) {
     uint8_t* const dst = static_cast<uint8_t*>(workspace) + table;
     BPLX_CUDA(cudaMemcpyAsync(dst, b->best_alloc, alloc_bytes(b), cudaMemcpyHostToDevice,
@@ -1018,6 +1028,19 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
     sp.ko.alloc = dst;
   }
   return launch_simulate_tournament(sp, static_cast<cudaStream_t>(stream));
+}
+
+int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                             const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b, int max_goals,
+                             int sims_per_draw, unsigned long long seed, long long first_draw,
+                             unsigned long long* position_counts, unsigned long long* points_counts,
+                             unsigned long long* reach_counts, unsigned long long* win_counts, uint8_t* positions,
+                             uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
+                             unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream) {
+  return bplx_simulate_tournament_ex(s, f, home_slot, away_slot, t, b, nullptr, max_goals, sims_per_draw, seed,
+                                     first_draw, position_counts, points_counts, reach_counts, win_counts, nullptr,
+                                     positions, scores, ko_entrants, ko_scores, ko_winners, nullptr, invalid, workspace,
+                                     workspace_bytes, stream);
 }
 
 void bplx_reload_env(void) {

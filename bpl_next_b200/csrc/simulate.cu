@@ -37,6 +37,7 @@ namespace bplx {
 namespace {
 
 __constant__ float c_sim_inv_k[64];  // 1 / k (k >= 1)
+constexpr float kExtraTimeFraction = 1.0f / 3.0f;  // BPLX_EXTRA_TIME_FRACTION: 30 of 90 minutes at constant rates
 
 // one fixture of one simulation; false when the rates or the normaliser are unusable
 __device__ __forceinline__ bool sample_score(float lh, float la, float c, float uh, float ua, int G, int& hg, int& ag) {
@@ -142,11 +143,17 @@ __device__ __forceinline__ void win_masses(float lh, float la, float c, int G, f
   }
 }
 
-// word w of the Philox sequence of simulation n (curand_init(seed, n, 0) followed by w + 1 curand()) without a state:
-// the tournament kernel reads the slot tie-break keys only when points, goal difference and goals for are level
+// words 4b .. 4b + 3 of the Philox sequence of simulation n (curand_init(seed, n, 0) followed by curand()) without a
+// state: one Philox4x32_10 block
+__device__ __forceinline__ uint4 philox_block(unsigned long long seed, unsigned long long n, unsigned b) {
+  return curand_Philox4x32_10(make_uint4(b, 0u, (unsigned)n, (unsigned)(n >> 32)),
+                              make_uint2((unsigned)seed, (unsigned)(seed >> 32)));
+}
+
+// word w of that sequence: the tournament kernel reads the slot tie-break keys only when points, goal difference and
+// goals for are level
 __device__ __forceinline__ uint32_t philox_word(unsigned long long seed, unsigned long long n, unsigned w) {
-  const uint4 o = curand_Philox4x32_10(make_uint4(w >> 2, 0u, (unsigned)n, (unsigned)(n >> 32)),
-                                       make_uint2((unsigned)seed, (unsigned)(seed >> 32)));
+  const uint4 o = philox_block(seed, n, w >> 2);
   const unsigned r = w & 3u;
   return r == 0 ? o.x : r == 1 ? o.y : r == 2 ? o.z : o.w;
 }
@@ -170,7 +177,9 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   unsigned* const h_pts = h_pos + NT * sp.P;
   unsigned* const h_reach = h_pts + (sp.points_in_smem ? NT * sp.B : 0);  // tournament: [NT][nr] each
   unsigned* const h_win = h_reach + (KO ? NT * ko.nr : 0);
-  int* const s_members = reinterpret_cast<int*>(h_win + (KO ? NT * ko.nr : 0));
+  // tournament: [K][2] ties settled in extra time / by u_d (the rest of the CTA's valid simulations: in normal time)
+  unsigned* const h_dec = h_win + (KO ? NT * ko.nr : 0);
+  int* const s_members = reinterpret_cast<int*>(h_dec + (KO ? 2 * ko.K : 0));
   int* const s_gbeg = s_members + NT;
   int* const s_gcnt = s_gbeg + NT;
   // Tournament: the keys are not stored (philox_word reads one when it is needed), so the s_key words hold bytes:
@@ -178,7 +187,8 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   // BEST j, k_gtab = per CTA, first member index [ng] and size [ng] of each group id.  The per-tie winner / loser bytes
   // go into the thread's OWN s_gf / s_gd words once its ranking and best-placed selection are done (byte b in byte
   // b % 4 of word [b / 4][thread], so a thread that reaches its ties early never touches the words another thread is
-  // still ranking), or after the member lists when 2K bytes exceed those 2 T_tab words.
+  // still ranking), or after the member lists when 2K bytes exceed those 2 T_tab words.  A slot fits 6 bits (T_tab <=
+  // 64): bits 6-7 of the winner byte hold how the tie was decided until the histograms are committed.
   uint8_t* const k_q = reinterpret_cast<uint8_t*>(s_key);
   uint8_t* const k_best = k_q + NT * kSimThreads;
   uint8_t* const k_gtab = k_best + (KO ? ko.bc : 0) * kSimThreads;
@@ -197,7 +207,7 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   if (sp.points_in_smem)
     for (int k = tid; k < NT * sp.B; k += kSimThreads) h_pts[k] = 0;
   if constexpr (KO) {
-    for (int k = tid; k < 2 * NT * ko.nr; k += kSimThreads) h_reach[k] = 0;  // h_win follows h_reach
+    for (int k = tid; k < 2 * (NT * ko.nr + ko.K); k += kSimThreads) h_reach[k] = 0;  // h_win, h_dec follow
     for (int g = tid; g < ko.ng; g += kSimThreads) {
       int beg = 0, cnt = 0;
       for (int u = 0; u < NT; u++) {
@@ -358,11 +368,13 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
           }
         }
       }
-      // the ties in play order; words 2F + T_tab + 3k, + 1 (the score) and + 2 (the decider) of tie k
+      // the ties in play order; words 2F + T_tab + 3k, + 1 (the first or only match) and + 2 (the decider) of tie k,
+      // and the Philox block E/4 + k (leg 2, extra time) of a tie of format 1 or 2
       skipahead((unsigned long long)NT, &rng);
       uint8_t* const ent = ko.entrants ? ko.entrants + (size_t)i * ko.K * 2 : nullptr;
       uint8_t* const ksc = ko.scores ? ko.scores + (size_t)i * ko.K * 2 : nullptr;
       uint8_t* const kwn = ko.winners ? ko.winners + (size_t)i * ko.K : nullptr;
+      uint8_t* const kex = ko.extra ? ko.extra + (size_t)i * ko.K * 4 : nullptr;
 #pragma unroll 1
       for (int k = 0; k < ko.K && ok; k++) {
         int e[2];
@@ -378,7 +390,7 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
               break;
             }
             case BPLX_ENTRANT_BEST: e[side] = BYTE(k_best, a0); break;
-            case BPLX_ENTRANT_WINNER: e[side] = WL(2 * a0); break;
+            case BPLX_ENTRANT_WINNER: e[side] = WL(2 * a0) & 63; break;
             default: e[side] = WL(2 * a0 + 1); break;
           }
         }
@@ -392,16 +404,52 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
         int hg = 0, ag = 0;
         ok = sample_score(lam.x, lam.y, c, uh, ua, sp.G, hg, ag);
         bool home_through = hg > ag;
-        if (ok && hg == ag) {  // a drawn tie: the home entrant goes through iff u_d (hw + aw) <= hw
-          float hw, aw;
-          win_masses(lam.x, lam.y, c, sp.G, hw, aw);
-          const float tot = hw + aw;
-          ok = tot > 0.0f;
-          home_through = ud * tot <= hw;
+        int how = 0;  // decided in normal time or on aggregate (0), in extra time (1), by u_d (2)
+        const int fmt = ko.format[k];
+        if (fmt == BPLX_TIE_ONE_MATCH) {
+          if (ok && hg == ag) {  // a drawn tie: the home entrant goes through iff u_d (hw + aw) <= hw
+            float hw, aw;
+            win_masses(lam.x, lam.y, c, sp.G, hw, aw);
+            const float tot = hw + aw;
+            ok = tot > 0.0f;
+            home_through = ud * tot <= hw;
+            how = 2;
+          }
+          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(0xFE, 0xFE, 0xFE, 0xFE);
+        } else if (ok) {
+          // goals of the home entrant A and the away entrant B; extra time at the venue of the last match
+          const uint4 xw = philox_block(sp.seed, n, (2u * gp.F + NT + 3u * ko.K + 3u) / 4u + k);
+          int tot_a = hg, tot_b = ag, l2a = 0xFE, l2b = 0xFE, eta = 0xFE, etb = 0xFE;
+          float2 last = lam;
+          const bool legs = fmt == BPLX_TIE_TWO_LEGS;
+          if (legs) {  // leg 2: B at home, never at a neutral venue
+            const FixtureOffsets off2 = fixture_offsets(L, ko.slot_team[as], ko.slot_team[hs], false, wc,
+                                                        wc ? ko.slot_conf[as] : 0, wc ? ko.slot_conf[hs] : 0);
+            last = fixture_rates(row, off2, false, wc);
+            ok = sample_score(last.x, last.y, c, _curand_uniform(xw.x), _curand_uniform(xw.y), sp.G, l2b, l2a);
+            tot_a += l2a;
+            tot_b += l2b;
+          }
+          if (ok && tot_a == tot_b) {
+            int eh = 0, ea = 0;
+            ok = sample_score(last.x * kExtraTimeFraction, last.y * kExtraTimeFraction, 0.0f, _curand_uniform(xw.z),
+                              _curand_uniform(xw.w), sp.G, eh, ea);
+            eta = legs ? ea : eh;
+            etb = legs ? eh : ea;
+            tot_a += eta;
+            tot_b += etb;
+            how = 1;
+          }
+          home_through = tot_a > tot_b;
+          if (tot_a == tot_b) {  // penalties
+            home_through = ud <= 0.5f;
+            how = 2;
+          }
+          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(l2a, l2b, eta, etb);
         }
         if (!ok) break;
         const int w = home_through ? hs : as;
-        WL(2 * k) = (uint8_t)w;
+        WL(2 * k) = (uint8_t)(w | how << 6);
         WL(2 * k + 1) = (uint8_t)(home_through ? as : hs);
         if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2((unsigned char)hs, (unsigned char)as);
         if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2((unsigned char)hg, (unsigned char)ag);
@@ -416,6 +464,7 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
           if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2(0xFF, 0xFF);
           if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2(0xFF, 0xFF);
           if (kwn) kwn[k] = 0xFF;
+          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(0xFF, 0xFF, 0xFF, 0xFF);
         }
       } else {
         for (int m = 0; m < NT; m++) {
@@ -427,10 +476,11 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
           else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
         }
         for (int k = 0; k < ko.K; k++) {
-          const int r = ko.round[k], w = WL(2 * k), l = WL(2 * k + 1);
+          const int r = ko.round[k], wb = WL(2 * k), w = wb & 63, l = WL(2 * k + 1);
           atomicAdd(&h_reach[w * ko.nr + r], 1u);
           atomicAdd(&h_reach[l * ko.nr + r], 1u);
           atomicAdd(&h_win[w * ko.nr + r], 1u);
+          if (wb >> 6) atomicAdd(&h_dec[2 * k + (wb >> 6) - 1], 1u);
         }
       }
     }
@@ -444,19 +494,30 @@ __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_cons
   if (sp.points_in_smem)
     for (int k = tid; k < NT * sp.B; k += kSimThreads)
       if (h_pts[k]) atomicAdd(&sp.pts_counts[k], (unsigned long long)h_pts[k]);
-  if constexpr (KO)
+  if constexpr (KO) {
     for (int k = tid; k < NT * ko.nr; k += kSimThreads) {
       if (h_reach[k]) atomicAdd(&ko.reach[k], (unsigned long long)h_reach[k]);
       if (h_win[k]) atomicAdd(&ko.win[k], (unsigned long long)h_win[k]);
     }
+    if (ko.decided) {
+      const unsigned valid = (unsigned)min(kSimThreads, sp.N - (int)blockIdx.x * kSimThreads) - s_invalid;
+      for (int k = tid; k < ko.K; k += kSimThreads) {
+        const unsigned et = h_dec[2 * k], ud = h_dec[2 * k + 1], nt = valid - et - ud;
+        if (nt) atomicAdd(&ko.decided[3 * k], (unsigned long long)nt);
+        if (et) atomicAdd(&ko.decided[3 * k + 1], (unsigned long long)et);
+        if (ud) atomicAdd(&ko.decided[3 * k + 2], (unsigned long long)ud);
+      }
+    }
+  }
   if (tid == 0 && s_invalid) atomicAdd(sp.invalid, (unsigned long long)s_invalid);
 }
 
 size_t simulate_smem_bytes(SimParams* sp) {
   size_t base = (size_t)sp->NT * kSimThreads * 16 + (size_t)sp->NT * sp->P * 4 + (size_t)sp->NT * 12;
   if (sp->ko.K > 0) {
-    // the reach / win histograms; the winner / loser bytes overlay s_gf and s_gd when they fit there (K <= 4 T_tab)
-    base += (size_t)sp->NT * sp->ko.nr * 8;
+    // the reach / win / decided histograms; the winner / loser bytes overlay s_gf and s_gd when they fit there (K <= 4
+    // T_tab)
+    base += (size_t)sp->NT * sp->ko.nr * 8 + (size_t)sp->ko.K * 8;
     sp->ko.wl_overlay = sp->ko.K <= 4 * sp->NT;
     if (!sp->ko.wl_overlay) base += (size_t)(2 * sp->ko.K + 3) / 4 * 4 * kSimThreads;
   }
@@ -494,6 +555,7 @@ static int launch_simulate_impl(SimParams& sp, cudaStream_t stream) {
   if (KO) {
     BPLX_CUDA(cudaMemsetAsync(sp.ko.reach, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
     BPLX_CUDA(cudaMemsetAsync(sp.ko.win, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
+    if (sp.ko.decided) BPLX_CUDA(cudaMemsetAsync(sp.ko.decided, 0, (size_t)sp.ko.K * 3 * 8, stream));
   }
   rc = launch_score_grid_tables(sp.gp, stream);
   if (rc != BPLX_OK) return rc;

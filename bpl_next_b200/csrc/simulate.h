@@ -18,12 +18,14 @@ struct KoParams {
   int wl_overlay;                 // the per-tie winner / loser bytes live in the dead s_gf / s_gd accumulators
   const uint8_t* alloc;           // device [2^ng][bc] allocation table or NULL (in the workspace)
   unsigned long long *reach, *win;  // [NT][nr]
-  uint8_t *entrants, *scores, *winners;  // [N][K][2], [N][K][2], [N][K] or NULL
+  unsigned long long* decided;    // [K][3] or NULL
+  uint8_t *entrants, *scores, *winners, *extra;  // [N][K][2], [N][K][2], [N][K], [N][K][4] or NULL
   uint8_t kind[2][kKoMaxTies];    // (home, away) entrant kinds: BPLX_ENTRANT_*
   uint8_t arg0[2][kKoMaxTies];    // slot / group / j / earlier tie
   uint8_t arg1[2][kKoMaxTies];    // position of GROUP_POS
   uint8_t round[kKoMaxTies];
   uint8_t neutral[kKoMaxTies];
+  uint8_t format[kKoMaxTies];     // BPLX_TIE_*
   uint16_t slot_team[kSimMaxTeams];
   uint8_t slot_conf[kSimMaxTeams];
 };

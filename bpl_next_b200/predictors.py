@@ -486,8 +486,8 @@ class _BplxPredictor:
         S, T, F = int(ds["attack"].shape[0]), len(table["teams"]), len(fx.get("home_team", ()))
         K = 0 if bracket is None else len(bracket["round"])
         step = (2 ** 31 - 1) // R  # simulations per call stay below 2^31
-        if return_simulations:  # bytes per simulation: positions, scores and the knockout entrants, scores, winners
-            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F + 5 * K))))
+        if return_simulations:  # bytes per simulation: positions, scores, the knockout entrants, scores, winners, extra
+            step = min(step, max(1, SIM_OUTPUT_BYTES // (R * (T + 2 * F + 9 * K))))
         if step < 1:
             raise ValueError(f"num_sims_per_draw={R} is too large for one draw per call")
         acc, invalid, raw = {}, 0, []
@@ -515,7 +515,8 @@ class _BplxPredictor:
                "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
                **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N)}
         if bracket is not None:
-            res.update(bseason.bracket_probabilities(bracket, cnt["reach_counts"], cnt["win_counts"], N))
+            res.update(bseason.bracket_probabilities(bracket, cnt["reach_counts"], cnt["win_counts"], N,
+                                                     cnt["decided_counts"]))
         res.update({"start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
                     "seed": seed})
         if return_simulations:
@@ -554,21 +555,35 @@ class _BplxPredictor:
         ``fixtures``, ``played``, ``teams``, ``groups``, ``points``, ``num_sims_per_draw``, ``random_state``,
         ``max_goals``: as ``simulate_table``; ``fixtures`` may be None or empty (a cup whose draw is made: the entrants
         are ``("team", name)``).  ``bracket``: the ties in play order, ``{"id", "round", "home", "away",
-        "neutral_venue"}``, entrants ``("group", label, position)``, ``("best", j)``, ``("winner", id)``,
+        "neutral_venue", "format"}``, entrants ``("group", label, position)``, ``("best", j)``, ``("winner", id)``,
         ``("loser", id)`` or ``("team", name)``; ``best``: the best-placed qualifiers, ``{"position", "count",
         "allocation"}`` (``season.build_bracket``).  ``team_conf`` (NeutralWC): team -> confederation, needed for the
         ties; inferred from the fixtures' confederations when they are consistent.
 
-        A tie is played like a group fixture from the draw's own grid.  A drawn tie goes to the home entrant with
-        probability ``hw_s / (hw_s + aw_s)``, the draw's own home and away win masses: the per-draw form of the
-        knockout renormalisation, which differs from ``predict_outcome_proba(knockout=True)`` (that renormalises after
-        averaging over the draws).  Extra time and penalties are not modelled; best-placed teams are ranked by points,
-        goal difference, goals for, then lot.
+        A tie's ``format`` is one of:
+
+        * ``"one_match"`` (default): one match, played like a group fixture from the draw's own grid.  A drawn tie goes
+          to the home entrant with probability ``hw_s / (hw_s + aw_s)``, the draw's own home and away win masses: the
+          per-draw form of the knockout renormalisation, which differs from ``predict_outcome_proba(knockout=True)``
+          (that renormalises after averaging over the draws).
+        * ``"extra_time"``: one match; if it is drawn, extra time is played at the same venue; if that is also level,
+          penalties.
+        * ``"two_legs"``: ``home`` hosts leg 1 and ``away`` hosts leg 2 with the venues swapped (never at a neutral
+          venue); the higher aggregate goes through (no away-goals rule); level on aggregate: extra time in leg 2, then
+          penalties.
+
+        Each leg is a 90-minute match from the draw's own grid.  Extra time uses the draw's rates times 1/3 (30 of 90
+        minutes at the model's constant rates) with no tau correction; the home entrant wins a shoot-out with
+        probability 1/2 (the model knows nothing of penalties).  Best-placed teams are ranked by points, goal
+        difference, goals for, then lot.
 
         Returns everything ``simulate_table`` returns, plus ``rounds`` (labels by first appearance), ``reach_proba`` /
-        ``win_proba [T, rounds]`` (the team plays / wins a tie of the round) and ``champion_proba [T]``.  With
-        ``return_simulations`` also ``positions [N, T]``, ``home_score`` / ``away_score [F, N]``, ``ko_entrants [N, K,
-        2]`` (table slots), ``ko_scores [N, K, 2]`` and ``ko_winners [N, K]``; the draws are then processed in ranges
+        ``win_proba [T, rounds]`` (the team plays / wins a tie of the round; a two-legged tie counts once),
+        ``champion_proba [T]``, ``tie_ids`` and ``decided_proba [K, 3]`` (tie k settled in normal time or on aggregate,
+        in extra time, or by penalties / the per-draw lot).  With ``return_simulations`` also ``positions [N, T]``,
+        ``home_score`` / ``away_score [F, N]``, ``ko_entrants [N, K, 2]`` (table slots), ``ko_scores [N, K, 2]`` (the
+        first or only match), ``ko_winners [N, K]`` and ``ko_extra [N, K, 4]`` (leg-2 goals of home and away entrant,
+        then their extra-time goals; 254 where not played); the draws are then processed in ranges
         within ``SIM_OUTPUT_BYTES`` and the results do not depend on the range size.  Raises if a simulation was invalid
         (a non-finite rate, or an allocation row the bracket does not cover)."""
         fixtures = fixtures if fixtures is not None and len(_str_to_list(fixtures["home_team"])[0]) else None

@@ -382,9 +382,19 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
     the decider of a drawn tie: the home entrant goes through iff ``u_d (hw_s + aw_s) <= hw_s`` with ``hw_s`` / ``aw_s``
     the draw's own home / away win masses, i.e. with probability ``hw_s / (hw_s + aw_s)`` per draw (the per-draw form of
     ``predict_outcome_proba(knockout=True)``, which renormalises after averaging over the draws).  Extra time and
-    penalties are not modelled.  Returns ``simulate_table``'s outputs plus ``reach_counts`` / ``win_counts`` (int64
-    ``[T_tab, num_rounds]``: ties of round r the slot played / won), and when ``want_knockout`` ``ko_entrants``,
-    ``ko_scores`` (uint8 ``[N, K, 2]``) and ``ko_winners`` (``[N, K]``); 255 marks an invalid simulation."""
+    penalties are not modelled in that format, ``_abi.TIE_ONE_MATCH``, the default.  ``bracket["tie_format"]`` (uint8
+    ``[K]``, optional) sets a format per tie: ``TIE_ONE_MATCH_ET`` (a drawn match goes to extra time, then penalties)
+    or ``TIE_TWO_LEGS`` (the away entrant B hosts leg 2 with the venues swapped; level on aggregate: extra time in leg
+    2, then penalties; no away-goals rule; never at a neutral venue).  Extra time is played at the venue of the last
+    match with the draw's rates times ``EXTRA_TIME_FRACTION`` = 1/3 and no tau correction; the home entrant A wins a
+    shoot-out iff ``u_d <= 1/2``.  Tie k's leg 2 and extra time use the Philox block ``E/4 + k``, ``E = 4 ceil((2F +
+    T_tab + 3K) / 4)`` (every word at a fixed address: a bracket of format-0 ties gives ``bplx_simulate_tournament``'s
+    outputs bit for bit).  Returns ``simulate_table``'s outputs plus ``reach_counts`` / ``win_counts`` (int64 ``[T_tab,
+    num_rounds]``: ties of round r the slot played / won; a two-legged tie counts once), ``decided_counts`` (int64
+    ``[K, 3]``: tie k settled in normal time or on aggregate / in extra time / by ``u_d``), and when ``want_knockout``
+    ``ko_entrants``, ``ko_scores`` (uint8 ``[N, K, 2]``, the first or only match), ``ko_winners`` (``[N, K]``) and
+    ``ko_extra`` (``[N, K, 4]``: leg-2 goals of A and B, then extra-time goals of A and B; 254 where not played); 255
+    marks an invalid simulation."""
     return _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw,
                      want_positions, want_scores, want_knockout, workspace, stream)
 
@@ -422,19 +432,30 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
            "points_counts": torch.empty((T_tab, t.num_points_bins), **i64)}
     if b is not None:
         out.update(reach_counts=torch.empty((T_tab, b.num_rounds), **i64),
-                   win_counts=torch.empty((T_tab, b.num_rounds), **i64))
+                   win_counts=torch.empty((T_tab, b.num_rounds), **i64),
+                   decided_counts=torch.empty((b.num_ties, 3), **i64))
     out.update(invalid=torch.empty(1, **i64), positions=torch.empty((N, T_tab), **u8) if want_positions else None,
                scores=torch.empty((N, F, 2), **u8) if want_scores else None)
     if b is not None:
         K = b.num_ties
         out.update(ko_entrants=torch.empty((N, K, 2), **u8) if want_knockout else None,
                    ko_scores=torch.empty((N, K, 2), **u8) if want_knockout else None,
-                   ko_winners=torch.empty((N, K), **u8) if want_knockout else None)
+                   ko_winners=torch.empty((N, K), **u8) if want_knockout else None,
+                   ko_extra=torch.empty((N, K, 4), **u8) if want_knockout else None)
     # the C functions take the outputs in the order of `out`, with `invalid` last
     outputs = [_dptr(v) for k, v in out.items() if k != "invalid"] + [_dptr(out["invalid"])]
     slots = (ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"])) if F else (None, None)
-    run = lib.bplx_simulate_table if b is None else lib.bplx_simulate_tournament
-    _abi.check(run(*structs[:2], *slots, *structs[2:], int(max_goals), int(sims_per_draw),
-                   int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw), *outputs, _dptr(workspace), workspace.numel(),
-                   _stream_ptr(stream)))
+    if b is None:
+        run, args = lib.bplx_simulate_table, structs[:2] + slots + structs[2:]
+    else:
+        fmt = bracket.get("tie_format")
+        if fmt is not None:
+            fmt = np.ascontiguousarray(fmt, dtype=np.uint8)
+            if fmt.shape != (b.num_ties,):
+                raise ValueError(f"tie_format has shape {fmt.shape}; the bracket has {b.num_ties} ties")
+            keep.append(fmt)
+        run, args = lib.bplx_simulate_tournament_ex, structs[:2] + slots + structs[2:] + (
+            None if fmt is None else fmt.ctypes.data,)
+    _abi.check(run(*args, int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
+                   *outputs, _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
     return out

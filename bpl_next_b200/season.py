@@ -16,7 +16,10 @@ from typing import Any, Dict, Optional, Sequence, Tuple
 import numpy as np
 
 from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_SLOT, ENTRANT_WINNER, KO_MAX_ALLOC_GROUPS,
-                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, SIM_MAX_TEAMS)
+                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, SIM_MAX_TEAMS, TIE_ONE_MATCH, TIE_ONE_MATCH_ET,
+                   TIE_TWO_LEGS)
+
+TIE_FORMATS = {"one_match": TIE_ONE_MATCH, "extra_time": TIE_ONE_MATCH_ET, "two_legs": TIE_TWO_LEGS}
 
 
 def _names(x) -> list:
@@ -153,7 +156,10 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
                   ) -> Dict[str, Any]:
     """The knockout bracket ``problem.simulate_tournament`` takes, from ties in play order.
 
-    Each tie is ``{"id", "round", "home", "away", "neutral_venue"}`` (``neutral_venue`` optional, default 0); an entrant
+    Each tie is ``{"id", "round", "home", "away", "neutral_venue", "format"}`` (``neutral_venue`` optional, default 0;
+    ``format`` optional: ``"one_match"`` (default: one match, a draw decided by the per-draw win masses),
+    ``"extra_time"`` (one match, then extra time and penalties) or ``"two_legs"`` (``home`` hosts leg 1, ``away`` leg
+    2; level on aggregate: extra time in leg 2, then penalties; not at a neutral venue)); an entrant
     is ``("group", label, position)`` (0-based position in the group; label None for a table without groups),
     ``("best", j)`` (the j-th best-placed qualifier), ``("winner", id)`` / ``("loser", id)`` of an earlier tie, or
     ``("team", name)`` (a table team already through).  Round labels are ordered by first appearance; the last tie is
@@ -161,7 +167,8 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
     {frozenset(group labels): [group label of BEST j for j < c]}}`` -- the best c of the teams placed p in their
     groups qualify, ranked across groups by points, goal difference, goals for, then lot; with an allocation every
     c-subset of the groups must have a row, and each row is a permutation of its subset.  ``slot_team`` / ``slot_conf``
-    are left to the caller (they need the model's team and confederation indices)."""
+    are left to the caller (they need the model's team and confederation indices).  ``tie_format`` holds the
+    ``_abi.TIE_*`` byte of every tie."""
     teams = list(table["teams"])
     slot = {t: i for i, t in enumerate(teams)}
     labels, sizes = _group_sizes(table)
@@ -183,6 +190,7 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
     arg1 = np.zeros((K, 2), np.uint8)
     rnd = np.zeros(K, np.uint8)
     nv = np.zeros(K, np.uint8)
+    fmt = np.zeros(K, np.uint8)
     for k, tie in enumerate(ties):
         tid = tie["id"]
         if tid in index:
@@ -191,6 +199,12 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
             rounds.append(tie["round"])
         rnd[k] = rounds.index(tie["round"])
         nv[k] = 1 if tie.get("neutral_venue", 0) else 0
+        f = tie.get("format", "one_match")
+        if f not in TIE_FORMATS:
+            raise ValueError(f"tie {tid!r}: unknown format {f!r} (one of {sorted(TIE_FORMATS)})")
+        fmt[k] = TIE_FORMATS[f]
+        if fmt[k] == TIE_TWO_LEGS and nv[k]:
+            raise ValueError(f"tie {tid!r}: a two-legged tie cannot be at a neutral venue")
         for side, key in enumerate(("home", "away")):
             e = tuple(tie[key])
             src = e
@@ -250,15 +264,18 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
             raise ValueError(f"the allocation has a row for {sorted(extra[0], key=str)}, not {bc} of the table's groups")
     return {"ids": [t["id"] for t in ties], "rounds": rounds, "num_rounds": len(rounds), "kind": kind, "arg0": arg0,
             "arg1": arg1, "round": rnd, "neutral_venue": nv, "num_groups": len(labels), "best_position": bp,
-            "best_count": bc, "best_alloc": best_alloc}
+            "best_count": bc, "best_alloc": best_alloc, "tie_format": fmt}
 
 
 def bracket_probabilities(bracket: Dict[str, Any], reach_counts: np.ndarray, win_counts: np.ndarray,
-                          num_simulations: int) -> Dict[str, np.ndarray]:
-    """Counts -> ``reach_proba`` / ``win_proba [T, rounds]`` (a team reaches / wins a tie of the round) and
-    ``champion_proba [T]`` (it wins the last tie)."""
+                          num_simulations: int, decided_counts: Optional[np.ndarray] = None) -> Dict[str, Any]:
+    """Counts -> ``reach_proba`` / ``win_proba [T, rounds]`` (a team reaches / wins a tie of the round),
+    ``champion_proba [T]`` (it wins the last tie), ``tie_ids`` and, from ``decided_counts``, ``decided_proba [K, 3]``
+    (tie k settled in normal time or on aggregate / in extra time / by the decider: penalties, or the per-draw lot of a
+    ``one_match`` tie)."""
     n = float(num_simulations)
     reach = np.asarray(reach_counts, np.float64) / n
     win = np.asarray(win_counts, np.float64) / n
     return {"rounds": list(bracket["rounds"]), "reach_proba": reach, "win_proba": win,
-            "champion_proba": win[:, int(bracket["round"][-1])].copy()}
+            "champion_proba": win[:, int(bracket["round"][-1])].copy(), "tie_ids": list(bracket["ids"]),
+            "decided_proba": None if decided_counts is None else np.asarray(decided_counts, np.float64) / n}

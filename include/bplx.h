@@ -350,19 +350,38 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
  * to the home entrant iff u_d (hw_s + aw_s) <= hw_s, hw_s = sum_{i > j} w(i, j) and aw_s = sum_{i < j} w(i, j) the
  * draw's own win masses on the same grid: P(home advances | draw s) = hw_s / (hw_s + aw_s), the per-draw form of the
  * knockout renormalisation of predict_outcome_proba(knockout=True), which renormalises AFTER averaging over the draws.
- * Extra time and penalties are not modelled (the model knows 90-minute scores only); two-legged ties are out of scope.
+ * That is tie format BPLX_TIE_ONE_MATCH; bplx_simulate_tournament_ex gives each tie a format byte:
+ *   0 BPLX_TIE_ONE_MATCH     one match; a draw is decided by u_d (hw_s + aw_s) <= hw_s (above)
+ *   1 BPLX_TIE_ONE_MATCH_ET  one match; drawn: extra time; still level: penalties
+ *   2 BPLX_TIE_TWO_LEGS      two legs; level on aggregate: extra time in leg 2; still level: penalties
+ * Legs: the home entrant A hosts leg 1, the away entrant B hosts leg 2 with the venues swapped (neutral_venue = 0 in
+ * both legs; NEUTRAL_WC: A's and B's confederations swap sides).  Each leg is a 90-minute match sampled like a group
+ * fixture (tau+ from the draw's own clamped, truncated grid).  Aggregate A = h1 + a2, B = a1 + h2; the higher goes
+ * through (no away-goals rule).  Extra time: at the venue of the last match (format 1: the tie's neutral flag
+ * included), the draw's rates times BPLX_EXTRA_TIME_FRACTION = 1/3 (30 of 90 minutes at the model's constant rates),
+ * no tau correction (tau is a 90-minute low-score term): independent Poissons truncated at G.  Penalties: A goes
+ * through iff u_d <= 1/2 (the model knows nothing of shoot-outs).  Neither constant is a parameter.
+ * Words: tie k keeps words 2F + T_tab + 3k, + 1 ((u_h, u_a) of its first or only match) and + 2 (u_d).  With
+ * E = 4 ceil((2F + T_tab + 3K) / 4), tie k owns words E + 4k .. E + 4k + 3: leg 2 (u_h, u_a), then extra time (u_h,
+ * u_a), i.e. the Philox4x32_10 block of counter E/4 + k.  Every word has a fixed address, used or not, so a bracket of
+ * format-0 ties reads exactly bplx_simulate_tournament's words and gives its outputs bit for bit.
  *
- * Invalid simulations (bplx_simulate_table's, and a tie with a non-finite rate or a bad normaliser, hw + aw not positive
- * on a drawn tie, a GROUP_POS beyond its group, fewer than best_count groups with a slot at best_position, or an
- * allocation entry of 0xFF) are counted in `invalid` and left out of every histogram; their positions, ko_entrants,
- * ko_scores and ko_winners rows are 0xFF.
+ * Invalid simulations (bplx_simulate_table's, and a tie with a non-finite rate or a bad normaliser in any of its
+ * matches or its extra time, hw + aw not positive on a drawn format-0 tie, a GROUP_POS beyond its group, fewer than
+ * best_count groups with a slot at best_position, or an allocation entry of 0xFF) are counted in `invalid` and left out
+ * of every histogram; their positions, ko_entrants, ko_scores, ko_winners and ko_extra rows are 0xFF.
  *
  * Outputs (device; integer counts, additive over draw ranges; overwritten): position_counts, points_counts and invalid
  * as bplx_simulate_table; reach_counts [T_tab, num_rounds]: ties of round r the slot played; win_counts [T_tab,
  * num_rounds]: ties of round r it won (the winner of the last tie is the champion).  Optional raw rows (NULL to skip):
- * positions [N, T_tab], scores [N, F, 2], ko_entrants [N, K, 2] (slots), ko_scores [N, K, 2], ko_winners [N, K].
+ * positions [N, T_tab], scores [N, F, 2], ko_entrants [N, K, 2] (slots), ko_scores [N, K, 2] (the first or only
+ * match, home and away), ko_winners [N, K].  A two-legged tie counts once in its round's reach / win counts.
+ * bplx_simulate_tournament_ex adds (NULL to skip): decided_counts [K, 3] (additive): how tie k was settled, in normal
+ * time or on aggregate / in extra time / by u_d (penalties, or the lot of format 0); ko_extra [N, K, 4] uint8: leg-2
+ * goals of (A, B), then extra-time goals of (A, B), in entrant order, 0xFE for a part not played.
  * Limits: K <= 64 ties, <= 16 rounds, best_count <= 16, num_groups <= 16 with an allocation table; T_tab <= 64 and
- * N < 2^31 per call as bplx_simulate_table; DYNAMIC: BPLX_E_UNSUPPORTED.
+ * N < 2^31 per call as bplx_simulate_table; DYNAMIC: BPLX_E_UNSUPPORTED; a format byte above 2, or format 2 on a tie
+ * with neutral_venue = 1: BPLX_E_INVALID.
  *
  * The bracket's arrays are HOST arrays: the call validates them (entrants reference earlier ties only, groups and
  * positions in range, BEST j < best_count, allocation entries are 0xFF or distinct groups of their mask) and passes
@@ -378,6 +397,10 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
 #define BPLX_ENTRANT_BEST 2
 #define BPLX_ENTRANT_WINNER 3
 #define BPLX_ENTRANT_LOSER 4
+#define BPLX_TIE_ONE_MATCH 0
+#define BPLX_TIE_ONE_MATCH_ET 1
+#define BPLX_TIE_TWO_LEGS 2
+#define BPLX_EXTRA_TIME_FRACTION (1.0 / 3.0)
 typedef struct {
   int32_t num_ties;               /* K, 1..64 */
   int32_t num_rounds;             /* 1..16 */
@@ -403,6 +426,18 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
                              unsigned long long* reach_counts, unsigned long long* win_counts, uint8_t* positions,
                              uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
                              unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream);
+/* bplx_simulate_tournament with a format per tie: tie_format is a HOST [K] array of BPLX_TIE_* (NULL: all
+ * BPLX_TIE_ONE_MATCH); decided_counts [K, 3] and ko_extra [N, K, 4] as above, or NULL.  bplx_simulate_tournament is
+ * this call with the three set to NULL; bplx_simulate_tournament_workspace_bytes serves both. */
+int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                const uint8_t* tie_format, int max_goals, int sims_per_draw, unsigned long long seed,
+                                long long first_draw, unsigned long long* position_counts,
+                                unsigned long long* points_counts, unsigned long long* reach_counts,
+                                unsigned long long* win_counts, unsigned long long* decided_counts, uint8_t* positions,
+                                uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
+                                uint8_t* ko_extra, unsigned long long* invalid, void* workspace,
+                                size_t workspace_bytes, void* stream);
 
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */

@@ -1027,7 +1027,7 @@ int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, c
                               static_cast<cudaStream_t>(stream)));
     sp.ko.alloc = dst;
   }
-  return launch_simulate_tournament(sp, static_cast<cudaStream_t>(stream));
+  return launch_simulate(sp, static_cast<cudaStream_t>(stream));
 }
 
 int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,

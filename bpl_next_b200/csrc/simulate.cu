@@ -161,7 +161,7 @@ __device__ __forceinline__ uint32_t philox_word(unsigned long long seed, unsigne
 }  // namespace
 
 // KO = false: season / group stage (bplx_simulate_table).  KO = true: the same group stage, then the knockout bracket
-// (bplx_simulate_tournament; see simulate_tournament_phase below).
+// (bplx_simulate_tournament / _ex).
 template <bool KO>
 __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_constant__ SimParams sp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -536,37 +536,36 @@ static int upload_sim_constants() {
   return BPLX_OK;
 }
 
-template <bool KO>
-static int launch_simulate_impl(SimParams& sp, cudaStream_t stream) {
+int launch_simulate(SimParams& sp, cudaStream_t stream) {
   int rc = upload_sim_constants();
   if (rc != BPLX_OK) return rc;
-  if (!KO) sp.ko.K = 0;
+  const bool ko = sp.ko.K > 0;
   const size_t smem = simulate_smem_bytes(&sp);
   BPLX_REQUIRE(smem <= (size_t)kSimSmemMax, BPLX_E_UNSUPPORTED,
                "simulate: %zu bytes of shared memory per CTA needed (max %d)", smem, kSimSmemMax);
-  static size_t smem_set = 48 * 1024;
-  if (smem > smem_set) {
-    BPLX_CUDA(cudaFuncSetAttribute(simulate_kernel<KO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_set = smem;
+  // the dynamic shared-memory limit is an attribute of each instantiation
+  static size_t smem_set[2] = {48 * 1024, 48 * 1024};
+  if (smem > smem_set[ko]) {
+    BPLX_CUDA(cudaFuncSetAttribute(ko ? simulate_kernel<true> : simulate_kernel<false>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    smem_set[ko] = smem;
   }
   BPLX_CUDA(cudaMemsetAsync(sp.pos_counts, 0, (size_t)sp.NT * sp.P * 8, stream));
   BPLX_CUDA(cudaMemsetAsync(sp.pts_counts, 0, (size_t)sp.NT * sp.B * 8, stream));
   BPLX_CUDA(cudaMemsetAsync(sp.invalid, 0, 8, stream));
-  if (KO) {
+  if (ko) {
     BPLX_CUDA(cudaMemsetAsync(sp.ko.reach, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
     BPLX_CUDA(cudaMemsetAsync(sp.ko.win, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
     if (sp.ko.decided) BPLX_CUDA(cudaMemsetAsync(sp.ko.decided, 0, (size_t)sp.ko.K * 3 * 8, stream));
   }
   rc = launch_score_grid_tables(sp.gp, stream);
   if (rc != BPLX_OK) return rc;
-  simulate_kernel<KO><<<(unsigned)((sp.N + kSimThreads - 1) / kSimThreads), kSimThreads, smem, stream>>>(sp);
+  const unsigned grid = (unsigned)((sp.N + kSimThreads - 1) / kSimThreads);
+  if (ko) simulate_kernel<true><<<grid, kSimThreads, smem, stream>>>(sp);
+  else simulate_kernel<false><<<grid, kSimThreads, smem, stream>>>(sp);
   BPLX_CUDA(cudaGetLastError());
   note_launch(1);
   return BPLX_OK;
 }
-
-int launch_simulate(SimParams& sp, cudaStream_t stream) { return launch_simulate_impl<false>(sp, stream); }
-
-int launch_simulate_tournament(SimParams& sp, cudaStream_t stream) { return launch_simulate_impl<true>(sp, stream); }
 
 }  // namespace bplx

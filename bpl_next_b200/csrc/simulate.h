@@ -50,8 +50,7 @@ struct SimParams {
 // shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
 // the tournament kernel (sets sp->ko.wl_overlay)
 size_t simulate_smem_bytes(SimParams* sp);
+// ko.K = 0: the group stage alone; ko.K >= 1: the tournament kernel, the same group stage, then the bracket of sp.ko
 int launch_simulate(SimParams& sp, cudaStream_t stream);
-// the tournament kernel: group stage as launch_simulate, then the bracket of sp.ko (ko.K >= 1)
-int launch_simulate_tournament(SimParams& sp, cudaStream_t stream);
 
 }  // namespace bplx

@@ -130,11 +130,15 @@ def tables(table, home_slot, away_slot, home, away):
 def rank_scores(table, home_slot, away_slot, home, away, keys, valid=None):
     """The ranking and histograms of given scores ``[n, F]`` with tie-break keys ``[n, T]``: ``positions [n, T]``
     (255 for invalid simulations), ``position_counts [T, P]``, ``points_counts [T, B]`` (gained points)."""
-    T = len(table["start_points"])
     n = np.asarray(home).shape[0]
     valid = np.ones(n, bool) if valid is None else np.asarray(valid, bool)
     pts, gd, gf = tables(table, home_slot, away_slot, np.where(valid[:, None], home, 0), np.where(valid[:, None], away, 0))
-    pos = rank(pts, gd, gf, keys, table.get("group"))
+    return histograms(table, pts, rank(pts, gd, gf, keys, table.get("group")), valid)
+
+
+def histograms(table, pts, pos, valid):
+    """``rank_scores``'s outputs from final points and positions ``[n, T]``, counting the simulations ``valid [n]``."""
+    T = len(table["start_points"])
     P, B = int(table["num_positions"]), int(table["num_points_bins"])
     pc = np.zeros((T, P), np.int64)
     bc = np.zeros((T, B), np.int64)
@@ -146,24 +150,26 @@ def rank_scores(table, home_slot, away_slot, home, away, keys, valid=None):
     return {"positions": pos, "position_counts": pc, "points_counts": bc}
 
 
-def simulate(model, samples, fixtures, home_slot, away_slot, table, max_goals, sims_per_draw, seed, first_draw=0):
-    """The simulations of draws ``samples`` (the call's range; ``first_draw`` is the global index of its first draw).
-    Returns ``home`` / ``away`` / ``margin`` ``[N, F]``, ``keys [N, T]``, ``valid [N]``, and ``rank_scores``'s
-    ``positions``, ``position_counts``, ``points_counts``, with ``invalid`` = the number of invalid simulations."""
+def philox_words(samples, sims_per_draw, seed, first_draw, count):
+    """Words ``0 .. count - 1`` of every simulation ``n = (first_draw + s) R + r`` (draw-major), ``[S R, count]``, and
+    the draw ``s`` of each simulation ``[S R]``."""
+    S, R = np.asarray(samples["attack"]).shape[0], int(sims_per_draw)
+    s_of = np.repeat(np.arange(S), R)
+    n_glob = (first_draw + s_of) * R + np.tile(np.arange(R), S)
+    return philox.stream(int(seed), n_glob.astype(np.uint64), 0, count), s_of
+
+
+def play_fixtures(model, samples, fixtures, home_slot, away_slot, T, max_goals, s_of, u):
+    """The fixtures of simulations of draws ``s_of [N]`` with uniforms ``u [N, 2F]`` (words ``2f``, ``2f + 1``):
+    ``home`` / ``away`` / ``margin [N, F]`` and ``valid [N]``; a fixture that makes its simulation invalid (a slot
+    outside the table of ``T`` slots included) has scores 255."""
     kw = {k: fixtures[k] for k in ("home_conf", "away_conf", "neutral_venue") if fixtures.get(k) is not None}
     if model in ("neutral", "neutral_wc") and "neutral_venue" not in kw:
         kw["neutral_venue"] = np.zeros(len(fixtures["home_team"]), np.uint8)
     with np.errstate(over="ignore", invalid="ignore"):
         lh, la = op.expected_goals(model, samples, fixtures["home_team"], fixtures["away_team"], **kw)  # [S, F]
     cc = np.asarray(samples["corr_coef"], np.float64)
-    S, F = lh.shape
-    T = len(table["start_points"])
-    R = int(sims_per_draw)
-    N = S * R
-    s_of = np.repeat(np.arange(S), R)
-    n_glob = (first_draw + s_of) * R + np.tile(np.arange(R), S)
-    words = philox.stream(int(seed), n_glob.astype(np.uint64), 0, 2 * F + T)  # [N, 2F + T]
-    u = philox.uniform(words[:, :2 * F]).astype(np.float64)
+    N, F = len(s_of), lh.shape[1]
     home = np.empty((N, F), np.int64)
     away = np.empty((N, F), np.int64)
     margin = np.empty((N, F))
@@ -174,7 +180,19 @@ def simulate(model, samples, fixtures, home_slot, away_slot, table, max_goals, s
         v &= (hs[f] < T) & (as_[f] < T)
         home[:, f], away[:, f], margin[:, f] = np.where(v, h, 255), np.where(v, a, 255), m
         valid &= v
+    return home, away, margin, valid
+
+
+def simulate(model, samples, fixtures, home_slot, away_slot, table, max_goals, sims_per_draw, seed, first_draw=0):
+    """The simulations of draws ``samples`` (the call's range; ``first_draw`` is the global index of its first draw).
+    Returns ``home`` / ``away`` / ``margin`` ``[N, F]``, ``keys [N, T]``, ``valid [N]``, and ``rank_scores``'s
+    ``positions``, ``position_counts``, ``points_counts``, with ``invalid`` = the number of invalid simulations."""
+    F, T = len(fixtures["home_team"]), len(table["start_points"])
+    words, s_of = philox_words(samples, sims_per_draw, seed, first_draw, 2 * F + T)  # [N, 2F + T]
+    home, away, margin, valid = play_fixtures(model, samples, fixtures, home_slot, away_slot, T, max_goals, s_of,
+                                              philox.uniform(words[:, :2 * F]).astype(np.float64))
     keys = words[:, 2 * F:].astype(np.int64)
-    out = rank_scores(table, np.minimum(hs, T - 1), np.minimum(as_, T - 1), home, away, keys, valid)
+    hs, as_ = np.minimum(np.asarray(home_slot, np.int64), T - 1), np.minimum(np.asarray(away_slot, np.int64), T - 1)
+    out = rank_scores(table, hs, as_, home, away, keys, valid)
     out.update(home=home, away=away, margin=margin, keys=keys, valid=valid, invalid=int((~valid).sum()))
     return out

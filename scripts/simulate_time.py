@@ -1,15 +1,17 @@
 """Times season / group-stage simulation (bplx_simulate_table) on one GPU.
 
-    python scripts/simulate_time.py [--samples 16384] [--reps 20] [--out FILE.json]
+    python scripts/simulate_time.py [--samples 16384] [--reps 20] [--baseline-lib OLD/libbplx.so] [--out FILE.json]
 
 Workloads (synthetic posterior draws, fixed seeds):
   league     20-team DixonColes league, F = 380 (a double round robin) and F = 190 (half a season), R = 64 and R = 1
   world cup  48-team group stage, 12 groups of four, 72 fixtures at neutral venues, NeutralWC draws of configs[5]'s shape
              (T = 220 model teams, Cf = 6), R = 64 and R = 1
-CUDA events around `--reps` calls after warm-up; a call is the whole entry point (count reset, exponential-table
-pre-pass, simulation kernel), issued straight through the C ABI so that no host synchronisation sits in the timed
-window.  Reports simulations/s and sampled scores/s, the GPU name and power limit read in the same run, and the float64
-oracle's CPU time on a few simulations of the league.
+With --baseline-lib, another build's bplx_simulate_table is timed on every workload, alternating with this build's, and
+its counts are checked equal.
+CUDA events around `--reps` calls after warm-up, best of three runs; a call is the whole entry point (count reset,
+exponential-table pre-pass, simulation kernel), issued straight through the C ABI so that no host synchronisation sits
+in the timed window.  Reports simulations/s and sampled scores/s, the GPU name and power limit read in the same run,
+and the float64 oracle's CPU time on a few simulations of the league.
 """
 from __future__ import annotations
 
@@ -88,13 +90,25 @@ def device_table(T_tab, group, hs, as_):
     return tab
 
 
-def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
-    """The bplx_simulate_table call with every argument built once; returns (call, outputs, keep-alive)."""
+def baseline_lib(path, names):
+    """Another build's libbplx.so, its entry points ``names`` typed as this build's."""
+    from bpl_next_b200 import _abi
+
+    lib = C.CDLL(os.path.abspath(path))
+    for name in names:
+        getattr(lib, name).argtypes = getattr(_abi.lib(), name).argtypes
+        getattr(lib, name).restype = getattr(_abi.lib(), name).restype
+    return lib
+
+
+def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1, lib=None):
+    """The bplx_simulate_table call with every argument built once; returns (call, outputs, keep-alive).  ``lib``:
+    another build's library (``baseline_lib``)."""
     import torch
 
     from bpl_next_b200 import _abi, problem
 
-    lib = _abi.lib()
+    lib = _abi.lib() if lib is None else lib
     keep = []
     ptr = problem._device_ptr_fn(keep)
     dev = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in s.items()}
@@ -114,7 +128,9 @@ def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1):
             ptr(ws), ws.numel(), stream)
 
     def call():
-        _abi.check(lib.bplx_simulate_table(*args))
+        rc = lib.bplx_simulate_table(*args)
+        if rc != _abi.OK:
+            raise _abi.BplxError(rc, lib.bplx_last_error().decode("utf-8", "replace"))
 
     return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, tab, ws)
 
@@ -134,6 +150,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--samples", type=int, default=16384)
     ap.add_argument("--reps", type=int, default=20)
+    ap.add_argument("--baseline-lib", default=None, help="another build's libbplx.so, timed on every workload")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
 
@@ -145,19 +162,37 @@ def main():
         raise SystemExit("simulate_time.py measures the GPU kernel and needs a CUDA device")
     S = a.samples
     rows = []
+    base = None
+    if a.baseline_lib:
+        base = baseline_lib(a.baseline_lib, ("bplx_simulate_table", "bplx_simulate_workspace_bytes", "bplx_last_error"))
     for name, make in (("league F=380", lambda: league(S, 380)), ("league F=190", lambda: league(S, 190)),
                        ("world cup groups", lambda: world_cup(S))):
         model, s, fx, hs, as_, T_tab, group = make()
         for R in (64, 1):
             call, out, _keep = prepared_call(model, s, fx, hs, as_, T_tab, group, R)
+            calls = [call]
+            if base is not None:
+                bcall, bout, _bk = prepared_call(model, s, fx, hs, as_, T_tab, group, R, lib=base)
+                calls.append(bcall)
             for _ in range(3):
-                call()
+                for c in calls:
+                    c()
             torch.cuda.synchronize()
             assert int(out["invalid"].item()) == 0
-            ms = time_ms(call, a.reps)
+            if base is not None:
+                for k in ("position_counts", "points_counts", "invalid"):
+                    assert torch.equal(out[k], bout[k]), k
+            ms_all = [[] for _ in calls]
+            for _ in range(3):  # alternate the builds
+                for c, m in zip(calls, ms_all):
+                    m.append(time_ms(c, a.reps))
+            ms = min(ms_all[0])
             N, F = S * R, len(hs)
             rows.append({"workload": name, "model": model, "S": S, "R": R, "N": N, "F": F, "T_tab": T_tab,
-                         "ms": ms, "sims_per_s": N / (ms * 1e-3), "scores_per_s": N * F / (ms * 1e-3)})
+                         "ms": ms, "ms_all": ms_all[0], "sims_per_s": N / (ms * 1e-3),
+                         "scores_per_s": N * F / (ms * 1e-3)})
+            if base is not None:
+                rows[-1].update(baseline_ms=min(ms_all[1]), baseline_ms_all=ms_all[1])
             print(json.dumps(rows[-1]), flush=True)
 
     # the float64 oracle on the CPU: 2 draws x 64 simulations of the F = 380 league

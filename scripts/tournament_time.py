@@ -39,7 +39,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
 sys.dont_write_bytecode = True
 
-from simulate_time import device_table, gpu_info, prepared_call, time_ms, world_cup  # noqa: E402
+from simulate_time import baseline_lib, device_table, gpu_info, prepared_call, time_ms, world_cup  # noqa: E402
 
 
 def _knockout(entrants):
@@ -196,12 +196,8 @@ def main():
     K = len(br["round"])
     base = None
     if a.baseline_lib:
-        from bpl_next_b200 import _abi
-
-        base = C.CDLL(os.path.abspath(a.baseline_lib))
-        for name in ("bplx_simulate_tournament", "bplx_simulate_tournament_workspace_bytes", "bplx_last_error"):
-            getattr(base, name).argtypes = getattr(_abi.lib(), name).argtypes
-            getattr(base, name).restype = getattr(_abi.lib(), name).restype
+        base = baseline_lib(a.baseline_lib, ("bplx_simulate_tournament", "bplx_simulate_tournament_workspace_bytes",
+                                             "bplx_last_error"))
     for R in (64, 1):
         gcall, gout, _gk = prepared_call(model, s, fx, hs, as_, T_tab, group, R)
         tcall, tout, _tk = tournament_call(model, s, fx, hs, as_, T_tab, group, br, R)

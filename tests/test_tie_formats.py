@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from bpl_next_b200 import _abi, season
-from tests import tie_format_oracle as oties
+from oracle import tournament
 from tests.test_score_grid_gpu import make_samples
 from tests.test_tournament import _euro
 
@@ -89,13 +89,13 @@ def test_resolve_bracket_by_hand():
     then D-C 0-3 (C through on aggregate, won in leg 2); third place A-D 1-1, A scores in extra time; final B-C 0-0,
     the lot to B.  The loser of the shoot-out, A, reaches the third-place match."""
     tab, b = _cup()
-    X = oties.NOT_PLAYED
+    X = tournament.NOT_PLAYED
     e = np.zeros((1, 0), np.int64)
     keys = np.zeros((1, 4), np.int64)
     ko_h, ko_a = np.array([[1, 0, 1, 0]]), np.array([[1, 2, 1, 0]])
     extra = np.array([[[2, 2, 0, 0], [3, 0, X, X], [X, X, 1, 0], [X, X, X, X]]])
     through = np.array([[0, 1, 1, 1]])  # read only where the tie is level after everything else
-    r = oties.resolve_bracket(tab, e[0], e[0], b, e, e, keys, ko_h, ko_a, through, ko_extra=extra)
+    r = tournament.resolve_bracket(tab, e[0], e[0], b, e, e, keys, ko_h, ko_a, through, ko_extra=extra)
     A, B, C_, D = range(4)
     np.testing.assert_array_equal(r["ko_entrants"][0], [[A, B], [C_, D], [A, D], [B, C_]])
     np.testing.assert_array_equal(r["ko_winners"][0], [B, C_, A, B])
@@ -105,16 +105,17 @@ def test_resolve_bracket_by_hand():
     np.testing.assert_array_equal(r["win_counts"], [[0, 1, 0], [1, 0, 1], [1, 0, 0], [0, 0, 0]])
     # the same scores, B losing the shoot-out instead: A goes through and meets C in the final
     through2 = np.array([[1, 1, 1, 1]])
-    r2 = oties.resolve_bracket(tab, e[0], e[0], b, e, e, keys, ko_h, ko_a, through2, ko_extra=extra)
+    r2 = tournament.resolve_bracket(tab, e[0], e[0], b, e, e, keys, ko_h, ko_a, through2, ko_extra=extra)
     np.testing.assert_array_equal(r2["ko_entrants"][0], [[A, B], [C_, D], [B, D], [A, C_]])
     # settle: a two-legged tie won on aggregate although its first leg was lost
-    th, how = oties.settle(oties.TWO_LEGS, np.array([0]), np.array([2]), np.array([[3, 0, X, X]]), np.array([False]))
+    th, how = tournament.settle(tournament.TWO_LEGS, np.array([0]), np.array([2]), np.array([[3, 0, X, X]]),
+                                np.array([False]))
     assert th[0] and how[0] == 0
 
 
-@pytest.mark.parametrize("model,fmt,neutral", [("dixon_coles", oties.TWO_LEGS, 0),
-                                               ("neutral_wc", oties.ONE_MATCH_ET, 1),
-                                               ("neutral", oties.TWO_LEGS, 0)])
+@pytest.mark.parametrize("model,fmt,neutral", [("dixon_coles", tournament.TWO_LEGS, 0),
+                                               ("neutral_wc", tournament.ONE_MATCH_ET, 1),
+                                               ("neutral", tournament.TWO_LEGS, 0)])
 def test_oracle_sampler_against_its_closed_form(model, fmt, neutral):
     """One tie at N = 2e5 (50 draws x 4,000): the oracle's shares of A through, extra time and penalties are within
     5 sigma of the mean over draws of ``tie_closed_form``; its decided counts add up to N."""
@@ -124,20 +125,20 @@ def test_oracle_sampler_against_its_closed_form(model, fmt, neutral):
     tab = season.build_table(["P", "Q"])
     season._size_histograms(tab)
     tie = {"id": "t", "round": "F", "home": ("team", "P"), "away": ("team", "Q"), "neutral_venue": neutral,
-           "format": {oties.ONE_MATCH_ET: "extra_time", oties.TWO_LEGS: "two_legs"}[fmt]}
+           "format": {tournament.ONE_MATCH_ET: "extra_time", tournament.TWO_LEGS: "two_legs"}[fmt]}
     br = season.build_bracket(tab, [tie])
     br["slot_team"] = np.array([2, 0], np.uint16)
     br["slot_conf"] = np.array([1, 2], np.uint8)
     e = np.zeros(0, np.uint8)
-    o = oties.simulate_tournament(model, s, None, e, e, tab, br, G, R, seed=5)
+    o = tournament.simulate_tournament(model, s, None, e, e, tab, br, G, R, seed=5)
     assert o["invalid"] == 0
     dec = o["decided_counts"][0]
     assert dec.sum() == N
-    p_through, p_et, p_pen = (x.mean() for x in oties.tie_closed_form(model, s, 2, 0, fmt, G, neutral, 1, 2))
+    p_through, p_et, p_pen = (x.mean() for x in tournament.tie_closed_form(model, s, 2, 0, fmt, G, neutral, 1, 2))
     for share, p in (((o["ko_winners"][:, 0] == 0).mean(), p_through), (dec[1:].sum() / N, p_et),
                      (dec[2] / N, p_pen)):
         assert abs(share - p) <= 5 * np.sqrt(p * (1 - p) / N), (share, p)
-    played = o["ko_extra"][:, 0, 2] != oties.NOT_PLAYED
+    played = o["ko_extra"][:, 0, 2] != tournament.NOT_PLAYED
     assert played.sum() == dec[1:].sum()
-    if fmt == oties.ONE_MATCH_ET:
-        assert (o["ko_extra"][:, 0, :2] == oties.NOT_PLAYED).all()
+    if fmt == tournament.ONE_MATCH_ET:
+        assert (o["ko_extra"][:, 0, :2] == tournament.NOT_PLAYED).all()

@@ -11,7 +11,7 @@ import pytest
 import torch
 
 from bpl_next_b200 import _abi, problem, season
-from tests import tie_format_oracle as oties
+from oracle import tournament
 from tests.test_score_grid_gpu import make_samples
 from tests.test_simulate_gpu import _dev, _dev_table
 from tests.test_tournament_gpu import REPLAY, _case, _raw_call, _run, _wc_predictor, _world_cup_48
@@ -85,7 +85,7 @@ def test_format_0_is_bitwise_the_legacy_call():
     assert old["invalid"][0] == 0
     for k, v in old.items():
         np.testing.assert_array_equal(new[k], v, err_msg=k)
-    assert (new["ko_extra"] == oties.NOT_PLAYED).all()
+    assert (new["ko_extra"] == tournament.NOT_PLAYED).all()
     d = new["decided_counts"]
     assert (d[:, 1] == 0).all() and (d.sum(axis=1) == S * R).all() and d[:, 2].sum() > 0
 
@@ -100,7 +100,7 @@ def test_exact_replay_with_formats(model, R, T_tab, grouped, best, F):
     s, fx, hs, as_, tab, br = _case(model, S, T_tab, grouped, F, seed, best=best)
     br = _mixed_formats(br)
     k = _run(model, s, fx, hs, as_, tab, br, 15, R, seed)
-    o = oties.simulate_tournament(model, s, fx if F else None, hs, as_, tab, br, 15, R, seed)
+    o = tournament.simulate_tournament(model, s, fx if F else None, hs, as_, tab, br, 15, R, seed)
     assert k["invalid"][0] == 0 and o["invalid"] == 0
     kh, ka = k["scores"][:, :, 0].astype(np.int64), k["scores"][:, :, 1].astype(np.int64)
     gdiff = (kh != o["home"]) | (ka != o["away"])
@@ -115,8 +115,8 @@ def test_exact_replay_with_formats(model, R, T_tab, grouped, best, F):
     assert gdiff.sum() <= max(1, 1e-3 * gdiff.size) and (diff | ~same_ent).sum() <= max(2, 1e-3 * diff.size)
     ent = kk["ko_entrants"]
     through = kk["ko_winners"] == ent[:, :, 0]
-    r = oties.resolve_bracket(tab, hs, as_, br, kh, ka, o["keys"], kk["ko_scores"][:, :, 0], kk["ko_scores"][:, :, 1],
-                             through, ko_extra=kk["ko_extra"])
+    r = tournament.resolve_bracket(tab, hs, as_, br, kh, ka, o["keys"], kk["ko_scores"][:, :, 0],
+                                   kk["ko_scores"][:, :, 1], through, ko_extra=kk["ko_extra"])
     for key in ("ko_entrants", "ko_winners", "ko_extra", "reach_counts", "win_counts", "decided_counts", "positions",
                 "position_counts", "points_counts"):
         np.testing.assert_array_equal(k[key], r[key], err_msg=key)
@@ -125,9 +125,9 @@ def test_exact_replay_with_formats(model, R, T_tab, grouped, best, F):
     assert (k["decided_counts"].sum(axis=1) == N).all()
     fmt = br["tie_format"]
     assert (k["decided_counts"][fmt == 0, 1] == 0).all()
-    assert (k["ko_extra"][:, fmt != 2, :2] == oties.NOT_PLAYED).all()
-    assert (k["ko_extra"][:, fmt == 0] == oties.NOT_PLAYED).all()
-    played = k["ko_extra"][:, :, 2] != oties.NOT_PLAYED
+    assert (k["ko_extra"][:, fmt != 2, :2] == tournament.NOT_PLAYED).all()
+    assert (k["ko_extra"][:, fmt == 0] == tournament.NOT_PLAYED).all()
+    played = k["ko_extra"][:, :, 2] != tournament.NOT_PLAYED
     np.testing.assert_array_equal(played.sum(axis=0), k["decided_counts"][:, 1:].sum(axis=1) * (fmt != 0))
 
 
@@ -168,11 +168,11 @@ def test_one_tie_against_the_closed_form(model, fmt, neutral):
     k = _run(model, s, {}, e, e, tab, br, G, R, seed=8)
     assert k["invalid"][0] == 0
     code = season.TIE_FORMATS[fmt]
-    p_through, p_et, p_pen = (x.mean() for x in oties.tie_closed_form(model, s, 3, 1, code, G, neutral, 2, 0))
+    p_through, p_et, p_pen = (x.mean() for x in tournament.tie_closed_form(model, s, 3, 1, code, G, neutral, 2, 0))
     d = k["decided_counts"][0]
     for share, p in (((k["ko_winners"][:, 0] == 0).mean(), p_through), (d[1:].sum() / N, p_et), (d[2] / N, p_pen)):
         assert abs(share - p) <= 5 * np.sqrt(p * (1 - p) / N), (share, p)
-    if code == oties.TWO_LEGS:
+    if code == tournament.TWO_LEGS:
         fx = {"home_team": np.array([1], np.uint16), "away_team": np.array([3], np.uint16)}
         grid, _ = score_grid(model, _dev(s), _dev(fx), G)
         pc = grid[0].double().cpu().numpy()
@@ -180,7 +180,7 @@ def test_one_tie_against_the_closed_form(model, fmt, neutral):
         counts = np.bincount(b_goals * 16 + a_goals, minlength=256).reshape(16, 16)
         assert (np.abs(counts - N * pc) <= 5 * np.sqrt(N * pc * (1 - pc)) + 1).all()
     else:
-        assert (k["ko_extra"][:, 0, :2] == oties.NOT_PLAYED).all()
+        assert (k["ko_extra"][:, 0, :2] == tournament.NOT_PLAYED).all()
 
 
 def _dc_predictor(T, S=256, seed=91):

@@ -10,7 +10,7 @@ import pytest
 from bpl_next_b200 import _abi, season
 from oracle import philox
 from oracle import simulate as osim
-from tests import tournament_oracle as otour
+from oracle import tournament
 
 
 def _groups(n_groups, size=4):
@@ -125,7 +125,7 @@ def test_best_placed_ranking_and_allocation_lookup():
     """Six groups of four, the four best thirds: the oracle's pool ranking by brute force over the thirds, and BEST j
     = the third of group alloc[mask][j] with the generated 15-row table."""
     tab, b, pts, gd, gf, keys, pos = _euro_case(1)
-    qmap, best, ok = otour.qualifiers(tab, b, pts, gd, gf, keys, pos)
+    qmap, best, ok = tournament.qualifiers(tab, b, pts, gd, gf, keys, pos)
     assert ok.all()
     group = tab["group"].astype(np.int64)
     for i in range(pts.shape[0]):
@@ -141,7 +141,7 @@ def test_best_placed_ranking_and_allocation_lookup():
                 assert pos[i, qmap[i, g, p]] == p and group[qmap[i, g, p]] == g
     # without an allocation, BEST j is the j-th best third
     nb = dict(b, best_alloc=None)
-    _, best2, ok2 = otour.qualifiers(tab, nb, pts, gd, gf, keys, pos)
+    _, best2, ok2 = tournament.qualifiers(tab, nb, pts, gd, gf, keys, pos)
     i = 0
     thirds = [int(np.flatnonzero((group == g) & (pos[i] == 2))[0]) for g in range(6)]
     order = sorted(thirds, key=lambda t: (-pts[i, t], -gd[i, t], -gf[i, t], -keys[i, t], t))
@@ -149,7 +149,7 @@ def test_best_placed_ranking_and_allocation_lookup():
     # an allocation row of 0xFF makes the simulation invalid
     bad = dict(b, best_alloc=b["best_alloc"].copy())
     bad["best_alloc"][:] = 255
-    assert not otour.qualifiers(tab, bad, pts, gd, gf, keys, pos)[2].any()
+    assert not tournament.qualifiers(tab, bad, pts, gd, gf, keys, pos)[2].any()
 
 
 @pytest.mark.parametrize("lh,la,c", [(1.6, 1.1, -0.12), (0.4, 2.7, 0.3), (1.0, 1.0, 0.0), (0.2, 0.3, 5.0)])
@@ -159,7 +159,7 @@ def test_decider_against_the_exact_per_draw_ratio(lh, la, c):
     from oracle import predict as op
 
     G = 15
-    hw, aw = otour.win_masses(np.array([lh]), np.array([la]), np.array([c]), G)
+    hw, aw = tournament.win_masses(np.array([lh]), np.array([la]), np.array([c]), G)
     samples = {"attack": np.array([[np.log(lh), np.log(la)]]), "defence": np.zeros((1, 2)),
                "home_advantage": np.zeros(1), "corr_coef": np.array([c])}
     grid, _, _ = op.predict_score_grid_proba("dixon_coles", samples, [0], [1], G)
@@ -196,8 +196,8 @@ def test_resolve_bracket_by_hand():
     ko_h = np.array([[1, 0, 3, 2, 0]])
     ko_a = np.array([[1, 2, 0, 2, 1]])
     through = np.array([[1, 0, 0, 0, 0]])
-    r = otour.resolve_bracket(dict(tab, num_positions=3, num_points_bins=7), hs, as_, b, home, away, keys, ko_h, ko_a,
-                             through)
+    r = tournament.resolve_bracket(dict(tab, num_positions=3, num_points_bins=7), hs, as_, b, home, away, keys, ko_h,
+                                   ko_a, through)
     slot = {t: i for i, t in enumerate(teams)}
     e = [[slot[x] for x in pair] for pair in (("X", "B0"), ("A0", "B2"), ("B1", "X"), ("A0", "X"), ("B2", "B1"))]
     np.testing.assert_array_equal(r["ko_entrants"][0], e)

@@ -1,5 +1,5 @@
-"""Tournament simulation on the GPU: the kernel replayed exactly by the float64 oracle (tests/tournament_oracle.py) on the same
-Philox words, the group stage bit-identical to bplx_simulate_table, draw ranges and seeds, the decider and the tie
+"""Tournament simulation on the GPU: the kernel replayed exactly by the float64 oracle (oracle/tournament.py) on the
+same Philox words, the group stage bit-identical to bplx_simulate_table, draw ranges and seeds, the decider and the tie
 scores against the per-draw grids, a knockout-only bracket, the 48-team World Cup format through the predictor, and
 refusals."""
 import ctypes as C
@@ -11,7 +11,7 @@ import torch
 
 from bpl_next_b200 import _abi, season
 from oracle import predict as op
-from tests import tournament_oracle as otour
+from oracle import tournament
 from tests.test_score_grid_gpu import make_samples
 from tests.test_simulate_gpu import _dev, _dev_table
 
@@ -113,7 +113,7 @@ def test_exact_replay(model, R, T_tab, grouped, best, F):
     S, seed = 149, 2000 + R * 100 + T_tab + F
     s, fx, hs, as_, tab, br = _case(model, S, T_tab, grouped, F, seed, best=best)
     k = _run(model, s, fx, hs, as_, tab, br, 15, R, seed)
-    o = otour.simulate_tournament(model, s, fx if F else None, hs, as_, tab, br, 15, R, seed)
+    o = tournament.simulate_tournament(model, s, fx if F else None, hs, as_, tab, br, 15, R, seed)
     assert k["invalid"][0] == 0 and o["invalid"] == 0
     kh, ka = k["scores"][:, :, 0].astype(np.int64), k["scores"][:, :, 1].astype(np.int64)
     gdiff = (kh != o["home"]) | (ka != o["away"])
@@ -127,8 +127,8 @@ def test_exact_replay(model, R, T_tab, grouped, best, F):
     assert gdiff.sum() <= max(1, 1e-3 * gdiff.size) and (diff | ~same_ent).sum() <= max(2, 1e-3 * diff.size)
     ent = kk["ko_entrants"]
     through = kk["ko_winners"] == ent[:, :, 0]
-    r = otour.resolve_bracket(tab, hs, as_, br, kh, ka, o["keys"], kk["ko_scores"][:, :, 0], kk["ko_scores"][:, :, 1],
-                             through)
+    r = tournament.resolve_bracket(tab, hs, as_, br, kh, ka, o["keys"], kk["ko_scores"][:, :, 0],
+                                   kk["ko_scores"][:, :, 1], through)
     for key in ("ko_entrants", "ko_winners", "reach_counts", "win_counts", "positions", "position_counts",
                 "points_counts"):
         np.testing.assert_array_equal(k[key], r[key], err_msg=key)
@@ -189,7 +189,7 @@ def test_one_neutral_tie_against_the_per_draw_grids():
           "neutral_venue": np.array([1], np.uint8)}
     lh, la = op.expected_goals("neutral_wc", s, fx["home_team"], fx["away_team"], home_conf=fx["home_conf"],
                                away_conf=fx["away_conf"], neutral_venue=fx["neutral_venue"])
-    hw, aw = otour.win_masses(lh[:, 0], la[:, 0], s["corr_coef"].astype(np.float64), 15)
+    hw, aw = tournament.win_masses(lh[:, 0], la[:, 0], s["corr_coef"].astype(np.float64), 15)
     p = (hw / (hw + aw)).mean()
     share = (k["ko_winners"][:, 0] == 0).mean()
     assert abs(share - p) <= 5 * np.sqrt(p * (1 - p) / N), (share, p)

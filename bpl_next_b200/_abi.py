@@ -76,6 +76,10 @@ class Bracket(C.Structure):
     ]
 
 
+class Ranking(C.Structure):
+    _fields_ = [("rule", C.c_int32), ("played_h2h", C.c_void_p)]
+
+
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
@@ -84,6 +88,8 @@ ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0
 # BPLX_TIE_*, BPLX_EXTRA_TIME_FRACTION
 TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS = 0, 1, 2
 EXTRA_TIME_FRACTION = 1.0 / 3.0
+# BPLX_RANK_*
+RANK_GOAL_DIFF, RANK_HEAD_TO_HEAD = 0, 1
 
 
 class BplxError(RuntimeError):
@@ -152,6 +158,22 @@ def declare(lib):
                                                 C.POINTER(Bracket), vp, i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp,
                                                 vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     lib.bplx_simulate_tournament_ex.restype = i
+    lib.bplx_simulate_table_ex_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), C.POINTER(Table),
+                                                           C.POINTER(Ranking)]
+    lib.bplx_simulate_table_ex_workspace_bytes.restype = sz
+    lib.bplx_simulate_table_ex.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                           C.POINTER(Ranking), i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp,
+                                           vp, sz, vp]
+    lib.bplx_simulate_table_ex.restype = i
+    lib.bplx_simulate_tournament_ranked_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures),
+                                                                    C.POINTER(Table), C.POINTER(Bracket),
+                                                                    C.POINTER(Ranking)]
+    lib.bplx_simulate_tournament_ranked_workspace_bytes.restype = sz
+    lib.bplx_simulate_tournament_ranked.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                                    C.POINTER(Bracket), vp, C.POINTER(Ranking), i, i, C.c_ulonglong,
+                                                    C.c_longlong, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                                                    sz, vp]
+    lib.bplx_simulate_tournament_ranked.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

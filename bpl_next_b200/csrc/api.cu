@@ -867,18 +867,81 @@ static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const u
   return BPLX_OK;
 }
 
+// ---- ranking rules --------------------------------------------------------------------------------------------
+static bool head_to_head(const bplx_ranking* r) { return r && r->rule == BPLX_RANK_HEAD_TO_HEAD; }
+
+// workspace bytes the ranking adds after `base` (256-aligned): head-to-head keeps the played matrix [NT][NT] int2, the
+// pair offsets [NT NT + 1] and the pair fixture list [F]
+static size_t ranking_bytes(const bplx_ranking* r, int NT, int F) {
+  if (!head_to_head(r)) return 0;
+  const size_t nn = (size_t)NT * NT;
+  return (nn * 8 + 255) / 256 * 256 + ((nn + 1) * 4 + 255) / 256 * 256 + ((size_t)(F > 0 ? F : 1) * 4 + 255) / 256 * 256;
+}
+
+static int check_ranking(const bplx_ranking* r, int NT, const char* what) {
+  if (!r) return BPLX_OK;
+  BPLX_REQUIRE(r->rule == BPLX_RANK_GOAL_DIFF || r->rule == BPLX_RANK_HEAD_TO_HEAD, BPLX_E_INVALID,
+               "%s: ranking rule %d is not a BPLX_RANK_* value", what, r->rule);
+  if (head_to_head(r) && r->played_h2h)
+    for (int k = 0; k < NT * NT * 2; k++)
+      BPLX_REQUIRE(r->played_h2h[k] >= 0, BPLX_E_INVALID,
+                   "%s: played_h2h (%d, %d) has a negative %s (%d)", what, k / 2 / NT, k / 2 % NT,
+                   k % 2 ? "goal count" : "points count", r->played_h2h[k]);
+  return BPLX_OK;
+}
+
+// fills the head-to-head fields of *sp from the workspace region at `base` (the played matrix is copied there)
+static int bind_ranking(const bplx_ranking* r, void* workspace, size_t base, SimParams* sp, cudaStream_t stream) {
+  sp->rule = r ? r->rule : BPLX_RANK_GOAL_DIFF;
+  if (!head_to_head(r)) return BPLX_OK;
+  const size_t nn = (size_t)sp->NT * sp->NT;
+  unsigned char* p = static_cast<unsigned char*>(workspace) + base;
+  if (r->played_h2h) {
+    BPLX_CUDA(cudaMemcpyAsync(p, r->played_h2h, nn * 8, cudaMemcpyHostToDevice, stream));
+    sp->h2h_played = reinterpret_cast<const int2*>(p);
+  }
+  p += (nn * 8 + 255) / 256 * 256;
+  sp->pair_beg = reinterpret_cast<int*>(p);
+  sp->pair_fix = reinterpret_cast<int*>(p + ((nn + 1) * 4 + 255) / 256 * 256);
+  return BPLX_OK;
+}
+
+size_t bplx_simulate_table_ex_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
+                                              const bplx_ranking* r) {
+  const size_t base = bplx_simulate_workspace_bytes(s, f, t);
+  if (!base || (r && r->rule != BPLX_RANK_GOAL_DIFF && r->rule != BPLX_RANK_HEAD_TO_HEAD)) return 0;
+  if (t->num_slots < 1 || t->num_slots > BPLX_SIM_MAX_TEAMS) return head_to_head(r) ? 0 : base;
+  return base + ranking_bytes(r, t->num_slots, f->num_fixtures);
+}
+
 int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
                         const bplx_table* t, int max_goals, int sims_per_draw, unsigned long long seed,
                         long long first_draw, unsigned long long* position_counts, unsigned long long* points_counts,
                         uint8_t* positions, uint8_t* scores, unsigned long long* invalid, void* workspace,
                         size_t workspace_bytes, void* stream) {
+  return bplx_simulate_table_ex(s, f, home_slot, away_slot, t, nullptr, max_goals, sims_per_draw, seed, first_draw,
+                                position_counts, points_counts, positions, scores, invalid, workspace, workspace_bytes,
+                                stream);
+}
+
+int bplx_simulate_table_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                           const uint8_t* away_slot, const bplx_table* t, const bplx_ranking* r, int max_goals,
+                           int sims_per_draw, unsigned long long seed, long long first_draw,
+                           unsigned long long* position_counts, unsigned long long* points_counts, uint8_t* positions,
+                           uint8_t* scores, unsigned long long* invalid, void* workspace, size_t workspace_bytes,
+                           void* stream) {
   SimParams sp{};
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "simulate", false, &sp);
   if (rc != BPLX_OK) return rc;
-  rc = check_workspace(workspace, workspace_bytes, simulate_plan_for(s, f, &sp));
+  rc = check_ranking(r, t->num_slots, "simulate");
+  if (rc != BPLX_OK) return rc;
+  const size_t table = simulate_plan_for(s, f, &sp);
+  rc = check_workspace(workspace, workspace_bytes, table + ranking_bytes(r, t->num_slots, f->num_fixtures));
   if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
+  rc = bind_ranking(r, workspace, table, &sp, static_cast<cudaStream_t>(stream));
+  if (rc != BPLX_OK) return rc;
   return launch_simulate(sp, static_cast<cudaStream_t>(stream));
 }
 
@@ -994,6 +1057,15 @@ static int check_bracket(const bplx_bracket* b, const uint8_t* tie_format, const
   return BPLX_OK;
 }
 
+size_t bplx_simulate_tournament_ranked_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f,
+                                                       const bplx_table* t, const bplx_bracket* b,
+                                                       const bplx_ranking* r) {
+  const size_t base = bplx_simulate_tournament_workspace_bytes(s, f, t, b);
+  if (!base || (r && r->rule != BPLX_RANK_GOAL_DIFF && r->rule != BPLX_RANK_HEAD_TO_HEAD)) return 0;
+  if (t->num_slots < 1 || t->num_slots > BPLX_SIM_MAX_TEAMS) return head_to_head(r) ? 0 : base;
+  return base + ranking_bytes(r, t->num_slots, f->num_fixtures);
+}
+
 int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
                                 const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
                                 const uint8_t* tie_format, int max_goals, int sims_per_draw, unsigned long long seed,
@@ -1003,6 +1075,21 @@ int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, c
                                 uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
                                 uint8_t* ko_extra, unsigned long long* invalid, void* workspace,
                                 size_t workspace_bytes, void* stream) {
+  return bplx_simulate_tournament_ranked(s, f, home_slot, away_slot, t, b, tie_format, nullptr, max_goals,
+                                         sims_per_draw, seed, first_draw, position_counts, points_counts, reach_counts,
+                                         win_counts, decided_counts, positions, scores, ko_entrants, ko_scores,
+                                         ko_winners, ko_extra, invalid, workspace, workspace_bytes, stream);
+}
+
+int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                    const uint8_t* tie_format, const bplx_ranking* r, int max_goals, int sims_per_draw,
+                                    unsigned long long seed, long long first_draw, unsigned long long* position_counts,
+                                    unsigned long long* points_counts, unsigned long long* reach_counts,
+                                    unsigned long long* win_counts, unsigned long long* decided_counts,
+                                    uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
+                                    uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
+                                    void* workspace, size_t workspace_bytes, void* stream) {
   SimParams sp{};
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "tournament", true, &sp);
@@ -1010,8 +1097,12 @@ int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, c
   rc = check_bracket(b, tie_format, s, t->num_slots, t->num_positions, &sp.ko);
   if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
-  const size_t table = simulate_plan_for(s, f, &sp);
-  rc = check_workspace(workspace, workspace_bytes, table + (alloc_bytes(b) + 255) / 256 * 256);
+  rc = check_ranking(r, t->num_slots, "tournament");
+  if (rc != BPLX_OK) return rc;
+  const size_t table = simulate_plan_for(s, f, &sp), alloc = (alloc_bytes(b) + 255) / 256 * 256;
+  rc = check_workspace(workspace, workspace_bytes, table + alloc + ranking_bytes(r, t->num_slots, f->num_fixtures));
+  if (rc != BPLX_OK) return rc;
+  rc = bind_ranking(r, workspace, table + alloc, &sp, static_cast<cudaStream_t>(stream));
   if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
   sp.ko.reach = reach_counts;

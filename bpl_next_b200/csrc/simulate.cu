@@ -15,7 +15,10 @@
 //   Table: points_win for a win, points_draw for a draw, goal difference and goals for added to the starting table.
 //   Teams are ranked within their group by points, goal difference, goals for, then the tie-break key, all descending,
 //   and the lower slot when even the keys are equal; position k (0-based) = the number of teams of the group ranked
-//   ahead.  Head-to-head and fair-play rules are not modelled: ties left after goals for are decided by lot.
+//   ahead.  That is BPLX_RANK_GOAL_DIFF; under BPLX_RANK_HEAD_TO_HEAD (simulate_h2h_kernel) a set of teams level on
+//   points is ordered by the points, goal difference and goals for of the matches among them (played and simulated),
+//   the parts still level again by the matches among themselves, and a set that this separates nobody in by goal
+//   difference, goals for, the key, then the lower slot.  Fair-play rules are not modelled.
 //   A simulation with a non-finite rate, a normaliser that is not positive and finite, or a slot outside the table is
 //   invalid: counted in `invalid`, left out of the histograms, its positions row 0xFF and that fixture's scores 0xFF.
 //
@@ -160,356 +163,208 @@ __device__ __forceinline__ uint32_t philox_word(unsigned long long seed, unsigne
 
 }  // namespace
 
-// KO = false: season / group stage (bplx_simulate_table).  KO = true: the same group stage, then the knockout bracket
-// (bplx_simulate_tournament / _ex).
-template <bool KO>
-__global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_constant__ SimParams sp) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
+// Head-to-head ranking of every group of a valid simulation into k_q (k_q[gbeg + position] = slot).  Each group
+// is sorted by points; bit 7 of a k_q byte marks the first position of a class of teams still level, bit 6 a class
+// whose head-to-head separates nobody.  A class of two or more is sorted by the points, goal difference and goals
+// for of the matches among its members (played, then this simulation's fixtures, re-sampled from their own Philox
+// words: the scores that built the table); the parts still level become classes and go through that again.  A
+// class that is not separated is sorted by goal difference, goals for, the key (word 2F + t), then the lower slot.
+__device__ __forceinline__ void rank_head_to_head(const SimParams& sp, int tid, unsigned long long n, const RowLayout& L,
+                                                  const float* row, float c, bool wc, const int* s_pts, const int* s_gf,
+                                                  const int* s_gd, const int* s_members, const int* s_gcnt,
+                                                  uint8_t* k_q) {
   const GridParams& gp = sp.gp;
-  const KoParams& ko = sp.ko;
-  const int NT = sp.NT, tid = threadIdx.x;
-  // [slot][thread] accumulators, then the histograms, then the group member lists
-  int* const s_pts = reinterpret_cast<int*>(smem_raw);
-  int* const s_gf = s_pts + NT * kSimThreads;
-  int* const s_gd = s_gf + NT * kSimThreads;  // goals against during the fixtures, goal difference for the ranking
-  uint32_t* const s_key = reinterpret_cast<uint32_t*>(s_gd + NT * kSimThreads);
-  unsigned* const h_pos = s_key + NT * kSimThreads;
-  unsigned* const h_pts = h_pos + NT * sp.P;
-  unsigned* const h_reach = h_pts + (sp.points_in_smem ? NT * sp.B : 0);  // tournament: [NT][nr] each
-  unsigned* const h_win = h_reach + (KO ? NT * ko.nr : 0);
-  // tournament: [K][2] ties settled in extra time / by u_d (the rest of the CTA's valid simulations: in normal time)
-  unsigned* const h_dec = h_win + (KO ? NT * ko.nr : 0);
-  int* const s_members = reinterpret_cast<int*>(h_dec + (KO ? 2 * ko.K : 0));
-  int* const s_gbeg = s_members + NT;
-  int* const s_gcnt = s_gbeg + NT;
-  // Tournament: the keys are not stored (philox_word reads one when it is needed), so the s_key words hold bytes:
-  // k_q [NT][thread] = the slot ranked p-th in its group at member index gbeg + p, k_best [bc][thread] = the slot of
-  // BEST j, k_gtab = per CTA, first member index [ng] and size [ng] of each group id.  The per-tie winner / loser bytes
-  // go into the thread's OWN s_gf / s_gd words once its ranking and best-placed selection are done (byte b in byte
-  // b % 4 of word [b / 4][thread], so a thread that reaches its ties early never touches the words another thread is
-  // still ranking), or after the member lists when 2K bytes exceed those 2 T_tab words.  A slot fits 6 bits (T_tab <=
-  // 64): bits 6-7 of the winner byte hold how the tie was decided until the histograms are committed.
-  uint8_t* const k_q = reinterpret_cast<uint8_t*>(s_key);
-  uint8_t* const k_best = k_q + NT * kSimThreads;
-  uint8_t* const k_gtab = k_best + (KO ? ko.bc : 0) * kSimThreads;
-  uint8_t* const k_wl = KO && !ko.wl_overlay ? reinterpret_cast<uint8_t*>(s_gcnt + NT) : reinterpret_cast<uint8_t*>(s_gf);
-  __shared__ unsigned s_invalid;
-  __shared__ int s_groups_fit;
+  const int NT = sp.NT;
 #define ACC(arr, t) arr[(t) * kSimThreads + tid]
 #define BYTE(arr, k) arr[(k) * kSimThreads + tid]
-#define WL(b) k_wl[(((b) >> 2) * kSimThreads + tid) * 4 + ((b) & 3)]
-
-  if (tid == 0) {
-    s_invalid = 0;
-    s_groups_fit = 1;
-  }
-  for (int k = tid; k < NT * sp.P; k += kSimThreads) h_pos[k] = 0;
-  if (sp.points_in_smem)
-    for (int k = tid; k < NT * sp.B; k += kSimThreads) h_pts[k] = 0;
-  if constexpr (KO) {
-    for (int k = tid; k < 2 * (NT * ko.nr + ko.K); k += kSimThreads) h_reach[k] = 0;  // h_win, h_dec follow
-    for (int g = tid; g < ko.ng; g += kSimThreads) {
-      int beg = 0, cnt = 0;
-      for (int u = 0; u < NT; u++) {
-        const int gu = sp.group ? sp.group[u] : 0;
-        beg += gu < g;
-        cnt += gu == g;
+  // fixture f's score again: words 2f, 2f + 1 are the (x, y) or (z, w) pair of Philox block f / 2
+  auto rescore = [&](int f, int& hg, int& ag) {
+    const uint4 w = philox_block(sp.seed, n, (unsigned)f >> 1);
+    const bool neutral = gp.ntab == 3 && gp.nv && gp.nv[f];
+    const FixtureOffsets off =
+        fixture_offsets(L, gp.home[f], gp.away[f], neutral, wc, wc ? gp.hconf[f] : 0, wc ? gp.aconf[f] : 0);
+    const float2 lam = fixture_rates(row, off, neutral, wc);
+    sample_score(lam.x, lam.y, c, _curand_uniform(f & 1 ? w.z : w.x), _curand_uniform(f & 1 ? w.w : w.y), sp.G,
+                 hg, ag);
+  };
+  // head-to-head points, goal difference and goals for of slot x against the other members of the class [a, b)
+  auto h2h = [&](int x, int a, int b, int& hp, int& hd, int& hf) {
+    hp = hd = hf = 0;
+    for (int q = a; q < b; q++) {
+      const int y = BYTE(k_q, q) & 63;
+      if (y == x) continue;
+      if (sp.h2h_played) {
+        const int2 xy = sp.h2h_played[x * NT + y], yx = sp.h2h_played[y * NT + x];
+        hp += xy.x;
+        hf += xy.y;
+        hd += xy.y - yx.y;
       }
-      k_gtab[g] = (uint8_t)beg;
-      k_gtab[ko.ng + g] = (uint8_t)cnt;
-    }
-  }
-  __syncthreads();
-  // group member lists: slots sorted by (group, slot); s_gbeg / s_gcnt = where a slot's group starts and its size
-  for (int t = tid; t < NT; t += kSimThreads) {
-    const int g = sp.group ? sp.group[t] : 0;
-    int beg = 0, before = 0, cnt = 0;
-    for (int u = 0; u < NT; u++) {
-      const int gu = sp.group ? sp.group[u] : 0;
-      beg += gu < g;
-      cnt += gu == g;
-      before += gu == g && u < t;
-    }
-    s_members[beg + before] = t;
-    s_gbeg[t] = beg;
-    s_gcnt[t] = cnt;
-    if (cnt > sp.P) s_groups_fit = 0;
-  }
-  __syncthreads();
-
-  const int i = blockIdx.x * kSimThreads + tid;  // (N < 2^31 per call)
-  if (i < sp.N) {
-    const int s = i / sp.R, r = i - s * sp.R;
-    const unsigned long long n = (unsigned long long)(sp.first_draw + s) * (unsigned long long)sp.R + (unsigned)r;
-    curandStatePhilox4_32_10_t rng;
-    curand_init(sp.seed, n, 0ull, &rng);
-    const RowLayout L = row_layout(gp.T, gp.Cf, gp.ntab);
-    const float* const row = gp.table + (size_t)s * gp.row_floats;
-    const float c = row[L.C];
-    const bool wc = gp.model == BPLX_NEUTRAL_WC;
-    for (int t = 0; t < NT; t++) {
-      ACC(s_pts, t) = sp.start_pts[t];
-      ACC(s_gf, t) = sp.start_gf[t];
-      ACC(s_gd, t) = sp.start_ga[t];
-    }
-    bool ok = true;
-    uint8_t* const sc = sp.scores ? sp.scores + (size_t)i * gp.F * 2 : nullptr;
+      const int pr = min(x, y) * NT + max(x, y);
 #pragma unroll 1
-    for (int f = 0; f < gp.F; f++) {
-      const int hs = sp.hslot[f], as = sp.aslot[f];
-      const bool neutral = gp.ntab == 3 && gp.nv && gp.nv[f];
-      const FixtureOffsets off =
-          fixture_offsets(L, gp.home[f], gp.away[f], neutral, wc, wc ? gp.hconf[f] : 0, wc ? gp.aconf[f] : 0);
-      const float2 lam = fixture_rates(row, off, neutral, wc);
-      const float uh = curand_uniform(&rng), ua = curand_uniform(&rng);
-      int hg = 0, ag = 0;
-      const bool fok = sample_score(lam.x, lam.y, c, uh, ua, sp.G, hg, ag) && hs < NT && as < NT;
-      if (fok) {
-        const int ph = hg > ag ? sp.pw : hg == ag ? sp.pd : 0;
-        const int pa = ag > hg ? sp.pw : hg == ag ? sp.pd : 0;
-        ACC(s_pts, hs) += ph;
-        ACC(s_gf, hs) += hg;
-        ACC(s_gd, hs) += ag;
-        ACC(s_pts, as) += pa;
-        ACC(s_gf, as) += ag;
-        ACC(s_gd, as) += hg;
-      } else {
-        ok = false;
-        hg = ag = 0xFF;
-      }
-      if (sc) *reinterpret_cast<uchar2*>(sc + 2 * f) = make_uchar2((unsigned char)hg, (unsigned char)ag);
-    }
-    if constexpr (!KO) {
-      for (int t = 0; t < NT; t++) {
-        ACC(s_key, t) = curand(&rng);
-        ACC(s_gd, t) = ACC(s_gf, t) - ACC(s_gd, t);
-        const int gained = ACC(s_pts, t) - sp.start_pts[t];
-        ok = ok && gained >= 0 && gained < sp.B;  // (bins sized by the caller: a short one is refused, never overrun)
-      }
-      ok = ok && s_groups_fit;
-      uint8_t* const prow = sp.positions ? sp.positions + (size_t)i * NT : nullptr;
-      if (!ok) {
-        atomicAdd(&s_invalid, 1u);
-        if (prow)
-          for (int t = 0; t < NT; t++) prow[t] = 0xFF;
-      } else {
-        for (int t = 0; t < NT; t++) {
-          const int pt = ACC(s_pts, t), dt = ACC(s_gd, t), ft = ACC(s_gf, t);
-          const uint32_t kt = ACC(s_key, t);
-          const int g0 = s_gbeg[t], gc = s_gcnt[t];
-          int pos = 0;
-          for (int m = 0; m < gc; m++) {
-            const int u = s_members[g0 + m];
-            const int pu = ACC(s_pts, u), du = ACC(s_gd, u), fu = ACC(s_gf, u);
-            const uint32_t ku = ACC(s_key, u);
-            pos += pu != pt ? pu > pt : du != dt ? du > dt : fu != ft ? fu > ft : ku != kt ? ku > kt : u < t;
-          }
-          if (prow) prow[t] = (uint8_t)pos;
-          atomicAdd(&h_pos[t * sp.P + pos], 1u);
-          const int gained = pt - sp.start_pts[t];
-          if (sp.points_in_smem) atomicAdd(&h_pts[t * sp.B + gained], 1u);
-          else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
-        }
-      }
-    } else {
-      for (int t = 0; t < NT; t++) {
-        ACC(s_gd, t) = ACC(s_gf, t) - ACC(s_gd, t);
-        const int gained = ACC(s_pts, t) - sp.start_pts[t];
-        ok = ok && gained >= 0 && gained < sp.B;
-      }
-      ok = ok && s_groups_fit;
-      const unsigned wkey = 2u * (unsigned)gp.F;  // word of slot 0's tie-break key
-      // a slot u ranked ahead of slot t (u != t): points, goal difference, goals for, the key, then the lower slot
-      auto ahead = [&](int u, int t) -> bool {
-        const int pu = ACC(s_pts, u), pt = ACC(s_pts, t);
-        if (pu != pt) return pu > pt;
-        const int du = ACC(s_gd, u), dt = ACC(s_gd, t);
-        if (du != dt) return du > dt;
-        const int fu = ACC(s_gf, u), ft = ACC(s_gf, t);
-        if (fu != ft) return fu > ft;
-        const uint32_t ku = philox_word(sp.seed, n, wkey + u), kt = philox_word(sp.seed, n, wkey + t);
-        return ku != kt ? ku > kt : u < t;
-      };
-      if (ok) {
-        // ranking within the groups: k_q[gbeg + position] = slot
-        for (int t = 0; t < NT; t++) {
-          const int g0 = s_gbeg[t], gc = s_gcnt[t];
-          int pos = 0;
-          for (int m = 0; m < gc; m++) {
-            const int u = s_members[g0 + m];
-            if (u != t) pos += ahead(u, t);
-          }
-          BYTE(k_q, g0 + pos) = (uint8_t)t;
-        }
-        // best-placed qualifiers: the slot at best_position of every group, ranked across groups
-        if (ko.bc > 0) {
-          unsigned mask = 0;
-          int nq = 0;
-          for (int g = 0; g < ko.ng; g++) {
-            if (k_gtab[ko.ng + g] <= ko.bp) continue;
-            const int t = BYTE(k_q, k_gtab[g] + ko.bp);
-            int rk = 0;
-            for (int h = 0; h < ko.ng; h++)
-              if (h != g && k_gtab[ko.ng + h] > ko.bp) rk += ahead(BYTE(k_q, k_gtab[h] + ko.bp), t);
-            if (rk < ko.bc) {
-              nq++;
-              if (ko.alloc) mask |= 1u << g;
-              else BYTE(k_best, rk) = (uint8_t)t;
-            }
-          }
-          ok = nq == ko.bc;
-          if (ok && ko.alloc) {
-            const uint8_t* const arow = ko.alloc + (size_t)mask * ko.bc;
-            for (int j = 0; j < ko.bc; j++) {
-              const int g = arow[j];
-              if (g < ko.ng && ((mask >> g) & 1u)) BYTE(k_best, j) = BYTE(k_q, k_gtab[g] + ko.bp);
-              else ok = false;  // an allocation row of 0xFF
-            }
-          }
-        }
-      }
-      // the ties in play order; words 2F + T_tab + 3k, + 1 (the first or only match) and + 2 (the decider) of tie k,
-      // and the Philox block E/4 + k (leg 2, extra time) of a tie of format 1 or 2
-      skipahead((unsigned long long)NT, &rng);
-      uint8_t* const ent = ko.entrants ? ko.entrants + (size_t)i * ko.K * 2 : nullptr;
-      uint8_t* const ksc = ko.scores ? ko.scores + (size_t)i * ko.K * 2 : nullptr;
-      uint8_t* const kwn = ko.winners ? ko.winners + (size_t)i * ko.K : nullptr;
-      uint8_t* const kex = ko.extra ? ko.extra + (size_t)i * ko.K * 4 : nullptr;
-#pragma unroll 1
-      for (int k = 0; k < ko.K && ok; k++) {
-        int e[2];
-#pragma unroll
-        for (int side = 0; side < 2; side++) {
-          const int a0 = ko.arg0[side][k];
-          switch (ko.kind[side][k]) {
-            case BPLX_ENTRANT_SLOT: e[side] = a0; break;
-            case BPLX_ENTRANT_GROUP_POS: {
-              const int p = ko.arg1[side][k];
-              ok = ok && p < k_gtab[ko.ng + a0];
-              e[side] = ok ? BYTE(k_q, k_gtab[a0] + p) : 0;
-              break;
-            }
-            case BPLX_ENTRANT_BEST: e[side] = BYTE(k_best, a0); break;
-            case BPLX_ENTRANT_WINNER: e[side] = WL(2 * a0) & 63; break;
-            default: e[side] = WL(2 * a0 + 1); break;
-          }
-        }
-        const float uh = curand_uniform(&rng), ua = curand_uniform(&rng), ud = curand_uniform(&rng);
-        if (!ok) break;
-        const int hs = e[0], as = e[1];
-        const bool neutral = gp.ntab == 3 && ko.neutral[k];
-        const FixtureOffsets off = fixture_offsets(L, ko.slot_team[hs], ko.slot_team[as], neutral, wc,
-                                                   wc ? ko.slot_conf[hs] : 0, wc ? ko.slot_conf[as] : 0);
-        const float2 lam = fixture_rates(row, off, neutral, wc);
+      for (int e = sp.pair_beg[pr]; e < sp.pair_beg[pr + 1]; e++) {
+        const int f = sp.pair_fix[e];
         int hg = 0, ag = 0;
-        ok = sample_score(lam.x, lam.y, c, uh, ua, sp.G, hg, ag);
-        bool home_through = hg > ag;
-        int how = 0;  // decided in normal time or on aggregate (0), in extra time (1), by u_d (2)
-        const int fmt = ko.format[k];
-        if (fmt == BPLX_TIE_ONE_MATCH) {
-          if (ok && hg == ag) {  // a drawn tie: the home entrant goes through iff u_d (hw + aw) <= hw
-            float hw, aw;
-            win_masses(lam.x, lam.y, c, sp.G, hw, aw);
-            const float tot = hw + aw;
-            ok = tot > 0.0f;
-            home_through = ud * tot <= hw;
-            how = 2;
-          }
-          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(0xFE, 0xFE, 0xFE, 0xFE);
-        } else if (ok) {
-          // goals of the home entrant A and the away entrant B; extra time at the venue of the last match
-          const uint4 xw = philox_block(sp.seed, n, (2u * gp.F + NT + 3u * ko.K + 3u) / 4u + k);
-          int tot_a = hg, tot_b = ag, l2a = 0xFE, l2b = 0xFE, eta = 0xFE, etb = 0xFE;
-          float2 last = lam;
-          const bool legs = fmt == BPLX_TIE_TWO_LEGS;
-          if (legs) {  // leg 2: B at home, never at a neutral venue
-            const FixtureOffsets off2 = fixture_offsets(L, ko.slot_team[as], ko.slot_team[hs], false, wc,
-                                                        wc ? ko.slot_conf[as] : 0, wc ? ko.slot_conf[hs] : 0);
-            last = fixture_rates(row, off2, false, wc);
-            ok = sample_score(last.x, last.y, c, _curand_uniform(xw.x), _curand_uniform(xw.y), sp.G, l2b, l2a);
-            tot_a += l2a;
-            tot_b += l2b;
-          }
-          if (ok && tot_a == tot_b) {
-            int eh = 0, ea = 0;
-            ok = sample_score(last.x * kExtraTimeFraction, last.y * kExtraTimeFraction, 0.0f, _curand_uniform(xw.z),
-                              _curand_uniform(xw.w), sp.G, eh, ea);
-            eta = legs ? ea : eh;
-            etb = legs ? eh : ea;
-            tot_a += eta;
-            tot_b += etb;
-            how = 1;
-          }
-          home_through = tot_a > tot_b;
-          if (tot_a == tot_b) {  // penalties
-            home_through = ud <= 0.5f;
-            how = 2;
-          }
-          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(l2a, l2b, eta, etb);
-        }
-        if (!ok) break;
-        const int w = home_through ? hs : as;
-        WL(2 * k) = (uint8_t)(w | how << 6);
-        WL(2 * k + 1) = (uint8_t)(home_through ? as : hs);
-        if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2((unsigned char)hs, (unsigned char)as);
-        if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2((unsigned char)hg, (unsigned char)ag);
-        if (kwn) kwn[k] = (uint8_t)w;
-      }
-      uint8_t* const prow = sp.positions ? sp.positions + (size_t)i * NT : nullptr;
-      if (!ok) {
-        atomicAdd(&s_invalid, 1u);
-        if (prow)
-          for (int t = 0; t < NT; t++) prow[t] = 0xFF;
-        for (int k = 0; k < ko.K; k++) {
-          if (ent) *reinterpret_cast<uchar2*>(ent + 2 * k) = make_uchar2(0xFF, 0xFF);
-          if (ksc) *reinterpret_cast<uchar2*>(ksc + 2 * k) = make_uchar2(0xFF, 0xFF);
-          if (kwn) kwn[k] = 0xFF;
-          if (kex) *reinterpret_cast<uchar4*>(kex + 4 * k) = make_uchar4(0xFF, 0xFF, 0xFF, 0xFF);
-        }
-      } else {
-        for (int m = 0; m < NT; m++) {
-          const int t = BYTE(k_q, m), pos = m - s_gbeg[t];
-          if (prow) prow[t] = (uint8_t)pos;
-          atomicAdd(&h_pos[t * sp.P + pos], 1u);
-          const int gained = ACC(s_pts, t) - sp.start_pts[t];
-          if (sp.points_in_smem) atomicAdd(&h_pts[t * sp.B + gained], 1u);
-          else atomicAdd(&sp.pts_counts[(size_t)t * sp.B + gained], 1ull);
-        }
-        for (int k = 0; k < ko.K; k++) {
-          const int r = ko.round[k], wb = WL(2 * k), w = wb & 63, l = WL(2 * k + 1);
-          atomicAdd(&h_reach[w * ko.nr + r], 1u);
-          atomicAdd(&h_reach[l * ko.nr + r], 1u);
-          atomicAdd(&h_win[w * ko.nr + r], 1u);
-          if (wb >> 6) atomicAdd(&h_dec[2 * k + (wb >> 6) - 1], 1u);
-        }
+        rescore(f, hg, ag);
+        const int gx = sp.hslot[f] == x ? hg : ag, gy = hg + ag - gx;
+        hp += gx > gy ? sp.pw : gx == gy ? sp.pd : 0;
+        hd += gx - gy;
+        hf += gx;
       }
     }
+  };
+  // the end of the class that starts at position a
+  auto class_end = [&](int a, int ge) {
+    int b = a + 1;
+    while (b < ge && !(BYTE(k_q, b) & 0x80)) b++;
+    return b;
+  };
+  const unsigned wkey = 2u * (unsigned)gp.F;
+  for (int g0 = 0; g0 < NT;) {
+    const int ge = g0 + s_gcnt[s_members[g0]];
+    for (int p = g0; p < ge; p++) {  // by points (insertion)
+      const int x = s_members[p], px = ACC(s_pts, x);
+      int q = p;
+      for (; q > g0 && ACC(s_pts, BYTE(k_q, q - 1)) < px; q--) BYTE(k_q, q) = BYTE(k_q, q - 1);
+      BYTE(k_q, q) = (uint8_t)x;
+    }
+    for (int p = g0, prev = 0; p < ge; p++) {
+      const int x = BYTE(k_q, p), px = ACC(s_pts, x);
+      if (p == g0 || px != prev) BYTE(k_q, p) = (uint8_t)(x | 0x80);
+      prev = px;
+    }
+#pragma unroll 1
+    for (int a = g0; a < ge;) {
+      const int b = class_end(a, ge);
+      if (b - a < 2 || (BYTE(k_q, a) & 0x40)) {
+        a = b;
+        continue;
+      }
+      BYTE(k_q, a) &= 63;
+      // by head-to-head (insertion: the class keeps its members while a place is searched for)
+#pragma unroll 1
+      for (int p = a + 1; p < b; p++) {
+        const int x = BYTE(k_q, p);
+        int xp, xd, xf;
+        h2h(x, a, b, xp, xd, xf);
+        int q = p;
+#pragma unroll 1
+        for (; q > a; q--) {
+          int yp, yd, yf;
+          h2h(BYTE(k_q, q - 1), a, b, yp, yd, yf);
+          if (!(xp != yp ? xp > yp : xd != yd ? xd > yd : xf > yf)) break;
+        }
+        for (int m = p; m > q; m--) BYTE(k_q, m) = BYTE(k_q, m - 1);
+        BYTE(k_q, q) = (uint8_t)x;
+      }
+      // mark the parts; a class that is not split is settled, a split one is refined from its first part
+      bool split = false;
+#pragma unroll 1
+      for (int p = a, pp = 0, pd = 0, pf = 0; p < b; p++) {
+        const int x = BYTE(k_q, p) & 63;
+        int xp, xd, xf;
+        h2h(x, a, b, xp, xd, xf);
+        const bool brk = p > a && (xp != pp || xd != pd || xf != pf);
+        if (p == a || brk) BYTE(k_q, p) = (uint8_t)(x | 0x80);
+        split = split || brk;
+        pp = xp;
+        pd = xd;
+        pf = xf;
+      }
+      if (!split) {
+        BYTE(k_q, a) |= 0x40;
+        a = b;
+      }
+    }
+    // the classes left level: goal difference, goals for, the key, then the lower slot
+#pragma unroll 1
+    for (int a = g0; a < ge;) {
+      const int b = class_end(a, ge);
+      BYTE(k_q, a) &= 63;
+#pragma unroll 1
+      for (int p = a + 1; p < b; p++) {
+        const int x = BYTE(k_q, p), dx = ACC(s_gd, x), fx = ACC(s_gf, x);
+        int q = p;
+        for (; q > a; q--) {
+          const int y = BYTE(k_q, q - 1), dy = ACC(s_gd, y), fy = ACC(s_gf, y);
+          if (dx != dy ? dx < dy : fx != fy ? fx < fy : false) break;
+          if (dx == dy && fx == fy) {
+            const uint32_t kx = philox_word(sp.seed, n, wkey + x), ky = philox_word(sp.seed, n, wkey + y);
+            if (kx != ky ? kx < ky : x > y) break;
+          }
+          BYTE(k_q, q) = (uint8_t)y;
+        }
+        BYTE(k_q, q) = (uint8_t)x;
+      }
+      a = b;
+    }
+    g0 = ge;
   }
 #undef ACC
 #undef BYTE
-#undef WL
+}
+
+// The kernels: simulate_body.inc with the ranking rule fixed at compile time
+template <bool KO>
+__global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_constant__ SimParams sp) {
+  constexpr bool H2H = false;
+#include "simulate_body.inc"
+}
+
+// the same, with the groups ranked by the head-to-head rule (bplx_ranking)
+template <bool KO>
+__global__ void __launch_bounds__(kSimThreads) simulate_h2h_kernel(const __grid_constant__ SimParams sp) {
+  constexpr bool H2H = true;
+#include "simulate_body.inc"
+}
+
+// the remaining fixtures by slot pair, for the head-to-head ranking: pair_fix[pair_beg[p] .. pair_beg[p + 1]) are the
+// fixtures between slots u < v, p = u NT + v, in no particular order (the ranking only sums over them).  One CTA of
+// 1024 threads; a fixture with a slot outside the table or a team playing itself is left out.
+__global__ void __launch_bounds__(1024) pair_index_kernel(const uint8_t* hslot, const uint8_t* aslot, int F, int NT,
+                                                          int* pair_beg, int* pair_fix) {
+  extern __shared__ int s_cnt[];  // [NT NT]: counts, then the cursors of the fill
+  __shared__ int s_warp[32];
+  const int np = NT * NT, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int p = tid; p < np; p += blockDim.x) s_cnt[p] = 0;
   __syncthreads();
-  for (int k = tid; k < NT * sp.P; k += kSimThreads)
-    if (h_pos[k]) atomicAdd(&sp.pos_counts[k], (unsigned long long)h_pos[k]);
-  if (sp.points_in_smem)
-    for (int k = tid; k < NT * sp.B; k += kSimThreads)
-      if (h_pts[k]) atomicAdd(&sp.pts_counts[k], (unsigned long long)h_pts[k]);
-  if constexpr (KO) {
-    for (int k = tid; k < NT * ko.nr; k += kSimThreads) {
-      if (h_reach[k]) atomicAdd(&ko.reach[k], (unsigned long long)h_reach[k]);
-      if (h_win[k]) atomicAdd(&ko.win[k], (unsigned long long)h_win[k]);
-    }
-    if (ko.decided) {
-      const unsigned valid = (unsigned)min(kSimThreads, sp.N - (int)blockIdx.x * kSimThreads) - s_invalid;
-      for (int k = tid; k < ko.K; k += kSimThreads) {
-        const unsigned et = h_dec[2 * k], ud = h_dec[2 * k + 1], nt = valid - et - ud;
-        if (nt) atomicAdd(&ko.decided[3 * k], (unsigned long long)nt);
-        if (et) atomicAdd(&ko.decided[3 * k + 1], (unsigned long long)et);
-        if (ud) atomicAdd(&ko.decided[3 * k + 2], (unsigned long long)ud);
-      }
-    }
+  for (int f = tid; f < F; f += blockDim.x) {
+    const int u = hslot[f], v = aslot[f];
+    if (u != v && u < NT && v < NT) atomicAdd(&s_cnt[min(u, v) * NT + max(u, v)], 1);
   }
-  if (tid == 0 && s_invalid) atomicAdd(sp.invalid, (unsigned long long)s_invalid);
+  __syncthreads();
+  // exclusive scan: a chunk of pairs per thread, the chunk sums scanned per warp, then across the warps
+  const int per = (np + blockDim.x - 1) / blockDim.x, lo = min(np, tid * per), hi = min(np, lo + per);
+  int sum = 0;
+  for (int p = lo; p < hi; p++) sum += s_cnt[p];
+  int incl = sum;
+  for (int d = 1; d < 32; d <<= 1) {
+    const int o = __shfl_up_sync(0xffffffffu, incl, d);
+    if (lane >= d) incl += o;
+  }
+  if (lane == 31) s_warp[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    int w = lane < (int)(blockDim.x >> 5) ? s_warp[lane] : 0;
+    for (int d = 1; d < 32; d <<= 1) {
+      const int o = __shfl_up_sync(0xffffffffu, w, d);
+      if (lane >= d) w += o;
+    }
+    s_warp[lane] = w;
+  }
+  __syncthreads();
+  int run = incl - sum + (warp ? s_warp[warp - 1] : 0);
+  for (int p = lo; p < hi; p++) {
+    const int c = s_cnt[p];
+    s_cnt[p] = run;
+    pair_beg[p] = run;
+    run += c;
+  }
+  if (tid == (int)blockDim.x - 1) pair_beg[np] = run;
+  __syncthreads();
+  for (int f = tid; f < F; f += blockDim.x) {
+    const int u = hslot[f], v = aslot[f];
+    if (u != v && u < NT && v < NT) pair_fix[atomicAdd(&s_cnt[min(u, v) * NT + max(u, v)], 1)] = f;
+  }
 }
 
 size_t simulate_smem_bytes(SimParams* sp) {
@@ -544,11 +399,13 @@ int launch_simulate(SimParams& sp, cudaStream_t stream) {
   BPLX_REQUIRE(smem <= (size_t)kSimSmemMax, BPLX_E_UNSUPPORTED,
                "simulate: %zu bytes of shared memory per CTA needed (max %d)", smem, kSimSmemMax);
   // the dynamic shared-memory limit is an attribute of each instantiation
-  static size_t smem_set[2] = {48 * 1024, 48 * 1024};
-  if (smem > smem_set[ko]) {
-    BPLX_CUDA(cudaFuncSetAttribute(ko ? simulate_kernel<true> : simulate_kernel<false>,
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_set[ko] = smem;
+  static void (*const kernels[4])(const SimParams) = {simulate_kernel<false>, simulate_kernel<true>,
+                                                      simulate_h2h_kernel<false>, simulate_h2h_kernel<true>};
+  static size_t smem_set[4] = {48 * 1024, 48 * 1024, 48 * 1024, 48 * 1024};
+  const int v = (int)ko + (sp.rule == BPLX_RANK_HEAD_TO_HEAD ? 2 : 0);
+  if (smem > smem_set[v]) {
+    BPLX_CUDA(cudaFuncSetAttribute(kernels[v], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    smem_set[v] = smem;
   }
   BPLX_CUDA(cudaMemsetAsync(sp.pos_counts, 0, (size_t)sp.NT * sp.P * 8, stream));
   BPLX_CUDA(cudaMemsetAsync(sp.pts_counts, 0, (size_t)sp.NT * sp.B * 8, stream));
@@ -560,9 +417,14 @@ int launch_simulate(SimParams& sp, cudaStream_t stream) {
   }
   rc = launch_score_grid_tables(sp.gp, stream);
   if (rc != BPLX_OK) return rc;
+  if (v >= 2) {
+    pair_index_kernel<<<1, 1024, (size_t)sp.NT * sp.NT * 4, stream>>>(sp.hslot, sp.aslot, sp.gp.F, sp.NT,
+                                                                     sp.pair_beg, sp.pair_fix);
+    BPLX_CUDA(cudaGetLastError());
+    note_launch(1);
+  }
   const unsigned grid = (unsigned)((sp.N + kSimThreads - 1) / kSimThreads);
-  if (ko) simulate_kernel<true><<<grid, kSimThreads, smem, stream>>>(sp);
-  else simulate_kernel<false><<<grid, kSimThreads, smem, stream>>>(sp);
+  kernels[v]<<<grid, kSimThreads, smem, stream>>>(sp);
   BPLX_CUDA(cudaGetLastError());
   note_launch(1);
   return BPLX_OK;

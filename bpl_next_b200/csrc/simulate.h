@@ -45,12 +45,17 @@ struct SimParams {
   unsigned long long *pos_counts, *pts_counts, *invalid;  // [NT][P], [NT][B], [1]
   uint8_t *positions, *scores;    // [N][NT], [N][F][2] or NULL
   KoParams ko;                    // the tournament kernel only
+  // the ranking rule (BPLX_RANK_*); head-to-head only: the played matches and the remaining fixtures by slot pair
+  int rule;
+  const int2* h2h_played;         // [NT][NT] (points, goals) of slot u against slot v in played matches, or NULL
+  int *pair_beg, *pair_fix;       // [NT NT + 1], [F] in the workspace (pair_index_kernel)
 };
 
 // shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
 // the tournament kernel (sets sp->ko.wl_overlay)
 size_t simulate_smem_bytes(SimParams* sp);
-// ko.K = 0: the group stage alone; ko.K >= 1: the tournament kernel, the same group stage, then the bracket of sp.ko
+// ko.K = 0: the group stage alone; ko.K >= 1: the tournament kernel, the same group stage, then the bracket of sp.ko.
+// rule = BPLX_RANK_HEAD_TO_HEAD: the head-to-head instantiation, after the pair index is built into pair_beg / pair_fix
 int launch_simulate(SimParams& sp, cudaStream_t stream);
 
 }  // namespace bplx

@@ -434,7 +434,7 @@ class _BplxPredictor:
     # ---- season / group-stage simulation -------------------------------------------------------------------------
     def simulate_table(self, fixtures, played=None, teams=None, groups=None, num_sims_per_draw: int = 1,
                        random_state: Optional[int] = None, max_goals: int = MAX_GOALS, points=(3, 1),
-                       return_simulations: bool = False) -> Dict[str, Any]:
+                       return_simulations: bool = False, tiebreak: str = "goal_difference") -> Dict[str, Any]:
         """Finishing-position and points probabilities of a league table or of group tables, simulated on the GPU.
 
         Every simulated season takes ONE posterior draw and plays every remaining fixture with that draw's rates, so a
@@ -451,11 +451,21 @@ class _BplxPredictor:
         ``points``: (win, draw).
 
         A fixture's score is drawn from the draw's own score grid up to ``max_goals`` (tau clamped at 0, normalised by
-        its sum); averaged over draws this is ``predict_score_grid_proba``.  Teams are ranked by points, goal
-        difference, goals for, then a random key: head-to-head and fair-play rules are NOT modelled, ties left after
-        goals for are decided by lot.
+        its sum); averaged over draws this is ``predict_score_grid_proba``.  ``tiebreak`` says how teams level on
+        points are ranked within their group:
 
-        Returns ``teams``, ``groups`` (each team's label, or None), ``position_proba [T, P]`` (P = the largest group;
+        * ``"goal_difference"`` (default): goal difference, goals for, then a random key.
+        * ``"head_to_head"`` (UEFA group stages, La Liga, Serie A): for a set of teams level on points, the points, goal
+          difference and goals for of the matches among them only (in ``played`` and the simulated ``fixtures``);
+          teams still level on all three go through that again with only the matches among themselves; a set it does
+          not separate at all (teams that have not met, say) is ordered by overall goal difference, goals for, then
+          the random key.
+
+        Fair-play rules are NOT modelled: ties left at the end are decided by lot.  Both rules read the same random
+        numbers, so with the same seed they differ only in the order of teams level on points.
+
+        Returns ``teams``, ``groups`` (each team's label, or None), ``tiebreak`` (the rule that ranked the table),
+        ``position_proba [T, P]`` (P = the largest group;
         position 0 = first), ``points_proba [T, B]`` (points GAINED in ``fixtures``), ``start_points``,
         ``expected_points`` (final), ``num_simulations``, ``sims_per_draw`` and ``seed`` (from the clock when
         ``random_state`` is None; pass it back to repeat the run).  With ``return_simulations`` also ``positions [N, T]``
@@ -464,7 +474,7 @@ class _BplxPredictor:
         size.  Raises if any simulation met a non-finite rate."""
         home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"])
         tteams = bseason.table_teams(home, away, played, teams)
-        table = bseason.build_table(tteams, played, groups, points)
+        table = bseason.build_table(tteams, played, groups, points, tiebreak)
         hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
         fx = {**self._fixture_arrays(home, away, fixtures), "home_slot": hs, "away_slot": as_}
         return self._simulate(table, fx, None, num_sims_per_draw, random_state, max_goals, return_simulations,
@@ -483,6 +493,7 @@ class _BplxPredictor:
         dtab = {k: None if table[k] is None else torch.from_numpy(table[k]).cuda()
                 for k in ("start_points", "start_goals_for", "start_goals_against", "group")}
         dtab.update({k: table[k] for k in ("num_positions", "num_points_bins", "points_win", "points_draw")})
+        dtab.update(tiebreak=table.get("tiebreak", "goal_difference"), played_h2h=table.get("played_h2h"))  # (host)
         S, T, F = int(ds["attack"].shape[0]), len(table["teams"]), len(fx.get("home_team", ()))
         K = 0 if bracket is None else len(bracket["round"])
         step = (2 ** 31 - 1) // R  # simulations per call stay below 2^31
@@ -513,6 +524,7 @@ class _BplxPredictor:
         cnt = {k: v.cpu().numpy() for k, v in acc.items()}
         res = {"teams": table["teams"],
                "groups": None if table["group"] is None else [table["group_labels"][g] for g in table["group"]],
+               "tiebreak": dtab["tiebreak"],
                **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N)}
         if bracket is not None:
             res.update(bseason.bracket_probabilities(bracket, cnt["reach_counts"], cnt["win_counts"], N,
@@ -546,14 +558,16 @@ class _BplxPredictor:
 
     def simulate_tournament(self, fixtures, bracket, played=None, teams=None, groups=None, best=None, team_conf=None,
                             num_sims_per_draw: int = 1, random_state: Optional[int] = None, max_goals: int = MAX_GOALS,
-                            points=(3, 1), return_simulations: bool = False) -> Dict[str, Any]:
+                            points=(3, 1), return_simulations: bool = False,
+                            tiebreak: str = "goal_difference") -> Dict[str, Any]:
         """A tournament simulated on the GPU: the group stage of ``simulate_table``, then a knockout bracket, with ONE
         posterior draw per simulated tournament, so a team that is stronger in a draw is stronger in every match of its
         path.  (Chaining ``predict_outcome_proba`` calls cannot give this: the opponent of a round depends on earlier
         results, and the same uncertain strengths run through all of a team's matches.)
 
         ``fixtures``, ``played``, ``teams``, ``groups``, ``points``, ``num_sims_per_draw``, ``random_state``,
-        ``max_goals``: as ``simulate_table``; ``fixtures`` may be None or empty (a cup whose draw is made: the entrants
+        ``max_goals``, ``tiebreak``: as ``simulate_table`` (``"head_to_head"`` ranks each group by the matches among
+        its teams level on points, as UEFA's and FIFA's group stages do); ``fixtures`` may be None or empty (a cup whose draw is made: the entrants
         are ``("team", name)``).  ``bracket``: the ties in play order, ``{"id", "round", "home", "away",
         "neutral_venue", "format"}``, entrants ``("group", label, position)``, ``("best", j)``, ``("winner", id)``,
         ``("loser", id)`` or ``("team", name)``; ``best``: the best-placed qualifiers, ``{"position", "count",
@@ -574,8 +588,9 @@ class _BplxPredictor:
 
         Each leg is a 90-minute match from the draw's own grid.  Extra time uses the draw's rates times 1/3 (30 of 90
         minutes at the model's constant rates) with no tau correction; the home entrant wins a shoot-out with
-        probability 1/2 (the model knows nothing of penalties).  Best-placed teams are ranked by points, goal
-        difference, goals for, then lot.
+        probability 1/2 (the model knows nothing of penalties).  Best-placed teams are ranked across groups by
+        points, goal difference, goals for, then lot, under either ``tiebreak`` (teams of different groups have no
+        head-to-head).
 
         Returns everything ``simulate_table`` returns, plus ``rounds`` (labels by first appearance), ``reach_proba`` /
         ``win_proba [T, rounds]`` (the team plays / wins a tie of the round; a two-legged tie counts once),
@@ -593,7 +608,7 @@ class _BplxPredictor:
             tteams = bseason.table_teams(home + named, away, played) if (home or named or played) else []
         else:
             tteams = bseason.table_teams(home, away, played, teams)
-        table = bseason.build_table(tteams, played, groups, points)
+        table = bseason.build_table(tteams, played, groups, points, tiebreak)
         br = bseason.build_bracket(table, bracket, best)
         known = set(np.asarray(self.teams).tolist())
         unknown = [t for t in tteams if t not in known]

@@ -13,6 +13,7 @@ import torch
 
 from . import _abi
 from .data import MatchArrays
+from .season import TIEBREAKS
 
 _STAT_NAMES = ("matches", "entries1", "entries1_padded", "entries2", "entries2_padded", "smem_bytes", "warps", "vteams")
 
@@ -319,12 +320,17 @@ def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[
     the first one).  ``fixtures``: the index tensors of ``score_grid`` plus ``home_slot`` / ``away_slot`` (uint8 table
     slots).  ``table``: ``start_points``, ``start_goals_for``, ``start_goals_against`` (int32 ``[T_tab]``), ``group``
     (uint8 ``[T_tab]`` or None) on the GPU, and the ints ``num_positions`` (largest group), ``num_points_bins``,
-    ``points_win``, ``points_draw`` (``season.build_table`` / ``season.fixture_slots`` make them).
+    ``points_win``, ``points_draw`` (``season.build_table`` / ``season.fixture_slots`` make them), and optionally
+    ``tiebreak`` (``"goal_difference"``, the default, or ``"head_to_head"``) with the host ``played_h2h`` (int32 ``[T_tab,
+    T_tab, 2]``: points and goals of slot u against slot v in played matches, or None).
 
     Simulation ``n = (first_draw + s) R + r`` uses draw s and the Philox words of ``curand_init(seed, n, 0)``: words 2f,
     2f+1 sample fixture f's score from the draw's own grid (tau clamped at 0, normalised by its sum), word 2F + t is slot
-    t's tie-break key.  Teams are ranked within their group by points, goal difference, goals for, then the key;
-    head-to-head and fair-play rules are not modelled, so ties left after goals for are decided by lot.  Returns
+    t's tie-break key.  Teams are ranked within their group by points, then under ``"goal_difference"`` by goal
+    difference, goals for, then the key (``bplx_simulate_table``); under ``"head_to_head"`` by the points, goal
+    difference and goals for of the matches among the teams level on points (played and simulated), reapplied to the
+    teams still level, then overall goal difference, goals for and the key (``bplx_simulate_table_ex``: the same Philox
+    words, only the group order can differ).  Fair-play rules are not modelled: ties left are decided by lot.  Returns
     ``position_counts [T_tab, P]`` and ``points_counts [T_tab, B]`` (points gained; int64), ``invalid`` (int64 ``[1]``:
     simulations with a non-finite rate or normaliser, left out of the counts), and when asked ``positions [N, T_tab]``
     and ``scores [N, F, 2]`` (uint8; 255 marks an invalid simulation / fixture), N = S R."""
@@ -342,6 +348,26 @@ def _table_struct(table: dict, ptr):
     for k in _TABLE_ARRAYS:
         setattr(t, k, ptr(table[k]))
     return t
+
+
+def _ranking_struct(table: dict, T_tab: int, keep: list):
+    """``_abi.Ranking`` of ``table["tiebreak"]`` over a host copy of ``played_h2h`` (kept alive in ``keep``), or None
+    for ``"goal_difference"`` (the calls without a ranking)."""
+    rule = table.get("tiebreak", "goal_difference")
+    if rule not in TIEBREAKS:
+        raise ValueError(f"unknown tiebreak {rule!r} (one of {sorted(TIEBREAKS)})")
+    if TIEBREAKS[rule] == _abi.RANK_GOAL_DIFF:
+        return None
+    r = _abi.Ranking()
+    r.rule = TIEBREAKS[rule]
+    h2h = table.get("played_h2h")
+    if h2h is not None:
+        h2h = np.ascontiguousarray(h2h, dtype=np.int32)
+        if h2h.shape != (T_tab, T_tab, 2):
+            raise ValueError(f"played_h2h has shape {h2h.shape}; the table needs ({T_tab}, {T_tab}, 2)")
+        keep.append(h2h)
+        r.played_h2h = h2h.ctypes.data
+    return r
 
 
 def _bracket_struct(bracket: dict, keep: list):
@@ -394,7 +420,9 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
     ``[K, 3]``: tie k settled in normal time or on aggregate / in extra time / by ``u_d``), and when ``want_knockout``
     ``ko_entrants``, ``ko_scores`` (uint8 ``[N, K, 2]``, the first or only match), ``ko_winners`` (``[N, K]``) and
     ``ko_extra`` (``[N, K, 4]``: leg-2 goals of A and B, then extra-time goals of A and B; 254 where not played); 255
-    marks an invalid simulation."""
+    marks an invalid simulation.  ``table["tiebreak"]`` ranks the groups as in ``simulate_table``
+    (``bplx_simulate_tournament_ranked``); best-placed qualifiers are ranked across groups by points, goal difference,
+    goals for, then the key under either rule."""
     return _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw,
                      want_positions, want_scores, want_knockout, workspace, stream)
 
@@ -421,10 +449,17 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     f = _fixtures_struct(fixtures, ptr) if F else _abi.Fixtures()
     t = _table_struct(table, ptr)
     b = None if bracket is None else _bracket_struct(bracket, keep)
+    r = _ranking_struct(table, T_tab, keep)
     structs = (C.byref(s), C.byref(f), C.byref(t)) + (() if b is None else (C.byref(b),))
-    ws_bytes = lib.bplx_simulate_workspace_bytes if b is None else lib.bplx_simulate_tournament_workspace_bytes
+    if r is None:
+        ws_bytes = lib.bplx_simulate_workspace_bytes if b is None else lib.bplx_simulate_tournament_workspace_bytes
+        need = int(ws_bytes(*structs))
+    else:
+        ws_bytes = (lib.bplx_simulate_table_ex_workspace_bytes if b is None
+                    else lib.bplx_simulate_tournament_ranked_workspace_bytes)
+        need = int(ws_bytes(*structs, C.byref(r)))
     dev = samples["attack"].device
-    workspace = _workspace(workspace, int(ws_bytes(*structs)), dev)
+    workspace = _workspace(workspace, need, dev)
     N = s.num_samples * int(sims_per_draw)
     i64 = dict(dtype=torch.int64, device=dev)
     u8 = dict(dtype=torch.uint8, device=dev)
@@ -447,6 +482,8 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     slots = (ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"])) if F else (None, None)
     if b is None:
         run, args = lib.bplx_simulate_table, structs[:2] + slots + structs[2:]
+        if r is not None:
+            run, args = lib.bplx_simulate_table_ex, args + (C.byref(r),)
     else:
         fmt = bracket.get("tie_format")
         if fmt is not None:
@@ -456,6 +493,8 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
             keep.append(fmt)
         run, args = lib.bplx_simulate_tournament_ex, structs[:2] + slots + structs[2:] + (
             None if fmt is None else fmt.ctypes.data,)
+        if r is not None:
+            run, args = lib.bplx_simulate_tournament_ranked, args + (C.byref(r),)
     _abi.check(run(*args, int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
                    *outputs, _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
     return out

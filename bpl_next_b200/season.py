@@ -4,8 +4,10 @@ The simulation itself is the CUDA kernel behind ``problem.simulate_table`` (``cs
 inputs from team names and played results and turns its integer counts into probabilities.  Definition, in short (the
 full text is in ``include/bplx.h``): every simulated season takes ONE posterior draw and plays every remaining fixture
 with that draw's rates, so a team that is stronger in a draw is stronger in all of its matches of that season.  Teams
-are ranked within their group by points, goal difference, goals for, then a random tie-break key; head-to-head and
-fair-play rules are not modelled, so ties left after goals for are decided by lot.  ``build_bracket`` and
+are ranked within their group by points, then by the table's ranking rule (``TIEBREAKS``): ``"goal_difference"`` (the
+default: goal difference, goals for, then a random tie-break key) or ``"head_to_head"`` (the matches among the teams
+level on points first, reapplied to those still level; then goal difference, goals for and the key).  Fair-play rules
+are not modelled: ties left at the end are decided by lot.  ``build_bracket`` and
 ``bracket_probabilities`` do the same for a knockout bracket played after the group stage (``problem.simulate_tournament``).
 """
 from __future__ import annotations
@@ -16,10 +18,11 @@ from typing import Any, Dict, Optional, Sequence, Tuple
 import numpy as np
 
 from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_SLOT, ENTRANT_WINNER, KO_MAX_ALLOC_GROUPS,
-                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, SIM_MAX_TEAMS, TIE_ONE_MATCH, TIE_ONE_MATCH_ET,
-                   TIE_TWO_LEGS)
+                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, RANK_GOAL_DIFF, RANK_HEAD_TO_HEAD, SIM_MAX_TEAMS,
+                   TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS)
 
 TIE_FORMATS = {"one_match": TIE_ONE_MATCH, "extra_time": TIE_ONE_MATCH_ET, "two_legs": TIE_TWO_LEGS}
+TIEBREAKS = {"goal_difference": RANK_GOAL_DIFF, "head_to_head": RANK_HEAD_TO_HEAD}
 
 
 def _names(x) -> list:
@@ -51,12 +54,17 @@ def check_points(points) -> Tuple[int, int]:
     return int(pw), int(pd)
 
 
-def build_table(teams: Sequence, played: Optional[Dict[str, Any]] = None, groups=None, points=(3, 1)) -> Dict[str, Any]:
+def build_table(teams: Sequence, played: Optional[Dict[str, Any]] = None, groups=None, points=(3, 1),
+                tiebreak: str = "goal_difference") -> Dict[str, Any]:
     """Starting table of ``teams`` from ``played`` results (reference ``training_data`` keys: ``home_team``,
     ``away_team``, ``home_goals``, ``away_goals``): points (``points = (win, draw)``), goals for and against.  ``groups``
     is a mapping team -> label or a sequence of labels aligned with ``teams`` (None: one table); labels become ids
-    0 .. K-1 in sorted order.  Returns the host table ``problem.simulate_table`` takes (int32 arrays, uint8 group ids)
-    plus ``group_labels``."""
+    0 .. K-1 in sorted order.  ``tiebreak``: how teams level on points are ranked, ``"goal_difference"`` or
+    ``"head_to_head"`` (``include/bplx.h``, BPLX_RANK_*).  Returns the host table ``problem.simulate_table`` takes
+    (int32 arrays, uint8 group ids) plus ``group_labels`` and ``tiebreak``; under ``"head_to_head"`` also
+    ``played_h2h`` (int32 ``[T, T, 2]``: points and goals of team u against team v in ``played``)."""
+    if tiebreak not in TIEBREAKS:
+        raise ValueError(f"unknown tiebreak {tiebreak!r} (one of {sorted(TIEBREAKS)})")
     teams = list(teams)
     T = len(teams)
     if T < 1:
@@ -66,6 +74,7 @@ def build_table(teams: Sequence, played: Optional[Dict[str, Any]] = None, groups
     pw, pd = check_points(points)
     slot = {t: i for i, t in enumerate(teams)}
     pts, gf, ga = np.zeros(T, np.int64), np.zeros(T, np.int64), np.zeros(T, np.int64)
+    h2h = np.zeros((T, T, 2), np.int64)
     if played is not None:
         ph, pa = _names(played["home_team"]), _names(played["away_team"])
         hg, ag = np.asarray(played["home_goals"]).astype(np.int64), np.asarray(played["away_goals"]).astype(np.int64)
@@ -84,8 +93,11 @@ def build_table(teams: Sequence, played: Optional[Dict[str, Any]] = None, groups
             ga[i] += y
             gf[j] += y
             ga[j] += x
-            pts[i] += pw if x > y else pd if x == y else 0
-            pts[j] += pw if y > x else pd if x == y else 0
+            pi, pj = (pw if x > y else pd if x == y else 0), (pw if y > x else pd if x == y else 0)
+            pts[i] += pi
+            pts[j] += pj
+            h2h[i, j] += (pi, x)
+            h2h[j, i] += (pj, y)
     group, labels = None, None
     if groups is not None:
         lab = [groups[t] for t in teams] if isinstance(groups, dict) else list(groups)
@@ -94,9 +106,12 @@ def build_table(teams: Sequence, played: Optional[Dict[str, Any]] = None, groups
         labels = sorted(set(lab))
         ids = {g: k for k, g in enumerate(labels)}
         group = np.asarray([ids[g] for g in lab], np.uint8)
-    return {"teams": teams, "start_points": pts.astype(np.int32), "start_goals_for": gf.astype(np.int32),
-            "start_goals_against": ga.astype(np.int32), "group": group, "group_labels": labels,
-            "points_win": pw, "points_draw": pd}
+    out = {"teams": teams, "start_points": pts.astype(np.int32), "start_goals_for": gf.astype(np.int32),
+           "start_goals_against": ga.astype(np.int32), "group": group, "group_labels": labels,
+           "points_win": pw, "points_draw": pd, "tiebreak": tiebreak}
+    if tiebreak == "head_to_head":
+        out["played_h2h"] = h2h.astype(np.int32)
+    return out
 
 
 def fixture_slots(table: Dict[str, Any], home, away, known_teams=None) -> Tuple[np.ndarray, np.ndarray]:

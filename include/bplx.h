@@ -287,8 +287,9 @@ int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t 
  * Table: points_win for a win, points_draw for a draw (0 <= points_draw <= points_win, points_win >= 1); goal
  * difference and goals for accumulate on top of the start.  Teams are ranked WITHIN THEIR GROUP by points, then goal
  * difference, then goals for, then the tie-break key, all descending; if even the keys are equal the lower slot ranks
- * first.  Position k (0-based) of slot t = the number of teams of its group ranked ahead of t.  Head-to-head and
- * fair-play rules are not modelled: ties left after goals for are decided by lot (the tie-break key).
+ * first.  Position k (0-based) of slot t = the number of teams of its group ranked ahead of t.  That is ranking rule
+ * BPLX_RANK_GOAL_DIFF; bplx_simulate_table_ex can rank by BPLX_RANK_HEAD_TO_HEAD instead (below).  Fair-play rules are
+ * not modelled: ties left after goals for are decided by lot (the tie-break key).
  *
  * Outputs (device; integer counts, so they are the same bits whatever order the atomics run in; overwritten):
  *   position_counts [T_tab, P]  P = num_positions, the largest group size
@@ -342,8 +343,9 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
  * points, goal difference, goals for, then the slot tie-break key (word 2F + t), then the lower slot; the first
  * best_count qualify.  Without an allocation table BEST j is the j-th best; with one (dense [2^num_groups][best_count]
  * group ids, indexed by the bit set of the groups whose team qualified: the form of FIFA's and UEFA's third-place
- * tables) BEST j is the position-best_position slot of group alloc[mask][j].  Fair play, rankings and head-to-head are
- * not modelled: ties left after goals for are decided by lot.
+ * tables) BEST j is the position-best_position slot of group alloc[mask][j].  This cross-group ranking is the same
+ * under either group ranking rule (bplx_ranking: teams of different groups have no head-to-head).  Fair play and
+ * rankings are not modelled: ties left after goals for are decided by lot.
  * A tie is played like a group fixture, from the draw's own clamped, truncated grid, with the rates of its entrants'
  * model teams (slot_team) and, for NEUTRAL_WC, their confederations (slot_conf).  Words 2F + T_tab + 3k and + 1 sample
  * its score, word + 2 is the decider u_d (curand_uniform); every word has a fixed address, used or not.  A drawn tie goes
@@ -438,6 +440,63 @@ int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, c
                                 uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores, uint8_t* ko_winners,
                                 uint8_t* ko_extra, unsigned long long* invalid, void* workspace,
                                 size_t workspace_bytes, void* stream);
+
+/* ---- ranking rules: head-to-head ------------------------------------------------------------------------------ */
+/*
+ * The calls above rank a group by BPLX_RANK_GOAL_DIFF: points, goal difference, goals for, then lot.  The _ex / _ranked
+ * calls below take a bplx_ranking; NULL, or rule BPLX_RANK_GOAL_DIFF, gives the calls above bit for bit.  Under
+ * BPLX_RANK_HEAD_TO_HEAD the teams of each group are ranked as follows:
+ *   1. Points.
+ *   2. Head-to-head among a level set.  For a set S of two or more teams level on points, each team's points, goal
+ *      difference and goals for are computed over the matches between teams of S only: the played matches (played_h2h)
+ *      and this simulation's simulated fixtures.  S is ordered by (head-to-head points, head-to-head goal difference,
+ *      head-to-head goals for), all descending.
+ *   3. Reapply to what is still level.  If step 2 splits S, any part of two or more teams still level on all three
+ *      values goes through step 2 again, with S being that part: only the matches among that part count.
+ *   4. Fall back when nobody separates.  A set in which step 2 separates nobody (its teams have not met, say) is
+ *      ordered by overall goal difference, overall goals for, the tie-break key (word 2F + t), then the lower slot.
+ * Position k is the team's index in this order.  This is the structure of UEFA's group-stage rule (criteria a-f); fair
+ * play, coefficient rankings and a shoot-out between two level teams who meet in the last round are replaced by lot.
+ * Best-placed qualifiers are still ranked across groups by points, goal difference, goals for, then lot (teams of
+ * different groups have no head-to-head).  No Philox word is added or moved: a simulation reads the same words under
+ * either rule, and only its group order can differ.
+ *
+ * played_h2h: HOST int32 [T_tab, T_tab, 2], entry (u, v) = (points of slot u, goals of slot u) in the played matches
+ * between u and v (NULL: none played); the diagonal is ignored, and a negative entry is refused.  The call copies it
+ * into the workspace (cudaMemcpyAsync: a pageable array makes the call wait for the stream) and indexes the remaining
+ * fixtures by slot pair there from home_slot / away_slot, so a level set costs only the fixtures among its members.  An
+ * unknown rule: BPLX_E_INVALID (and 0 from the workspace-size calls).
+ */
+#define BPLX_RANK_GOAL_DIFF 0
+#define BPLX_RANK_HEAD_TO_HEAD 1
+typedef struct {
+  int32_t rule;                   /* BPLX_RANK_* */
+  const int32_t* played_h2h;      /* host [T_tab, T_tab, 2] (points, goals) of slot u against slot v, or NULL */
+} bplx_ranking;
+
+size_t bplx_simulate_table_ex_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
+                                              const bplx_ranking* r);
+/* bplx_simulate_table with a ranking rule; bplx_simulate_table is this call with r = NULL. */
+int bplx_simulate_table_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                           const uint8_t* away_slot, const bplx_table* t, const bplx_ranking* r, int max_goals,
+                           int sims_per_draw, unsigned long long seed, long long first_draw,
+                           unsigned long long* position_counts, unsigned long long* points_counts, uint8_t* positions,
+                           uint8_t* scores, unsigned long long* invalid, void* workspace, size_t workspace_bytes,
+                           void* stream);
+size_t bplx_simulate_tournament_ranked_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f,
+                                                       const bplx_table* t, const bplx_bracket* b,
+                                                       const bplx_ranking* r);
+/* bplx_simulate_tournament_ex with a ranking rule for the group stage; bplx_simulate_tournament_ex is this call with
+ * r = NULL. */
+int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                    const uint8_t* tie_format, const bplx_ranking* r, int max_goals, int sims_per_draw,
+                                    unsigned long long seed, long long first_draw, unsigned long long* position_counts,
+                                    unsigned long long* points_counts, unsigned long long* reach_counts,
+                                    unsigned long long* win_counts, unsigned long long* decided_counts,
+                                    uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
+                                    uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
+                                    void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */

@@ -7,7 +7,8 @@ Workloads (synthetic posterior draws, fixed seeds):
   world cup  48-team group stage, 12 groups of four, 72 fixtures at neutral venues, NeutralWC draws of configs[5]'s shape
              (T = 220 model teams, Cf = 6), R = 64 and R = 1
 With --baseline-lib, another build's bplx_simulate_table is timed on every workload, alternating with this build's, and
-its counts are checked equal.
+its counts are checked equal.  Every workload is also timed under the head-to-head ranking rule (bplx_simulate_table_ex,
+no played matches), alternating with the goal-difference call in the same run: h2h_ms, h2h_cost = h2h_ms / ms - 1.
 CUDA events around `--reps` calls after warm-up, best of three runs; a call is the whole entry point (count reset,
 exponential-table pre-pass, simulation kernel), issued straight through the C ABI so that no host synchronisation sits
 in the timed window.  Reports simulations/s and sampled scores/s, the GPU name and power limit read in the same run,
@@ -101,9 +102,9 @@ def baseline_lib(path, names):
     return lib
 
 
-def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1, lib=None):
+def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1, lib=None, head_to_head=False):
     """The bplx_simulate_table call with every argument built once; returns (call, outputs, keep-alive).  ``lib``:
-    another build's library (``baseline_lib``)."""
+    another build's library (``baseline_lib``).  ``head_to_head``: bplx_simulate_table_ex under that ranking rule."""
     import torch
 
     from bpl_next_b200 import _abi, problem
@@ -121,18 +122,23 @@ def prepared_call(model, s, fx, hs, as_, T_tab, group, R, seed=1, lib=None):
     pc = torch.empty((T_tab, t.num_positions), dtype=torch.int64, device="cuda")
     bc = torch.empty((T_tab, t.num_points_bins), dtype=torch.int64, device="cuda")
     inv = torch.empty(1, dtype=torch.int64, device="cuda")
-    need = int(lib.bplx_simulate_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t)))
+    rk = _abi.Ranking(_abi.RANK_HEAD_TO_HEAD, None)
+    if head_to_head:
+        need = int(lib.bplx_simulate_table_ex_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t), C.byref(rk)))
+    else:
+        need = int(lib.bplx_simulate_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t)))
     ws = torch.empty(need, dtype=torch.uint8, device="cuda")
     stream = torch.cuda.current_stream().cuda_stream
-    args = (C.byref(st), C.byref(ft), d_hs, d_as, C.byref(t), 15, R, seed, 0, ptr(pc), ptr(bc), None, None, ptr(inv),
-            ptr(ws), ws.numel(), stream)
+    args = (C.byref(st), C.byref(ft), d_hs, d_as, C.byref(t)) + ((C.byref(rk),) if head_to_head else ()) + (
+        15, R, seed, 0, ptr(pc), ptr(bc), None, None, ptr(inv), ptr(ws), ws.numel(), stream)
+    fn = lib.bplx_simulate_table_ex if head_to_head else lib.bplx_simulate_table
 
     def call():
-        rc = lib.bplx_simulate_table(*args)
+        rc = fn(*args)
         if rc != _abi.OK:
             raise _abi.BplxError(rc, lib.bplx_last_error().decode("utf-8", "replace"))
 
-    return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, tab, ws)
+    return call, {"position_counts": pc, "points_counts": bc, "invalid": inv}, (keep, st, ft, t, dev, dfx, tab, ws, rk)
 
 
 def time_ms(fn, reps):
@@ -174,11 +180,14 @@ def main():
             if base is not None:
                 bcall, bout, _bk = prepared_call(model, s, fx, hs, as_, T_tab, group, R, lib=base)
                 calls.append(bcall)
+            hcall, hout, _hk = prepared_call(model, s, fx, hs, as_, T_tab, group, R, head_to_head=True)
+            calls.append(hcall)
             for _ in range(3):
                 for c in calls:
                     c()
             torch.cuda.synchronize()
-            assert int(out["invalid"].item()) == 0
+            assert int(out["invalid"].item()) == 0 and int(hout["invalid"].item()) == 0
+            assert torch.equal(out["points_counts"], hout["points_counts"])  # the rule moves positions only
             if base is not None:
                 for k in ("position_counts", "points_counts", "invalid"):
                     assert torch.equal(out[k], bout[k]), k
@@ -193,6 +202,8 @@ def main():
                          "scores_per_s": N * F / (ms * 1e-3)})
             if base is not None:
                 rows[-1].update(baseline_ms=min(ms_all[1]), baseline_ms_all=ms_all[1])
+            rows[-1].update(h2h_ms=min(ms_all[-1]), h2h_ms_all=ms_all[-1], h2h_cost=min(ms_all[-1]) / ms - 1,
+                            h2h_changed_positions=int((out["position_counts"] != hout["position_counts"]).sum()))
             print(json.dumps(rows[-1]), flush=True)
 
     # the float64 oracle on the CPU: 2 draws x 64 simulations of the F = 380 league

@@ -18,7 +18,9 @@ Workloads (synthetic posterior draws, fixed seeds):
              priced against a one-match tie per (simulation, tie).
 The world-cup calls go through bplx_simulate_tournament_ex (tie_format all 0, decided_counts on: what
 problem.simulate_tournament issues).  With --baseline-lib, another build's bplx_simulate_tournament is timed on the
-same world-cup call, alternating with this build's, and its counts are checked equal.
+same world-cup call, alternating with this build's, and its counts are checked equal.  The world-cup group stage and
+tournament are also timed under the head-to-head ranking rule (bplx_simulate_table_ex / _tournament_ranked, no played
+matches), alternating with the goal-difference calls in the same run: h2h_*_ms and h2h_*_cost.
 CUDA events around `--reps` calls after warm-up; a call is the whole entry point (count resets, exponential-table
 pre-pass, kernel), issued straight through the C ABI.  Reports the GPU name and power limit read in the same run and
 the shared memory per CTA of both kernels at the world-cup shape.
@@ -113,9 +115,10 @@ def champions_league(S):
     return s, fx, hs.astype(np.uint8), as_.astype(np.uint8), br
 
 
-def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1, lib=None):
+def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1, lib=None, head_to_head=False):
     """The bplx_simulate_tournament_ex call (the bracket's tie_format, decided_counts on) with every argument built once;
-    returns (call, outputs, keep-alive).  ``lib``: another build's library, called through its bplx_simulate_tournament."""
+    returns (call, outputs, keep-alive).  ``lib``: another build's library, called through its bplx_simulate_tournament.
+    ``head_to_head``: bplx_simulate_tournament_ranked under that ranking rule."""
     import torch
 
     from bpl_next_b200 import _abi, problem
@@ -139,7 +142,12 @@ def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1, lib=None
     cnt = {k: torch.empty(n, dtype=torch.int64, device="cuda") for k, n in
            (("pos", T_tab * t.num_positions), ("pts", T_tab * t.num_points_bins), ("reach", T_tab * b.num_rounds),
             ("win", T_tab * b.num_rounds), ("decided", 3 * b.num_ties), ("invalid", 1))}
-    need = int(lib.bplx_simulate_tournament_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t), C.byref(b)))
+    rk = _abi.Ranking(_abi.RANK_HEAD_TO_HEAD, None)
+    if head_to_head:
+        need = int(lib.bplx_simulate_tournament_ranked_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t),
+                                                                        C.byref(b), C.byref(rk)))
+    else:
+        need = int(lib.bplx_simulate_tournament_workspace_bytes(C.byref(st), C.byref(ft), C.byref(t), C.byref(b)))
     ws = torch.empty(need, dtype=torch.uint8, device="cuda")
     stream = torch.cuda.current_stream().cuda_stream
     head = (C.byref(st), C.byref(ft), d_hs, d_as, C.byref(t), C.byref(b))
@@ -155,13 +163,15 @@ def tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, seed=1, lib=None
                                                             ptr(cnt["pts"]), ptr(cnt["reach"]), ptr(cnt["win"]),
                                                             ptr(cnt["decided"]), None, None, None, None, None,
                                                             None) + tail
+        if head_to_head:
+            fn, args = lib.bplx_simulate_tournament_ranked, args[:7] + (C.byref(rk),) + args[7:]
 
     def call():
         rc = fn(*args)
         if rc != _abi.OK:
             raise _abi.BplxError(rc, lib.bplx_last_error().decode("utf-8", "replace"))
 
-    return call, cnt, (keep, st, ft, t, b, dev, tab, ws)
+    return call, cnt, (keep, st, ft, t, b, dev, tab, ws, rk)
 
 
 def smem_bytes(T_tab, P, B, nr=0, K=0):
@@ -205,11 +215,17 @@ def main():
         if base is not None:
             bcall, bout, _bk = tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, lib=base)
             calls.append(bcall)
+        # the group stage and the tournament under the head-to-head rule: the last two calls
+        hgcall, hgout, _hgk = prepared_call(model, s, fx, hs, as_, T_tab, group, R, head_to_head=True)
+        htcall, htout, _htk = tournament_call(model, s, fx, hs, as_, T_tab, group, br, R, head_to_head=True)
+        calls += [hgcall, htcall]
         for _ in range(3):
             for c in calls:
                 c()
         torch.cuda.synchronize()
         assert int(gout["invalid"].item()) == 0 and int(tout["invalid"].item()) == 0
+        assert int(hgout["invalid"].item()) == 0 and int(htout["invalid"].item()) == 0
+        assert torch.equal(hgout["position_counts"].flatten(), htout["pos"])
         assert torch.equal(gout["position_counts"].flatten(), tout["pos"])
         if base is not None:
             for k in ("pos", "pts", "reach", "win", "invalid"):
@@ -226,6 +242,9 @@ def main():
                      "ps_per_sim_tie": (t - g) * 1e9 / (N * K), "tournaments_per_s": N / (t * 1e-3)})
         if base is not None:
             rows[-1].update(baseline_tournament_ms=min(ms[2]), baseline_tournament_ms_all=ms[2])
+        hg, ht = min(ms[-2]), min(ms[-1])
+        rows[-1].update(h2h_group_stage_ms=hg, h2h_tournament_ms=ht, h2h_group_stage_ms_all=ms[-2],
+                        h2h_tournament_ms_all=ms[-1], h2h_group_stage_cost=hg / g - 1, h2h_tournament_cost=ht / t - 1)
         print(json.dumps(rows[-1]), flush=True)
     # the Champions League: its bracket with the real formats and with every tie one match, the league phase alone
     s_cl, fx_cl, hs_cl, as_cl, br_cl = champions_league(S)

@@ -229,7 +229,7 @@ __device__ __forceinline__ void walk16(uint32_t& a, const uint32_t e_end, F&& it
 // min(x, 15) = x and every guard true, bit for bit, minus the instructions.
 enum { kTauPlain = 0, kTauUnclipped = 1, kTauClipped = 2 };
 template <int MODE>
-__device__ __forceinline__ void tau_piece(uint32_t& a, const Hdr& L, const float2 own, const bool home, const float cc,
+__device__ __forceinline__ void tau_terms(uint32_t& a, const Hdr& L, const float2 own, const bool home, const float cc,
                                           const uint32_t tab, float& lt_out, float& du_out, float& gx_out, float& gy_out) {
   // every 16 bytes hold two entries (opponent row offset, w): their arithmetic runs as packed pairs (.x = first entry)
   const float2 one = make_float2(1.0f, 1.0f);
@@ -295,6 +295,15 @@ __device__ __forceinline__ void tau_piece(uint32_t& a, const Hdr& L, const float
   du_out = u1[0] + u1[1] - uxy_s;
   gx_out = cc * (s1[0] - sx);
   gy_out = cc * (s1[1] - sy);
+}
+// Home and away lists get their own copy of the walk, with `home` a constant: an away list then issues none of the
+// predicated-off MUFU.LG2 / FFMA2 that one shared walk carries through it (2 + 1 issue slots per item).  Same arithmetic,
+// same bits.
+template <int MODE>
+__device__ __forceinline__ void tau_piece(uint32_t& a, const Hdr& L, const float2 own, const bool home, const float cc,
+                                          const uint32_t tab, float& lt_out, float& du_out, float& gx_out, float& gy_out) {
+  if (home) tau_terms<MODE>(a, L, own, true, cc, tab, lt_out, du_out, gx_out, gy_out);
+  else tau_terms<MODE>(a, L, own, false, cc, tab, lt_out, du_out, gx_out, gy_out);
 }
 
 // the two arg-max matches of a chain (SURVEY Appendix B.3), as every warp needs them in the team pass

@@ -10,7 +10,7 @@ __version__ = "0.1.0"
 
 def __getattr__(name):  # lazy: importing torch is slow and not needed for host-only users
     if name in ("Problem", "score_grid", "score_grid_host", "pointwise_loglik", "psis_loo",
-                "simulate_table", "simulate_tournament"):
+                "simulate_table", "simulate_tournament", "posterior_predictive"):
         from . import problem
         return getattr(problem, name)
     if name in ("DixonColesMatchPredictor", "ExtendedDixonColesMatchPredictor", "NeutralDixonColesMatchPredictor",

@@ -80,6 +80,14 @@ class Ranking(C.Structure):
     _fields_ = [("rule", C.c_int32), ("played_h2h", C.c_void_p)]
 
 
+class PpcOutput(C.Structure):
+    _fields_ = [
+        ("score_counts", C.c_void_p), ("outcome_counts", C.c_void_p), ("goals", C.c_void_p),
+        ("total_goals_sq", C.c_void_p), ("team_points", C.c_void_p), ("team_goals_for", C.c_void_p),
+        ("team_goals_against", C.c_void_p), ("scores", C.c_void_p), ("invalid", C.c_void_p),
+    ]
+
+
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
@@ -174,6 +182,11 @@ def declare(lib):
                                                     C.c_longlong, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                                     sz, vp]
     lib.bplx_simulate_tournament_ranked.restype = i
+    lib.bplx_posterior_predictive_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Observations)]
+    lib.bplx_posterior_predictive_workspace_bytes.restype = sz
+    lib.bplx_posterior_predictive.argtypes = [C.POINTER(Samples), C.POINTER(Observations), i, i, i, i, i, C.c_ulonglong,
+                                              C.c_longlong, C.POINTER(PpcOutput), vp, sz, vp]
+    lib.bplx_posterior_predictive.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

@@ -8,8 +8,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "lib", "libbplx.so")
-SOURCES = ["api.cu", "logdensity.cu", "logdensity_dynamic.cu", "score_grid.cu", "loo.cu", "simulate.cu", "nuts.cu", "peer_sum.cu", "plan.cc"]
-HEADERS = ["common.cuh", "k1_common.cuh", "plan.h", "plan_dynamic.inc", "problem.h", "score_grid.h", "loo.h", "simulate.h", "simulate_body.inc", "nuts.h", os.path.join("..", "..", "include", "bplx_nuts.h"), os.path.join("..", "..", "include", "bplx.h")]
+SOURCES = ["api.cu", "logdensity.cu", "logdensity_dynamic.cu", "score_grid.cu", "loo.cu", "simulate.cu", "ppc.cu", "nuts.cu", "peer_sum.cu", "plan.cc"]
+HEADERS = ["common.cuh", "k1_common.cuh", "plan.h", "plan_dynamic.inc", "problem.h", "score_grid.h", "loo.h", "simulate.h", "simulate_body.inc", "sample_score.cuh", "ppc.h", "nuts.h", os.path.join("..", "..", "include", "bplx_nuts.h"), os.path.join("..", "..", "include", "bplx.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

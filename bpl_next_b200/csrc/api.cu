@@ -13,6 +13,7 @@
 #include "plan.h"
 #include "problem.h"
 #include "loo.h"
+#include "ppc.h"
 #include "score_grid.h"
 #include "simulate.h"
 
@@ -1132,6 +1133,69 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
                                      first_draw, position_counts, points_counts, reach_counts, win_counts, nullptr,
                                      positions, scores, ko_entrants, ko_scores, ko_winners, nullptr, invalid, workspace,
                                      workspace_bytes, stream);
+}
+
+// ---- posterior predictive checks ------------------------------------------------------------------------------
+// the workspace is the [S][row_floats] exponential table, as for a simulation
+size_t bplx_posterior_predictive_workspace_bytes(const bplx_samples* s, const bplx_observations* obs) {
+  if (!s || !obs || s->num_samples <= 0 || s->num_teams <= 0 || obs->fixtures.num_fixtures <= 0) return 0;
+  GridParams gp{};
+  bind_samples(s, &obs->fixtures, &gp);
+  return table_layout(&gp);
+}
+
+int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* obs, int max_goals, int score_bins,
+                              int points_win, int points_draw, int sims_per_draw, unsigned long long seed,
+                              long long first_draw, const bplx_ppc_output* out, void* workspace,
+                              size_t workspace_bytes, void* stream) {
+  const char* what = "posterior predictive";
+  BPLX_REQUIRE(obs != nullptr && out != nullptr, BPLX_E_INVALID, "%s: observations / out is NULL", what);
+  int rc = check_sample_args(s, &obs->fixtures, what);
+  if (rc != BPLX_OK) return rc;
+  const int M = obs->fixtures.num_fixtures;
+  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
+               what);
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
+               max_goals);
+  BPLX_REQUIRE(score_bins >= 2 && score_bins <= 16, BPLX_E_INVALID, "%s: score_bins must be in [2, 16] (got %d)", what,
+               score_bins);
+  BPLX_REQUIRE(points_win >= 1 && points_draw >= 0 && points_draw <= points_win, BPLX_E_INVALID,
+               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
+               points_win, points_draw);
+  BPLX_REQUIRE((long long)std::max(points_win, max_goals) * M <= INT_MAX, BPLX_E_INVALID,
+               "%s: max(points_win, max_goals) * num_matches must be below 2^31 (a team count could overflow)", what);
+  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
+  BPLX_REQUIRE(first_draw >= 0 && first_draw + s->num_samples <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
+               "%s: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits", what);
+  BPLX_REQUIRE((long long)s->num_samples * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
+               "%s: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
+               what, (long long)s->num_samples * sims_per_draw);
+  BPLX_REQUIRE(out->score_counts && out->outcome_counts && out->goals && out->total_goals_sq && out->team_points &&
+                   out->team_goals_for && out->team_goals_against && out->invalid,
+               BPLX_E_INVALID, "%s: every output but scores must be given", what);
+  PpcParams pp{};
+  bind_samples(s, &obs->fixtures, &pp.gp);
+  rc = check_workspace(workspace, workspace_bytes, table_layout(&pp.gp));
+  if (rc != BPLX_OK) return rc;
+  pp.gp.table = static_cast<float*>(workspace);
+  pp.G = max_goals;
+  pp.B = score_bins;
+  pp.R = sims_per_draw;
+  pp.pw = points_win;
+  pp.pd = points_draw;
+  pp.seed = seed;
+  pp.first_draw = first_draw;
+  pp.N = s->num_samples * sims_per_draw;
+  pp.score_counts = out->score_counts;
+  pp.outcome_counts = out->outcome_counts;
+  pp.goals = reinterpret_cast<long long*>(out->goals);
+  pp.total_goals_sq = reinterpret_cast<long long*>(out->total_goals_sq);
+  pp.team_points = out->team_points;
+  pp.team_goals_for = out->team_goals_for;
+  pp.team_goals_against = out->team_goals_against;
+  pp.scores = out->scores;
+  pp.invalid = out->invalid;
+  return launch_ppc(pp, static_cast<cudaStream_t>(stream));
 }
 
 void bplx_reload_env(void) {

@@ -391,6 +391,73 @@ class _BplxPredictor:
         lppd = bcompare.lppd_from_stats(st.cpu().numpy(), int(ds["attack"].shape[0]))
         return {"log_score": float(lppd.sum()), "pointwise": lppd, "num_matches": len(lppd)}
 
+    # ---- posterior predictive checks ------------------------------------------------------------------------------
+    def posterior_predictive_check(self, data=None, num_sims_per_draw: int = 1, random_state: Optional[int] = None,
+                                   max_goals: int = MAX_GOALS, score_bins: int = 6, points=(3, 1),
+                                   return_replicates: bool = False) -> Dict[str, Any]:
+        """Does the fit reproduce the data? Replicated datasets of the observed matches of ``data`` (reference
+        ``training_data`` keys; default: the training data) are drawn on the GPU, one posterior draw per replicate, and
+        their statistics are set beside those of the observed scores.
+
+        Replicate ``n = (first_draw + s) R + r`` (R = ``num_sims_per_draw``) uses draw s; every match of it is drawn by
+        ``simulate_table``'s sampler (the draw's own grid up to ``max_goals``, tau clamped at 0, normalised by its sum;
+        the rates of ``predict_*``), from Philox words 2m and 2m + 1 of ``curand_init(seed, n, 0)``, so with the same
+        seed and matches the replicated scores are ``simulate_table``'s.  Match weights are ignored: for a time-decayed
+        fit every match counts equally; pass ``data`` (the last season, say) to check recent form.
+
+        Statistics: ``score_counts [B, B]`` (matches per cell ``min(hg, B-1), min(ag, B-1)``, B = ``score_bins``: with 6,
+        0-4 and "5+"), ``outcome_counts [3]`` (home wins, draws, away wins), ``goals [2]`` (home, away),
+        ``total_goals_sq`` (sum of squared match totals), ``total_goals_dispersion`` (variance over mean of total goals
+        per match: 1 for Poisson totals), and per team ``team_points`` (``points`` = (win, draw)), ``team_goals_for``,
+        ``team_goals_against [T]`` in the order of ``teams``.  Each maps to ``observed``, ``mean`` and ``sd`` over the
+        N = S R replicates and ``p_value``, the mid-p ``P(T_rep > T_obs) + 1/2 P(T_rep = T_obs)``: near 0.5 the data
+        sit inside what the model predicts, near 0 or 1 the model misses (a team with no matches gets 0.5).  Observed
+        goals above ``max_goals`` count as they are; replicated goals cannot exceed it.
+
+        Also returned: ``teams``, ``score_bins``, ``max_goals``, ``num_replicates``, ``sims_per_draw``, ``seed`` (from
+        the clock when ``random_state`` is None; pass it back to repeat the run) and ``match_key`` (names the matches).
+        With ``return_replicates``, ``replicates`` (each statistic per replicate, ``[N, ...]``) and ``home_score`` /
+        ``away_score [M, N]`` (``sample_score``'s shape).  The draws run in ranges within ``SIM_OUTPUT_BYTES`` of device
+        output; the results do not depend on the range size.  Raises if a replicate met a non-finite rate."""
+        if self.teams is None:
+            raise ValueError("the model is not fitted: fit it first")
+        from . import ppc as bppc
+        from .problem import posterior_predictive
+
+        seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
+        R, B = int(num_sims_per_draw), int(score_bins)
+        if R < 1:
+            raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
+        ds, do, key = self._comparison_inputs(data)
+        S, T, M = int(ds["attack"].shape[0]), int(ds["attack"].shape[1]), int(do["home_team"].shape[0])
+        step = (2 ** 31 - 1) // R  # replicates per call stay below 2^31
+        per_rep = 4 * (B * B + 3 + 3 * T) + 8 * 3 + (2 * M if return_replicates else 0)  # device output bytes
+        step = min(step, max(1, SIM_OUTPUT_BYTES // (R * per_rep)))
+        parts, scores, invalid = [], [], 0
+        for lo in range(0, S, step):
+            hi = min(S, lo + step)
+            out = posterior_predictive(self.model, {k: v[lo:hi] for k, v in ds.items()}, do, max_goals, B, points, R,
+                                       seed, first_draw=lo, want_scores=return_replicates)
+            invalid += int(out["invalid"].item())
+            parts.append({k: out[k].cpu().numpy() for k in bppc.STATISTICS})
+            if return_replicates:
+                scores.append(out["scores"].cpu().numpy())
+        N = S * R
+        if invalid:
+            raise ValueError(f"{invalid} of {N} replicates met a non-finite scoring rate or score-grid normaliser: "
+                             "check the posterior draws")
+        reps = {k: np.concatenate([p[k] for p in parts]) for k in bppc.STATISTICS}
+        h = {k: do[k].cpu().numpy() for k in ("home_team", "away_team", "home_goals", "away_goals")}
+        observed = bppc.statistics(h["home_team"], h["away_team"], h["home_goals"], h["away_goals"], T, B, points)
+        res = bppc.summarize(observed, reps, M)
+        res.update(teams=list(np.asarray(self.teams).tolist()), score_bins=B, max_goals=int(max_goals),
+                   num_replicates=N, sims_per_draw=R, seed=seed, match_key=key)
+        if return_replicates:
+            sc = np.concatenate(scores)
+            res.update(replicates=reps, home_score=np.ascontiguousarray(sc[:, :, 0].T),
+                       away_score=np.ascontiguousarray(sc[:, :, 1].T))
+        return res
+
     # ---- simulation from the grid (bpl/base.py:150-246, bpl/_util.py:96-112) -----------------------------------
     @staticmethod
     def _choice(probs: np.ndarray, num_samples: int, random_state) -> np.ndarray:
@@ -926,6 +993,10 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
     def simulate_tournament(self, *args, **kwargs):
         raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
                                   "cannot run in the reference (SURVEY.md D3)")
+
+    def posterior_predictive_check(self, *args, **kwargs):
+        raise NotImplementedError("posterior predictive checks need the predictive distribution, and the dynamic model's "
+                                  "predict methods cannot run in the reference (SURVEY.md D3)")
 
     def _comparison_inputs(self, data):
         raise NotImplementedError("model comparison needs the predictive distribution, and the dynamic model's predict "

@@ -1,5 +1,5 @@
 """Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik``,
-``psis_loo`` and ``simulate_table``.
+``psis_loo``, ``simulate_table``, ``simulate_tournament`` and ``posterior_predictive``.
 
 torch is used only for device memory and streams; every number comes from ``libbplx.so``.
 """
@@ -498,3 +498,51 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     _abi.check(run(*args, int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
                    *outputs, _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
     return out
+
+
+
+def posterior_predictive(model: str, samples: Dict[str, torch.Tensor], observations: Dict[str, torch.Tensor],
+                         max_goals: int = 15, score_bins: int = 6, points=(3, 1), sims_per_draw: int = 1, seed: int = 0,
+                         first_draw: int = 0, want_scores: bool = False, workspace=None,
+                         stream=None) -> Dict[str, Optional[torch.Tensor]]:
+    """Device path of ``bplx_posterior_predictive``: replicated datasets of the observed matches, one posterior draw per
+    replicate, each reduced to its statistics on the GPU.
+
+    ``samples``: posterior arrays ``[S, T]`` on the GPU (the draws of this call; ``first_draw`` is the global index of
+    the first one).  ``observations``: the index tensors of ``score_grid`` plus ``home_goals`` / ``away_goals`` (uint8),
+    as for ``pointwise_loglik``.
+
+    Replicate ``n = (first_draw + s) R + r`` (R = ``sims_per_draw``) uses draw s; words 2m and 2m + 1 of
+    ``curand_init(seed, n, 0)`` sample match m's score with the season simulation's sampler (the draw's own grid up to
+    ``max_goals``, tau clamped at 0, normalised by its sum), so with the same seed, draws and matches the scores equal
+    ``simulate_table``'s.  Match weights are ignored.  Returns per replicate (row ``s R + r``, N = S R):
+    ``score_counts [N, B, B]`` (cells ``min(hg, B-1), min(ag, B-1)``, B = ``score_bins``), ``outcome_counts [N, 3]``
+    (home wins, draws, away wins), ``team_points``, ``team_goals_for``, ``team_goals_against [N, T]`` (int32),
+    ``goals [N, 2]`` (home, away) and ``total_goals_sq [N]`` (sum of squared match totals; int64); ``invalid`` (int64
+    ``[1]``: replicates with a non-finite rate or normaliser, whose rows are -1), and when ``want_scores`` the raw
+    ``scores [N, M, 2]`` (uint8; 255 marks the match that made a replicate invalid)."""
+    lib = _abi.lib()
+    keep = []
+    ptr = _device_ptr_fn(keep)
+    _check_inputs(samples, observations, ("home_goals", "away_goals"))
+    s = _samples_struct(model, samples, ptr)
+    o = _abi.Observations()
+    o.fixtures = _fixtures_struct(observations, ptr)
+    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    M, S, T, B = o.fixtures.num_fixtures, s.num_samples, s.num_teams, int(score_bins)
+    N = S * int(sims_per_draw)
+    dev = samples["attack"].device
+    workspace = _workspace(workspace, int(lib.bplx_posterior_predictive_workspace_bytes(C.byref(s), C.byref(o))), dev)
+    i32, i64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.int64, device=dev)
+    shapes = {"score_counts": ((N, B, B), i32), "outcome_counts": ((N, 3), i32), "goals": ((N, 2), i64),
+              "total_goals_sq": ((N,), i64), "team_points": ((N, T), i32), "team_goals_for": ((N, T), i32),
+              "team_goals_against": ((N, T), i32)}
+    res = {k: torch.empty(shp, **kw) for k, (shp, kw) in shapes.items()}
+    res["invalid"] = torch.empty(1, **i64)
+    res["scores"] = torch.empty((N, M, 2), dtype=torch.uint8, device=dev) if want_scores else None
+    out = _abi.PpcOutput(**{k: _dptr(v) for k, v in res.items()})
+    pw, pd = (int(x) for x in points)
+    _abi.check(lib.bplx_posterior_predictive(C.byref(s), C.byref(o), int(max_goals), B, pw, pd, int(sims_per_draw),
+                                             int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw), C.byref(out),
+                                             _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    return res

@@ -498,6 +498,58 @@ int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* 
                                     uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
                                     void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- posterior predictive checks: replicated scores of the observed matches and their statistics ------------ */
+/*
+ * Replicate and random numbers.  Replicate n = (first_draw + s) * R + r (R = sims_per_draw) uses posterior draw s.  Its
+ * random numbers are curand_init(seed, n, 0) followed by curand() (Philox4_32_10).  Words 2m and 2m + 1 become u_h and
+ * u_a of observed match m through curand_uniform.  These are exactly the word addresses bplx_simulate_table gives
+ * fixture f.
+ *
+ * One match of one replicate.  The score is drawn by the season simulation's sampler, unchanged: the predict path's
+ * rates (neutral venues and confederations included, Extended's clip not applied); the draw's own grid up to max_goals
+ * (1..63), with tau clamped at 0, normalised by its sum; inverse CDF over home goals, then over away goals given home
+ * goals.  As a result, with the same seed, draws and matches, the replicated scores equal bplx_simulate_table's scores.
+ * A replicate that meets a non-finite rate or normaliser is counted in `invalid`, as in simulation.  Match weights are
+ * ignored, as in bplx_pointwise_loglik.
+ *
+ * Statistics per replicate.  All are integers, so device atomics give the same bits in any order:
+ *   score_counts [B, B]         matches with min(hg, B - 1) = i, min(ag, B - 1) = j (B = score_bins, 2..16)
+ *   outcome_counts [3]          home wins, draws, away wins ("home" = the listed home team, neutral venue or not)
+ *   goals [2]                   total home goals, total away goals
+ *   total_goals_sq []           sum_m (hg + ag)^2
+ *   team_points [T]             points of each model team over the matches (points_win for a win, points_draw for a draw)
+ *   team_goals_for [T], team_goals_against [T]   per model team
+ * Replicated goals cannot exceed max_goals.  The host computes the dispersion of total goals, the statistics of the
+ * observed scores and the posterior predictive p-values (bpl_next_b200/ppc.py).
+ *
+ * Outputs (device; overwritten): row q = s * R + r of this call, q < N = num_samples * R.  An invalid replicate (also: a
+ * match naming a team >= num_teams or a confederation >= num_conferences) has -1 in every statistic of its row and
+ * 0xFF as the scores of the offending match.  scores [N, M, 2] uint8 (home, away) is optional, in the layout of
+ * bplx_simulate_table's scores.  The statistics depend neither on the launch geometry nor on the draw range of the
+ * call: calls on draws [0, k) and [k, S) give the rows of the single call.  The workspace holds the [S, row]
+ * exponential table of bplx_score_grid's pre-pass (bplx_posterior_predictive_workspace_bytes).
+ * Refusals: DYNAMIC, N >= 2^31, or more teams than one CTA's shared memory holds (about 6,000): BPLX_E_UNSUPPORTED;
+ * max_goals outside 1..63, score_bins outside 2..16, R < 1, missing goals or outputs, points outside 0 <= points_draw <=
+ * points_win, points_win >= 1, or max(points_win, max_goals) * M >= 2^31 (a count that could overflow): BPLX_E_INVALID.
+ */
+typedef struct {
+  int32_t* score_counts;          /* device [N, B, B] */
+  int32_t* outcome_counts;        /* device [N, 3] */
+  int64_t* goals;                 /* device [N, 2] */
+  int64_t* total_goals_sq;        /* device [N] */
+  int32_t* team_points;           /* device [N, T] */
+  int32_t* team_goals_for;        /* device [N, T] */
+  int32_t* team_goals_against;    /* device [N, T] */
+  uint8_t* scores;                /* device [N, M, 2] or NULL */
+  unsigned long long* invalid;    /* device [1]: invalid replicates */
+} bplx_ppc_output;
+
+size_t bplx_posterior_predictive_workspace_bytes(const bplx_samples* s, const bplx_observations* obs);
+int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* obs, int max_goals, int score_bins,
+                              int points_win, int points_draw, int sims_per_draw, unsigned long long seed,
+                              long long first_draw, const bplx_ppc_output* out, void* workspace,
+                              size_t workspace_bytes, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

@@ -298,6 +298,25 @@ def _idx(a):
     return torch.as_tensor(np.asarray(a, dtype=np.int64))
 
 
+_tap: Optional[list] = None  # while set (``_prior_terms``), every prior and Jacobian term a model adds is appended
+
+
+def _term(x, parts=None):
+    """One group of elementary prior / Jacobian terms (one per element of ``x``), as the model adds it to lp; ``parts``
+    (summing to ``x``) are recorded in its place when ``x`` cancels inside itself."""
+    if _tap is not None:
+        _tap.extend([x] if parts is None else parts)
+    return x
+
+
+def _conditional_normal(zd, loc, s2):
+    """N(zd | loc, sqrt(s2)) log-prob; recorded as the parts of its expanded square, so that the error scale sees
+    zd and loc rather than their (possibly cancelling) difference."""
+    x = _normal_lp(zd, loc, torch.sqrt(s2))
+    parts = [-0.5 * zd * zd / s2, zd * loc / s2, -0.5 * loc * loc / s2, -0.5 * torch.log(s2) - LOG_SQRT_2PI]
+    return _term(x, [p.expand_as(x) for p in parts])
+
+
 def _prior_means(d: MatchData, mean_defence, beta_a, beta_d, dtype):
     """Attack/defence prior means, with covariates ``extended_dixon_coles.py:123-146``."""
     if d.covariates is not None:
@@ -319,17 +338,17 @@ def _dixon_coles(d: MatchData, theta):
     T = d.num_teams
     s = _split(theta, site_layout("dixon_coles", T))
     dt = theta.dtype
-    lp = _normal_lp(s["home_advantage"], 0.1, 0.2) + _normal_lp(s["mean_defence"], 0.0, 1.0)
-    std_a, j = _exp_site(s["std_attack"]); lp = lp + _halfnormal_lp(std_a, 1.0) + j
-    std_d, j = _exp_site(s["std_defence"]); lp = lp + _halfnormal_lp(std_d, 1.0) + j
-    lp = lp + _normal_lp(s["attack_decentered"], 0.0, 1.0).sum(-1)
-    lp = lp + _normal_lp(s["defence_decentered"], 0.0, 1.0).sum(-1)
+    lp = _term(_normal_lp(s["home_advantage"], 0.1, 0.2)) + _term(_normal_lp(s["mean_defence"], 0.0, 1.0))
+    std_a, j = _exp_site(s["std_attack"]); lp = lp + _term(_halfnormal_lp(std_a, 1.0)) + _term(j)
+    std_d, j = _exp_site(s["std_defence"]); lp = lp + _term(_halfnormal_lp(std_d, 1.0)) + _term(j)
+    lp = lp + _term(_normal_lp(s["attack_decentered"], 0.0, 1.0)).sum(-1)
+    lp = lp + _term(_normal_lp(s["defence_decentered"], 0.0, 1.0)).sum(-1)
     attack = 0.0 + std_a[..., None] * s["attack_decentered"]
     defence = s["mean_defence"][..., None] + std_d[..., None] * s["defence_decentered"]
     h, a = _idx(d.home_team), _idx(d.away_team)
     lam_h = torch.exp(attack[..., h] - defence[..., a] + s["home_advantage"][..., None])
     lam_a = torch.exp(attack[..., a] - defence[..., h])
-    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _beta_lp(raw, 2.0, 2.0) + j
+    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _term(_beta_lp(raw, 2.0, 2.0)) + _term(j)
     ll, cc = _likelihood(d, lam_h, lam_a, raw, dt)
     return lp + ll, {"attack": attack, "defence": defence, "home_advantage": s["home_advantage"],
                      "corr_coef": cc, "lam_h": lam_h, "lam_a": lam_a}
@@ -338,11 +357,11 @@ def _dixon_coles(d: MatchData, theta):
 def _rho_block(s, lp):
     """u ~ Beta(2,4), rho = 2u-1, za ~ N(0,1), zd ~ N(rho za, sqrt(1-rho^2))
     (``extended_dixon_coles.py:152-174``)."""
-    u, j = _sigmoid_site(s["u"]); lp = lp + _beta_lp(u, 2.0, 4.0) + j
+    u, j = _sigmoid_site(s["u"]); lp = lp + _term(_beta_lp(u, 2.0, 4.0)) + _term(j)
     rho = 2.0 * u - 1.0
     za, zd = s["standardised_attack"], s["standardised_defence"]
-    lp = lp + _normal_lp(za, 0.0, 1.0).sum(-1)
-    lp = lp + _normal_lp(zd, rho[..., None] * za, torch.sqrt(1.0 - rho**2.0)[..., None]).sum(-1)
+    lp = lp + _term(_normal_lp(za, 0.0, 1.0)).sum(-1)
+    lp = lp + _conditional_normal(zd, rho[..., None] * za, (1.0 - rho**2.0)[..., None]).sum(-1)
     return lp, rho
 
 
@@ -351,17 +370,17 @@ def _extended(d: MatchData, theta):
     T, K = d.num_teams, d.num_covariates
     s = _split(theta, site_layout("extended", T, K))
     dt = theta.dtype
-    lp = _normal_lp(s["mean_home_advantage"], 0.1, 0.2)
-    std_ha, j = _exp_site(s["std_home_advantage"]); lp = lp + _halfnormal_lp(std_ha, 1.0) + j
-    lp = lp + _normal_lp(s["mean_defence"], 0.0, 1.0)
-    std_a, j = _exp_site(s["std_attack"]); lp = lp + _halfnormal_lp(std_a, 1.0) + j
-    std_d, j = _exp_site(s["std_defence"]); lp = lp + _halfnormal_lp(std_d, 1.0) + j
+    lp = _term(_normal_lp(s["mean_home_advantage"], 0.1, 0.2))
+    std_ha, j = _exp_site(s["std_home_advantage"]); lp = lp + _term(_halfnormal_lp(std_ha, 1.0)) + _term(j)
+    lp = lp + _term(_normal_lp(s["mean_defence"], 0.0, 1.0))
+    std_a, j = _exp_site(s["std_attack"]); lp = lp + _term(_halfnormal_lp(std_a, 1.0)) + _term(j)
+    std_d, j = _exp_site(s["std_defence"]); lp = lp + _term(_halfnormal_lp(std_d, 1.0)) + _term(j)
     if K:
-        lp = lp + _normal_lp(s["attack_coefficients"], 0.0, 1.0).sum(-1)
-        lp = lp + _normal_lp(s["defence_coefficients"], 0.0, 1.0).sum(-1)
+        lp = lp + _term(_normal_lp(s["attack_coefficients"], 0.0, 1.0)).sum(-1)
+        lp = lp + _term(_normal_lp(s["defence_coefficients"], 0.0, 1.0)).sum(-1)
     a_mean, d_mean = _prior_means(d, s["mean_defence"], s["attack_coefficients"], s["defence_coefficients"], dt)
     lp, rho = _rho_block(s, lp)
-    lp = lp + _normal_lp(s["home_advantage_decentered"], 0.0, 1.0).sum(-1)
+    lp = lp + _term(_normal_lp(s["home_advantage_decentered"], 0.0, 1.0)).sum(-1)
     home_adv = s["mean_home_advantage"][..., None] + std_ha[..., None] * s["home_advantage_decentered"]
     attack = a_mean + s["standardised_attack"] * std_a[..., None]
     defence = d_mean + s["standardised_defence"] * std_d[..., None]
@@ -370,7 +389,7 @@ def _extended(d: MatchData, theta):
     lam_a = torch.exp(attack[..., a] - defence[..., h])
     lam_h = torch.clamp(lam_h, max=15.0)  # :197-198
     lam_a = torch.clamp(lam_a, max=15.0)
-    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _beta_lp(raw, 2.0, 2.0) + j
+    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _term(_beta_lp(raw, 2.0, 2.0)) + _term(j)
     ll, cc = _likelihood(d, lam_h, lam_a, raw, dt)
     return lp + ll, {"attack": attack, "defence": defence, "home_advantage": home_adv, "rho": rho,
                      "corr_coef": cc, "lam_h": lam_h, "lam_a": lam_a}
@@ -381,24 +400,24 @@ def _neutral_family(d: MatchData, theta, wc: bool):
     T, K, Cf = d.num_teams, d.num_covariates, (d.num_conferences if wc else 0)
     s = _split(theta, site_layout("neutral_wc" if wc else "neutral", T, K, Cf))
     dt = theta.dtype
-    lp = _normal_lp(s["mean_defence"], 0.0, 1.0)
-    std_a, j = _exp_site(s["std_attack"]); lp = lp + _halfnormal_lp(std_a, 0.5) + j
-    std_d, j = _exp_site(s["std_defence"]); lp = lp + _halfnormal_lp(std_d, 0.5) + j
-    lp = lp + _normal_lp(s["mean_home_attack"], 0.1, 0.2) + _normal_lp(s["mean_away_attack"], -0.1, 0.2)
-    lp = lp + _normal_lp(s["mean_home_defence"], 0.1, 0.2) + _normal_lp(s["mean_away_defence"], -0.1, 0.2)
+    lp = _term(_normal_lp(s["mean_defence"], 0.0, 1.0))
+    std_a, j = _exp_site(s["std_attack"]); lp = lp + _term(_halfnormal_lp(std_a, 0.5)) + _term(j)
+    std_d, j = _exp_site(s["std_defence"]); lp = lp + _term(_halfnormal_lp(std_d, 0.5)) + _term(j)
+    lp = lp + _term(_normal_lp(s["mean_home_attack"], 0.1, 0.2)) + _term(_normal_lp(s["mean_away_attack"], -0.1, 0.2))
+    lp = lp + _term(_normal_lp(s["mean_home_defence"], 0.1, 0.2)) + _term(_normal_lp(s["mean_away_defence"], -0.1, 0.2))
     stds = {}
     for nm in ("home_attack", "away_attack", "home_defence", "away_defence"):
-        v, j = _exp_site(s["std_" + nm]); lp = lp + _halfnormal_lp(v, 1.0) + j
+        v, j = _exp_site(s["std_" + nm]); lp = lp + _term(_halfnormal_lp(v, 1.0)) + _term(j)
         stds[nm] = v
     if K:
-        lp = lp + _normal_lp(s["attack_coefficients"], 0.0, 1.0).sum(-1)
-        lp = lp + _normal_lp(s["defence_coefficients"], 0.0, 1.0).sum(-1)
+        lp = lp + _term(_normal_lp(s["attack_coefficients"], 0.0, 1.0)).sum(-1)
+        lp = lp + _term(_normal_lp(s["defence_coefficients"], 0.0, 1.0)).sum(-1)
     a_mean, d_mean = _prior_means(d, s["mean_defence"], s["attack_coefficients"], s["defence_coefficients"], dt)
     lp, rho = _rho_block(s, lp)
     eff = {}
     for nm in ("home_attack", "away_attack", "home_defence", "away_defence"):
         dec = s[nm + "_decentered"]
-        lp = lp + _normal_lp(dec, 0.0, 1.0).sum(-1)
+        lp = lp + _term(_normal_lp(dec, 0.0, 1.0)).sum(-1)
         eff[nm] = s["mean_" + nm][..., None] + stds[nm][..., None] * dec
     attack = a_mean + s["standardised_attack"] * std_a[..., None]
     defence = d_mean + s["standardised_defence"] * std_d[..., None]
@@ -409,13 +428,13 @@ def _neutral_family(d: MatchData, theta, wc: bool):
     det = {}
     if wc:  # confederation_strength ~ N(0,1), LocScaleReparam -> identity (..._WC.py:180-203)
         conf = s["confederation_strength_decentered"]
-        lp = lp + _normal_lp(conf, 0.0, 1.0).sum(-1)
+        lp = lp + _term(_normal_lp(conf, 0.0, 1.0)).sum(-1)
         hc, ac = _idx(d.home_conf), _idx(d.away_conf)
         eta_h = eta_h + conf[..., hc] - conf[..., ac]
         eta_a = eta_a + conf[..., ac] - conf[..., hc]
         det["confederation_strength"] = conf
     lam_h, lam_a = torch.exp(eta_h), torch.exp(eta_a)
-    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _beta_lp(raw, 2.0, 2.0) + j
+    raw, j = _sigmoid_site(s["corr_coef_raw"]); lp = lp + _term(_beta_lp(raw, 2.0, 2.0)) + _term(j)
     ll, cc = _likelihood(d, lam_h, lam_a, raw, dt)
     det.update({"attack": attack, "defence": defence, "rho": rho, "corr_coef": cc, "lam_h": lam_h,
                 "lam_a": lam_a, **eff})
@@ -433,28 +452,28 @@ def _dynamic(d: MatchData, theta):
     T, K, G = d.num_teams, d.num_covariates, d.num_gameweeks
     s = _split(theta, site_layout("dynamic", T, K, 0, G))
     dt = theta.dtype
-    lp = _normal_lp(s["mean_home_attack"], 0.1, 0.2).sum(-1) + _normal_lp(s["mean_away_attack"], -0.1, 0.2).sum(-1)
-    lp = lp + _normal_lp(s["mean_home_defence"], 0.1, 0.2).sum(-1) + _normal_lp(s["mean_away_defence"], -0.1, 0.2).sum(-1)
+    lp = _term(_normal_lp(s["mean_home_attack"], 0.1, 0.2)).sum(-1) + _term(_normal_lp(s["mean_away_attack"], -0.1, 0.2)).sum(-1)
+    lp = lp + _term(_normal_lp(s["mean_home_defence"], 0.1, 0.2)).sum(-1) + _term(_normal_lp(s["mean_away_defence"], -0.1, 0.2)).sum(-1)
     stds = {}
     for nm in ("home_attack", "away_attack", "home_defence", "away_defence", "attack", "defence"):
         v, j = _exp_site(s["std_" + nm])
-        lp = lp + (_halfnormal_lp(v, 1.0) + j).sum(-1)
+        lp = lp + (_term(_halfnormal_lp(v, 1.0)) + _term(j)).sum(-1)
         stds[nm] = v  # [C, G]
-    lp = lp + _normal_lp(s["mean_defence"], 0.0, 1.0)
+    lp = lp + _term(_normal_lp(s["mean_defence"], 0.0, 1.0))
     if K:
-        lp = lp + _normal_lp(s["attack_coefficients"], 0.0, 1.0).sum(-1)
-        lp = lp + _normal_lp(s["defence_coefficients"], 0.0, 1.0).sum(-1)
+        lp = lp + _term(_normal_lp(s["attack_coefficients"], 0.0, 1.0)).sum(-1)
+        lp = lp + _term(_normal_lp(s["defence_coefficients"], 0.0, 1.0)).sum(-1)
     a_mean, d_mean = _prior_means(d, s["mean_defence"], s["attack_coefficients"], s["defence_coefficients"], dt)
     u, j = _sigmoid_site(s["u"])  # [C, G, T]
-    lp = lp + (_beta_lp(u, 2.0, 4.0) + j).sum((-1, -2))
+    lp = lp + (_term(_beta_lp(u, 2.0, 4.0)) + _term(j)).sum((-1, -2))
     rho = 2.0 * u - 1.0
     za, zd = s["standardised_attack"], s["standardised_defence"]
-    lp = lp + _normal_lp(za, 0.0, 1.0).sum((-1, -2))
-    lp = lp + _normal_lp(zd, rho * za, torch.sqrt(1.0 - rho**2.0)).sum((-1, -2))
+    lp = lp + _term(_normal_lp(za, 0.0, 1.0)).sum((-1, -2))
+    lp = lp + _conditional_normal(zd, rho * za, 1.0 - rho**2.0).sum((-1, -2))
     eff = {}
     for nm in ("home_attack", "away_attack", "home_defence", "away_defence"):
         dec = s[nm + "_decentered"]
-        lp = lp + _normal_lp(dec, 0.0, 1.0).sum((-1, -2))
+        lp = lp + _term(_normal_lp(dec, 0.0, 1.0)).sum((-1, -2))
         eff[nm] = s["mean_" + nm][..., None] + stds[nm][..., None] * dec  # [C, G, T]
     step_a = za * stds["attack"][..., None]
     step_d = zd * stds["defence"][..., None]
@@ -473,7 +492,7 @@ def _dynamic(d: MatchData, theta):
     lam_a = torch.exp(attack[..., g, a] - defence[..., g, h]
                       + n * eff["away_attack"][..., g, a] - n * eff["home_defence"][..., g, h])
     raw, j = _sigmoid_site(s["corr_coef_raw"])  # Uniform(0,1): log_prob 0 (:241)
-    lp = lp + j
+    lp = lp + _term(j)
     ll, cc = _likelihood(d, lam_h, lam_a, raw, dt)
     return lp + ll, {"attack": attack, "defence": defence, "rho": rho, "corr_coef": cc,
                      "lam_h": lam_h, "lam_a": lam_a, **eff}
@@ -500,6 +519,207 @@ def log_density_and_grad(d: MatchData, theta, dtype=torch.float64):
     lp, det = log_density(d, th)
     (g,) = torch.autograd.grad(lp.sum(), th)
     return lp.detach().numpy(), g.numpy(), det["corr_coef"].detach().numpy()
+
+
+# --------------------------------------------------------------------------------------
+# error scale of a float32 evaluation: sum over the elementary terms of |d term / d theta_i|
+# --------------------------------------------------------------------------------------
+def _prior_terms(d: MatchData, theta):
+    """Every prior and Jacobian term of the log density, ``[C, N]`` (the likelihood's terms are not in it)."""
+    global _tap
+    _tap = []
+    try:
+        log_density(d, theta)
+        C = theta.shape[0]
+        return torch.cat([x.reshape(C, -1) for x in _tap], dim=-1)
+    finally:
+        _tap = None
+
+
+def _rate_jacobian(d: MatchData, theta):
+    """d eta / d theta of the log-rates eta_h, eta_a of every match (before any clip), sparse: per side a list of
+    (theta index [M], value [C, M]); row m of the Jacobian is the sum over the list (an index may repeat)."""
+    model, T, K, G = d.model, d.num_teams, d.num_covariates, d.num_gameweeks
+    Cf = d.num_conferences if model == "neutral_wc" else 0
+    lay = site_layout(model, T, K, Cf, G)
+    off = layout_offsets(lay)
+    s = _split(theta, lay)
+    C = theta.shape[0]
+    h, a = np.asarray(d.home_team, np.int64), np.asarray(d.away_team, np.int64)
+    M = len(h)
+    o = lambda name: off[name][0]  # noqa: E731
+    full = lambda i: np.full(M, i, np.int64)  # noqa: E731
+    ones = torch.ones((C, M), dtype=theta.dtype)
+    X = None
+    if K:
+        X = np.asarray(d.covariates if d.covariates_prestandardised else standardise_covariates(d.covariates), np.float64)
+    n = ones if model in ("dixon_coles", "extended") else ones * torch.as_tensor(
+        1 - np.asarray(d.neutral_venue, np.int64), dtype=theta.dtype)
+    jh, ja = [], []
+    if model == "dynamic":
+        g = np.asarray(d.gameweek, np.int64)
+        sa, sd = torch.exp(s["std_attack"]), torch.exp(s["std_defence"])  # [C, G]
+
+        def strength(side, t, sign, out):  # sign * attack[g, t] or sign * defence[g, t]: the walk up to gameweek g
+            if d.walk == "as_written":  # (attack and defence stay zero)
+                return
+            z, ls, sg = ("standardised_" + side, "std_" + side, sa if side == "attack" else sd)
+            for j in range(G):
+                on = torch.as_tensor((j <= g).astype(np.float64), dtype=theta.dtype)
+                out.append((o(z) + j * T + t, sign * sg[:, j, None] * on))
+                out.append((full(o(ls) + j), sign * sg[:, j, None] * s[z][:, j, t] * on))
+            if side == "defence":
+                out.append((full(o("mean_defence")), sign * ones))
+            for k in range(K):
+                out.append((full(o(side + "_coefficients") + k), sign * torch.as_tensor(X[t, k], dtype=theta.dtype).expand(C, M)))
+
+        def effect(nm, t, coef, out):  # coef * effect[g, t]
+            sg = torch.exp(s["std_" + nm])
+            out.append((o("mean_" + nm) + g, coef))
+            out.append((o("std_" + nm) + g, coef * sg[:, g] * s[nm + "_decentered"][:, g, t]))
+            out.append((o(nm + "_decentered") + g * T + t, coef * sg[:, g]))
+
+        strength("attack", h, 1.0, jh); strength("defence", a, -1.0, jh)
+        effect("home_attack", h, n, jh); effect("away_defence", a, -n, jh)
+        strength("attack", a, 1.0, ja); strength("defence", h, -1.0, ja)
+        effect("away_attack", a, n, ja); effect("home_defence", h, -n, ja)
+        return jh, ja
+    dc = model == "dixon_coles"
+    za_n, zd_n = ("attack_decentered", "defence_decentered") if dc else ("standardised_attack", "standardised_defence")
+    sa, sd = torch.exp(s["std_attack"]), torch.exp(s["std_defence"])
+
+    def attack(t, out):
+        out.append((o(za_n) + t, sa[:, None] * ones))
+        out.append((full(o("std_attack")), sa[:, None] * s[za_n][:, t]))
+        for k in range(K):
+            out.append((full(o("attack_coefficients") + k), torch.as_tensor(X[t, k], dtype=theta.dtype).expand(C, M)))
+
+    def minus_defence(t, out):
+        out.append((o(zd_n) + t, -sd[:, None] * ones))
+        out.append((full(o("std_defence")), -sd[:, None] * s[zd_n][:, t]))
+        out.append((full(o("mean_defence")), -ones))
+        for k in range(K):
+            out.append((full(o("defence_coefficients") + k), -torch.as_tensor(X[t, k], dtype=theta.dtype).expand(C, M)))
+
+    def effect(nm, mean, std, t, coef, out):  # coef * (mean + std * decentred[t])
+        sg = torch.exp(s[std])
+        out.append((full(o(mean)), coef))
+        out.append((full(o(std)), coef * sg[:, None] * s[nm + "_decentered"][:, t]))
+        out.append((o(nm + "_decentered") + t, coef * sg[:, None]))
+
+    attack(h, jh); minus_defence(a, jh); attack(a, ja); minus_defence(h, ja)
+    if dc:
+        jh.append((full(o("home_advantage")), ones))
+    elif model == "extended":
+        effect("home_advantage", "mean_home_advantage", "std_home_advantage", h, ones, jh)
+    else:
+        for nm, t, sign, out in (("home_attack", h, 1, jh), ("away_defence", a, -1, jh),
+                                 ("away_attack", a, 1, ja), ("home_defence", h, -1, ja)):
+            effect(nm, "mean_" + nm, "std_" + nm, t, sign * n, out)
+    if Cf:
+        hc, ac = np.asarray(d.home_conf, np.int64), np.asarray(d.away_conf, np.int64)
+        oc = o("confederation_strength_decentered")
+        jh += [(oc + hc, ones), (oc + ac, -ones)]
+        ja += [(oc + ac, ones), (oc + hc, -ones)]
+    return jh, ja
+
+
+def _gradient_terms(d: MatchData, theta):
+    """float64 (kappa [C, D], lp scale [C], gradient [C, D], lp [C]): kappa_i = sum over the elementary terms, and
+    over the paths by which a term reaches theta_i, of |d term / d theta_i|; the lp scale = sum of |term|.  The
+    gradient and lp are the same pieces summed with their signs (they equal ``log_density_and_grad``: a check of the
+    decomposition).
+
+    Elementary terms: per match w y_h log lam_h, -w lam_h, w y_a log lam_a, -w lam_a, -w log(y_h! y_a!) and, for low
+    scores, w log tau (tau through corr_coef and its bounds); every prior and Jacobian term, one per element (the
+    conditional normal of the standardised defence as the parts of its expanded square).  A match term reaches theta
+    through eta_h, eta_a and corr_coef, and each rate through each table entry it reads (attack[h], confederation
+    strength[home conf], ... -- separately even when two cancel, as two entries of one confederation do): float32
+    evaluates each path on its own.  The match terms are differentiated through the sparse rows of d eta / d theta (per
+    chain, ``scipy.sparse``), the prior terms site by site: inside one site every prior term reads at most one element,
+    so a forward derivative along the whole site gives each term's derivative and a reverse pass weighted by its sign
+    sums their moduli."""
+    import scipy.sparse as sp
+
+    th = torch.as_tensor(np.asarray(theta), dtype=torch.float64).clone().requires_grad_(True)
+    C, D = th.shape
+    lp_o, det = log_density(d, th)
+    cc = det["corr_coef"]
+    (dc_dth,) = torch.autograd.grad(cc.sum(), th)  # d corr_coef / d theta: raw and the two arg-max matches' rates
+    dc_dth = dc_dth.numpy()
+    lam_h, lam_a, c = det["lam_h"].detach(), det["lam_a"].detach(), cc.detach()[:, None]
+    # ---- match terms: derivatives with respect to eta_h, eta_a and c (the rates are clipped only in "extended") ----
+    M = d.num_matches
+    w = torch.ones(M, dtype=torch.float64) if d.weights is None else torch.as_tensor(np.asarray(d.weights, np.float64))
+    hg, ag = np.asarray(d.home_goals, np.int64), np.asarray(d.away_goals, np.int64)
+    yh, ya = torch.as_tensor(hg, dtype=torch.float64), torch.as_tensor(ag, dtype=torch.float64)
+    fh = (lam_h < 15.0).double() if d.model == "extended" else torch.ones_like(lam_h)
+    fa = (lam_a < 15.0).double() if d.model == "extended" else torch.ones_like(lam_a)
+    t_pois = [w * yh * torch.log(lam_h), -w * lam_h, w * ya * torch.log(lam_a), -w * lam_a,
+              (-w * (torch.lgamma(yh + 1.0) + torch.lgamma(ya + 1.0))).expand(C, M)]
+    k00 = torch.as_tensor((hg == 0) & (ag == 0)).double()
+    k10 = torch.as_tensor((hg == 1) & (ag == 0)).double()
+    k01 = torch.as_tensor((hg == 0) & (ag == 1)).double()
+    k11 = torch.as_tensor((hg == 1) & (ag == 1)).double()
+    low = (k00 + k10 + k01 + k11) > 0
+    x = lam_h * lam_a
+    tau = 1.0 + c * (-k00 * x + k10 * lam_a + k01 * lam_h - k11)  # 1 - c x, 1 + c lam_a, 1 + c lam_h, 1 - c
+    tau = torch.where(low, tau, torch.ones_like(tau))
+    t_tau = w * torch.log(tau) * low
+    a_h = w * (yh - lam_h) * fh  # Poisson terms, d / d eta_h (both terms: |.| taken per term below)
+    p_h = w * (yh + lam_h) * fh  # sum of the two terms' moduli
+    a_a, p_a = w * (ya - lam_a) * fa, w * (ya + lam_a) * fa
+    q_h = w * c * (-k00 * x + k01 * lam_h) / tau * fh  # tau term, d / d eta_h
+    q_a = w * c * (-k00 * x + k10 * lam_a) / tau * fa
+    q_c = w * (-k00 * x + k10 * lam_a + k01 * lam_h - k11) / tau  # d / d c
+    # ---- prior terms --------------------------------------------------------------------------------------------
+    pri = _prior_terms(d, th.detach())
+    kappa = np.zeros((C, D))
+    grad = np.zeros((C, D))
+    f = lambda t: _prior_terms(d, t)  # noqa: E731
+    _, vjp = torch.func.vjp(f, th.detach())
+    grad += vjp(torch.ones_like(pri))[0].numpy()
+    off = layout_offsets(site_layout(d.model, d.num_teams, d.num_covariates,
+                                     d.num_conferences if d.model == "neutral_wc" else 0, d.num_gameweeks))
+    for name, (o, shape, _) in off.items():
+        n = int(np.prod(shape)) if shape else 1
+        if name == "__D__" or n == 0:
+            continue
+        e = torch.zeros_like(th.detach())
+        e[:, o:o + n] = 1.0
+        _, along = torch.func.jvp(f, (th.detach(),), (e,))
+        kappa[:, o:o + n] += vjp(torch.sign(along))[0][:, o:o + n].numpy()
+    lp_scale = pri.abs().sum(-1).numpy() + sum(t.abs().sum(-1) for t in t_pois).numpy() + t_tau.abs().sum(-1).numpy()
+    lp = pri.sum(-1).numpy() + sum(t.sum(-1) for t in t_pois).numpy() + t_tau.sum(-1).numpy()
+    # ---- match terms through the sparse rate Jacobian, chain by chain ---------------------------------------------
+    jh, ja = _rate_jacobian(d, th.detach())
+    rows = np.arange(M)
+
+    def csr(parts, c_, absolute=False):  # duplicate (row, column) pairs are summed: after |.| with absolute=True
+        r = np.concatenate([rows] * len(parts))
+        i = np.concatenate([np.broadcast_to(ix, (M,)) for ix, _ in parts])
+        v = np.concatenate([val[c_].numpy() for _, val in parts])
+        return sp.csr_matrix((np.abs(v) if absolute else v, (r, i)), shape=(M, D))
+
+    lowi = np.nonzero(low.numpy())[0]
+    for c_ in range(C):
+        Jh, Ja = csr(jh, c_), csr(ja, c_)
+        Ph, Pa = csr(jh, c_, absolute=True), csr(ja, c_, absolute=True)
+        kappa[c_] += Ph.T @ (p_h[c_] + q_h[c_].abs()).numpy() + Pa.T @ (p_a[c_] + q_a[c_].abs()).numpy()
+        grad[c_] += Jh.T @ (a_h[c_] + q_h[c_]).numpy() + Ja.T @ (a_a[c_] + q_a[c_]).numpy()
+        qc = q_c[c_].numpy()[lowi]  # the path through corr_coef: d c / d theta is dense over few components
+        kappa[c_] += np.abs(qc).sum() * np.abs(dc_dth[c_])
+        grad[c_] += qc.sum() * dc_dth[c_]
+    return kappa, lp_scale, grad, lp
+
+
+def gradient_scale(d: MatchData, theta):
+    """Error scale of a float32 evaluation of (lp, d lp / d theta) at ``theta [C, D]``, in float64: returns
+    ``(kappa [C, D], lp_scale [C])`` with kappa_i = sum over the elementary terms (and the paths by which they reach
+    theta_i) of |d term / d theta_i| and lp_scale = sum of |term| (terms and paths as in ``_gradient_terms``).  A float32 evaluation that rounds each term and each partial sum
+    once errs by a small multiple of 2^-24 of these, component by component, however the terms cancel."""
+    kappa, lp_scale, _, _ = _gradient_terms(d, theta)
+    return kappa, lp_scale
 
 
 # --------------------------------------------------------------------------------------

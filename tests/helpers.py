@@ -83,6 +83,53 @@ def random_theta(D, C, seed=0, radius=1.0, dtype=np.float64):
 
 
 # --------------------------------------------------------------------------------------
+# per-component error criterion of a float32 log density + gradient (tests/test_gradient_criterion.py calibrates it)
+# --------------------------------------------------------------------------------------
+EPS32 = 2.0 ** -24
+# |g_i - g_o,i| <= CRIT_C * 2^-24 * kappa_i, kappa_i = sum over the elementary terms (and the paths by which they reach
+# theta_i) of |d term / d theta_i|; the same with lp and sum |term| (oracle.models.gradient_scale).  The two float32
+# restatements of the oracle (closed_form.ClosedForm and models in float32) reach a gradient ratio of 163 (configs[2]
+# data at radius 2: a confederation strength, a sum over 40,000 matches) and an lp ratio of 32 on the cases of
+# tests/test_gradient_criterion.py.  CRIT_C is about three times the larger.
+CRIT_C = 512.0
+
+
+def criterion_ratios(d: om.MatchData, theta64, lp, grad, ref=None):
+    """(|lp - lp_o| / (2^-24 sum |term|) [C], |g - g_o| / (2^-24 kappa) [C, D]) against the float64 oracle;
+    ``ref`` = (lp_o, g_o, kappa, lp_scale) when the caller has them."""
+    if ref is None:
+        lp_o, g_o, _ = om.log_density_and_grad(d, theta64)
+        kappa, lp_scale = om.gradient_scale(d, theta64)
+    else:
+        lp_o, g_o, kappa, lp_scale = ref
+    with np.errstate(divide="ignore", invalid="ignore"):
+        rg = np.abs(np.asarray(grad, np.float64) - g_o) / (EPS32 * kappa)
+        rl = np.abs(np.asarray(lp, np.float64) - lp_o) / (EPS32 * lp_scale)
+    rg[(kappa == 0) & (np.asarray(grad) == g_o)] = 0.0  # a component no term depends on (K = 0 sites are absent)
+    return rl, rg
+
+
+def criterion_failures(d: om.MatchData, theta64, lp, grad, c: float = CRIT_C, limit: int = 8, ref=None):
+    """Components that break the criterion, as 'chain c: site[index] ratio r' (worst first); [] when it holds."""
+    rl, rg = criterion_ratios(d, theta64, lp, grad, ref)
+    names = []
+    for name, shape, _ in om.site_layout(d.model, d.num_teams, d.num_covariates,
+                                         d.num_conferences if d.model == "neutral_wc" else 0, d.num_gameweeks):
+        n = int(np.prod(shape)) if shape else 1
+        names += [name] if shape == () else [f"{name}{list(np.unravel_index(i, shape))}" for i in range(n)]
+    out = [(r, f"chain {ch}: lp ratio {r:.3g}") for ch, r in enumerate(rl) if not r <= c]
+    bad = np.argwhere(~(rg <= c))
+    out += [(rg[ch, i], f"chain {ch}: {names[i]} ratio {rg[ch, i]:.3g}") for ch, i in bad]
+    out.sort(key=lambda x: -x[0] if np.isfinite(x[0]) else -np.inf)
+    return [s for _, s in out[:limit]] + ([f"... {len(out) - limit} more"] if len(out) > limit else [])
+
+
+def assert_criterion(d: om.MatchData, theta64, lp, grad, what: str = "", ref=None):
+    bad = criterion_failures(d, theta64, lp, grad, ref=ref)
+    assert not bad, f"{what}: per-component criterion (c = {CRIT_C:g}) fails: " + "; ".join(bad)
+
+
+# --------------------------------------------------------------------------------------
 _plancheck = None
 
 

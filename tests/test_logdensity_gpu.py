@@ -1,6 +1,8 @@
 """GPU parity: K1 (C ABI) vs the float64 oracle restatement of the reference models.
 
 Tolerances are BASELINE.json's: log-density 1e-5 relative, gradient 1e-4 relative (float32)."""
+import hashlib
+
 import numpy as np
 import pytest
 
@@ -13,14 +15,24 @@ LP_RTOL = 1e-5
 GRAD_RTOL = 1e-4
 
 
-def _check(arr, theta64, lp, grad, cc):
-    d = H.to_oracle(arr)
-    lp_o, g_o, cc_o = om.log_density_and_grad(d, theta64)
+_ORACLE = {}
+
+
+def _check(arr, theta64, lp, grad, cc, what=""):
+    """Against the float64 oracle: lp and corr_coef relative, the gradient scaled by its largest component, and every
+    component within the per-component criterion (tests/helpers.py: CRIT_C 2^-24 sum |d term / d theta_i|)."""
+    key = (id(arr), hashlib.sha1(np.ascontiguousarray(theta64).tobytes()).hexdigest())
+    if key not in _ORACLE:  # (geometry sweeps check many calls on one problem and one theta)
+        _ORACLE.clear()
+        d = H.to_oracle(arr)
+        _ORACLE[key] = (d, arr) + om.log_density_and_grad(d, theta64) + om.gradient_scale(d, theta64)
+    d, _, lp_o, g_o, cc_o, kappa, lp_scale = _ORACLE[key]
     np.testing.assert_allclose(lp, lp_o, rtol=LP_RTOL)
     np.testing.assert_allclose(cc, cc_o, rtol=1e-4, atol=1e-6)
     scale = np.abs(g_o).max(axis=1, keepdims=True)
     err = np.abs(grad - g_o) / scale
     assert err.max() < GRAD_RTOL, f"max scaled gradient error {err.max():.3e} at {np.unravel_index(err.argmax(), err.shape)}"
+    H.assert_criterion(d, theta64, lp, grad, what or arr.model, ref=(lp_o, g_o, kappa, lp_scale))
 
 
 CASES = [

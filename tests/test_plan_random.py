@@ -46,3 +46,42 @@ def test_random_problem_plan_matches_oracle(seed):
         np.testing.assert_allclose(cc_p, cc_o, rtol=1e-9, atol=1e-12)
         scale = np.abs(g_o).max(axis=1, keepdims=True)
         np.testing.assert_allclose(g_p / scale, g_o / scale, rtol=0, atol=3e-7)
+
+
+GEOMETRY_WARPS = (1, 2, 3, 5, 7, 13, 24, 30)
+
+
+@pytest.mark.parametrize("seed", range(0, 40, 2))
+def test_plan_geometries_match_oracle(seed, monkeypatch):
+    """The plan under forced geometries (BPLX_NWARPS warps per CTA, 512 / 1024-byte stages, phase 2 by (team, side) or
+    by whole team; K1d: hyper table in shared memory or the workspace) walked in double == the oracle, for 1, 2 and 8 CTAs
+    per chain group -- on the randomised problems and, for the covariate models, the same problem with K = 4 ... 16."""
+    model, kw = _random_problem(seed)
+    problems = [H.small_problem(model, seed=100 + seed, **kw)]
+    if model != "dixon_coles" and kw["T"] >= 3:
+        problems.append(H.small_problem(model, seed=100 + seed, **dict(kw, K=(4, 5, 8, 16)[seed % 4])))
+    for arr in problems:
+        d = H.to_oracle(arr)
+        D = om.num_params(model, arr.num_teams, arr.num_covariates, arr.num_conferences, arr.num_gameweeks)
+        theta = H.random_theta(D, 1, seed=seed, radius=0.8)
+        lp_o, g_o, cc_o = om.log_density_and_grad(d, theta)
+        scale = np.abs(g_o).max(axis=1, keepdims=True)
+        if model == "dynamic":
+            geoms = [dict(BPLX_NWARPS=W, BPLX_DYN_HYP_WS=h) for W in GEOMETRY_WARPS for h in (0, 1)]
+            splits = (0,)
+        else:
+            geoms = [dict(BPLX_NWARPS=W, BPLX_STAGE=st, BPLX_NO_P2SPLIT=p2) for W in GEOMETRY_WARPS for st in (512, 1024)
+                     for p2 in (None, 1)]
+            splits = (0, 1, 3)
+        for g in geoms:
+            for k, v in g.items():
+                if v is None:
+                    monkeypatch.delenv(k, raising=False)
+                else:
+                    monkeypatch.setenv(k, str(v))
+            for si in splits:
+                lp_p, g_p, cc_p = H.plancheck_eval(arr, theta, si)
+                msg = f"{model} K={arr.num_covariates} {g} split {1 << si}"
+                np.testing.assert_allclose(lp_p, lp_o, rtol=2e-7, err_msg=msg)
+                np.testing.assert_allclose(cc_p, cc_o, rtol=1e-9, atol=1e-12, err_msg=msg)
+                np.testing.assert_allclose(g_p / scale, g_o / scale, rtol=0, atol=3e-7, err_msg=msg)

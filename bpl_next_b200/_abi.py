@@ -80,6 +80,14 @@ class Ranking(C.Structure):
     _fields_ = [("rule", C.c_int32), ("played_h2h", C.c_void_p)]
 
 
+class Pairings(C.Structure):
+    _fields_ = [
+        ("num_pairings", C.c_int32), ("mode", C.c_void_p), ("protect", C.c_void_p), ("host_pot", C.c_void_p),
+        ("pool_size", C.c_void_p), ("pool_kind", C.c_void_p), ("pool_arg0", C.c_void_p), ("pool_arg1", C.c_void_p),
+        ("pool_pot", C.c_void_p), ("slot_assoc", C.c_void_p),
+    ]
+
+
 class PpcOutput(C.Structure):
     _fields_ = [
         ("score_counts", C.c_void_p), ("outcome_counts", C.c_void_p), ("goals", C.c_void_p),
@@ -92,7 +100,11 @@ PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
 # BPLX_ENTRANT_*
-ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER = 0, 1, 2, 3, 4
+ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER, ENTRANT_PAIRED = 0, 1, 2, 3, 4, 5
+# BPLX_MAX_PAIRINGS, BPLX_PAIRING_MAX_POOL, BPLX_PAIRING_MAX_POT, BPLX_PAIRING_*, BPLX_PROTECT_*
+MAX_PAIRINGS, PAIRING_MAX_POOL, PAIRING_MAX_POT = 16, 64, 16
+PAIRING_OPEN, PAIRING_SEEDED = 0, 1
+PROTECT_GROUP, PROTECT_ASSOCIATION = 1, 2
 # BPLX_TIE_*, BPLX_EXTRA_TIME_FRACTION
 TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS = 0, 1, 2
 EXTRA_TIME_FRACTION = 1.0 / 3.0
@@ -182,6 +194,15 @@ def declare(lib):
                                                     C.c_longlong, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                                     sz, vp]
     lib.bplx_simulate_tournament_ranked.restype = i
+    lib.bplx_simulate_tournament_paired_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures),
+                                                                    C.POINTER(Table), C.POINTER(Bracket),
+                                                                    C.POINTER(Ranking), C.POINTER(Pairings)]
+    lib.bplx_simulate_tournament_paired_workspace_bytes.restype = sz
+    lib.bplx_simulate_tournament_paired.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                                    C.POINTER(Bracket), vp, C.POINTER(Ranking), C.POINTER(Pairings), i,
+                                                    i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                                                    vp, vp, vp, vp, vp, sz, vp]
+    lib.bplx_simulate_tournament_paired.restype = i
     lib.bplx_posterior_predictive_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Observations)]
     lib.bplx_posterior_predictive_workspace_bytes.restype = sz
     lib.bplx_posterior_predictive.argtypes = [C.POINTER(Samples), C.POINTER(Observations), i, i, i, i, i, C.c_ulonglong,

@@ -962,7 +962,7 @@ size_t bplx_simulate_tournament_workspace_bytes(const bplx_samples* s, const bpl
 
 // the bracket checks the kernel relies on; fills sp->ko
 static int check_bracket(const bplx_bracket* b, const uint8_t* tie_format, const bplx_samples* s, int NT, int P,
-                         KoParams* ko) {
+                         KoParams* ko, bool allow_paired = false) {
   BPLX_REQUIRE(b != nullptr, BPLX_E_INVALID, "tournament: bracket is NULL");
   const int K = b->num_ties;
   BPLX_REQUIRE(K >= 1, BPLX_E_INVALID, "tournament: the bracket needs at least one tie (got %d)", K);
@@ -1014,6 +1014,11 @@ static int check_bracket(const bplx_bracket* b, const uint8_t* tie_format, const
           BPLX_REQUIRE(a0 < k, BPLX_E_INVALID, "tournament: tie %d %s: refers to tie %d, which is not earlier", k, sd,
                        a0);
           break;
+        case BPLX_ENTRANT_PAIRED:  // (check_pairings validates it; the kernel takes the entrant from the pairing)
+          BPLX_REQUIRE(allow_paired, BPLX_E_INVALID, "tournament: tie %d %s: a PAIRED entrant needs pairings", k, sd);
+          ko->kind[side][k] = BPLX_ENTRANT_SLOT;
+          ko->arg0[side][k] = ko->arg1[side][k] = 0;
+          continue;
         default:
           BPLX_REQUIRE(false, BPLX_E_INVALID, "tournament: tie %d %s: unknown entrant kind %d", k, sd, kind);
       }
@@ -1082,12 +1087,15 @@ int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, c
                                          ko_winners, ko_extra, invalid, workspace, workspace_bytes, stream);
 }
 
-int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+static int check_pairings(const bplx_pairings* p, const bplx_bracket* b, const bplx_table* t, int F, PairParams* pr);
+
+int bplx_simulate_tournament_paired(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
                                     const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
-                                    const uint8_t* tie_format, const bplx_ranking* r, int max_goals, int sims_per_draw,
-                                    unsigned long long seed, long long first_draw, unsigned long long* position_counts,
-                                    unsigned long long* points_counts, unsigned long long* reach_counts,
-                                    unsigned long long* win_counts, unsigned long long* decided_counts,
+                                    const uint8_t* tie_format, const bplx_ranking* r, const bplx_pairings* p,
+                                    int max_goals, int sims_per_draw, unsigned long long seed, long long first_draw,
+                                    unsigned long long* position_counts, unsigned long long* points_counts,
+                                    unsigned long long* reach_counts, unsigned long long* win_counts,
+                                    unsigned long long* decided_counts, unsigned long long* pairing_counts,
                                     uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
                                     uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
                                     void* workspace, size_t workspace_bytes, void* stream) {
@@ -1095,8 +1103,14 @@ int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* 
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "tournament", true, &sp);
   if (rc != BPLX_OK) return rc;
-  rc = check_bracket(b, tie_format, s, t->num_slots, t->num_positions, &sp.ko);
+  const bool paired = p && p->num_pairings != 0;
+  rc = check_bracket(b, tie_format, s, t->num_slots, t->num_positions, &sp.ko, paired);
   if (rc != BPLX_OK) return rc;
+  if (paired) {
+    rc = check_pairings(p, b, t, f->num_fixtures, &sp.pr);
+    if (rc != BPLX_OK) return rc;
+    sp.pr.counts = pairing_counts;
+  }
   BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
   rc = check_ranking(r, t->num_slots, "tournament");
   if (rc != BPLX_OK) return rc;
@@ -1133,6 +1147,136 @@ int bplx_simulate_tournament(const bplx_samples* s, const bplx_fixtures* f, cons
                                      first_draw, position_counts, points_counts, reach_counts, win_counts, nullptr,
                                      positions, scores, ko_entrants, ko_scores, ko_winners, nullptr, invalid, workspace,
                                      workspace_bytes, stream);
+}
+
+// ---- pairings drawn by lot -------------------------------------------------------------------------------------
+// the pairing checks the kernel relies on (the bracket already checked, PAIRED entrants allowed); fills *pr
+static int check_pairings(const bplx_pairings* p, const bplx_bracket* b, const bplx_table* t, int F, PairParams* pr) {
+  const int P = p->num_pairings, K = b->num_ties, NT = t->num_slots;
+  BPLX_REQUIRE(P >= 0 && P <= BPLX_MAX_PAIRINGS, BPLX_E_INVALID, "pairings: num_pairings must be in [0, %d] (got %d)",
+               BPLX_MAX_PAIRINGS, P);
+  BPLX_REQUIRE(P == 0 || (p->mode && p->pool_size && p->pool_kind && p->pool_arg0 && p->pool_arg1), BPLX_E_INVALID,
+               "pairings: mode, pool_size, pool_kind, pool_arg0 and pool_arg1 must not be NULL");
+  memset(pr->made_at, 0xFF, sizeof(pr->made_at));
+  memset(pr->of_tie, 0xFF, sizeof(pr->of_tie));
+  memset(pr->assoc, 0xFF, sizeof(pr->assoc));
+  if (p->slot_assoc)
+    for (int u = 0; u < NT; u++) pr->assoc[u] = p->slot_assoc[u];
+  // the ties that take pairs: home (d, 2i) and away (d, 2i + 1) of one pair, each pair once
+  unsigned long long used[BPLX_MAX_PAIRINGS] = {};
+  unsigned made = 0;
+  for (int k = 0; k < K; k++) {
+    const int kh = b->kind[2 * k], ka = b->kind[2 * k + 1];
+    if (kh != BPLX_ENTRANT_PAIRED && ka != BPLX_ENTRANT_PAIRED) continue;
+    const int d = b->arg0[2 * k], h = b->arg1[2 * k];
+    BPLX_REQUIRE(kh == BPLX_ENTRANT_PAIRED && ka == BPLX_ENTRANT_PAIRED && b->arg0[2 * k + 1] == d && h % 2 == 0 &&
+                     b->arg1[2 * k + 1] == h + 1,
+                 BPLX_E_INVALID, "pairings: tie %d must take home 2i and away 2i + 1 of one pair of one pairing", k);
+    BPLX_REQUIRE(d < P && h / 2 < p->pool_size[d] / 2, BPLX_E_INVALID,
+                 "pairings: tie %d takes pair %d of pairing %d, which does not exist", k, h / 2, d);
+    BPLX_REQUIRE(!((used[d] >> (h / 2)) & 1ull), BPLX_E_INVALID, "pairings: pair %d of pairing %d is taken twice", h / 2,
+                 d);
+    used[d] |= 1ull << (h / 2);
+    pr->tie[d][h / 2] = (uint8_t)k;
+    pr->of_tie[k] = (uint8_t)d;
+    if (!((made >> d) & 1u)) pr->made_at[k] = (uint8_t)d;  // the pairing is made at its first tie
+    made |= 1u << d;
+  }
+  int nbuf = 0;
+  for (int d = 0; d < P; d++) {
+    const int n = p->pool_size[d], mode = p->mode[d], prot = p->protect ? p->protect[d] : 0;
+    BPLX_REQUIRE(mode == BPLX_PAIRING_OPEN || mode == BPLX_PAIRING_SEEDED, BPLX_E_INVALID,
+                 "pairings: pairing %d: mode %d is not a BPLX_PAIRING_* value", d, mode);
+    BPLX_REQUIRE(n >= 2 && n % 2 == 0 && n <= BPLX_PAIRING_MAX_POOL, BPLX_E_INVALID,
+                 "pairings: pairing %d: the pool must have an even size in [2, %d] (got %d)", d, BPLX_PAIRING_MAX_POOL,
+                 n);
+    BPLX_REQUIRE(prot >= 0 && prot <= (BPLX_PROTECT_GROUP | BPLX_PROTECT_ASSOCIATION), BPLX_E_INVALID,
+                 "pairings: pairing %d: unknown protection bits 0x%x", d, prot);
+    BPLX_REQUIRE(mode == BPLX_PAIRING_SEEDED || prot == 0, BPLX_E_INVALID,
+                 "pairings: pairing %d: protections need a seeded pairing", d);
+    BPLX_REQUIRE(!(prot & BPLX_PROTECT_GROUP) || t->group, BPLX_E_INVALID,
+                 "pairings: pairing %d: group protection needs a table with groups", d);
+    BPLX_REQUIRE(!(prot & BPLX_PROTECT_ASSOCIATION) || p->slot_assoc, BPLX_E_INVALID,
+                 "pairings: pairing %d: association protection needs slot_assoc", d);
+    int first = 0;  // the pairing's first tie (K when no tie takes a pair: refused below)
+    while (first < K && pr->made_at[first] != d) first++;
+    int in_pot[2] = {0, 0};
+    for (int j = 0; j < n; j++) {
+      const int kind = p->pool_kind[d * BPLX_PAIRING_MAX_POOL + j], a0 = p->pool_arg0[d * BPLX_PAIRING_MAX_POOL + j],
+                a1 = p->pool_arg1[d * BPLX_PAIRING_MAX_POOL + j];
+      switch (kind) {
+        case BPLX_ENTRANT_SLOT:
+          BPLX_REQUIRE(a0 < NT, BPLX_E_INVALID, "pairings: pairing %d entry %d: slot %d outside the table", d, j, a0);
+          break;
+        case BPLX_ENTRANT_GROUP_POS:
+          BPLX_REQUIRE(a0 < b->num_groups && a1 < t->num_positions, BPLX_E_INVALID,
+                       "pairings: pairing %d entry %d: group %d position %d out of range", d, j, a0, a1);
+          break;
+        case BPLX_ENTRANT_BEST:
+          BPLX_REQUIRE(a0 < b->best_count, BPLX_E_INVALID, "pairings: pairing %d entry %d: BEST %d >= best_count", d, j,
+                       a0);
+          break;
+        case BPLX_ENTRANT_WINNER:
+        case BPLX_ENTRANT_LOSER:
+          BPLX_REQUIRE(a0 < first, BPLX_E_INVALID,
+                       "pairings: pairing %d entry %d: tie %d is not settled before the pairing's first tie %d", d, j,
+                       a0, first);
+          break;
+        case BPLX_ENTRANT_PAIRED:
+          BPLX_REQUIRE(false, BPLX_E_INVALID, "pairings: pairing %d entry %d: a PAIRED entrant inside a pool", d, j);
+        default:
+          BPLX_REQUIRE(false, BPLX_E_INVALID, "pairings: pairing %d entry %d: unknown entrant kind %d", d, j, kind);
+      }
+      int dst = j;
+      if (mode == BPLX_PAIRING_SEEDED) {
+        const int pot = p->pool_pot ? p->pool_pot[d * BPLX_PAIRING_MAX_POOL + j] : 2;
+        BPLX_REQUIRE(pot <= 1, BPLX_E_INVALID, "pairings: pairing %d entry %d: pot must be 0 or 1", d, j);
+        BPLX_REQUIRE(in_pot[pot] < BPLX_PAIRING_MAX_POT, BPLX_E_INVALID,
+                     "pairings: pairing %d: a pot holds at most %d entrants", d, BPLX_PAIRING_MAX_POT);
+        dst = 16 * pot + in_pot[pot]++;
+      }
+      pr->kind[d][j] = (uint8_t)kind;
+      pr->arg0[d][j] = (uint8_t)a0;
+      pr->arg1[d][j] = (uint8_t)a1;
+      pr->dst[d][j] = (uint8_t)dst;
+    }
+    BPLX_REQUIRE(mode == BPLX_PAIRING_OPEN || in_pot[0] == in_pot[1], BPLX_E_INVALID,
+                 "pairings: pairing %d: the pots differ in size (%d and %d)", d, in_pot[0], in_pot[1]);
+    BPLX_REQUIRE(used[d] == (1ull << (n / 2)) - 1, BPLX_E_INVALID, "pairings: pairing %d: a pair is taken by no tie",
+                 d);
+    pr->mode[d] = (uint8_t)mode;
+    pr->protect[d] = (uint8_t)prot;
+    pr->host_b[d] = p->host_pot ? (p->host_pot[d] != 0) : 0;
+    pr->size[d] = (uint8_t)n;
+    nbuf = max(nbuf, mode == BPLX_PAIRING_SEEDED ? 64 : n);
+  }
+  pr->num = P;
+  pr->nbuf = nbuf;
+  const unsigned E = (unsigned)(2 * F + NT + 3 * K + 3) / 4 * 4;
+  pr->P0 = E / 4 + (unsigned)K;
+  return BPLX_OK;
+}
+
+size_t bplx_simulate_tournament_paired_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f,
+                                                       const bplx_table* t, const bplx_bracket* b,
+                                                       const bplx_ranking* r, const bplx_pairings* p) {
+  if (p && (p->num_pairings < 0 || p->num_pairings > BPLX_MAX_PAIRINGS)) return 0;
+  return bplx_simulate_tournament_ranked_workspace_bytes(s, f, t, b, r);
+}
+
+int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                    const uint8_t* tie_format, const bplx_ranking* r, int max_goals, int sims_per_draw,
+                                    unsigned long long seed, long long first_draw, unsigned long long* position_counts,
+                                    unsigned long long* points_counts, unsigned long long* reach_counts,
+                                    unsigned long long* win_counts, unsigned long long* decided_counts,
+                                    uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
+                                    uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
+                                    void* workspace, size_t workspace_bytes, void* stream) {
+  return bplx_simulate_tournament_paired(s, f, home_slot, away_slot, t, b, tie_format, r, nullptr, max_goals,
+                                         sims_per_draw, seed, first_draw, position_counts, points_counts, reach_counts,
+                                         win_counts, decided_counts, nullptr, positions, scores, ko_entrants, ko_scores,
+                                         ko_winners, ko_extra, invalid, workspace, workspace_bytes, stream);
 }
 
 // ---- posterior predictive checks ------------------------------------------------------------------------------

@@ -64,7 +64,139 @@ __device__ __forceinline__ uint32_t philox_word(unsigned long long seed, unsigne
   return r == 0 ? o.x : r == 1 ? o.y : r == 2 ? o.z : o.w;
 }
 
+__device__ __forceinline__ int nibble(unsigned long long x, int i) { return (int)(x >> (4 * i)) & 15; }
+__device__ __forceinline__ unsigned long long set_nibble(unsigned long long x, int i, int v) {
+  return (x & ~(0xFull << (4 * i))) | ((unsigned long long)v << (4 * i));
+}
+// the index of the r-th set bit of m (r < popc(m))
+__device__ __forceinline__ int nth_bit(unsigned m, int r) {
+  for (; r > 0; r--) m &= m - 1;
+  return __ffs(m) - 1;
+}
+
 }  // namespace
+
+// Pairing d of a simulation, its pool already resolved into the thread's pool bytes (PB(j): byte [j][thread]); the
+// drawn entrants of pair i go into the winner / loser bytes of tie pr.tie[d][i], home first.  Word j of the pairing is
+// component j mod 4 of Philox block P0 + 16 d + j / 4; an index uniform in [0, m) is (uint64(w) m) >> 32.
+// Open: the pool in pool order, swapped in place (p[i] <-> p[i + ((w_i (n - i)) >> 32)] for i < n - 1), pair i =
+// (p[2i], p[2i + 1]).  Seeded: pot A's slots at bytes [0, m), pot B's at [16, 16 + m), in pool order; adj[a] (u16
+// [a][thread] at byte row 32) = the pot-B entrants a may meet.  One perfect matching of the remaining entrants is kept as
+// nibbles (mate_a, mate_b, in registers); a pot-A candidate a for the drawn b is eligible iff it may meet b and either
+// is b's mate or an augmenting path joins b's mate to a's mate once a and b are gone: one alternating-path search per
+// candidate on bit masks, not a new matching.  Returns false when the seeded pool cannot be fully paired.
+__device__ __forceinline__ bool draw_pairing(const PairParams& pr, int d, uint8_t* k_pool, const uint8_t* k_ptab,
+                                             uint8_t* k_wl, int tid, unsigned long long seed, unsigned long long n) {
+#define PB(j) k_pool[(j) * kSimThreads + tid]
+#define WL(b) k_wl[(((b) >> 2) * kSimThreads + tid) * 4 + ((b) & 3)]
+  const unsigned blk0 = pr.P0 + 16u * (unsigned)d;
+  const int nd = pr.size[d];
+  uint4 w4 = make_uint4(0, 0, 0, 0);
+  if (pr.mode[d] == BPLX_PAIRING_OPEN) {
+#pragma unroll 1
+    for (int i = 0; i < nd - 1; i++) {
+      if ((i & 3) == 0) w4 = philox_block(seed, n, blk0 + (unsigned)(i >> 2));
+      const uint32_t w = (i & 3) == 0 ? w4.x : (i & 3) == 1 ? w4.y : (i & 3) == 2 ? w4.z : w4.w;
+      const int j = i + (int)(((unsigned long long)w * (unsigned)(nd - i)) >> 32);
+      const uint8_t x = PB(i);
+      PB(i) = PB(j);
+      PB(j) = x;
+    }
+#pragma unroll 1
+    for (int i = 0; i < nd / 2; i++) {
+      const int k = pr.tie[d][i];
+      WL(2 * k) = PB(2 * i);
+      WL(2 * k + 1) = PB(2 * i + 1);
+    }
+    return true;
+  }
+  const int m = nd >> 1, prot = pr.protect[d];
+  uint16_t* const adj = reinterpret_cast<uint16_t*>(k_pool + 32 * kSimThreads);
+#define ADJ(a) adj[(a) * kSimThreads + tid]
+#pragma unroll 1
+  for (int a = 0; a < m; a++) {
+    const int sa = PB(a), ga = k_ptab[sa], xa = k_ptab[64 + sa];
+    unsigned row = 0;
+#pragma unroll 1
+    for (int b = 0; b < m; b++) {
+      const int sb = PB(16 + b);
+      const bool clash = ((prot & BPLX_PROTECT_GROUP) && k_ptab[sb] == ga) ||
+                         ((prot & BPLX_PROTECT_ASSOCIATION) && xa != 0xFF && k_ptab[64 + sb] == xa);
+      row |= (unsigned)!clash << b;
+    }
+    ADJ(a) = (uint16_t)row;
+  }
+  unsigned long long mate_a = 0, mate_b = 0, parent = 0;
+  // breadth-first over alternating paths from pot-A entrant src inside (ra, rb): the first pot-B entrant of `targets`
+  // reached, or -1; nibble b of `parent` = the pot-A entrant b was reached from.  Every other pot-B entrant reached is
+  // matched, and its mate is the next pot-A entrant of the path.
+  auto search = [&](int src, unsigned ra, unsigned rb, unsigned targets) -> int {
+    unsigned frontier = 1u << src, seen = 0;
+    while (frontier) {
+      unsigned next = 0;
+      for (unsigned f = frontier; f; f &= f - 1) {
+        const int a = __ffs(f) - 1;
+        const unsigned nb = ADJ(a) & rb & ~seen;
+        seen |= nb;
+        for (unsigned g = nb; g; g &= g - 1) {
+          const int b = __ffs(g) - 1;
+          parent = set_nibble(parent, b, a);
+          if ((targets >> b) & 1u) return b;
+          next |= 1u << nibble(mate_b, b);
+        }
+      }
+      frontier = next & ra;
+    }
+    return -1;
+  };
+  // flips the path that search(src, ...) found to b
+  auto augment = [&](int src, int b) {
+    for (;;) {
+      const int a = nibble(parent, b), prev = nibble(mate_a, a);
+      mate_a = set_nibble(mate_a, a, b);
+      mate_b = set_nibble(mate_b, b, a);
+      if (a == src) break;
+      b = prev;
+    }
+  };
+  const unsigned full = (1u << m) - 1u;
+  unsigned free_b = full;
+#pragma unroll 1
+  for (int a = 0; a < m; a++) {
+    const int b = search(a, full, full, free_b);
+    if (b < 0) return false;
+    augment(a, b);
+    free_b &= ~(1u << b);
+  }
+  unsigned ra = full, rb = full;
+#pragma unroll 1
+  for (int i = 0; i < m; i++) {
+    if ((i & 1) == 0) w4 = philox_block(seed, n, blk0 + (unsigned)(i >> 1));
+    const uint32_t wb = i & 1 ? w4.z : w4.x, wa = i & 1 ? w4.w : w4.y;  // w_{2i}, w_{2i+1}
+    const int b = nth_bit(rb, (int)(((unsigned long long)wb * (unsigned)__popc(rb)) >> 32));
+    const int ab = nibble(mate_b, b);
+    const unsigned rb2 = rb & ~(1u << b);
+    unsigned elig = 0;
+#pragma unroll 1
+    for (unsigned f = ra; f; f &= f - 1) {
+      const int a = __ffs(f) - 1;
+      if (!((ADJ(a) >> b) & 1u)) continue;
+      if (a == ab || search(ab, ra & ~(1u << a), rb2, 1u << nibble(mate_a, a)) >= 0) elig |= 1u << a;
+    }
+    // (never empty: b's mate is eligible)
+    const int a = nth_bit(elig, (int)(((unsigned long long)wa * (unsigned)__popc(elig)) >> 32));
+    if (a != ab) augment(ab, search(ab, ra & ~(1u << a), rb2, 1u << nibble(mate_a, a)));
+    const int sa = PB(a), sb = PB(16 + b), k = pr.tie[d][i];
+    WL(2 * k) = (uint8_t)(pr.host_b[d] ? sb : sa);
+    WL(2 * k + 1) = (uint8_t)(pr.host_b[d] ? sa : sb);
+    ra &= ~(1u << a);
+    rb = rb2;
+  }
+  return true;
+#undef PB
+#undef WL
+#undef ADJ
+}
 
 // Head-to-head ranking of every group of a valid simulation into k_q (k_q[gbeg + position] = slot).  Each group
 // is sorted by points; bit 7 of a k_q byte marks the first position of a class of teams still level, bit 6 a class
@@ -209,14 +341,21 @@ __device__ __forceinline__ void rank_head_to_head(const SimParams& sp, int tid, 
 // The kernels: simulate_body.inc with the ranking rule fixed at compile time
 template <bool KO>
 __global__ void __launch_bounds__(kSimThreads) simulate_kernel(const __grid_constant__ SimParams sp) {
-  constexpr bool H2H = false;
+  constexpr bool H2H = false, PAIRED = false;
 #include "simulate_body.inc"
 }
 
 // the same, with the groups ranked by the head-to-head rule (bplx_ranking)
 template <bool KO>
 __global__ void __launch_bounds__(kSimThreads) simulate_h2h_kernel(const __grid_constant__ SimParams sp) {
-  constexpr bool H2H = true;
+  constexpr bool H2H = true, PAIRED = false;
+#include "simulate_body.inc"
+}
+
+// the tournament with pairings drawn by lot (bplx_pairings), under either ranking rule
+template <bool H2H_RULE>
+__global__ void __launch_bounds__(kSimThreads) simulate_paired_kernel(const __grid_constant__ SimParams sp) {
+  constexpr bool KO = true, H2H = H2H_RULE, PAIRED = true;
 #include "simulate_body.inc"
 }
 
@@ -279,9 +418,19 @@ size_t simulate_smem_bytes(SimParams* sp) {
     sp->ko.wl_overlay = sp->ko.K <= 4 * sp->NT;
     if (!sp->ko.wl_overlay) base += (size_t)(2 * sp->ko.K + 3) / 4 * 4 * kSimThreads;
   }
+  // the pool bytes of the paired kernel: in the s_key words past the qualifier map, the BEST bytes and the two 128-byte
+  // per-CTA tables (row NT + bc + 2 of [row][thread]) when they fit there (4 T_tab rows), else appended
+  size_t pool = 0;
+  if (sp->pr.num > 0) {
+    const int row = sp->NT + sp->ko.bc + 2;
+    if (row + sp->pr.nbuf <= 4 * sp->NT) sp->pr.buf_off = (12 * sp->NT + row) * kSimThreads;
+    else pool = (size_t)sp->pr.nbuf * kSimThreads;
+  }
   const size_t pts = (size_t)sp->NT * sp->B * 4;
-  sp->points_in_smem = base + pts <= (size_t)kSimSmemMax;
-  return base + (sp->points_in_smem ? pts : 0);
+  sp->points_in_smem = base + pool + pts <= (size_t)kSimSmemMax;
+  const size_t end = base + (sp->points_in_smem ? pts : 0);
+  if (pool) sp->pr.buf_off = (int)end;
+  return end + pool;
 }
 
 int launch_simulate(SimParams& sp, cudaStream_t stream) {
@@ -292,10 +441,12 @@ int launch_simulate(SimParams& sp, cudaStream_t stream) {
   BPLX_REQUIRE(smem <= (size_t)kSimSmemMax, BPLX_E_UNSUPPORTED,
                "simulate: %zu bytes of shared memory per CTA needed (max %d)", smem, kSimSmemMax);
   // the dynamic shared-memory limit is an attribute of each instantiation
-  static void (*const kernels[4])(const SimParams) = {simulate_kernel<false>, simulate_kernel<true>,
-                                                      simulate_h2h_kernel<false>, simulate_h2h_kernel<true>};
-  static size_t smem_set[4] = {48 * 1024, 48 * 1024, 48 * 1024, 48 * 1024};
-  const int v = (int)ko + (sp.rule == BPLX_RANK_HEAD_TO_HEAD ? 2 : 0);
+  static void (*const kernels[6])(const SimParams) = {
+      simulate_kernel<false>,        simulate_kernel<true>,        simulate_h2h_kernel<false>,
+      simulate_h2h_kernel<true>,     simulate_paired_kernel<false>, simulate_paired_kernel<true>};
+  static size_t smem_set[6] = {48 * 1024, 48 * 1024, 48 * 1024, 48 * 1024, 48 * 1024, 48 * 1024};
+  const bool h2h = sp.rule == BPLX_RANK_HEAD_TO_HEAD;
+  const int v = ko && sp.pr.num > 0 ? 4 + (int)h2h : (int)ko + (h2h ? 2 : 0);
   if (smem > smem_set[v]) {
     BPLX_CUDA(cudaFuncSetAttribute(kernels[v], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set[v] = smem;
@@ -307,10 +458,12 @@ int launch_simulate(SimParams& sp, cudaStream_t stream) {
     BPLX_CUDA(cudaMemsetAsync(sp.ko.reach, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
     BPLX_CUDA(cudaMemsetAsync(sp.ko.win, 0, (size_t)sp.NT * sp.ko.nr * 8, stream));
     if (sp.ko.decided) BPLX_CUDA(cudaMemsetAsync(sp.ko.decided, 0, (size_t)sp.ko.K * 3 * 8, stream));
+    if (sp.pr.counts)
+      BPLX_CUDA(cudaMemsetAsync(sp.pr.counts, 0, (size_t)sp.pr.num * sp.NT * sp.NT * 8, stream));
   }
   rc = launch_score_grid_tables(sp.gp, stream);
   if (rc != BPLX_OK) return rc;
-  if (v >= 2) {
+  if (h2h) {
     pair_index_kernel<<<1, 1024, (size_t)sp.NT * sp.NT * 4, stream>>>(sp.hslot, sp.aslot, sp.gp.F, sp.NT,
                                                                      sp.pair_beg, sp.pair_fix);
     BPLX_CUDA(cudaGetLastError());

@@ -30,6 +30,31 @@ struct KoParams {
   uint8_t slot_conf[kSimMaxTeams];
 };
 
+constexpr int kMaxPairings = 16;      // BPLX_MAX_PAIRINGS
+constexpr int kPairingMaxPool = 64;   // BPLX_PAIRING_MAX_POOL
+constexpr int kPairingMaxPot = 16;    // BPLX_PAIRING_MAX_POT
+
+// the pairings drawn by lot of a tournament (num = 0: none, the kernels without pairings).  A tie that takes a pair
+// has entrant kind SLOT 0 in KoParams; the pairing writes its drawn entrants into the tie's winner / loser bytes, which
+// are free until the tie is played.
+struct PairParams {
+  int num;
+  int buf_off;                    // byte offset in dynamic shared memory of the per-thread pool bytes [nbuf][thread]
+  int nbuf;                       // bytes per thread: the largest open pool, 64 for a seeded pairing
+  unsigned P0;                    // Philox counter of pairing 0's first block: E/4 + K
+  unsigned long long* counts;     // [num][NT][NT] or NULL
+  uint8_t mode[kMaxPairings];     // BPLX_PAIRING_*
+  uint8_t protect[kMaxPairings];  // BPLX_PROTECT_* bits
+  uint8_t host_b[kMaxPairings];   // seeded: the pot-B entrant is at home
+  uint8_t size[kMaxPairings];     // n_d
+  uint8_t made_at[kKoMaxTies];    // the pairing made when tie k is reached, or 0xFF
+  uint8_t of_tie[kKoMaxTies];     // the pairing tie k takes a pair of, or 0xFF
+  uint8_t tie[kMaxPairings][kPairingMaxPool / 2];  // the tie that takes pair i
+  uint8_t kind[kMaxPairings][kPairingMaxPool], arg0[kMaxPairings][kPairingMaxPool], arg1[kMaxPairings][kPairingMaxPool];
+  uint8_t dst[kMaxPairings][kPairingMaxPool];  // pool byte of entry j: j (open); 16 pot + index in the pot (seeded)
+  uint8_t assoc[kSimMaxTeams];    // slot associations, 0xFF = none
+};
+
 struct SimParams {
   GridParams gp;                  // samples (S = draws of this call), fixtures (F), table layout; gp.table = workspace
   const uint8_t *hslot, *aslot;   // [F] table slots
@@ -49,10 +74,12 @@ struct SimParams {
   int rule;
   const int2* h2h_played;         // [NT][NT] (points, goals) of slot u against slot v in played matches, or NULL
   int *pair_beg, *pair_fix;       // [NT NT + 1], [F] in the workspace (pair_index_kernel)
+  PairParams pr;                  // the paired tournament kernels only (last, so the other kernels' parameters keep
+                                  // their offsets)
 };
 
 // shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
-// the tournament kernel (sets sp->ko.wl_overlay)
+// the tournament kernel (sets sp->ko.wl_overlay), with pr.num > 0 that of the paired kernel (sets sp->pr.buf_off)
 size_t simulate_smem_bytes(SimParams* sp);
 // ko.K = 0: the group stage alone; ko.K >= 1: the tournament kernel, the same group stage, then the bracket of sp.ko.
 // rule = BPLX_RANK_HEAD_TO_HEAD: the head-to-head instantiation, after the pair index is built into pair_beg / pair_fix

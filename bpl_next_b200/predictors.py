@@ -595,7 +595,7 @@ class _BplxPredictor:
                **bseason.probabilities(table, cnt["position_counts"], cnt["points_counts"], N)}
         if bracket is not None:
             res.update(bseason.bracket_probabilities(bracket, cnt["reach_counts"], cnt["win_counts"], N,
-                                                     cnt["decided_counts"]))
+                                                     cnt["decided_counts"], cnt.get("pairing_counts")))
         res.update({"start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
                     "seed": seed})
         if return_simulations:
@@ -626,7 +626,7 @@ class _BplxPredictor:
     def simulate_tournament(self, fixtures, bracket, played=None, teams=None, groups=None, best=None, team_conf=None,
                             num_sims_per_draw: int = 1, random_state: Optional[int] = None, max_goals: int = MAX_GOALS,
                             points=(3, 1), return_simulations: bool = False,
-                            tiebreak: str = "goal_difference") -> Dict[str, Any]:
+                            tiebreak: str = "goal_difference", pairings=None, association=None) -> Dict[str, Any]:
         """A tournament simulated on the GPU: the group stage of ``simulate_table``, then a knockout bracket, with ONE
         posterior draw per simulated tournament, so a team that is stronger in a draw is stronger in every match of its
         path.  (Chaining ``predict_outcome_proba`` calls cannot give this: the opponent of a round depends on earlier
@@ -634,8 +634,8 @@ class _BplxPredictor:
 
         ``fixtures``, ``played``, ``teams``, ``groups``, ``points``, ``num_sims_per_draw``, ``random_state``,
         ``max_goals``, ``tiebreak``: as ``simulate_table`` (``"head_to_head"`` ranks each group by the matches among
-        its teams level on points, as UEFA's and FIFA's group stages do); ``fixtures`` may be None or empty (a cup whose draw is made: the entrants
-        are ``("team", name)``).  ``bracket``: the ties in play order, ``{"id", "round", "home", "away",
+        its teams level on points, as UEFA's and FIFA's group stages do); ``fixtures`` may be None or empty (a cup: the entrants
+        are ``("team", name)``, in fixed ties or in the pools of ``pairings``).  ``bracket``: the ties in play order, ``{"id", "round", "home", "away",
         "neutral_venue", "format"}``, entrants ``("group", label, position)``, ``("best", j)``, ``("winner", id)``,
         ``("loser", id)`` or ``("team", name)``; ``best``: the best-placed qualifiers, ``{"position", "count",
         "allocation"}`` (``season.build_bracket``).  ``team_conf`` (NeutralWC): team -> confederation, needed for the
@@ -659,6 +659,18 @@ class _BplxPredictor:
         points, goal difference, goals for, then lot, under either ``tiebreak`` (teams of different groups have no
         head-to-head).
 
+        Draws by lot (``pairings``, ``association``; ``season.build_bracket``): domestic cups, the UEFA round of 16,
+        open quarter-final draws.  A pairing turns a pool of entrants into pairs when the first tie that takes one of
+        its pairs is reached (a tie takes ``"pair": (pairing id, i)`` instead of ``home`` / ``away``), so the opponent
+        distribution is part of every simulation.  ``{"id", "pool", "pots": None, ...}`` is an open draw: the pool is
+        shuffled and the first team of each pair drawn is at home.  With ``"pots"`` (0 seeded, 1 unseeded, equal in
+        size, at most 16 each) it is UEFA's sequential procedure: draw an unseeded team, then one of the seeded teams
+        it may meet (``"protect"``: not of the same ``"group"``, not of the same ``"association"``, ``association``
+        mapping team -> label) for which the teams left can still be paired; the unseeded team is at home unless
+        ``"seeded_home"``.  This is not a uniform choice among the valid pairings, and its pair probabilities differ
+        from those.  Adds ``pairing_ids`` and ``pairing_proba [P, T, T]`` (pairing d drew team u at home against team
+        v).
+
         Returns everything ``simulate_table`` returns, plus ``rounds`` (labels by first appearance), ``reach_proba`` /
         ``win_proba [T, rounds]`` (the team plays / wins a tie of the round; a two-legged tie counts once),
         ``champion_proba [T]``, ``tie_ids`` and ``decided_proba [K, 3]`` (tie k settled in normal time or on aggregate,
@@ -670,13 +682,15 @@ class _BplxPredictor:
         (a non-finite rate, or an allocation row the bracket does not cover)."""
         fixtures = fixtures if fixtures is not None and len(_str_to_list(fixtures["home_team"])[0]) else None
         home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"]) if fixtures else ([], [])
-        named = [e[1] for tie in bracket for e in (tuple(tie["home"]), tuple(tie["away"])) if e[0] == "team"]
+        named = [e[1] for tie in bracket if "pair" not in tie for e in (tuple(tie["home"]), tuple(tie["away"]))
+                 if e[0] == "team"]
+        named += [tuple(e)[1] for pg in pairings or () for e in pg["pool"] if tuple(e)[0] == "team"]
         if teams is None:
             tteams = bseason.table_teams(home + named, away, played) if (home or named or played) else []
         else:
             tteams = bseason.table_teams(home, away, played, teams)
         table = bseason.build_table(tteams, played, groups, points, tiebreak)
-        br = bseason.build_bracket(table, bracket, best)
+        br = bseason.build_bracket(table, bracket, best, pairings, association)
         known = set(np.asarray(self.teams).tolist())
         unknown = [t for t in tteams if t not in known]
         if unknown:
@@ -692,7 +706,8 @@ class _BplxPredictor:
             bseason._size_histograms(table)
         return self._simulate(table, fx, br, num_sims_per_draw, random_state, max_goals, return_simulations,
                               "were invalid: a non-finite scoring rate or score-grid normaliser (check the posterior "
-                              "draws), or best-placed qualifiers the bracket does not place")
+                              "draws), best-placed qualifiers the bracket does not place, or a pool of a draw "
+                              "that could not be paired")
 
     # ---- a team the model has not seen (extended_dixon_coles.py:401-462 and the neutral siblings) ---------------
     def _new_team_pair(self, team_name, team_covariates):

@@ -389,6 +389,34 @@ def _bracket_struct(bracket: dict, keep: list):
     return b
 
 
+def _pairings_struct(bracket: dict, T_tab: int, keep: list):
+    """``_abi.Pairings`` over host copies of the pairing arrays of ``bracket`` (kept alive in ``keep``), or None for a
+    bracket without pairings."""
+    if bracket.get("pool_kind") is None:
+        return None
+
+    def host(k, shape=None):
+        v = bracket.get(k)
+        if v is None:
+            return None
+        a = np.ascontiguousarray(v, dtype=np.uint8)
+        if shape is not None and a.shape != shape:
+            raise ValueError(f"{k} has shape {a.shape}; expected {shape}")
+        keep.append(a)
+        return a.ctypes.data
+
+    P = int(len(bracket["pool_size"]))
+    p = _abi.Pairings()
+    p.num_pairings = P
+    for k in ("mode", "protect", "host_pot"):
+        setattr(p, k, host("pairing_" + k, (P,)))
+    p.pool_size = host("pool_size", (P,))
+    for k in ("pool_kind", "pool_arg0", "pool_arg1", "pool_pot"):
+        setattr(p, k, host(k, (P, _abi.PAIRING_MAX_POOL)))
+    p.slot_assoc = host("slot_assoc", (T_tab,))
+    return p
+
+
 def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor], table: dict,
                         bracket: dict, max_goals: int, sims_per_draw: int, seed: int, first_draw: int = 0,
                         want_positions: bool = False, want_scores: bool = False, want_knockout: bool = False,
@@ -422,7 +450,19 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
     ``ko_extra`` (``[N, K, 4]``: leg-2 goals of A and B, then extra-time goals of A and B; 254 where not played); 255
     marks an invalid simulation.  ``table["tiebreak"]`` ranks the groups as in ``simulate_table``
     (``bplx_simulate_tournament_ranked``); best-placed qualifiers are ranked across groups by points, goal difference,
-    goals for, then the key under either rule."""
+    goals for, then the key under either rule.
+
+    Pairings drawn by lot (``bplx_simulate_tournament_paired``): ``bracket`` may also hold ``pairing_mode``,
+    ``pairing_protect``, ``pairing_host_pot``, ``pool_size`` (uint8 ``[P]``), ``pool_kind``, ``pool_arg0``,
+    ``pool_arg1``, ``pool_pot`` (``[P, 64]``) and ``slot_assoc`` (``[T_tab]`` or None), as ``season.build_bracket``
+    makes them; a tie then takes both sides from pair i of pairing d (``_abi.ENTRANT_PAIRED``, arg0 d, arg1 2i and 2i + 1).
+    Pairing d is made when its first tie is reached, on the Philox words of blocks ``E/4 + K + 16 d`` onwards: an open
+    draw shuffles the pool (``j = i + ((w_i (n - i)) >> 32)``, swap; pair i = the entrants drawn 2i and 2i + 1, the first
+    at home); a seeded draw takes an unseeded entrant b (``(w_2i |B left|) >> 32``), then one of the seeded entrants
+    left that b may meet (group / association protection) for which the rest can still be paired (``(w_2i+1
+    |eligible|) >> 32``), in pool order.  A pool that cannot be paired makes the simulation invalid.  Adds
+    ``pairing_counts`` (int64 ``[P, T_tab, T_tab]``: pairing d drew slot u at home against slot v).  A bracket
+    without pairings takes ``bplx_simulate_tournament_ranked``'s path and words."""
     return _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw,
                      want_positions, want_scores, want_knockout, workspace, stream)
 
@@ -450,8 +490,12 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     t = _table_struct(table, ptr)
     b = None if bracket is None else _bracket_struct(bracket, keep)
     r = _ranking_struct(table, T_tab, keep)
+    pg = None if b is None else _pairings_struct(bracket, T_tab, keep)
     structs = (C.byref(s), C.byref(f), C.byref(t)) + (() if b is None else (C.byref(b),))
-    if r is None:
+    if pg is not None:
+        need = int(lib.bplx_simulate_tournament_paired_workspace_bytes(*structs, None if r is None else C.byref(r),
+                                                                        C.byref(pg)))
+    elif r is None:
         ws_bytes = lib.bplx_simulate_workspace_bytes if b is None else lib.bplx_simulate_tournament_workspace_bytes
         need = int(ws_bytes(*structs))
     else:
@@ -469,6 +513,8 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
         out.update(reach_counts=torch.empty((T_tab, b.num_rounds), **i64),
                    win_counts=torch.empty((T_tab, b.num_rounds), **i64),
                    decided_counts=torch.empty((b.num_ties, 3), **i64))
+        if pg is not None:
+            out["pairing_counts"] = torch.empty((pg.num_pairings, T_tab, T_tab), **i64)
     out.update(invalid=torch.empty(1, **i64), positions=torch.empty((N, T_tab), **u8) if want_positions else None,
                scores=torch.empty((N, F, 2), **u8) if want_scores else None)
     if b is not None:
@@ -493,7 +539,9 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
             keep.append(fmt)
         run, args = lib.bplx_simulate_tournament_ex, structs[:2] + slots + structs[2:] + (
             None if fmt is None else fmt.ctypes.data,)
-        if r is not None:
+        if pg is not None:
+            run, args = lib.bplx_simulate_tournament_paired, args + (None if r is None else C.byref(r), C.byref(pg))
+        elif r is not None:
             run, args = lib.bplx_simulate_tournament_ranked, args + (C.byref(r),)
     _abi.check(run(*args, int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
                    *outputs, _dptr(workspace), workspace.numel(), _stream_ptr(stream)))

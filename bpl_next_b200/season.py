@@ -17,12 +17,14 @@ from typing import Any, Dict, Optional, Sequence, Tuple
 
 import numpy as np
 
-from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_SLOT, ENTRANT_WINNER, KO_MAX_ALLOC_GROUPS,
-                   KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, RANK_GOAL_DIFF, RANK_HEAD_TO_HEAD, SIM_MAX_TEAMS,
-                   TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS)
+from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_PAIRED, ENTRANT_SLOT, ENTRANT_WINNER,
+                   KO_MAX_ALLOC_GROUPS, KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, MAX_PAIRINGS, PAIRING_MAX_POOL,
+                   PAIRING_MAX_POT, PAIRING_OPEN, PAIRING_SEEDED, PROTECT_ASSOCIATION, PROTECT_GROUP, RANK_GOAL_DIFF,
+                   RANK_HEAD_TO_HEAD, SIM_MAX_TEAMS, TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS)
 
 TIE_FORMATS = {"one_match": TIE_ONE_MATCH, "extra_time": TIE_ONE_MATCH_ET, "two_legs": TIE_TWO_LEGS}
 TIEBREAKS = {"goal_difference": RANK_GOAL_DIFF, "head_to_head": RANK_HEAD_TO_HEAD}
+PROTECTIONS = {"group": PROTECT_GROUP, "association": PROTECT_ASSOCIATION}
 
 
 def _names(x) -> list:
@@ -167,8 +169,8 @@ def _group_sizes(table: Dict[str, Any]) -> Tuple[list, np.ndarray]:
     return list(table["group_labels"]), np.bincount(table["group"], minlength=len(table["group_labels"]))
 
 
-def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: Optional[Dict[str, Any]] = None
-                  ) -> Dict[str, Any]:
+def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: Optional[Dict[str, Any]] = None,
+                  pairings: Optional[Sequence[Dict[str, Any]]] = None, association=None) -> Dict[str, Any]:
     """The knockout bracket ``problem.simulate_tournament`` takes, from ties in play order.
 
     Each tie is ``{"id", "round", "home", "away", "neutral_venue", "format"}`` (``neutral_venue`` optional, default 0;
@@ -183,7 +185,18 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
     groups qualify, ranked across groups by points, goal difference, goals for, then lot; with an allocation every
     c-subset of the groups must have a row, and each row is a permutation of its subset.  ``slot_team`` / ``slot_conf``
     are left to the caller (they need the model's team and confederation indices).  ``tie_format`` holds the
-    ``_abi.TIE_*`` byte of every tie."""
+    ``_abi.TIE_*`` byte of every tie.
+
+    ``pairings``: draws by lot that pair a pool of entrants when the first tie taking one of their pairs is reached
+    (``include/bplx.h``, bplx_pairings), each ``{"id", "pool": [entrants], "pots": None or [0 / 1 per entrant],
+    "protect": a set of "group" / "association", "seeded_home": bool}``.  ``pots`` None is an open draw (at most 64
+    entrants, an even number, no protection): the pool is shuffled and the first team drawn of each pair is at home.
+    With pots, pot 0 is seeded and pot 1 unseeded, at most 16 each and equal in size: UEFA's sequential procedure
+    draws an unseeded team, then one of the seeded teams it may meet for which the rest can still be paired; the
+    unseeded team is at home unless ``seeded_home``.  ``protect`` forbids pairs of the same group or of the same
+    ``association`` (a mapping team -> label, or labels aligned with the table's teams; a team without one never
+    clashes).  A tie takes pair i of a pairing with ``"pair": (pairing id, i)`` instead of ``home`` / ``away``; every
+    pair feeds exactly one tie, and a pool's winners / losers must come from ties played before the first such tie."""
     teams = list(table["teams"])
     slot = {t: i for i, t in enumerate(teams)}
     labels, sizes = _group_sizes(table)
@@ -206,6 +219,90 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
     rnd = np.zeros(K, np.uint8)
     nv = np.zeros(K, np.uint8)
     fmt = np.zeros(K, np.uint8)
+    def entrant(e, where):
+        """(kind, arg0, arg1, source key) of entrant ``e``."""
+        e = tuple(e)
+        if e[0] == "group":
+            _, g, p = e
+            if g not in gid:
+                raise ValueError(f"{where}: unknown group {g!r}")
+            if not 0 <= int(p) < sizes[gid[g]]:
+                raise ValueError(f"{where}: group {g!r} has no position {p}")
+            return ENTRANT_GROUP_POS, gid[g], int(p), ("group", g, int(p))
+        if e[0] == "best":
+            j = int(e[1])
+            if not 0 <= j < bc:
+                raise ValueError(f"{where}: best {j} is not one of the {bc} best-placed qualifiers")
+            return ENTRANT_BEST, j, 0, ("best", j)
+        if e[0] in ("winner", "loser"):
+            ref = e[1]
+            if ref not in index:
+                if any(t["id"] == ref for t in ties):
+                    raise ValueError(f"{where} refers to tie {ref!r}, which is not played before it")
+                raise ValueError(f"{where} refers to an unknown tie id {ref!r}")
+            return ENTRANT_WINNER if e[0] == "winner" else ENTRANT_LOSER, index[ref], 0, e
+        if e[0] == "team":
+            if e[1] not in slot:
+                raise ValueError(f"{where}: team {e[1]!r} is not in the table")
+            return ENTRANT_SLOT, slot[e[1]], 0, e
+        raise ValueError(f"{where}: unknown entrant {e!r}")
+
+    def take(src, where):
+        if src in used:
+            raise ValueError(f"{where}: entrant {src!r} is used twice")
+        used.add(src)
+
+    pairings = None if pairings is None else list(pairings)
+    P = 0 if pairings is None else len(pairings)
+    if P > MAX_PAIRINGS:
+        raise ValueError(f"a bracket has at most {MAX_PAIRINGS} pairings, got {P}")
+    pid = {}
+    for d, pg in enumerate(pairings or ()):
+        if pg["id"] in pid:
+            raise ValueError(f"pairing id {pg['id']!r} is used twice")
+        pid[pg["id"]] = d
+    pmode, pprot, phost, psize = (np.zeros(P, np.uint8) for _ in range(4))
+    pkind, parg0, parg1, ppot = (np.zeros((P, PAIRING_MAX_POOL), np.uint8) for _ in range(4))
+    made, taken = set(), [set() for _ in range(P)]
+
+    def make_pairing(d):
+        """Pairing d's pool, read when its first tie is reached (so its winners / losers are of earlier ties)."""
+        pg = pairings[d]
+        where = f"pairing {pg['id']!r}"
+        pool, pots = list(pg["pool"]), pg.get("pots")
+        n = len(pool)
+        prot = 0
+        for name in pg.get("protect") or ():
+            if name not in PROTECTIONS:
+                raise ValueError(f"{where}: unknown protection {name!r} (one of {sorted(PROTECTIONS)})")
+            prot |= PROTECTIONS[name]
+        if pots is None:
+            if prot:
+                raise ValueError(f"{where}: protections need a seeded draw (pots)")
+            if not (2 <= n <= PAIRING_MAX_POOL and n % 2 == 0):
+                raise ValueError(f"{where}: an open draw needs an even pool of 2 to {PAIRING_MAX_POOL}, got {n}")
+        else:
+            pots = [int(x) for x in pots]
+            if len(pots) != n or any(x not in (0, 1) for x in pots):
+                raise ValueError(f"{where}: pots must give 0 or 1 for every pool entrant")
+            m = pots.count(0)
+            if 2 * m != n or not 1 <= m <= PAIRING_MAX_POT:
+                raise ValueError(f"{where}: the pots must be equal in size, 1 to {PAIRING_MAX_POT} each "
+                                 f"(got {m} and {n - m})")
+            if prot & PROTECT_GROUP and table.get("group") is None:
+                raise ValueError(f"{where}: group protection needs a table with groups")
+            if prot & PROTECT_ASSOCIATION and association is None:
+                raise ValueError(f"{where}: association protection needs association")
+        for j, e in enumerate(pool):
+            kd, a0, a1, src = entrant(e, where)
+            take(src, where)
+            pkind[d, j], parg0[d, j], parg1[d, j] = kd, a0, a1
+            ppot[d, j] = 0 if pots is None else pots[j]
+        pmode[d] = PAIRING_OPEN if pots is None else PAIRING_SEEDED
+        pprot[d], psize[d] = prot, n
+        phost[d] = 0 if pots is None or pg.get("seeded_home", False) else 1
+        made.add(d)
+
     for k, tie in enumerate(ties):
         tid = tie["id"]
         if tid in index:
@@ -220,40 +317,26 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
         fmt[k] = TIE_FORMATS[f]
         if fmt[k] == TIE_TWO_LEGS and nv[k]:
             raise ValueError(f"tie {tid!r}: a two-legged tie cannot be at a neutral venue")
-        for side, key in enumerate(("home", "away")):
-            e = tuple(tie[key])
-            src = e
-            if e[0] == "group":
-                _, g, p = e
-                if g not in gid:
-                    raise ValueError(f"tie {tid!r}: unknown group {g!r}")
-                if not 0 <= int(p) < sizes[gid[g]]:
-                    raise ValueError(f"tie {tid!r}: group {g!r} has no position {p}")
-                kind[k, side], arg0[k, side], arg1[k, side] = ENTRANT_GROUP_POS, gid[g], int(p)
-                src = ("group", g, int(p))
-            elif e[0] == "best":
-                j = int(e[1])
-                if not 0 <= j < bc:
-                    raise ValueError(f"tie {tid!r}: best {j} is not one of the {bc} best-placed qualifiers")
-                kind[k, side], arg0[k, side] = ENTRANT_BEST, j
-                src = ("best", j)
-            elif e[0] in ("winner", "loser"):
-                ref = e[1]
-                if ref not in index:
-                    if any(t["id"] == ref for t in ties[k:]):
-                        raise ValueError(f"tie {tid!r} refers to tie {ref!r}, which is not played before it")
-                    raise ValueError(f"tie {tid!r} refers to an unknown tie id {ref!r}")
-                kind[k, side] = ENTRANT_WINNER if e[0] == "winner" else ENTRANT_LOSER
-                arg0[k, side] = index[ref]
-            elif e[0] == "team":
-                if e[1] not in slot:
-                    raise ValueError(f"tie {tid!r}: team {e[1]!r} is not in the table")
-                kind[k, side], arg0[k, side] = ENTRANT_SLOT, slot[e[1]]
-            else:
-                raise ValueError(f"tie {tid!r}: unknown entrant {e!r}")
-            if src in used:
-                raise ValueError(f"tie {tid!r}: entrant {src!r} is used twice")
-            used.add(src)
+        if "pair" in tie:
+            if "home" in tie or "away" in tie:
+                raise ValueError(f"tie {tid!r}: a tie takes a pair or a home and an away entrant, not both")
+            ref, i = tie["pair"]
+            if ref not in pid:
+                raise ValueError(f"tie {tid!r}: unknown pairing {ref!r}")
+            d, i = pid[ref], int(i)
+            if d not in made:
+                make_pairing(d)
+            if not 0 <= i < psize[d] // 2:
+                raise ValueError(f"tie {tid!r}: pairing {ref!r} has no pair {i}")
+            if i in taken[d]:
+                raise ValueError(f"tie {tid!r}: pair {i} of pairing {ref!r} is taken twice")
+            taken[d].add(i)
+            kind[k] = ENTRANT_PAIRED
+            arg0[k], arg1[k] = d, (2 * i, 2 * i + 1)
+        else:
+            for side, key in enumerate(("home", "away")):
+                kind[k, side], arg0[k, side], arg1[k, side], src = entrant(tie[key], f"tie {tid!r}")
+                take(src, f"tie {tid!r}")
         index[tid] = k
     if len(rounds) > KO_MAX_ROUNDS:
         raise ValueError(f"a bracket has at most {KO_MAX_ROUNDS} rounds, got {len(rounds)}")
@@ -277,20 +360,43 @@ def build_bracket(table: Dict[str, Any], ties: Sequence[Dict[str, Any]], best: O
         extra = [k for k in rows if len(k) != bc or not k <= set(labels)]
         if extra:
             raise ValueError(f"the allocation has a row for {sorted(extra[0], key=str)}, not {bc} of the table's groups")
-    return {"ids": [t["id"] for t in ties], "rounds": rounds, "num_rounds": len(rounds), "kind": kind, "arg0": arg0,
-            "arg1": arg1, "round": rnd, "neutral_venue": nv, "num_groups": len(labels), "best_position": bp,
-            "best_count": bc, "best_alloc": best_alloc, "tie_format": fmt}
+    out = {"ids": [t["id"] for t in ties], "rounds": rounds, "num_rounds": len(rounds), "kind": kind, "arg0": arg0,
+           "arg1": arg1, "round": rnd, "neutral_venue": nv, "num_groups": len(labels), "best_position": bp,
+           "best_count": bc, "best_alloc": best_alloc, "tie_format": fmt}
+    if pairings is not None:
+        for d, pg in enumerate(pairings):
+            if len(taken[d]) != psize[d] // 2:
+                raise ValueError(f"pairing {pg['id']!r}: {psize[d] // 2 - len(taken[d])} of its pairs feed no tie")
+        slot_assoc = None
+        if association is not None:
+            lab = [association.get(t) for t in teams] if isinstance(association, dict) else list(association)
+            if len(lab) != len(teams):
+                raise ValueError(f"association has {len(lab)} labels for {len(teams)} teams")
+            ids = {a: i for i, a in enumerate(sorted({a for a in lab if a is not None}, key=str))}
+            if len(ids) > 255:
+                raise ValueError("at most 255 associations are supported")
+            slot_assoc = np.asarray([0xFF if a is None else ids[a] for a in lab], np.uint8)
+        out.update(pairing_ids=list(pid), pairing_mode=pmode, pairing_protect=pprot, pairing_host_pot=phost,
+                   pool_size=psize, pool_kind=pkind, pool_arg0=parg0, pool_arg1=parg1, pool_pot=ppot,
+                   slot_assoc=slot_assoc)
+    return out
 
 
 def bracket_probabilities(bracket: Dict[str, Any], reach_counts: np.ndarray, win_counts: np.ndarray,
-                          num_simulations: int, decided_counts: Optional[np.ndarray] = None) -> Dict[str, Any]:
+                          num_simulations: int, decided_counts: Optional[np.ndarray] = None,
+                          pairing_counts: Optional[np.ndarray] = None) -> Dict[str, Any]:
     """Counts -> ``reach_proba`` / ``win_proba [T, rounds]`` (a team reaches / wins a tie of the round),
     ``champion_proba [T]`` (it wins the last tie), ``tie_ids`` and, from ``decided_counts``, ``decided_proba [K, 3]``
     (tie k settled in normal time or on aggregate / in extra time / by the decider: penalties, or the per-draw lot of a
-    ``one_match`` tie)."""
+    ``one_match`` tie); from ``pairing_counts``, ``pairing_ids`` and ``pairing_proba [P, T, T]`` (pairing d drew team
+    u at home against team v)."""
     n = float(num_simulations)
     reach = np.asarray(reach_counts, np.float64) / n
     win = np.asarray(win_counts, np.float64) / n
-    return {"rounds": list(bracket["rounds"]), "reach_proba": reach, "win_proba": win,
-            "champion_proba": win[:, int(bracket["round"][-1])].copy(), "tie_ids": list(bracket["ids"]),
-            "decided_proba": None if decided_counts is None else np.asarray(decided_counts, np.float64) / n}
+    out = {"rounds": list(bracket["rounds"]), "reach_proba": reach, "win_proba": win,
+           "champion_proba": win[:, int(bracket["round"][-1])].copy(), "tie_ids": list(bracket["ids"]),
+           "decided_proba": None if decided_counts is None else np.asarray(decided_counts, np.float64) / n}
+    if pairing_counts is not None:
+        out.update(pairing_ids=list(bracket["pairing_ids"]),
+                   pairing_proba=np.asarray(pairing_counts, np.float64) / n)
+    return out

@@ -330,7 +330,7 @@ int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uin
 /*
  * Group stage: exactly bplx_simulate_table's definition (same simulation index n, same Philox words 2f, 2f+1 and
  * 2F + t, same ranking); with the same seed its outputs are bit-identical to a bplx_simulate_table call, except that a
- * simulation made invalid by its bracket is left out here.  F = 0 is allowed (a cup whose draw is already made).
+ * simulation made invalid by its bracket is left out here.  F = 0 is allowed (a cup: fixed ties, or pools drawn by lot, below).
  *
  * Bracket: K ties in play order.  Each tie has a home and an away entrant, a round id and (neutral models) a
  * neutral-venue flag; for DIXON_COLES and EXTENDED the home entrant is at home.  An entrant is
@@ -494,6 +494,88 @@ int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* 
                                     unsigned long long seed, long long first_draw, unsigned long long* position_counts,
                                     unsigned long long* points_counts, unsigned long long* reach_counts,
                                     unsigned long long* win_counts, unsigned long long* decided_counts,
+                                    uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
+                                    uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
+                                    void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- knockout pairings drawn by lot ------------------------------------------------------------------------- */
+/*
+ * A pairing is a lot-drawing event that turns a pool of entrants into pairs: a domestic cup's open draw, the UEFA round
+ * of 16 (group winners against runners-up under group and association protection), an open quarter-final draw.
+ * ("Draw" already names a posterior draw and a level match here, so the object is a pairing.)
+ *
+ * Pairing and entrants.  A bracket may carry up to 16 pairings.  Pairing d has a pool of n_d entrants, each one of the
+ * entrant kinds SLOT, GROUP_POS, BEST, WINNER, LOSER.  It produces n_d / 2 pairs; pair i has a home and an away
+ * entrant.  Entrant kind BPLX_ENTRANT_PAIRED (5) takes arg0 = d and arg1 = 2i (home) or 2i + 1 (away).  A tie that uses
+ * pair i takes both of its sides from that pair: home = 2i, away = 2i + 1.  Each pair of each pairing feeds exactly one
+ * tie.  Every pool source must be settled before the first tie that takes a pair of the pairing: group-stage entrants,
+ * or winners / losers of ties earlier in play order.  The pairing is made when that first tie is reached.
+ *
+ * Random words.  With E as above and K ties, the first Philox4x32_10 counter after the tie blocks is P0 = E/4 + K.
+ * Pairing d owns the 16 blocks P0 + 16d .. P0 + 16d + 15: words w_0 .. w_63, word j being component j mod 4 of block
+ * j / 4.  Every word has a fixed address, used or not; a bracket with no pairings reads exactly the words of
+ * bplx_simulate_tournament_ranked, and its outputs are bit-identical.  An index uniform in [0, m) is
+ * (uint64(w) * m) >> 32, exact integer arithmetic.
+ *
+ * BPLX_PAIRING_OPEN: n <= 64, n even, no protections.  Start from pool order p[0..n).  For i = 0 .. n - 2:
+ * j = i + ((w_i * (n - i)) >> 32), swap p[i] and p[j].  Pair i = (p[2i], p[2i + 1]): the first team drawn is at home.
+ *
+ * BPLX_PAIRING_SEEDED: pot A (seeded, pot byte 0) and pot B (unseeded, pot byte 1) are equal in size, at most 16 each.
+ * The sequential procedure UEFA used for its round of 16 (not a uniform choice among valid pairings); for pair
+ * i = 0 .. n/2 - 1:
+ *   1. the unseeded entrant b is the ((w_{2i} * |remaining B|) >> 32)-th remaining pot-B entrant, in pool order;
+ *   2. the eligible seeded entrants are the remaining pot-A entrants a that b may meet and for which the teams left
+ *      after removing a and b can still be fully paired;
+ *   3. a is the ((w_{2i+1} * |eligible|) >> 32)-th eligible entrant, in pool order.
+ * host_pot = 1: the unseeded entrant is at home (UEFA: the unseeded team hosts leg 1); 0: the seeded one.
+ * Protections (seeded only), evaluated on the table slots the pool entrants resolve to in the simulation: bit 0
+ * (BPLX_PROTECT_GROUP) forbids a pair of slots with the same group id; bit 1 (BPLX_PROTECT_ASSOCIATION) a pair with the
+ * same slot_assoc entry (0xFF: no association, never clashes).  A pool that cannot be fully paired at the start makes
+ * the simulation invalid: counted in `invalid`, left out of every histogram, its raw rows 0xFF.
+ *
+ * Output: pairing_counts [num_pairings, T_tab, T_tab] (uint64, NULL to skip): entry (d, u, v) counts the valid
+ * simulations in which pairing d drew slot u at home against slot v; additive over draw ranges.  ko_entrants records
+ * who met whom.
+ *
+ * The arrays are HOST arrays, validated by the call: refused (BPLX_E_INVALID) are more than 16 pairings, an unknown
+ * mode, an odd open pool or one above 64, unequal pots or pots above 16, protections on an open pairing, group
+ * protection without table groups, association protection without slot_assoc, a PAIRED entrant inside a pool, a pool
+ * source not settled before the pairing's first tie, a tie with one PAIRED side or with sides of different pairs or
+ * out of order, and a pair that no tie or two ties take.
+ */
+#define BPLX_ENTRANT_PAIRED 5
+#define BPLX_MAX_PAIRINGS 16
+#define BPLX_PAIRING_MAX_POOL 64
+#define BPLX_PAIRING_MAX_POT 16
+#define BPLX_PAIRING_OPEN 0
+#define BPLX_PAIRING_SEEDED 1
+#define BPLX_PROTECT_GROUP 1
+#define BPLX_PROTECT_ASSOCIATION 2
+typedef struct {
+  int32_t num_pairings;           /* 0..16 */
+  const uint8_t* mode;            /* host [P] BPLX_PAIRING_* */
+  const uint8_t* protect;         /* host [P] BPLX_PROTECT_* bits (seeded only), or NULL (none) */
+  const uint8_t* host_pot;        /* host [P] seeded: 1 = the unseeded entrant is at home, 0 = the seeded one; or NULL */
+  const uint8_t* pool_size;       /* host [P] n_d */
+  const uint8_t* pool_kind;       /* host [P, 64] BPLX_ENTRANT_* (not PAIRED), entries j < n_d read */
+  const uint8_t* pool_arg0;       /* host [P, 64] */
+  const uint8_t* pool_arg1;       /* host [P, 64] */
+  const uint8_t* pool_pot;        /* host [P, 64] seeded: 0 = pot A (seeded), 1 = pot B; or NULL (all open) */
+  const uint8_t* slot_assoc;      /* host [T_tab] association of each slot, 0xFF = none; or NULL */
+} bplx_pairings;
+
+size_t bplx_simulate_tournament_paired_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f,
+                                                       const bplx_table* t, const bplx_bracket* b,
+                                                       const bplx_ranking* r, const bplx_pairings* p);
+/* bplx_simulate_tournament_ranked with pairings drawn by lot (NULL or num_pairings = 0: none) and pairing_counts;
+ * bplx_simulate_tournament_ranked is this call with p = NULL and pairing_counts = NULL. */
+int bplx_simulate_tournament_paired(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_bracket* b,
+                                    const uint8_t* tie_format, const bplx_ranking* r, const bplx_pairings* p,
+                                    int max_goals, int sims_per_draw, unsigned long long seed, long long first_draw,
+                                    unsigned long long* position_counts, unsigned long long* points_counts,
+                                    unsigned long long* reach_counts, unsigned long long* win_counts,
+                                    unsigned long long* decided_counts, unsigned long long* pairing_counts,
                                     uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
                                     uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
                                     void* workspace, size_t workspace_bytes, void* stream);

@@ -10,12 +10,13 @@ __version__ = "0.1.0"
 
 def __getattr__(name):  # lazy: importing torch is slow and not needed for host-only users
     if name in ("Problem", "score_grid", "score_grid_host", "pointwise_loglik", "psis_loo",
-                "simulate_table", "simulate_tournament", "posterior_predictive"):
+                "simulate_table", "simulate_tournament", "posterior_predictive", "dynamic_forecast",
+                "pointwise_loglik_gameweeks", "posterior_predictive_gameweeks"):
         from . import problem
         return getattr(problem, name)
     if name in ("DixonColesMatchPredictor", "ExtendedDixonColesMatchPredictor", "NeutralDixonColesMatchPredictor",
                 "NeutralDixonColesMatchPredictorWC",  # the four classes bpl/__init__.py:4-7 exports
-                "DynamicNeutralDixonColesMatchPredictor"):  # not exported by the reference; fit only (SURVEY D3)
+                "DynamicNeutralDixonColesMatchPredictor"):  # not exported by the reference
         from . import predictors
         return getattr(predictors, name)
     raise AttributeError(name)

@@ -110,6 +110,8 @@ TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS = 0, 1, 2
 EXTRA_TIME_FRACTION = 1.0 / 3.0
 # BPLX_RANK_*
 RANK_GOAL_DIFF, RANK_HEAD_TO_HEAD = 0, 1
+FORECAST_KEY = 0x9E3779B97F4A7C15  # BPLX_FORECAST_KEY
+FORECAST_MAX_TEAMS = 256  # BPLX_FORECAST_MAX_TEAMS
 
 
 class BplxError(RuntimeError):
@@ -208,6 +210,19 @@ def declare(lib):
     lib.bplx_posterior_predictive.argtypes = [C.POINTER(Samples), C.POINTER(Observations), i, i, i, i, i, C.c_ulonglong,
                                               C.c_longlong, C.POINTER(PpcOutput), vp, sz, vp]
     lib.bplx_posterior_predictive.restype = i
+    lib.bplx_dynamic_forecast.argtypes = [vp, vp, i, i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp, vp, vp]
+    lib.bplx_dynamic_forecast.restype = i
+    lib.bplx_pointwise_loglik_gameweeks_workspace_bytes.argtypes = [C.POINTER(Samples), i, C.POINTER(Observations)]
+    lib.bplx_pointwise_loglik_gameweeks_workspace_bytes.restype = sz
+    lib.bplx_pointwise_loglik_gameweeks.argtypes = [C.POINTER(Samples), i, C.POINTER(Observations), vp, vp, sz, vp, vp,
+                                                    sz, vp]
+    lib.bplx_pointwise_loglik_gameweeks.restype = i
+    lib.bplx_posterior_predictive_gameweeks_workspace_bytes.argtypes = [C.POINTER(Samples), i, C.POINTER(Observations)]
+    lib.bplx_posterior_predictive_gameweeks_workspace_bytes.restype = sz
+    lib.bplx_posterior_predictive_gameweeks.argtypes = [C.POINTER(Samples), i, C.POINTER(Observations), vp, i, i, i, i,
+                                                        i, C.c_ulonglong, C.c_longlong, C.POINTER(PpcOutput), vp, sz,
+                                                        vp]
+    lib.bplx_posterior_predictive_gameweeks.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

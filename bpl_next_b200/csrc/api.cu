@@ -10,6 +10,7 @@
 #include <new>
 
 #include "common.cuh"
+#include "dynamic_predict.h"
 #include "plan.h"
 #include "problem.h"
 #include "loo.h"
@@ -1340,6 +1341,199 @@ int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* ob
   pp.scores = out->scores;
   pp.invalid = out->invalid;
   return launch_ppc(pp, static_cast<cudaStream_t>(stream));
+}
+
+// ---- the dynamic model's predictive distribution: forecast, and matches spread over gameweeks --------------------
+int bplx_dynamic_forecast(const float* attack_last, const float* defence_last, int num_samples, int num_teams,
+                          int horizon, unsigned long long seed, long long first_draw, float* attack, float* defence,
+                          float* home_attack, float* away_attack, float* home_defence, float* away_defence,
+                          void* stream) {
+  const char* what = "dynamic forecast";
+  BPLX_REQUIRE(attack_last && defence_last && attack && defence && home_attack && away_attack && home_defence &&
+                   away_defence,
+               BPLX_E_INVALID, "%s: every input and output must be given", what);
+  BPLX_REQUIRE(num_samples > 0 && num_teams > 0, BPLX_E_INVALID, "%s: num_samples and num_teams must be positive", what);
+  BPLX_REQUIRE(horizon >= 1, BPLX_E_INVALID, "%s: horizon must be >= 1 (got %d)", what, horizon);
+  BPLX_REQUIRE(first_draw >= 0 && first_draw <= LLONG_MAX - num_samples, BPLX_E_INVALID,
+               "%s: first_draw must be >= 0", what);
+  BPLX_REQUIRE(num_teams <= kForecastMaxTeams, BPLX_E_UNSUPPORTED, "%s: %d teams (max %d: BPLX_FORECAST_MAX_TEAMS)", what,
+               num_teams, kForecastMaxTeams);
+  BPLX_REQUIRE((3ull + 3ull * num_teams) * (unsigned long long)horizon < (1ull << 32), BPLX_E_UNSUPPORTED,
+               "%s: (3 + 3T) * horizon must be below 2^32 (the counter blocks of one draw)", what);
+  ForecastParams fp{};
+  fp.attack = attack_last;
+  fp.defence = defence_last;
+  float* outs[6] = {attack, defence, home_attack, away_attack, home_defence, away_defence};
+  for (int k = 0; k < 6; k++) fp.out[k] = outs[k];
+  fp.S = num_samples;
+  fp.T = num_teams;
+  fp.h = horizon;
+  fp.key = seed ^ BPLX_FORECAST_KEY;
+  fp.first_draw = first_draw;
+  return launch_dynamic_forecast(fp, static_cast<cudaStream_t>(stream));
+}
+
+// the shape of a gameweek-major call: S = num_samples / num_gameweeks draws per gameweek, every gameweek in range and,
+// when `grouped`, non-decreasing
+static int check_gameweeks(const bplx_samples* s, int ngw, const bplx_observations* obs, const int32_t* gw, bool grouped,
+                           const char* what) {
+  BPLX_REQUIRE(ngw >= 1 && s->num_samples % ngw == 0, BPLX_E_INVALID,
+               "%s: num_gameweeks (%d) must be >= 1 and divide num_samples (%d): the samples are gameweek-major", what,
+               ngw, s->num_samples);
+  BPLX_REQUIRE(gw != nullptr, BPLX_E_INVALID, "%s: gameweek is NULL", what);
+  const int M = obs->fixtures.num_fixtures;
+  for (int m = 0; m < M; m++) {
+    BPLX_REQUIRE(gw[m] >= 0 && gw[m] < ngw, BPLX_E_INVALID, "%s: match %d has gameweek %d outside [0, %d)", what, m,
+                 gw[m], ngw);
+    BPLX_REQUIRE(!grouped || m == 0 || gw[m] >= gw[m - 1], BPLX_E_INVALID,
+                 "%s: the matches are not grouped by gameweek (match %d has gameweek %d after %d)", what, m, gw[m],
+                 gw[m - 1]);
+  }
+  return BPLX_OK;
+}
+
+// workspace of the segmented log-likelihood: [G' S] table rows | partial stats [nsplit][M][4] | CTA descriptors (at most
+// one per gameweek plus one per kPwThreads matches)
+static size_t pointwise_gw_plan(const bplx_samples* s, int ngw, const bplx_observations* o, PointwiseParams* pp,
+                                const char** err, size_t* off_partial, size_t* off_seg) {
+  bind_samples(s, &o->fixtures, &pp->gp);
+  pp->gp.S = s->num_samples / ngw;
+  if (pointwise_plan(pp, err) == 0) return 0;
+  GridParams all = pp->gp;
+  all.S = s->num_samples;
+  *off_partial = table_layout(&all);
+  *off_seg = align256(*off_partial + (size_t)pp->gp.nsplit * pp->gp.F * 4 * sizeof(double));
+  const size_t max_seg = (size_t)(pp->gp.F + kPwThreads - 1) / kPwThreads + ngw;
+  return *off_seg + max_seg * sizeof(int4);
+}
+
+size_t bplx_pointwise_loglik_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
+                                                       const bplx_observations* obs) {
+  if (!s || !obs || num_gameweeks < 1 || s->num_samples <= 0 || s->num_samples % num_gameweeks || s->num_teams <= 0 ||
+      obs->fixtures.num_fixtures <= 0)
+    return 0;
+  PointwiseParams pp{};
+  size_t a, b;
+  return pointwise_gw_plan(s, num_gameweeks, obs, &pp, nullptr, &a, &b);
+}
+
+int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
+                                    const int32_t* gameweek, float* loglik, size_t ld, double* stats, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  const char* what = "pointwise log-likelihood over gameweeks";
+  BPLX_REQUIRE(obs != nullptr, BPLX_E_INVALID, "observations is NULL");
+  int rc = check_sample_args(s, &obs->fixtures, what);
+  if (rc != BPLX_OK) return rc;
+  rc = check_gameweeks(s, num_gameweeks, obs, gameweek, true, what);
+  if (rc != BPLX_OK) return rc;
+  const int S = s->num_samples / num_gameweeks, M = obs->fixtures.num_fixtures;
+  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
+               what);
+  BPLX_REQUIRE(stats != nullptr, BPLX_E_INVALID, "%s: stats is NULL", what);
+  BPLX_REQUIRE(!loglik || ld >= (size_t)S, BPLX_E_INVALID, "%s: ld (%zu) < draws per gameweek (%d)", what, ld, S);
+  PointwiseParams pp{};
+  const char* perr = nullptr;
+  size_t off_partial = 0, off_seg = 0;
+  const size_t need = pointwise_gw_plan(s, num_gameweeks, obs, &pp, &perr, &off_partial, &off_seg);
+  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
+  rc = check_workspace(workspace, workspace_bytes, need);
+  if (rc != BPLX_OK) return rc;
+  // one descriptor per (gameweek, run of up to kPwThreads of its matches): CTAs are cut at gameweek boundaries
+  std::vector<int4> seg;
+  for (int lo = 0; lo < M;) {
+    int hi = lo;
+    while (hi < M && gameweek[hi] == gameweek[lo]) hi++;
+    for (int m0 = lo; m0 < hi; m0 += kPwThreads) seg.push_back(make_int4(gameweek[lo], m0, std::min(kPwThreads, hi - m0), 0));
+    lo = hi;
+  }
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  BPLX_CUDA(cudaMemcpyAsync(ws + off_seg, seg.data(), seg.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+  pp.gp.table = reinterpret_cast<float*>(ws);
+  pp.partial = reinterpret_cast<double*>(ws + off_partial);
+  pp.seg = reinterpret_cast<const int4*>(ws + off_seg);
+  pp.nseg = (int)seg.size();
+  pp.hg = obs->home_goals;
+  pp.ag = obs->away_goals;
+  pp.ll = loglik;
+  pp.ld = ld;
+  pp.stats = stats;
+  return launch_pointwise_segmented(pp, num_gameweeks, st);
+}
+
+// workspace of the multi-gameweek predictive check: [G' S] table rows | the matches' gameweeks [M]
+size_t bplx_posterior_predictive_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
+                                                           const bplx_observations* obs) {
+  if (!s || !obs || num_gameweeks < 1 || s->num_samples <= 0 || s->num_samples % num_gameweeks || s->num_teams <= 0 ||
+      obs->fixtures.num_fixtures <= 0)
+    return 0;
+  GridParams gp{};
+  bind_samples(s, &obs->fixtures, &gp);
+  return table_layout(&gp) + (size_t)obs->fixtures.num_fixtures * sizeof(int32_t);
+}
+
+int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
+                                        const int32_t* gameweek, int max_goals, int score_bins, int points_win,
+                                        int points_draw, int sims_per_draw, unsigned long long seed,
+                                        long long first_draw, const bplx_ppc_output* out, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+  const char* what = "posterior predictive over gameweeks";
+  BPLX_REQUIRE(obs != nullptr && out != nullptr, BPLX_E_INVALID, "%s: observations / out is NULL", what);
+  int rc = check_sample_args(s, &obs->fixtures, what);
+  if (rc != BPLX_OK) return rc;
+  rc = check_gameweeks(s, num_gameweeks, obs, gameweek, false, what);
+  if (rc != BPLX_OK) return rc;
+  const int S = s->num_samples / num_gameweeks, M = obs->fixtures.num_fixtures;
+  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
+               what);
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
+               max_goals);
+  BPLX_REQUIRE(score_bins >= 2 && score_bins <= 16, BPLX_E_INVALID, "%s: score_bins must be in [2, 16] (got %d)", what,
+               score_bins);
+  BPLX_REQUIRE(points_win >= 1 && points_draw >= 0 && points_draw <= points_win, BPLX_E_INVALID,
+               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
+               points_win, points_draw);
+  BPLX_REQUIRE((long long)std::max(points_win, max_goals) * M <= INT_MAX, BPLX_E_INVALID,
+               "%s: max(points_win, max_goals) * num_matches must be below 2^31 (a team count could overflow)", what);
+  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
+  BPLX_REQUIRE(first_draw >= 0 && first_draw + S <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
+               "%s: first_draw must be >= 0 and (first_draw + S) * sims_per_draw must fit 63 bits", what);
+  BPLX_REQUIRE((long long)S * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
+               "%s: draws * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges", what,
+               (long long)S * sims_per_draw);
+  BPLX_REQUIRE(out->score_counts && out->outcome_counts && out->goals && out->total_goals_sq && out->team_points &&
+                   out->team_goals_for && out->team_goals_against && out->invalid,
+               BPLX_E_INVALID, "%s: every output but scores must be given", what);
+  PpcParams pp{};
+  bind_samples(s, &obs->fixtures, &pp.gp);
+  const size_t off_gw = table_layout(&pp.gp);
+  rc = check_workspace(workspace, workspace_bytes, off_gw + (size_t)M * sizeof(int32_t));
+  if (rc != BPLX_OK) return rc;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  BPLX_CUDA(cudaMemcpyAsync(ws + off_gw, gameweek, (size_t)M * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  pp.gp.S = S;
+  pp.gp.table = reinterpret_cast<float*>(ws);
+  pp.gw = reinterpret_cast<const int32_t*>(ws + off_gw);
+  pp.ngw = num_gameweeks;
+  pp.G = max_goals;
+  pp.B = score_bins;
+  pp.R = sims_per_draw;
+  pp.pw = points_win;
+  pp.pd = points_draw;
+  pp.seed = seed;
+  pp.first_draw = first_draw;
+  pp.N = S * sims_per_draw;
+  pp.score_counts = out->score_counts;
+  pp.outcome_counts = out->outcome_counts;
+  pp.goals = reinterpret_cast<long long*>(out->goals);
+  pp.total_goals_sq = reinterpret_cast<long long*>(out->total_goals_sq);
+  pp.team_points = out->team_points;
+  pp.team_goals_for = out->team_goals_for;
+  pp.team_goals_against = out->team_goals_against;
+  pp.scores = out->scores;
+  pp.invalid = out->invalid;
+  return launch_ppc_gameweeks(pp, st);
 }
 
 void bplx_reload_env(void) {

@@ -13,6 +13,8 @@
 //              no transpose) and keeps the running max, sum exp(ll - max), sum ll and sum ll^2 (float64).  Few matches:
 //              the samples are split over CTAs (up to 64 splits, planned from S alone); a finalize kernel combines the
 //              splits in a fixed order.
+//              pointwise_kernel<true>: matches grouped by gameweek over a gameweek-major table ([G'][S] rows); each CTA
+//              takes up to 256 matches of ONE gameweek (a host-built descriptor) and streams only that gameweek's rows.
 //   psis       one CTA per match (row of the matrix), ArviZ's _psislw / _gpdfit:
 //              (1) min ll, non-finite check and the histogram of the top 11 key bits in one pass; (2) two more radix
 //              passes (11 + 10 bits) select the (Mt+1)-th smallest ll = the (Mt+1)-th largest log-ratio x = -ll;
@@ -27,6 +29,9 @@
 namespace bplx {
 
 // ---- pointwise kernel ------------------------------------------------------------------------------------------------
+// SEG: matches grouped by gameweek, one gameweek per CTA (its descriptor pp.seg[blockIdx.x]); the CTA streams that
+// gameweek's S rows of the gameweek-major table.  Otherwise 256 consecutive matches per CTA over the S rows.
+template <bool SEG>
 __global__ void __launch_bounds__(kPwThreads, 3) pointwise_kernel(const __grid_constant__ PointwiseParams pp) {
   const GridParams& gp = pp.gp;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -34,9 +39,19 @@ __global__ void __launch_bounds__(kPwThreads, 3) pointwise_kernel(const __grid_c
   const uint32_t bar0 = smem_u32(smem_raw);
   const int tid = threadIdx.x;
   const RowLayout L = row_layout(gp.T, gp.Cf, gp.ntab);
-  const int f_raw = blockIdx.x * kPwThreads + tid;
-  const bool live = f_raw < gp.F;
-  const int f = min(f_raw, gp.F - 1);
+  int f_raw, f_end;
+  const float* table = gp.table;
+  if (SEG) {
+    const int4 d = pp.seg[blockIdx.x];
+    f_raw = d.y + tid;
+    f_end = d.y + d.z;
+    table += (size_t)d.x * gp.S * gp.row_floats;
+  } else {
+    f_raw = blockIdx.x * kPwThreads + tid;
+    f_end = gp.F;
+  }
+  const bool live = f_raw < f_end;
+  const int f = min(f_raw, f_end - 1);
   const int split = blockIdx.y;
   const int s_begin = split * gp.samples_per_split;
   const int s_end = min(gp.S, s_begin + gp.samples_per_split);
@@ -64,7 +79,7 @@ __global__ void __launch_bounds__(kPwThreads, 3) pointwise_kernel(const __grid_c
     const uint32_t bytes = (uint32_t)min(NS, s_end - s0) * row_bytes;
     const uint32_t slot = (uint32_t)st % kPwStages;
     mbar_arrive_expect_tx(bar0 + 8 * slot, bytes);
-    tma_load_1d(smem_u32(buf0 + slot * stage_floats), gp.table + (size_t)s0 * gp.row_floats, bytes, bar0 + 8 * slot);
+    tma_load_1d(smem_u32(buf0 + slot * stage_floats), table + (size_t)s0 * gp.row_floats, bytes, bar0 + 8 * slot);
   };
   if (tid == 0) {
 #pragma unroll
@@ -191,11 +206,33 @@ int launch_pointwise(PointwiseParams& pp, cudaStream_t stream) {
   const size_t smem = 128 + (size_t)kPwStages * gp.ns_stage * gp.row_floats * 4;
   static size_t smem_set = 48 * 1024;
   if (smem > smem_set) {
-    BPLX_CUDA(cudaFuncSetAttribute(pointwise_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BPLX_CUDA(cudaFuncSetAttribute(pointwise_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set = smem;
   }
   dim3 grid((gp.F + kPwThreads - 1) / kPwThreads, gp.nsplit);
-  pointwise_kernel<<<grid, kPwThreads, smem, stream>>>(pp);
+  pointwise_kernel<false><<<grid, kPwThreads, smem, stream>>>(pp);
+  BPLX_CUDA(cudaGetLastError());
+  pointwise_finalize<<<(gp.F + 255) / 256, 256, 0, stream>>>(pp);
+  BPLX_CUDA(cudaGetLastError());
+  note_launch(2);
+  return BPLX_OK;
+}
+
+int launch_pointwise_segmented(PointwiseParams& pp, int ngw, cudaStream_t stream) {
+  GridParams& gp = pp.gp;
+  pp.vec = pp.ll && pp.ld % 4 == 0 && gp.ns_stage % 4 == 0 && (reinterpret_cast<uintptr_t>(pp.ll) & 15u) == 0;
+  GridParams all = gp;  // the pre-pass builds every gameweek's rows in one launch: (gameweek, draw) is a pseudo-draw
+  all.S = ngw * gp.S;
+  int rc = launch_score_grid_tables(all, stream);
+  if (rc != BPLX_OK) return rc;
+  const size_t smem = 128 + (size_t)kPwStages * gp.ns_stage * gp.row_floats * 4;
+  static size_t smem_set = 48 * 1024;
+  if (smem > smem_set) {
+    BPLX_CUDA(cudaFuncSetAttribute(pointwise_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    smem_set = smem;
+  }
+  dim3 grid(pp.nseg, gp.nsplit);
+  pointwise_kernel<true><<<grid, kPwThreads, smem, stream>>>(pp);
   BPLX_CUDA(cudaGetLastError());
   pointwise_finalize<<<(gp.F + 255) / 256, 256, 0, stream>>>(pp);
   BPLX_CUDA(cudaGetLastError());

@@ -18,6 +18,10 @@ struct PointwiseParams {
   int vec;                  // rows and stages are 16-byte aligned: the matrix is written with 16-byte stores
   double* partial;          // [nsplit][M][4]
   double* stats;            // [M][4]
+  // gameweek-segmented call (pointwise_kernel<true>): CTA c takes matches [seg[c].y, seg[c].y + seg[c].z), all of
+  // gameweek seg[c].x, whose draws are rows [seg[c].x * S, (seg[c].x + 1) * S) of a gameweek-major table (gp.S = S)
+  const int4* seg;
+  int nseg;
 };
 
 struct PsisParams {
@@ -34,6 +38,8 @@ struct PsisParams {
 // 0 with *err set when a sample row does not fit a stage buffer
 size_t pointwise_plan(PointwiseParams* pp, const char** err);
 int launch_pointwise(PointwiseParams& pp, cudaStream_t stream);
+// the segmented call: the pre-pass over the ngw * S rows of the gameweek-major table, one CTA per descriptor of pp.seg
+int launch_pointwise_segmented(PointwiseParams& pp, int ngw, cudaStream_t stream);
 
 // tail length of PSIS for S draws at relative efficiency r_eff
 int psis_tail_length(int S, double r_eff);

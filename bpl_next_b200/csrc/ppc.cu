@@ -29,12 +29,15 @@ namespace bplx {
 
 namespace {
 
+// MULTI: the draw's rows of pp.ngw gameweeks side by side in shared memory, match m on the row of gameweek pp.gw[m]
+template <bool MULTI>
 __global__ void __launch_bounds__(kPpcThreads) ppc_kernel(const __grid_constant__ PpcParams pp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const GridParams& gp = pp.gp;
   const int T = gp.T, M = gp.F, B = pp.B, tid = threadIdx.x;
+  const int rows = MULTI ? pp.ngw : 1;
   float* const s_row = reinterpret_cast<float*>(smem_raw);
-  int* const s_cells = reinterpret_cast<int*>(s_row + gp.row_floats);  // [B][B]
+  int* const s_cells = reinterpret_cast<int*>(s_row + rows * gp.row_floats);  // [B][B]
   int* const s_pts = s_cells + B * B;                                   // [T]
   int* const s_gf = s_pts + T;
   int* const s_ga = s_gf + T;
@@ -45,8 +48,17 @@ __global__ void __launch_bounds__(kPpcThreads) ppc_kernel(const __grid_constant_
   const int i = blockIdx.x;  // (N < 2^31 per call)
   const int s = i / pp.R, r = i - s * pp.R;
   const unsigned long long n = (unsigned long long)(pp.first_draw + s) * (unsigned long long)pp.R + (unsigned)r;
-  const float4* const src = reinterpret_cast<const float4*>(gp.table + (size_t)s * gp.row_floats);
-  for (int k = tid; k < gp.row_floats / 4; k += kPpcThreads) reinterpret_cast<float4*>(s_row)[k] = src[k];
+  if (MULTI) {
+    const int q = gp.row_floats / 4;
+    for (int k = tid; k < rows * q; k += kPpcThreads) {
+      const int g = k / q;
+      reinterpret_cast<float4*>(s_row)[k] =
+          reinterpret_cast<const float4*>(gp.table + ((size_t)g * gp.S + s) * gp.row_floats)[k - g * q];
+    }
+  } else {
+    const float4* const src = reinterpret_cast<const float4*>(gp.table + (size_t)s * gp.row_floats);
+    for (int k = tid; k < gp.row_floats / 4; k += kPpcThreads) reinterpret_cast<float4*>(s_row)[k] = src[k];
+  }
   for (int k = tid; k < B * B + 3 * T; k += kPpcThreads) s_cells[k] = 0;
   if (tid < 3) {
     s_outcome[tid] = 0;
@@ -73,8 +85,9 @@ __global__ void __launch_bounds__(kPpcThreads) ppc_kernel(const __grid_constant_
     bool ok = ht < T && at < T && (!wc || (hc < gp.Cf && ac < gp.Cf));
     if (ok) {
       const FixtureOffsets off = fixture_offsets(L, ht, at, neutral, wc, hc, ac);
-      const float2 lam = fixture_rates(s_row, off, neutral, wc);
-      ok = sample_score(lam.x, lam.y, c, _curand_uniform(wh), _curand_uniform(wa), pp.G, hg, ag);
+      const float* const row = MULTI ? s_row + pp.gw[m] * gp.row_floats : s_row;
+      const float2 lam = fixture_rates(row, off, neutral, wc);
+      ok = sample_score(lam.x, lam.y, MULTI ? row[L.C] : c, _curand_uniform(wh), _curand_uniform(wa), pp.G, hg, ag);
     }
     if (ok) {
       atomicAdd(&s_cells[min(hg, B - 1) * B + min(ag, B - 1)], 1);
@@ -139,29 +152,36 @@ __global__ void __launch_bounds__(kPpcThreads) ppc_kernel(const __grid_constant_
 
 }  // namespace
 
-size_t ppc_smem_bytes(const PpcParams& pp) {
-  return (size_t)pp.gp.row_floats * 4 + ((size_t)pp.B * pp.B + 3 * (size_t)pp.gp.T) * 4;
+size_t ppc_smem_bytes(const PpcParams& pp, int rows) {
+  return (size_t)rows * pp.gp.row_floats * 4 + ((size_t)pp.B * pp.B + 3 * (size_t)pp.gp.T) * 4;
 }
 
-int launch_ppc(const PpcParams& pp, cudaStream_t stream) {
+template <bool MULTI>
+static int launch(const PpcParams& pp, cudaStream_t stream) {
   int rc = upload_sim_constants();
   if (rc != BPLX_OK) return rc;
-  const size_t smem = ppc_smem_bytes(pp);
+  const int rows = MULTI ? pp.ngw : 1;
+  const size_t smem = ppc_smem_bytes(pp, rows);
   BPLX_REQUIRE(smem <= (size_t)kPpcSmemMax, BPLX_E_UNSUPPORTED,
-               "posterior predictive: %zu bytes of shared memory per CTA needed for %d teams (max %d)", smem, pp.gp.T,
-               kPpcSmemMax);
-  static size_t smem_set = 48 * 1024;
+               "posterior predictive: %zu bytes of shared memory per CTA needed for %d teams and %d gameweeks (max %d)",
+               smem, pp.gp.T, rows, kPpcSmemMax);
+  static size_t smem_set = 48 * 1024;  // per instantiation
   if (smem > smem_set) {
-    BPLX_CUDA(cudaFuncSetAttribute(ppc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BPLX_CUDA(cudaFuncSetAttribute(ppc_kernel<MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set = smem;
   }
   BPLX_CUDA(cudaMemsetAsync(pp.invalid, 0, 8, stream));
-  rc = launch_score_grid_tables(pp.gp, stream);
+  GridParams all = pp.gp;  // (gameweek, draw) pairs are the pseudo-draws of the pre-pass
+  all.S = rows * pp.gp.S;
+  rc = launch_score_grid_tables(all, stream);
   if (rc != BPLX_OK) return rc;
-  ppc_kernel<<<(unsigned)pp.N, kPpcThreads, smem, stream>>>(pp);
+  ppc_kernel<MULTI><<<(unsigned)pp.N, kPpcThreads, smem, stream>>>(pp);
   BPLX_CUDA(cudaGetLastError());
   note_launch(1);
   return BPLX_OK;
 }
+
+int launch_ppc(const PpcParams& pp, cudaStream_t stream) { return launch<false>(pp, stream); }
+int launch_ppc_gameweeks(const PpcParams& pp, cudaStream_t stream) { return launch<true>(pp, stream); }
 
 }  // namespace bplx

@@ -23,7 +23,7 @@ from . import data as bdata
 from . import nuts as bnuts
 from . import parallel
 from . import season as bseason
-from .problem import Problem, pointwise_loglik, psis_loo, score_grid_host
+from .problem import Problem, pointwise_loglik, psis_loo, score_grid_host, take_rows
 from .problem import simulate_table as _simulate_table
 from .problem import simulate_tournament as _simulate_tournament
 
@@ -320,7 +320,7 @@ class _BplxPredictor:
         key.update(obs["home_goals"].tobytes() + obs["away_goals"].tobytes())
         return obs, key.hexdigest()
 
-    def _comparison_inputs(self, data):
+    def _comparison_inputs(self, data, random_state=None):
         obs, key = self._observations(data)
         ds = self._device_samples()
         do = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in obs.items()}
@@ -422,22 +422,20 @@ class _BplxPredictor:
         if self.teams is None:
             raise ValueError("the model is not fitted: fit it first")
         from . import ppc as bppc
-        from .problem import posterior_predictive
 
         seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
         R, B = int(num_sims_per_draw), int(score_bins)
         if R < 1:
             raise ValueError(f"num_sims_per_draw must be >= 1, got {num_sims_per_draw}")
-        ds, do, key = self._comparison_inputs(data)
-        S, T, M = int(ds["attack"].shape[0]), int(ds["attack"].shape[1]), int(do["home_team"].shape[0])
+        ds, do, key = self._comparison_inputs(data, seed)
+        S, T, M = int(ds["attack"].shape[-2]), int(ds["attack"].shape[-1]), int(do["home_team"].shape[0])
         step = (2 ** 31 - 1) // R  # replicates per call stay below 2^31
         per_rep = 4 * (B * B + 3 + 3 * T) + 8 * 3 + (2 * M if return_replicates else 0)  # device output bytes
         step = min(step, max(1, SIM_OUTPUT_BYTES // (R * per_rep)))
         parts, scores, invalid = [], [], 0
         for lo in range(0, S, step):
             hi = min(S, lo + step)
-            out = posterior_predictive(self.model, {k: v[lo:hi] for k, v in ds.items()}, do, max_goals, B, points, R,
-                                       seed, first_draw=lo, want_scores=return_replicates)
+            out = self._replicates(ds, do, lo, hi, max_goals, B, points, R, seed, return_replicates)
             invalid += int(out["invalid"].item())
             parts.append({k: out[k].cpu().numpy() for k in bppc.STATISTICS})
             if return_replicates:
@@ -457,6 +455,13 @@ class _BplxPredictor:
             res.update(replicates=reps, home_score=np.ascontiguousarray(sc[:, :, 0].T),
                        away_score=np.ascontiguousarray(sc[:, :, 1].T))
         return res
+
+    def _replicates(self, ds, do, lo, hi, max_goals, B, points, R, seed, want_scores):
+        """``posterior_predictive`` on draws ``[lo, hi)``."""
+        from .problem import posterior_predictive
+
+        return posterior_predictive(self.model, {k: v[lo:hi] for k, v in ds.items()}, do, max_goals, B, points, R, seed,
+                                    first_draw=lo, want_scores=want_scores)
 
     # ---- simulation from the grid (bpl/base.py:150-246, bpl/_util.py:96-112) -----------------------------------
     @staticmethod
@@ -936,11 +941,31 @@ class NeutralDixonColesMatchPredictorWC(NeutralDixonColesMatchPredictor):
 
 
 class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
-    """``bpl/dynamic_dixon_coles.py:23-334`` -- ``fit`` only.  The reference's predict methods index a Python list with a
-    tuple and cannot run (SURVEY.md D3), so they are not mirrored.  ``walk="intended"`` (default) makes attack / defence the
-    cumulative random walk the model describes; ``walk="as_written"`` reproduces ``:192-218`` literally (SURVEY D1).
-    Gameweeks are 0-based and G = max + 1 (the reference passes ``max``, SURVEY D2)."""
+    """``bpl/dynamic_dixon_coles.py:23-334``.  ``walk="intended"`` (default) makes attack / defence the cumulative random
+    walk the model describes; ``walk="as_written"`` reproduces ``:192-218`` literally (SURVEY D1).  Gameweeks are 0-based
+    and G = max + 1 (the reference passes ``max``, SURVEY D2).
+
+    Predictive distribution.  The reference's predict methods index a Python list with a tuple and cannot run (SURVEY
+    D3), and their venue signs disagree with ``_model``; they are not mirrored.  Instead, at a fixed gameweek the model's
+    rates are exactly the NEUTRAL model's rates, so every predictive method works on one gameweek of the posterior at a
+    time (``at_gameweek``), with the rates of ``_model``:
+
+    * Scope: only a fit with ``walk="intended"`` has a predictive distribution (an ``as_written`` fit's likelihood never
+      reaches the walk); otherwise every predictive method raises ``NotImplementedError``.
+    * Fitted gameweek (g < G): per draw, ``attack[g]``, ``defence[g]``, the four venue effects ``[:, g]`` and
+      ``corr_coef``, as ``fit`` records them.
+    * Forecast gameweek (g >= G): the model's own generative process continued from the last fitted state.  For each
+      draw and each gameweek j = G .. g in order, fresh sites from their priors (means N(+-0.1, 0.2), the six spreads
+      HalfNormal(1), per team u ~ Beta(2, 4), rho = 2u - 1, za ~ N(0, 1), zd = rho za + sqrt(1 - rho^2) eps, the four
+      decentred effects N(0, 1)); ``attack[j] = attack[j - 1] + za std_attack[j]`` (defence likewise with zd), venue
+      effects ``mean[j] + std[j] decentered[j]`` (not cumulative).  With HalfNormal(1) venue spreads this forecast is
+      WIDE: it is what the model says about gameweeks it has not seen, nothing more.  Its random numbers are Philox words
+      under ``random_state`` (include/bplx.h gives the word map), the same for any cut of the draws.
+    * ``gameweek`` defaults to G - 1, the latest fitted state (not a forecast).
+    """
     model = "dynamic"
+    _effects = NeutralDixonColesMatchPredictor._effects
+    _fixture_extras = NeutralDixonColesMatchPredictor._fixture_extras
 
     def __init__(self, walk: str = "intended"):
         super().__init__()
@@ -959,6 +984,7 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         arr.as_written = self.walk == "as_written"
         self.teams, self._teams_dict = list(meta["teams"]), meta["teams_dict"]
         self.problem = p = Problem(arr)
+        self._train_arrays = arr  # the matches log_likelihood() / waic() / loo() evaluate by default
         G, T = arr.num_gameweeks, arr.num_teams
         flat_dev, cc = _run_chains(p, num_chains, random_state, num_warmup, num_samples, thin, kw, self)
         flat = flat_dev.cpu().numpy()
@@ -1001,18 +1027,241 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         self.defence = [dfn[:, j] for j in range(G)]
         return self
 
-    def simulate_table(self, *args, **kwargs):
-        raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
-                                  "cannot run in the reference (SURVEY.md D3)")
+    # ---- the predictive distribution: one gameweek of the posterior is a NEUTRAL sample set ----------------------
+    def _require_predictive(self):
+        if getattr(self, "attack", None) is None or self.walk != "intended":
+            raise NotImplementedError(
+                "the dynamic model's predictive distribution needs a fit of a predictor built with walk=\"intended\" "
+                "(the constructor argument): an as_written fit's likelihood never reaches the walk (SURVEY D1)")
 
-    def simulate_tournament(self, *args, **kwargs):
-        raise NotImplementedError("simulation needs the predictive distribution, and the dynamic model's predict methods "
-                                  "cannot run in the reference (SURVEY.md D3)")
+    @staticmethod
+    def _seed(random_state) -> int:
+        return int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
 
-    def posterior_predictive_check(self, *args, **kwargs):
-        raise NotImplementedError("posterior predictive checks need the predictive distribution, and the dynamic model's "
-                                  "predict methods cannot run in the reference (SURVEY.md D3)")
+    def _fixture_gameweeks(self, gameweek, n: int) -> np.ndarray:
+        """``[n]`` gameweeks of the fixtures: None -> G - 1, a scalar for all, or one per fixture."""
+        if gameweek is None:
+            return np.full(n, len(self.attack) - 1, np.int64)
+        g = np.asarray(gameweek)
+        if g.dtype.kind not in "iu" or (g.ndim == 1 and len(g) not in (1, n)) or g.ndim > 1:
+            raise ValueError(f"gameweek must be an integer or one integer per fixture (got {gameweek!r})")
+        if (g < 0).any():
+            raise ValueError(f"gameweek must be >= 0 (got {gameweek!r})")
+        return np.resize(g.astype(np.int64), n)
 
-    def _comparison_inputs(self, data):
-        raise NotImplementedError("model comparison needs the predictive distribution, and the dynamic model's predict "
-                                  "methods cannot run in the reference (SURVEY.md D3)")
+    def _one_gameweek(self, gameweek) -> int:
+        if np.ndim(gameweek) > 0:
+            if len(np.unique(np.asarray(gameweek))) != 1:
+                raise ValueError("every fixture of this call is played at one gameweek: pass a single gameweek")
+            gameweek = np.asarray(gameweek)[0]
+        return int(self._fixture_gameweeks(gameweek, 1)[0])
+
+    def _slabs(self, gameweeks, seed: int) -> Dict[int, Dict[str, np.ndarray]]:
+        """NEUTRAL sample sets ``{g: {attack, defence, four venue effects [S, T], corr_coef [S]}}`` of the gameweeks, the
+        forecast ones drawn in one call under ``seed``."""
+        from .problem import dynamic_forecast
+
+        G = len(self.attack)
+        gws = sorted({int(g) for g in gameweeks})
+        fc = None
+        if gws and gws[-1] >= G:
+            dev = lambda x: torch.from_numpy(np.ascontiguousarray(x, np.float32)).cuda()  # noqa: E731
+            out = dynamic_forecast(dev(self.attack[G - 1]), dev(self.defence[G - 1]), gws[-1] - G + 1, seed)
+            fc = {k: v.cpu().numpy() for k, v in out.items()}
+        slabs = {}
+        for g in gws:
+            if g < G:
+                d = {"attack": self.attack[g], "defence": self.defence[g],
+                     **{nm: getattr(self, nm)[:, g] for nm in self._effects}}
+            else:
+                d = {k: fc[k][g - G] for k in fc}
+            d = {k: np.ascontiguousarray(v, np.float32) for k, v in d.items()}
+            d["corr_coef"] = np.ascontiguousarray(self.corr_coef, np.float32)
+            slabs[g] = d
+        return slabs
+
+    def at_gameweek(self, gameweek: int, random_state: int = 0) -> "NeutralDixonColesMatchPredictor":
+        """A ``NeutralDixonColesMatchPredictor`` with the same teams and this gameweek's draws (fitted for g < G, else
+        the forecast under ``random_state``): every single-gameweek question goes through the NEUTRAL class."""
+        self._require_predictive()
+        g = self._one_gameweek(gameweek)
+        p = NeutralDixonColesMatchPredictor()
+        p.teams, p._teams_dict = list(self.teams), dict(self._teams_dict)
+        for k, v in self._slabs([g], self._seed(random_state))[g].items():
+            setattr(p, k, v)
+        return p
+
+    def _grid(self, home_team, away_team, max_goals, gameweek=None, forecast_seed=0, **kw):
+        """The base class's grid, per fixture at its gameweek: the fixtures are grouped by gameweek, each group through
+        the NEUTRAL grid of that gameweek's draws."""
+        h, a = self._parse_fixture_args(home_team, away_team)
+        fx = {"home_team": h, "away_team": a, **self._fixture_extras(len(h), **kw)}
+        gw = self._fixture_gameweeks(gameweek, len(h))
+        g = max_goals + 1
+        grid, outcome = np.empty((len(h), g, g), np.float32), np.empty((len(h), 3), np.float32)
+        for gv, smp in self._slabs(np.unique(gw), int(forecast_seed)).items():
+            idx = np.flatnonzero(gw == gv)
+            grid[idx], outcome[idx] = score_grid_host("neutral", smp, {k: v[idx] for k, v in fx.items()}, max_goals)
+        return grid, outcome
+
+    def predict_score_grid_proba(self, home_team, away_team, neutral_venue, max_goals: int = MAX_GOALS, gameweek=None,
+                                 random_state: int = 0):
+        """NEUTRAL's ``predict_score_grid_proba`` at ``gameweek`` (scalar or per fixture; default G - 1); forecast
+        gameweeks under ``random_state``."""
+        self._require_predictive()
+        return _BplxPredictor.predict_score_grid_proba(self, home_team, away_team, max_goals=max_goals,
+                                                       neutral_venue=neutral_venue, gameweek=gameweek,
+                                                       forecast_seed=random_state)
+
+    def predict_outcome_proba(self, home_team, away_team, neutral_venue, knockout: bool = False,
+                              max_goals: int = MAX_GOALS, gameweek=None, random_state: int = 0):
+        """NEUTRAL's ``predict_outcome_proba`` at ``gameweek`` (see ``predict_score_grid_proba``)."""
+        self._require_predictive()
+        return _BplxPredictor.predict_outcome_proba(self, home_team, away_team, max_goals=max_goals, knockout=knockout,
+                                                    neutral_venue=neutral_venue, gameweek=gameweek,
+                                                    forecast_seed=random_state)
+
+    def predict_score_proba(self, home_team, away_team, home_goals, away_goals, neutral_venue, gameweek=None,
+                            random_state: int = 0):
+        """NEUTRAL's ``predict_score_proba`` at ``gameweek`` (see ``predict_score_grid_proba``)."""
+        self._require_predictive()
+        return _BplxPredictor.predict_score_proba(self, home_team, away_team, home_goals, away_goals,
+                                                  neutral_venue=neutral_venue, gameweek=gameweek,
+                                                  forecast_seed=random_state)
+
+    def predict_score_n_proba(self, n, team, opponent, home: bool = True, neutral_venue: int = 0,
+                              max_goals: int = MAX_GOALS, gameweek=None, random_state: int = 0):
+        self._require_predictive()
+        return self._n_proba(n, team, opponent, home, max_goals, True, neutral_venue=neutral_venue,
+                             gameweek=self._one_gameweek(gameweek), forecast_seed=random_state)
+
+    def predict_concede_n_proba(self, n, team, opponent, home: bool = True, neutral_venue: int = 0,
+                                max_goals: int = MAX_GOALS, gameweek=None, random_state: int = 0):
+        self._require_predictive()
+        return self._n_proba(n, team, opponent, home, max_goals, False, neutral_venue=neutral_venue,
+                             gameweek=self._one_gameweek(gameweek), forecast_seed=random_state)
+
+    def sample_score(self, home_team, away_team, neutral_venue, num_samples: int = 1, random_state: Optional[int] = None,
+                     max_goals: int = MAX_GOALS, gameweek=None):
+        """NEUTRAL's ``sample_score`` at ``gameweek``; ``random_state`` seeds both the forecast and the sampling."""
+        self._require_predictive()
+        seed = self._seed(random_state)
+        return self._sample_score(home_team, away_team, num_samples, seed, max_goals, neutral_venue=neutral_venue,
+                                  gameweek=gameweek, forecast_seed=seed)
+
+    def sample_outcome(self, home_team, away_team, neutral_venue, knockout: bool = False, num_samples: int = 1,
+                       random_state: Optional[int] = None, max_goals: int = MAX_GOALS, gameweek=None):
+        """NEUTRAL's ``sample_outcome`` at ``gameweek``; ``random_state`` seeds both the forecast and the sampling."""
+        self._require_predictive()
+        seed = self._seed(random_state)
+        return self._sample_outcome(home_team, away_team, num_samples, seed, max_goals, knockout=knockout,
+                                    neutral_venue=neutral_venue, gameweek=gameweek, forecast_seed=seed)
+
+    def simulate_table(self, fixtures, played=None, teams=None, groups=None, num_sims_per_draw: int = 1,
+                       random_state: Optional[int] = None, max_goals: int = MAX_GOALS, points=(3, 1),
+                       return_simulations: bool = False, tiebreak: str = "goal_difference", gameweek=None):
+        """NEUTRAL's ``simulate_table`` with every fixture played at one ``gameweek`` (default G - 1; "the next season"
+        is ``gameweek=G`` when the gameweeks are seasons).  ``random_state`` seeds the forecast and the simulation."""
+        self._require_predictive()
+        seed = self._seed(random_state)
+        return self.at_gameweek(self._one_gameweek(gameweek), seed).simulate_table(
+            fixtures, played, teams, groups, num_sims_per_draw, seed, max_goals, points, return_simulations, tiebreak)
+
+    def simulate_tournament(self, fixtures, bracket, played=None, teams=None, groups=None, best=None, team_conf=None,
+                            num_sims_per_draw: int = 1, random_state: Optional[int] = None, max_goals: int = MAX_GOALS,
+                            points=(3, 1), return_simulations: bool = False, tiebreak: str = "goal_difference",
+                            pairings=None, association=None, gameweek=None):
+        """NEUTRAL's ``simulate_tournament`` with every match played at one ``gameweek`` (see ``simulate_table``)."""
+        self._require_predictive()
+        seed = self._seed(random_state)
+        return self.at_gameweek(self._one_gameweek(gameweek), seed).simulate_tournament(
+            fixtures, bracket, played, teams, groups, best, team_conf, num_sims_per_draw, seed, max_goals, points,
+            return_simulations, tiebreak, pairings, association)
+
+    # ---- model comparison and predictive checks over the gameweeks of the data --------------------------------------
+    def _comparison_inputs(self, data, random_state=0):
+        """Device samples ``[G', S, T]`` of the gameweeks the matches of ``data`` (default: the training data) use, the
+        device observations with ``gameweek`` (host, each match's index into the G' gameweeks) and the match key."""
+        self._require_predictive()
+        obs, key = self._observations(data)
+        if data is None:
+            gw = np.asarray(self._train_arrays.gameweek, np.int64)
+            obs.setdefault("neutral_venue", np.zeros(len(gw), np.uint8))
+        else:
+            if "gameweek" not in data:
+                raise ValueError("the dynamic model scores each match at its gameweek: data needs the key 'gameweek'")
+            gw = self._fixture_gameweeks(np.asarray(data["gameweek"]), len(obs["home_team"]))
+        used, index = np.unique(gw, return_inverse=True)
+        slabs = self._slabs(used, self._seed(random_state))
+        ds = {k: torch.from_numpy(np.stack([slabs[g][k] for g in used])).cuda() for k in slabs[int(used[0])]}
+        do = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in obs.items()}
+        do["gameweek"] = index.astype(np.int32)
+        return ds, do, key
+
+    def _pointwise(self, ds, do, **kw):
+        from .problem import pointwise_loglik_gameweeks
+
+        dev = {k: v for k, v in do.items() if k != "gameweek"}
+        return pointwise_loglik_gameweeks("neutral", ds, dev, do["gameweek"], **kw)
+
+    def log_likelihood(self, data=None, random_state: int = 0) -> np.ndarray:
+        """The base class's ``log_likelihood`` with each match scored at its gameweek (``data["gameweek"]``; held-out
+        gameweeks >= G on the forecast under ``random_state``), in one launch over all gameweeks."""
+        ds, do, _ = self._comparison_inputs(data, random_state)
+        ll, _ = self._pointwise(ds, do)
+        return np.ascontiguousarray(ll.cpu().numpy().T)
+
+    def waic(self, data=None, random_state: int = 0) -> Dict[str, Any]:
+        """The base class's ``waic`` with each match scored at its gameweek (see ``log_likelihood``)."""
+        ds, do, key = self._comparison_inputs(data, random_state)
+        _, st = self._pointwise(ds, do, want_matrix=False)
+        return bcompare.waic_from_stats(st.cpu().numpy(), int(ds["attack"].shape[1]), key)
+
+    def log_score(self, data, random_state: int = 0) -> Dict[str, Any]:
+        """The base class's ``log_score`` with each match scored at its gameweek: later gameweeks (>= G) on the forecast
+        under ``random_state``, so "does the walk forecast the next season better than a static fit?" is one comparison
+        of the two log scores."""
+        ds, do, _ = self._comparison_inputs(data, random_state)
+        _, st = self._pointwise(ds, do, want_matrix=False)
+        lppd = bcompare.lppd_from_stats(st.cpu().numpy(), int(ds["attack"].shape[1]))
+        return {"log_score": float(lppd.sum()), "pointwise": lppd, "num_matches": len(lppd)}
+
+    def loo(self, r_eff: float = 1.0) -> Dict[str, Any]:
+        """The base class's ``loo`` on the training data, each match scored at its (fitted) gameweek: the matrix of the
+        matches grouped by gameweek comes from one launch per range of ``LOO_MATRIX_BYTES``; results in match order."""
+        ds, do, key = self._comparison_inputs(None)
+        S, M = int(ds["attack"].shape[1]), int(do["home_team"].shape[0])
+        order = np.argsort(do["gameweek"], kind="stable")
+        idx = torch.from_numpy(order).cuda()
+        srt = {k: (v[order] if k == "gameweek" else take_rows(v, idx)) for k, v in do.items()}
+        rows = max(1, min(M, LOO_MATRIX_BYTES // (4 * S)))
+        buf = torch.empty((rows, S), dtype=torch.float32, device="cuda")
+        elpd, khat, lppd = [], [], []
+        for lo in range(0, M, rows):
+            hi = min(M, lo + rows)
+            ll, st = self._pointwise(ds, {k: v[lo:hi] for k, v in srt.items()}, loglik=buf)
+            e, k = psis_loo(ll, r_eff)
+            elpd.append(e.cpu().numpy())
+            khat.append(k.cpu().numpy())
+            lppd.append(bcompare.lppd_from_stats(st.cpu().numpy(), S))
+        inv = np.argsort(order, kind="stable")
+        return bcompare.loo_from_pointwise(np.concatenate(elpd)[inv], np.concatenate(khat)[inv],
+                                           np.concatenate(lppd)[inv], S, r_eff, key)
+
+    def posterior_predictive_check(self, data=None, num_sims_per_draw: int = 1, random_state: Optional[int] = None,
+                                   max_goals: int = MAX_GOALS, score_bins: int = 6, points=(3, 1),
+                                   return_replicates: bool = False) -> Dict[str, Any]:
+        """The base class's ``posterior_predictive_check`` with each match replicated at its gameweek
+        (``data["gameweek"]``, default the training data; ``random_state`` also seeds forecast gameweeks): the same
+        replicate index, words and statistics, one launch per range of draws."""
+        self._require_predictive()
+        return super().posterior_predictive_check(data, num_sims_per_draw, random_state, max_goals, score_bins, points,
+                                                  return_replicates)
+
+    def _replicates(self, ds, do, lo, hi, max_goals, B, points, R, seed, want_scores):
+        from .problem import posterior_predictive_gameweeks
+
+        dev = {k: v for k, v in do.items() if k != "gameweek"}
+        return posterior_predictive_gameweeks("neutral", {k: v[:, lo:hi].contiguous() for k, v in ds.items()}, dev,
+                                              do["gameweek"], max_goals, B, points, R, seed, first_draw=lo,
+                                              want_scores=want_scores)

@@ -1,5 +1,6 @@
 """Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik``,
-``psis_loo``, ``simulate_table``, ``simulate_tournament`` and ``posterior_predictive``.
+``psis_loo``, ``simulate_table``, ``simulate_tournament`` and ``posterior_predictive``; for the dynamic model's
+gameweeks ``dynamic_forecast``, ``pointwise_loglik_gameweeks`` and ``posterior_predictive_gameweeks``.
 
 torch is used only for device memory and streams; every number comes from ``libbplx.so``.
 """
@@ -593,4 +594,127 @@ def posterior_predictive(model: str, samples: Dict[str, torch.Tensor], observati
     _abi.check(lib.bplx_posterior_predictive(C.byref(s), C.byref(o), int(max_goals), B, pw, pd, int(sims_per_draw),
                                              int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw), C.byref(out),
                                              _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    return res
+
+
+# ---- the dynamic model's predictive distribution ----------------------------------------------------------------
+_FORECAST_SITES = ("attack", "defence", "home_attack", "away_attack", "home_defence", "away_defence")
+
+
+def dynamic_forecast(attack_last: torch.Tensor, defence_last: torch.Tensor, horizon: int, seed: int,
+                     first_draw: int = 0, stream=None) -> Dict[str, torch.Tensor]:
+    """Device path of ``bplx_dynamic_forecast``: the dynamic model's gameweeks ``G .. G + horizon - 1`` drawn from its
+    own generative process, continued from the walk at gameweek ``G - 1`` (``attack_last`` / ``defence_last [S, T]``
+    float32 on the GPU, draws ``first_draw ..``).  Returns the six NEUTRAL sites ``[horizon, S, T]``: ``attack``,
+    ``defence``, ``home_attack``, ``away_attack``, ``home_defence``, ``away_defence`` (word map in include/bplx.h)."""
+    lib = _abi.lib()
+    assert attack_last.is_cuda and attack_last.dtype == torch.float32 and attack_last.is_contiguous()
+    assert defence_last.shape == attack_last.shape and defence_last.dtype == torch.float32 and defence_last.is_contiguous()
+    S, T = int(attack_last.shape[0]), int(attack_last.shape[1])
+    out = {k: torch.empty((int(horizon), S, T), dtype=torch.float32, device=attack_last.device) for k in _FORECAST_SITES}
+    _abi.check(lib.bplx_dynamic_forecast(_dptr(attack_last), _dptr(defence_last), S, T, int(horizon),
+                                         int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
+                                         *(_dptr(out[k]) for k in _FORECAST_SITES), _stream_ptr(stream)))
+    return out
+
+
+def _gameweek_major(samples: Dict[str, torch.Tensor]):
+    """``[G', S, T]`` sample arrays (``corr_coef [G', S]``) -> the ``[G' S, ...]`` pseudo-draws the C ABI takes, G', S."""
+    G, S = int(samples["attack"].shape[0]), int(samples["attack"].shape[1])
+    flat = {k: None if v is None else v.reshape((G * S,) + tuple(v.shape[2:])) for k, v in samples.items()}
+    return flat, G, S
+
+
+def take_rows(v: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
+    """``v[idx]`` along the first axis; uint16 team indices go through their int16 view (torch has no uint16 gather)."""
+    if v.dtype == torch.uint16:
+        return v.view(torch.int16).index_select(0, idx).view(torch.uint16)
+    return v.index_select(0, idx)
+
+
+def _gw_observations(samples, observations, gameweek, keep):
+    ptr = _device_ptr_fn(keep)
+    _check_inputs(samples, observations, ("home_goals", "away_goals"))
+    o = _abi.Observations()
+    o.fixtures = _fixtures_struct(observations, ptr)
+    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    gw = np.ascontiguousarray(gameweek, dtype=np.int32)
+    keep.append(gw)
+    return o, gw
+
+
+def pointwise_loglik_gameweeks(model: str, samples: Dict[str, torch.Tensor], observations: Dict[str, torch.Tensor],
+                               gameweek, want_matrix: bool = True, loglik: Optional[torch.Tensor] = None,
+                               workspace=None, stream=None):
+    """``pointwise_loglik`` for matches spread over gameweeks, in one launch (``bplx_pointwise_loglik_gameweeks``).
+    ``samples``: NEUTRAL-form arrays ``[G', S, T]`` (``corr_coef [G', S]``) on the GPU, gameweek-major; ``gameweek``:
+    host ints ``[M]`` in ``[0, G')``, match m's gameweek.  The matches are grouped by gameweek here (a stable sort) and
+    the outputs returned in the order given: ``(loglik [M, S] or None, stats [M, 4])``.  ``loglik`` (an ``[M, ld]``
+    buffer) is only filled in place when the matches are already grouped."""
+    lib = _abi.lib()
+    gw = np.asarray(gameweek, dtype=np.int64)
+    order = np.argsort(gw, kind="stable")
+    grouped = bool((np.diff(gw) >= 0).all())
+    if not grouped:
+        idx = torch.from_numpy(order).to(observations["home_team"].device)
+        observations = {k: take_rows(v, idx) for k, v in observations.items()}
+        gw, loglik = gw[order], None
+    flat, G, S = _gameweek_major(samples)
+    keep = []
+    s = _samples_struct(model, flat, _device_ptr_fn(keep))
+    o, gw32 = _gw_observations(flat, observations, gw, keep)
+    M = o.fixtures.num_fixtures
+    dev = samples["attack"].device
+    workspace = _workspace(workspace, int(lib.bplx_pointwise_loglik_gameweeks_workspace_bytes(C.byref(s), G,
+                                                                                              C.byref(o))), dev)
+    ld = 0
+    if want_matrix:
+        if loglik is None:
+            loglik = torch.empty((M, S), dtype=torch.float32, device=dev)
+        assert loglik.dtype == torch.float32 and loglik.shape[0] >= M and loglik.stride(1) == 1
+        ld = int(loglik.stride(0)) if M > 1 else max(S, int(loglik.shape[1]))
+    stats = torch.empty((M, 4), dtype=torch.float64, device=dev)
+    _abi.check(lib.bplx_pointwise_loglik_gameweeks(C.byref(s), G, C.byref(o), gw32.ctypes.data,
+                                                   _dptr(loglik) if want_matrix else None, ld, _dptr(stats),
+                                                   _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    ll = loglik[:M, :S] if want_matrix else None
+    if not grouped:
+        inv = torch.from_numpy(np.argsort(order, kind="stable")).to(dev)
+        stats = stats.index_select(0, inv)
+        ll = None if ll is None else ll.index_select(0, inv)
+    return ll, stats
+
+
+def posterior_predictive_gameweeks(model: str, samples: Dict[str, torch.Tensor], observations: Dict[str, torch.Tensor],
+                                   gameweek, max_goals: int = 15, score_bins: int = 6, points=(3, 1),
+                                   sims_per_draw: int = 1, seed: int = 0, first_draw: int = 0,
+                                   want_scores: bool = False, workspace=None,
+                                   stream=None) -> Dict[str, Optional[torch.Tensor]]:
+    """``posterior_predictive`` for matches spread over gameweeks (``bplx_posterior_predictive_gameweeks``):
+    ``samples`` NEUTRAL-form ``[G', S, T]`` (``corr_coef [G', S]``) on the GPU, ``gameweek`` host ints ``[M]`` in
+    ``[0, G')``; match m of draw s is sampled from gameweek ``gameweek[m]``'s row, with the replicate index, words and
+    statistics of ``posterior_predictive`` (matches in the order given).  Same outputs."""
+    lib = _abi.lib()
+    flat, G, S = _gameweek_major(samples)
+    keep = []
+    s = _samples_struct(model, flat, _device_ptr_fn(keep))
+    o, gw32 = _gw_observations(flat, observations, gameweek, keep)
+    M, T, B = o.fixtures.num_fixtures, s.num_teams, int(score_bins)
+    N = S * int(sims_per_draw)
+    dev = samples["attack"].device
+    workspace = _workspace(workspace, int(lib.bplx_posterior_predictive_gameweeks_workspace_bytes(C.byref(s), G,
+                                                                                                  C.byref(o))), dev)
+    i32, i64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.int64, device=dev)
+    shapes = {"score_counts": ((N, B, B), i32), "outcome_counts": ((N, 3), i32), "goals": ((N, 2), i64),
+              "total_goals_sq": ((N,), i64), "team_points": ((N, T), i32), "team_goals_for": ((N, T), i32),
+              "team_goals_against": ((N, T), i32)}
+    res = {k: torch.empty(shp, **kw) for k, (shp, kw) in shapes.items()}
+    res["invalid"] = torch.empty(1, **i64)
+    res["scores"] = torch.empty((N, M, 2), dtype=torch.uint8, device=dev) if want_scores else None
+    out = _abi.PpcOutput(**{k: _dptr(v) for k, v in res.items()})
+    pw, pd = (int(x) for x in points)
+    _abi.check(lib.bplx_posterior_predictive_gameweeks(C.byref(s), G, C.byref(o), gw32.ctypes.data, int(max_goals), B,
+                                                       pw, pd, int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                                       int(first_draw), C.byref(out), _dptr(workspace),
+                                                       workspace.numel(), _stream_ptr(stream)))
     return res

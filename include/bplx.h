@@ -632,6 +632,85 @@ int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* ob
                               long long first_draw, const bplx_ppc_output* out, void* workspace,
                               size_t workspace_bytes, void* stream);
 
+/* ---- the dynamic model's predictive distribution: fitted and forecast gameweeks ------------------------------ */
+/*
+ * Scope.  Only fits of the intended walk have a predictive distribution (BPLX_FLAG_DYNAMIC_AS_WRITTEN: the likelihood
+ * never reaches the walk, SURVEY D1).  Gameweeks are 0-based and G = max + 1, as in the fit; "gameweek g" is g as the
+ * training data numbers it.
+ *
+ * Fitted gameweek (g < G).  For each draw s, the walk and venue effects the fit records: attack[g], defence[g] and the
+ * four venue effects at g, plus corr_coef.  At one gameweek the dynamic likelihood's rates ARE the NEUTRAL model's
+ * rates (term by term against the P1 / Q1 / P0 tables of the score grid's pre-pass), so one gameweek of the posterior is
+ * a NEUTRAL bplx_samples and every call above consumes it.
+ *
+ * Forecast gameweek (g >= G): the model's own generative process, continued from the last fitted state.  For each draw
+ * s and each gameweek j = G .. g in order, fresh sites from their priors: mean_home_attack, mean_home_defence ~
+ * N(0.1, 0.2); mean_away_attack, mean_away_defence ~ N(-0.1, 0.2); the six std_* ~ HalfNormal(1); per team u ~
+ * Beta(2, 4), rho = 2u - 1, za ~ N(0, 1), zd = rho za + sqrt(1 - rho^2) eps with eps ~ N(0, 1), and the four
+ * *_decentered ~ N(0, 1).  Then attack[j] = attack[j - 1] + za std_attack[j] (defence likewise with zd), and the venue
+ * effects are mean[j] + std[j] decentered[j] (not cumulative).  With HalfNormal(1) venue spreads the forecast is wide.
+ *
+ * Random numbers of the forecast: Philox4_32_10 under the key seed ^ BPLX_FORECAST_KEY (so that they never coincide
+ * with the match-sampling words of the simulation and predictive-check calls under the same seed), subsequence = the
+ * global draw index first_draw + s, counter block b = words 4b .. 4b + 3 (curand_init(key, first_draw + s, 0) followed by
+ * curand()).  Gameweek k = j - G, P = 3 + 3T blocks per gameweek:
+ *   block kP + 0   words (0, 1) -> _curand_box_muller -> (mean_home_attack, mean_away_attack) as 0.1 + 0.2 n, -0.1 + 0.2 n
+ *                  words (2, 3) -> (mean_home_defence, mean_away_defence), the same way
+ *   block kP + 1   words (0, 1) -> |n| -> (std_home_attack, std_away_attack); words (2, 3) -> (std_home_defence,
+ *                  std_away_defence)
+ *   block kP + 2   words (0, 1) -> |n| -> (std_attack, std_defence); words 2, 3 unused
+ *   team t: blocks kP + 3 + 3t + (0, 1, 2) = words w0 .. w11:
+ *                  u = the 2nd smallest of curand_uniform(w0 .. w4); w5 unused; (w6, w7) -> (za, eps);
+ *                  (w8, w9) -> (home_attack_decentered, away_attack_decentered); (w10, w11) -> (home_defence_decentered,
+ *                  away_defence_decentered)
+ * The forecast depends neither on the launch geometry, nor on how the draws are cut into ranges, nor on sims_per_draw.
+ */
+#define BPLX_FORECAST_KEY 0x9E3779B97F4A7C15ull
+#define BPLX_FORECAST_MAX_TEAMS 256
+
+/*
+ * attack_last / defence_last: device [S, T], the walk at gameweek G - 1 of draws first_draw .. first_draw + S - 1.
+ * Outputs (device [horizon, S, T] each, overwritten): the six sites of gameweeks G .. G + horizon - 1 in NEUTRAL
+ * bplx_samples form (corr_coef is the fitted one).  No workspace.  Refusals: NULL pointers, S, T or horizon < 1,
+ * first_draw < 0: BPLX_E_INVALID; T > BPLX_FORECAST_MAX_TEAMS or (3 + 3T) * horizon >= 2^32: BPLX_E_UNSUPPORTED.
+ */
+int bplx_dynamic_forecast(const float* attack_last, const float* defence_last, int num_samples, int num_teams,
+                          int horizon, unsigned long long seed, long long first_draw, float* attack, float* defence,
+                          float* home_attack, float* away_attack, float* home_defence, float* away_defence,
+                          void* stream);
+
+/*
+ * Matches spread over gameweeks.  Samples are GAMEWEEK-MAJOR: s->num_samples = G' * S rows, row g * S + s = draw s at
+ * gameweek g (g < G' = num_gameweeks; the arrays of a NEUTRAL bplx_samples stacked [G', S, T], corr_coef repeated per
+ * gameweek).  gameweek: HOST int32 [M], match m's row block.  Any static model's samples are accepted (the calls do not
+ * know about walks).
+ *
+ * bplx_pointwise_loglik_gameweeks: bplx_pointwise_loglik with match m scored on the draws of its gameweek; loglik
+ * [M, ld] (ld >= S) and stats [M, 4] as there, in the order of the matches given.  The matches must be grouped by
+ * gameweek (gameweek[] non-decreasing): one launch covers every gameweek, each CTA on one gameweek's rows.  The rows of
+ * a gameweek's matches are bit-equal to a bplx_pointwise_loglik call on that gameweek's samples.
+ *
+ * bplx_posterior_predictive_gameweeks: bplx_posterior_predictive with match m sampled from its gameweek's row of draw
+ * s; the same replicate index, word addresses (2m, 2m + 1) and statistics, in the order of the matches given (no
+ * grouping needed).  Each replicate holds its draw's G' rows in shared memory: BPLX_E_UNSUPPORTED when they do not fit.
+ * With G' = 1 the outputs are bit-equal to bplx_posterior_predictive's.
+ *
+ * Refusals (both): what the single-gameweek call refuses; num_gameweeks < 1, num_samples not a multiple of it, a
+ * gameweek outside [0, G'), a NULL gameweek array, or (loglik) matches not grouped by gameweek: BPLX_E_INVALID.
+ */
+size_t bplx_pointwise_loglik_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
+                                                       const bplx_observations* obs);
+int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
+                                    const int32_t* gameweek, float* loglik, size_t ld, double* stats, void* workspace,
+                                    size_t workspace_bytes, void* stream);
+size_t bplx_posterior_predictive_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
+                                                           const bplx_observations* obs);
+int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
+                                        const int32_t* gameweek, int max_goals, int score_bins, int points_win,
+                                        int points_draw, int sims_per_draw, unsigned long long seed,
+                                        long long first_draw, const bplx_ppc_output* out, void* workspace,
+                                        size_t workspace_bytes, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

@@ -88,6 +88,13 @@ class Pairings(C.Structure):
     ]
 
 
+class Conditions(C.Structure):
+    _fields_ = [
+        ("num_key_fixtures", C.c_int32), ("key_fixture", C.c_void_p), ("num_events", C.c_int32),
+        ("event_slot", C.c_void_p), ("event_positions", C.c_void_p),
+    ]
+
+
 class PpcOutput(C.Structure):
     _fields_ = [
         ("score_counts", C.c_void_p), ("outcome_counts", C.c_void_p), ("goals", C.c_void_p),
@@ -98,6 +105,7 @@ class PpcOutput(C.Structure):
 
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
+SIM_MAX_KEY_FIXTURES, SIM_MAX_EVENTS = 64, 64  # BPLX_SIM_MAX_KEY_FIXTURES, BPLX_SIM_MAX_EVENTS
 KO_MAX_TIES, KO_MAX_ROUNDS, KO_MAX_BEST, KO_MAX_ALLOC_GROUPS = 64, 16, 16, 16  # BPLX_KO_MAX_*
 # BPLX_ENTRANT_*
 ENTRANT_SLOT, ENTRANT_GROUP_POS, ENTRANT_BEST, ENTRANT_WINNER, ENTRANT_LOSER, ENTRANT_PAIRED = 0, 1, 2, 3, 4, 5
@@ -187,6 +195,10 @@ def declare(lib):
                                            C.POINTER(Ranking), i, i, C.c_ulonglong, C.c_longlong, vp, vp, vp, vp, vp,
                                            vp, sz, vp]
     lib.bplx_simulate_table_ex.restype = i
+    lib.bplx_simulate_table_conditional.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), vp, vp, C.POINTER(Table),
+                                                    C.POINTER(Ranking), C.POINTER(Conditions), i, i, C.c_ulonglong,
+                                                    C.c_longlong, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.bplx_simulate_table_conditional.restype = i
     lib.bplx_simulate_tournament_ranked_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures),
                                                                     C.POINTER(Table), C.POINTER(Bracket),
                                                                     C.POINTER(Ranking)]

@@ -932,12 +932,70 @@ int bplx_simulate_table_ex(const bplx_samples* s, const bplx_fixtures* f, const 
                            unsigned long long* position_counts, unsigned long long* points_counts, uint8_t* positions,
                            uint8_t* scores, unsigned long long* invalid, void* workspace, size_t workspace_bytes,
                            void* stream) {
+  return bplx_simulate_table_conditional(s, f, home_slot, away_slot, t, r, nullptr, max_goals, sims_per_draw, seed,
+                                         first_draw, position_counts, points_counts, nullptr, nullptr, positions,
+                                         scores, invalid, workspace, workspace_bytes, stream);
+}
+
+// the conditions the conditional kernel relies on; fills sp->cd (tables: slot events, event positions, keys)
+static int check_conditions(const bplx_conditions* c, int NT, int P, int F, unsigned long long* outcome_counts,
+                            unsigned long long* conditional_counts, CondParams* cd) {
+  const char* what = "simulate_table_conditional";
+  const int K = c->num_key_fixtures, E = c->num_events;
+  BPLX_REQUIRE(K >= 1 && K <= BPLX_SIM_MAX_KEY_FIXTURES, BPLX_E_INVALID,
+               "%s: num_key_fixtures must be in [1, %d] (got %d)", what, BPLX_SIM_MAX_KEY_FIXTURES, K);
+  BPLX_REQUIRE(E >= 1 && E <= BPLX_SIM_MAX_EVENTS, BPLX_E_INVALID, "%s: num_events must be in [1, %d] (got %d)", what,
+               BPLX_SIM_MAX_EVENTS, E);
+  BPLX_REQUIRE(c->key_fixture && c->event_slot && c->event_positions, BPLX_E_INVALID,
+               "%s: key_fixture, event_slot and event_positions must not be NULL", what);
+  BPLX_REQUIRE(outcome_counts && conditional_counts, BPLX_E_INVALID,
+               "%s: outcome_counts and conditional_counts must not be NULL", what);
+  int32_t* const keys = reinterpret_cast<int32_t*>(cd->tables + kSimMaxTeams + kCondMaxEvents);
+  for (int j = 0; j < K; j++) {
+    const int32_t k = c->key_fixture[j];
+    BPLX_REQUIRE(k >= 0 && k < F, BPLX_E_INVALID, "%s: key fixture %d: index %d outside the %d fixtures", what, j, k,
+                 F);
+    BPLX_REQUIRE(j == 0 || k > c->key_fixture[j - 1], BPLX_E_INVALID,
+                 "%s: key fixture %d: index %d is not above the previous one (%d): the keys must be strictly increasing",
+                 what, j, k, c->key_fixture[j - 1]);
+    keys[j] = k;
+  }
+  for (int e = 0; e < E; e++) {
+    const int t = c->event_slot[e];
+    const uint64_t m = c->event_positions[e];
+    BPLX_REQUIRE(t < NT, BPLX_E_INVALID, "%s: event %d: slot %d outside the table (%d slots)", what, e, t, NT);
+    BPLX_REQUIRE(m != 0 && (P >= 64 || (m >> P) == 0), BPLX_E_INVALID,
+                 "%s: event %d: position mask 0x%llx is empty or has a bit at %d positions or above", what, e,
+                 (unsigned long long)m, P);
+    cd->tables[t] |= 1ull << e;
+    cd->tables[kSimMaxTeams + e] = m;
+  }
+  cd->nk = K;
+  cd->ne = E;
+  cd->outcome_counts = outcome_counts;
+  cd->cond_counts = conditional_counts;
+  return BPLX_OK;
+}
+
+int bplx_simulate_table_conditional(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_ranking* r,
+                                    const bplx_conditions* c, int max_goals, int sims_per_draw, unsigned long long seed,
+                                    long long first_draw, unsigned long long* position_counts,
+                                    unsigned long long* points_counts, unsigned long long* outcome_counts,
+                                    unsigned long long* conditional_counts, uint8_t* positions, uint8_t* scores,
+                                    unsigned long long* invalid, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
   SimParams sp{};
   int rc = simulate_setup(s, f, home_slot, away_slot, t, max_goals, sims_per_draw, seed, first_draw, position_counts,
                           points_counts, positions, scores, invalid, "simulate", false, &sp);
   if (rc != BPLX_OK) return rc;
   rc = check_ranking(r, t->num_slots, "simulate");
   if (rc != BPLX_OK) return rc;
+  if (c) {
+    rc = check_conditions(c, t->num_slots, t->num_positions, f->num_fixtures, outcome_counts, conditional_counts,
+                          &sp.cd);
+    if (rc != BPLX_OK) return rc;
+  }
   const size_t table = simulate_plan_for(s, f, &sp);
   rc = check_workspace(workspace, workspace_bytes, table + ranking_bytes(r, t->num_slots, f->num_fixtures));
   if (rc != BPLX_OK) return rc;

@@ -55,6 +55,22 @@ struct PairParams {
   uint8_t assoc[kSimMaxTeams];    // slot associations, 0xFF = none
 };
 
+constexpr int kCondMaxKeys = 64;      // BPLX_SIM_MAX_KEY_FIXTURES
+constexpr int kCondMaxEvents = 64;    // BPLX_SIM_MAX_EVENTS
+
+constexpr int kCondTableWords = kSimMaxTeams + kCondMaxEvents + kCondMaxKeys / 2;
+
+// the key fixtures and events of a conditional table simulation (nk = 0: none, the kernels without conditions)
+struct CondParams {
+  int nk, ne;                     // key fixtures, events
+  int tab_off;                    // byte offset in dynamic shared memory of the per-CTA copy of `tables`
+  int buf_off;                    // byte offset of the per-warp partial counts [2][7][kSimThreads] (uint32)
+  unsigned long long *outcome_counts, *cond_counts;  // [nk][3], [nk][3][ne]
+  // the events of each slot [64] (bit e: event e is about the slot), the positions of each event [64] (bit p:
+  // position p is in its set), then the key fixtures as int32 [64], strictly increasing
+  unsigned long long tables[kCondTableWords];
+};
+
 struct SimParams {
   GridParams gp;                  // samples (S = draws of this call), fixtures (F), table layout; gp.table = workspace
   const uint8_t *hslot, *aslot;   // [F] table slots
@@ -74,15 +90,25 @@ struct SimParams {
   int rule;
   const int2* h2h_played;         // [NT][NT] (points, goals) of slot u against slot v in played matches, or NULL
   int *pair_beg, *pair_fix;       // [NT NT + 1], [F] in the workspace (pair_index_kernel)
-  PairParams pr;                  // the paired tournament kernels only (last, so the other kernels' parameters keep
-                                  // their offsets)
+  // last, so the other kernels' parameters keep their offsets.  cd shares pr's bytes: the paired tournament kernels
+  // never read cd and the conditional table kernels never read pr, and a larger parameter block changed the register
+  // allocation of simulate_h2h_kernel<true>.  A table call (ko.K = 0) leaves pr unused.
+  union {
+    PairParams pr;                // the paired tournament kernels only
+    CondParams cd;                // the conditional table kernels only (cd.nk = 0 otherwise)
+  };
 };
+static_assert(sizeof(CondParams) <= sizeof(PairParams), "cd must fit in pr's bytes");
 
 // shared memory per CTA, and whether the points histogram fits in it (sets sp->points_in_smem); with ko.K > 0 that of
-// the tournament kernel (sets sp->ko.wl_overlay), with pr.num > 0 that of the paired kernel (sets sp->pr.buf_off)
+// the tournament kernel (sets sp->ko.wl_overlay), with pr.num > 0 that of the paired kernel (sets sp->pr.buf_off), with
+// cd.nk > 0 that of the conditional kernel (sets sp->cd.tab_off, sp->cd.buf_off)
 size_t simulate_smem_bytes(SimParams* sp);
 // ko.K = 0: the group stage alone; ko.K >= 1: the tournament kernel, the same group stage, then the bracket of sp.ko.
 // rule = BPLX_RANK_HEAD_TO_HEAD: the head-to-head instantiation, after the pair index is built into pair_beg / pair_fix
 int launch_simulate(SimParams& sp, cudaStream_t stream);
+// launch_simulate's last step for a table with conditions (cd.nk >= 1, ko.K = 0): simulate_cond_kernel, which lives in
+// its own translation unit (simulate_cond.cu) so that the instantiations of simulate.cu keep their instructions
+int launch_simulate_cond(const SimParams& sp, unsigned grid, size_t smem, cudaStream_t stream);
 
 }  // namespace bplx

@@ -506,7 +506,8 @@ class _BplxPredictor:
     # ---- season / group-stage simulation -------------------------------------------------------------------------
     def simulate_table(self, fixtures, played=None, teams=None, groups=None, num_sims_per_draw: int = 1,
                        random_state: Optional[int] = None, max_goals: int = MAX_GOALS, points=(3, 1),
-                       return_simulations: bool = False, tiebreak: str = "goal_difference") -> Dict[str, Any]:
+                       return_simulations: bool = False, tiebreak: str = "goal_difference", key_fixtures=None,
+                       events=None) -> Dict[str, Any]:
         """Finishing-position and points probabilities of a league table or of group tables, simulated on the GPU.
 
         Every simulated season takes ONE posterior draw and plays every remaining fixture with that draw's rates, so a
@@ -543,19 +544,52 @@ class _BplxPredictor:
         ``random_state`` is None; pass it back to repeat the run).  With ``return_simulations`` also ``positions [N, T]``
         and ``home_score`` / ``away_score`` ``[F, N]`` (``sample_score``'s shape); the draws are then processed in
         ranges that keep these within ``SIM_OUTPUT_BYTES`` of device memory, and the results do not depend on the range
-        size.  Raises if any simulation met a non-finite rate."""
+        size.  Raises if any simulation met a non-finite rate.
+
+        Match importance (``key_fixtures`` and ``events``, both or neither): which remaining fixtures decide the title,
+        the top four, relegation or who goes through.  ``key_fixtures``: indices into ``fixtures``, in any order and
+        any number; ``events``: a mapping label -> ``(team, positions)``, ``positions`` an int or an iterable of 0-based
+        positions within the team's group (title: 0; top four: range(4); relegation: (17, 18, 19); through from a
+        group: (0, 1)), at most 64 events.  Key fixture j has outcome o in {0 home win, 1 draw, 2 away win} from its
+        simulated score; the GPU counts, in the same simulated seasons, how often each outcome occurred and how often
+        each event held with it.  Adds ``key_fixtures``, ``events`` (the labels), ``outcome_proba [Kc, 3]``,
+        ``event_proba [E]``, ``conditional_proba [Kc, 3, E]`` (P(event | outcome); NaN where the outcome never
+        occurred), ``importance [Kc, E]`` (the largest minus the smallest ``conditional_proba`` over the outcomes that
+        occurred, 0 if fewer than two did) and the integer ``outcome_counts`` / ``conditional_counts``: a conditional
+        probability needs its sample size, and with ``num_sims_per_draw > 1`` the seasons of one draw are correlated,
+        so the effective sample size is smaller than the count.  More than 64 key fixtures run in groups of at most 64
+        with the same seed, so every group sees the same simulated seasons; each group costs one simulation."""
+        if (key_fixtures is None) != (events is None):
+            raise ValueError("key_fixtures and events go together: give both or neither")
         home, away = _str_to_list(fixtures["home_team"], fixtures["away_team"])
         tteams = bseason.table_teams(home, away, played, teams)
         table = bseason.build_table(tteams, played, groups, points, tiebreak)
         hs, as_ = bseason.fixture_slots(table, home, away, known_teams=self.teams)
         fx = {**self._fixture_arrays(home, away, fixtures), "home_slot": hs, "away_slot": as_}
-        return self._simulate(table, fx, None, num_sims_per_draw, random_state, max_goals, return_simulations,
-                              "met a non-finite scoring rate or score-grid normaliser: check the posterior draws")
+        why = "met a non-finite scoring rate or score-grid normaliser: check the posterior draws"
+        if key_fixtures is None:
+            return self._simulate(table, fx, None, num_sims_per_draw, random_state, max_goals, return_simulations, why)
+        cond = bseason.build_conditions(table, len(home), key_fixtures, events)
+        if random_state is None:
+            random_state = int(datetime.now().timestamp() * 100)  # one seed for every group
+        Kc, E = len(cond["key_fixtures"]), len(cond["events"])
+        oc, cc = np.zeros((Kc, 3), np.int64), np.zeros((Kc, 3, E), np.int64)
+        res = None
+        for g in cond["groups"]:
+            part = dict(g, event_slot=cond["event_slot"], event_positions=cond["event_positions"])
+            out = self._simulate(table, fx, None, num_sims_per_draw, random_state, max_goals,
+                                 return_simulations and res is None, why, part)
+            oc[g["rows"]], cc[g["rows"]] = out.pop("outcome_counts"), out.pop("conditional_counts")
+            res = out if res is None else res
+        res.update(bseason.conditional_probabilities(cond, oc, cc, res["num_simulations"]))
+        return res
 
     def _simulate(self, table, fx, bracket, num_sims_per_draw, random_state, max_goals, return_simulations,
-                  invalid_reason) -> Dict[str, Any]:
+                  invalid_reason, conditions=None) -> Dict[str, Any]:
         """``simulate_table`` (``bracket`` None) and ``simulate_tournament`` from the host table, fixture arrays (with
-        their slots; ``{}`` for none) and bracket: the draws in ranges, counts summed over the ranges, probabilities."""
+        their slots; ``{}`` for none) and bracket: the draws in ranges, counts summed over the ranges, probabilities.
+        With ``conditions`` (one group of ``season.build_conditions``) the result also holds the summed
+        ``outcome_counts`` and ``conditional_counts``."""
         seed = int(datetime.now().timestamp() * 100) if random_state is None else int(random_state)
         R = int(num_sims_per_draw)
         if R < 1:
@@ -579,7 +613,8 @@ class _BplxPredictor:
             draws = {k: v[lo:hi] for k, v in ds.items()}
             if bracket is None:
                 out = _simulate_table(self.model, draws, dfx, dtab, max_goals, R, seed, first_draw=lo,
-                                      want_positions=return_simulations, want_scores=return_simulations)
+                                      want_positions=return_simulations, want_scores=return_simulations,
+                                      conditions=conditions)
             else:
                 out = _simulate_tournament(self.model, draws, dfx, dtab, bracket, max_goals, R, seed, first_draw=lo,
                                            want_positions=return_simulations, want_scores=return_simulations,
@@ -603,6 +638,8 @@ class _BplxPredictor:
                                                      cnt["decided_counts"], cnt.get("pairing_counts")))
         res.update({"start_points": table["start_points"].astype(np.int64), "num_simulations": N, "sims_per_draw": R,
                     "seed": seed})
+        if conditions is not None:
+            res.update(outcome_counts=cnt["outcome_counts"], conditional_counts=cnt["conditional_counts"])
         if return_simulations:
             cat = {k: np.concatenate([r[k] for r in raw]) for k in raw[0]}
             sc = cat.pop("scores")
@@ -1159,13 +1196,16 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
 
     def simulate_table(self, fixtures, played=None, teams=None, groups=None, num_sims_per_draw: int = 1,
                        random_state: Optional[int] = None, max_goals: int = MAX_GOALS, points=(3, 1),
-                       return_simulations: bool = False, tiebreak: str = "goal_difference", gameweek=None):
+                       return_simulations: bool = False, tiebreak: str = "goal_difference", gameweek=None,
+                       key_fixtures=None, events=None):
         """NEUTRAL's ``simulate_table`` with every fixture played at one ``gameweek`` (default G - 1; "the next season"
-        is ``gameweek=G`` when the gameweeks are seasons).  ``random_state`` seeds the forecast and the simulation."""
+        is ``gameweek=G`` when the gameweeks are seasons).  ``random_state`` seeds the forecast and the simulation;
+        ``key_fixtures`` / ``events`` give match importance as there."""
         self._require_predictive()
         seed = self._seed(random_state)
         return self.at_gameweek(self._one_gameweek(gameweek), seed).simulate_table(
-            fixtures, played, teams, groups, num_sims_per_draw, seed, max_goals, points, return_simulations, tiebreak)
+            fixtures, played, teams, groups, num_sims_per_draw, seed, max_goals, points, return_simulations, tiebreak,
+            key_fixtures, events)
 
     def simulate_tournament(self, fixtures, bracket, played=None, teams=None, groups=None, best=None, team_conf=None,
                             num_sims_per_draw: int = 1, random_state: Optional[int] = None, max_goals: int = MAX_GOALS,

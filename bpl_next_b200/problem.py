@@ -314,7 +314,8 @@ _TABLE_ARRAYS = ("start_points", "start_goals_for", "start_goals_against")
 
 def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor], table: dict,
                    max_goals: int, sims_per_draw: int, seed: int, first_draw: int = 0, want_positions: bool = False,
-                   want_scores: bool = False, workspace=None, stream=None) -> Dict[str, Optional[torch.Tensor]]:
+                   want_scores: bool = False, workspace=None, stream=None,
+                   conditions: Optional[dict] = None) -> Dict[str, Optional[torch.Tensor]]:
     """Device path of ``bplx_simulate_table``: season / group-stage simulation, one posterior draw per simulated season.
 
     ``samples``: posterior arrays ``[S, T]`` on the GPU (the draws of this call; ``first_draw`` is the global index of
@@ -334,9 +335,17 @@ def simulate_table(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[
     words, only the group order can differ).  Fair-play rules are not modelled: ties left are decided by lot.  Returns
     ``position_counts [T_tab, P]`` and ``points_counts [T_tab, B]`` (points gained; int64), ``invalid`` (int64 ``[1]``:
     simulations with a non-finite rate or normaliser, left out of the counts), and when asked ``positions [N, T_tab]``
-    and ``scores [N, F, 2]`` (uint8; 255 marks an invalid simulation / fixture), N = S R."""
+    and ``scores [N, F, 2]`` (uint8; 255 marks an invalid simulation / fixture), N = S R.
+
+    ``conditions`` (``bplx_simulate_table_conditional``; ``season.build_conditions`` makes it): host arrays
+    ``key_fixture`` (int32 ``[Kc]``, strictly increasing fixture indices, 1 <= Kc <= 64), ``event_slot`` (uint8
+    ``[E]``) and ``event_positions`` (uint64 ``[E]``: bit p = position p within the slot's group, 1 <= E <= 64).  Key
+    fixture j has outcome o in {0 home win, 1 draw, 2 away win} from its sampled score; event e holds iff slot
+    ``event_slot[e]``'s position is a bit of ``event_positions[e]``.  Adds ``outcome_counts`` (int64 ``[Kc, 3]``: valid
+    simulations in which key fixture j ended in o) and ``conditional_counts`` (int64 ``[Kc, 3, E]``: ... and event e
+    held).  No random word is added or moved: every other output is the same bits as without ``conditions``."""
     return _simulate(model, samples, fixtures, table, None, max_goals, sims_per_draw, seed, first_draw, want_positions,
-                     want_scores, False, workspace, stream)
+                     want_scores, False, workspace, stream, conditions)
 
 
 def _table_struct(table: dict, ptr):
@@ -468,8 +477,22 @@ def simulate_tournament(model: str, samples: Dict[str, torch.Tensor], fixtures: 
                      want_positions, want_scores, want_knockout, workspace, stream)
 
 
+def _conditions_struct(conditions: dict, keep: list):
+    """``_abi.Conditions`` over host copies of the arrays of ``conditions`` (kept alive in ``keep``)."""
+    arrays = {k: np.ascontiguousarray(conditions[k], dtype=dt).ravel()
+              for k, dt in (("key_fixture", np.int32), ("event_slot", np.uint8), ("event_positions", np.uint64))}
+    if len(arrays["event_slot"]) != len(arrays["event_positions"]):
+        raise ValueError("event_slot and event_positions differ in length")
+    keep.extend(arrays.values())
+    c = _abi.Conditions()
+    c.num_key_fixtures, c.num_events = len(arrays["key_fixture"]), len(arrays["event_slot"])
+    for k, a in arrays.items():
+        setattr(c, k, a.ctypes.data)
+    return c
+
+
 def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw, seed, first_draw, want_positions,
-              want_scores, want_knockout, workspace, stream):
+              want_scores, want_knockout, workspace, stream, conditions=None):
     """``simulate_tournament``, and ``simulate_table`` when ``bracket`` is None (``bplx_simulate_table``: the group
     stage kernel)."""
     lib = _abi.lib()
@@ -492,6 +515,7 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     b = None if bracket is None else _bracket_struct(bracket, keep)
     r = _ranking_struct(table, T_tab, keep)
     pg = None if b is None else _pairings_struct(bracket, T_tab, keep)
+    cd = None if conditions is None else _conditions_struct(conditions, keep)
     structs = (C.byref(s), C.byref(f), C.byref(t)) + (() if b is None else (C.byref(b),))
     if pg is not None:
         need = int(lib.bplx_simulate_tournament_paired_workspace_bytes(*structs, None if r is None else C.byref(r),
@@ -510,6 +534,9 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     u8 = dict(dtype=torch.uint8, device=dev)
     out = {"position_counts": torch.empty((T_tab, t.num_positions), **i64),
            "points_counts": torch.empty((T_tab, t.num_points_bins), **i64)}
+    if cd is not None:
+        out.update(outcome_counts=torch.empty((cd.num_key_fixtures, 3), **i64),
+                   conditional_counts=torch.empty((cd.num_key_fixtures, 3, cd.num_events), **i64))
     if b is not None:
         out.update(reach_counts=torch.empty((T_tab, b.num_rounds), **i64),
                    win_counts=torch.empty((T_tab, b.num_rounds), **i64),
@@ -529,7 +556,9 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
     slots = (ptr(fixtures["home_slot"]), ptr(fixtures["away_slot"])) if F else (None, None)
     if b is None:
         run, args = lib.bplx_simulate_table, structs[:2] + slots + structs[2:]
-        if r is not None:
+        if cd is not None:
+            run, args = lib.bplx_simulate_table_conditional, args + (None if r is None else C.byref(r), C.byref(cd))
+        elif r is not None:
             run, args = lib.bplx_simulate_table_ex, args + (C.byref(r),)
     else:
         fmt = bracket.get("tie_format")

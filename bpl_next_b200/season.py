@@ -9,6 +9,8 @@ default: goal difference, goals for, then a random tie-break key) or ``"head_to_
 level on points first, reapplied to those still level; then goal difference, goals for and the key).  Fair-play rules
 are not modelled: ties left at the end are decided by lot.  ``build_bracket`` and
 ``bracket_probabilities`` do the same for a knockout bracket played after the group stage (``problem.simulate_tournament``).
+``build_conditions`` and ``conditional_probabilities`` give match importance: finishing probabilities conditioned on the
+outcome of key fixtures (``problem.simulate_table(conditions=...)``).
 """
 from __future__ import annotations
 
@@ -20,7 +22,8 @@ import numpy as np
 from ._abi import (ENTRANT_BEST, ENTRANT_GROUP_POS, ENTRANT_LOSER, ENTRANT_PAIRED, ENTRANT_SLOT, ENTRANT_WINNER,
                    KO_MAX_ALLOC_GROUPS, KO_MAX_BEST, KO_MAX_ROUNDS, KO_MAX_TIES, MAX_PAIRINGS, PAIRING_MAX_POOL,
                    PAIRING_MAX_POT, PAIRING_OPEN, PAIRING_SEEDED, PROTECT_ASSOCIATION, PROTECT_GROUP, RANK_GOAL_DIFF,
-                   RANK_HEAD_TO_HEAD, SIM_MAX_TEAMS, TIE_ONE_MATCH, TIE_ONE_MATCH_ET, TIE_TWO_LEGS)
+                   RANK_HEAD_TO_HEAD, SIM_MAX_EVENTS, SIM_MAX_KEY_FIXTURES, SIM_MAX_TEAMS, TIE_ONE_MATCH, TIE_ONE_MATCH_ET,
+                   TIE_TWO_LEGS)
 
 TIE_FORMATS = {"one_match": TIE_ONE_MATCH, "extra_time": TIE_ONE_MATCH_ET, "two_legs": TIE_TWO_LEGS}
 TIEBREAKS = {"goal_difference": RANK_GOAL_DIFF, "head_to_head": RANK_HEAD_TO_HEAD}
@@ -158,6 +161,80 @@ def probabilities(table: Dict[str, Any], position_counts: np.ndarray, points_cou
     start = np.asarray(table["start_points"], np.int64)
     return {"position_proba": pos, "points_proba": pts,
             "expected_points": start + pts @ np.arange(pts.shape[1], dtype=np.float64)}
+
+
+# ---- match importance: finishing probabilities conditioned on key fixtures' results ----------------------------------
+def build_conditions(table: Dict[str, Any], num_fixtures: int, key_fixtures: Sequence[int],
+                     events: Dict[Any, Tuple[Any, Any]]) -> Dict[str, Any]:
+    """The conditions ``problem.simulate_table`` takes, from fixture indices and events on team names.
+
+    Key fixture j has outcome o in {0 home win, 1 draw, 2 away win}, taken from its sampled score; event e = (team,
+    positions) holds in a simulation iff the team's 0-based position within its group is one of ``positions`` (an int or
+    an iterable).  ``key_fixtures``: distinct indices into the ``num_fixtures`` fixtures, in any order and any number;
+    ``events``: label -> (team, positions), 1 to 64 of them.  Returns ``key_fixtures`` and ``events`` (the labels) in
+    the caller's order, ``event_slot`` (uint8 ``[E]``), ``event_positions`` (uint64 ``[E]``, bit p = position p) and
+    ``groups``: the key fixtures sorted and cut into runs of at most 64, each ``{"key_fixture": int32 [Kc], "rows":
+    int64 [Kc]}`` with ``rows`` the index in ``key_fixtures`` of each key.  Each run is one simulation."""
+    keys = [int(k) for k in key_fixtures]
+    if not keys:
+        raise ValueError("key_fixtures is empty")
+    for k in keys:
+        if not 0 <= k < num_fixtures:
+            raise ValueError(f"key fixture {k} is not one of the {num_fixtures} fixtures")
+    if len(set(keys)) != len(keys):
+        raise ValueError("key_fixtures lists a fixture more than once")
+    events = dict(events)
+    if not 1 <= len(events) <= SIM_MAX_EVENTS:
+        raise ValueError(f"between 1 and {SIM_MAX_EVENTS} events are supported, got {len(events)}")
+    slot = {t: i for i, t in enumerate(table["teams"])}
+    labels, sizes = _group_sizes(table)
+    group = np.zeros(len(slot), np.int64) if table.get("group") is None else np.asarray(table["group"], np.int64)
+    eslot = np.zeros(len(events), np.uint8)
+    emask = np.zeros(len(events), np.uint64)
+    for e, (label, ev) in enumerate(events.items()):
+        try:
+            team, positions = ev
+        except (TypeError, ValueError):
+            raise ValueError(f"event {label!r}: expected (team, positions), got {ev!r}") from None
+        if team not in slot:
+            raise ValueError(f"event {label!r}: team {team!r} is not in the table")
+        size = int(sizes[group[slot[team]]])
+        pos = [positions] if isinstance(positions, (int, np.integer)) else list(positions)
+        if not pos:
+            raise ValueError(f"event {label!r}: no positions")
+        m = 0
+        for p in pos:
+            if not isinstance(p, (int, np.integer)) or isinstance(p, bool) or not 0 <= p < size:
+                raise ValueError(f"event {label!r}: position {p!r} is not a position of a group of {size}")
+            m |= 1 << int(p)
+        eslot[e], emask[e] = slot[team], m
+    order = np.argsort(keys, kind="stable")
+    groups = [{"key_fixture": np.asarray([keys[i] for i in order[lo:lo + SIM_MAX_KEY_FIXTURES]], np.int32),
+               "rows": order[lo:lo + SIM_MAX_KEY_FIXTURES].astype(np.int64)}
+              for lo in range(0, len(keys), SIM_MAX_KEY_FIXTURES)]
+    return {"key_fixtures": keys, "events": list(events), "event_slot": eslot, "event_positions": emask,
+            "groups": groups}
+
+
+def conditional_probabilities(conditions: Dict[str, Any], outcome_counts: np.ndarray, conditional_counts: np.ndarray,
+                              num_simulations: int) -> Dict[str, Any]:
+    """Counts -> ``outcome_proba [Kc, 3]`` (key fixture j ends in a home win / draw / away win), ``event_proba [E]``,
+    ``conditional_proba [Kc, 3, E]`` (P(event e | key fixture j ended in o); NaN where o never occurred) and
+    ``importance [Kc, E]`` (the largest minus the smallest ``conditional_proba`` over the outcomes that occurred; 0 if
+    fewer than two occurred), with ``key_fixtures``, ``events`` and the integer counts.  Rows follow
+    ``conditions["key_fixtures"]``."""
+    oc = np.asarray(outcome_counts, np.int64)
+    cc = np.asarray(conditional_counts, np.int64)
+    n = float(num_simulations)
+    seen = oc > 0
+    with np.errstate(invalid="ignore", divide="ignore"):
+        cond = np.where(seen[:, :, None], cc / oc[:, :, None].astype(np.float64), np.nan)
+    hi = np.where(seen[:, :, None], cond, -np.inf).max(axis=1)
+    lo = np.where(seen[:, :, None], cond, np.inf).min(axis=1)
+    importance = np.where((seen.sum(axis=1) >= 2)[:, None], hi - lo, 0.0)
+    return {"key_fixtures": list(conditions["key_fixtures"]), "events": list(conditions["events"]),
+            "outcome_proba": oc / n, "event_proba": cc[0].sum(axis=0) / n, "conditional_proba": cond,
+            "importance": importance, "outcome_counts": oc, "conditional_counts": cc}
 
 
 # ---- tournament: a knockout bracket after the group stage ---------------------------------------------------------

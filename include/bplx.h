@@ -476,7 +476,8 @@ typedef struct {
 
 size_t bplx_simulate_table_ex_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
                                               const bplx_ranking* r);
-/* bplx_simulate_table with a ranking rule; bplx_simulate_table is this call with r = NULL. */
+/* bplx_simulate_table with a ranking rule; bplx_simulate_table is this call with r = NULL.  It is
+ * bplx_simulate_table_conditional (below) with c = NULL. */
 int bplx_simulate_table_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
                            const uint8_t* away_slot, const bplx_table* t, const bplx_ranking* r, int max_goals,
                            int sims_per_draw, unsigned long long seed, long long first_draw,
@@ -497,6 +498,50 @@ int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* 
                                     uint8_t* positions, uint8_t* scores, uint8_t* ko_entrants, uint8_t* ko_scores,
                                     uint8_t* ko_winners, uint8_t* ko_extra, unsigned long long* invalid,
                                     void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- match importance: finishing probabilities conditioned on key fixtures' results ---------------------------- */
+/*
+ * bplx_simulate_table_ex, plus counts of each simulation's key-fixture outcomes jointly with events on the final table.
+ *
+ * Key fixtures: 1 <= Kc <= BPLX_SIM_MAX_KEY_FIXTURES distinct indices into the call's F fixtures.  In a simulation, key
+ * fixture j has outcome o in {0 home win, 1 draw, 2 away win}, taken from its sampled score (hg > ag, hg = ag, hg < ag).
+ * Events: 1 <= E <= BPLX_SIM_MAX_EVENTS.  Event e is a pair (slot t_e, position set M_e); M_e is a uint64 bit mask over
+ * 0-based positions within t_e's group, so P <= 64 always fits.  Event e holds in a simulation iff t_e's position is in
+ * M_e.  Examples: title = {0}, top four = {0..3}, relegation = {17, 18, 19}, through from a group = {0, 1}.
+ *
+ * Outputs (device; integer counts, additive over draw ranges, the same bits whatever order the atomics run in;
+ * overwritten):
+ *   outcome_counts     [Kc, 3]     valid simulations in which key fixture j ended in outcome o
+ *   conditional_counts [Kc, 3, E]  valid simulations in which key fixture j ended in o and event e held
+ * Invalid simulations are excluded exactly as they are from position_counts.  No random word is added or moved: with
+ * the same seed, position_counts, points_counts, invalid, positions and scores are bit-identical to
+ * bplx_simulate_table_ex under either ranking rule.  For every j and e:
+ *   sum_o conditional_counts[j, o, e] = sum_{p in M_e} position_counts[t_e, p],
+ *   sum_o outcome_counts[j, o] = N - invalid.
+ *
+ * The arrays of bplx_conditions are HOST arrays, validated by the call (BPLX_E_INVALID): Kc or E outside 1..64, a key
+ * index out of range or not strictly increasing, a slot >= T_tab, an empty mask or one with a bit >= P, and NULL count
+ * outputs when c is not NULL.  c = NULL gives bplx_simulate_table_ex (which is this call with c = NULL).  DYNAMIC:
+ * BPLX_E_UNSUPPORTED.  The call needs no more workspace than bplx_simulate_table_ex:
+ * bplx_simulate_table_ex_workspace_bytes serves both.
+ */
+#define BPLX_SIM_MAX_KEY_FIXTURES 64
+#define BPLX_SIM_MAX_EVENTS 64
+typedef struct {
+  int32_t num_key_fixtures;       /* Kc, 1..64 */
+  const int32_t* key_fixture;     /* host [Kc] fixture indices < F, strictly increasing */
+  int32_t num_events;             /* E, 1..64 */
+  const uint8_t* event_slot;      /* host [E] table slot t_e < T_tab */
+  const uint64_t* event_positions; /* host [E] M_e: non-zero, no bit at P or above */
+} bplx_conditions;
+
+int bplx_simulate_table_conditional(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
+                                    const uint8_t* away_slot, const bplx_table* t, const bplx_ranking* r,
+                                    const bplx_conditions* c, int max_goals, int sims_per_draw, unsigned long long seed,
+                                    long long first_draw, unsigned long long* position_counts,
+                                    unsigned long long* points_counts, unsigned long long* outcome_counts,
+                                    unsigned long long* conditional_counts, uint8_t* positions, uint8_t* scores,
+                                    unsigned long long* invalid, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- knockout pairings drawn by lot ------------------------------------------------------------------------- */
 /*

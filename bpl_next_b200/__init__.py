@@ -11,7 +11,7 @@ __version__ = "0.1.0"
 def __getattr__(name):  # lazy: importing torch is slow and not needed for host-only users
     if name in ("Problem", "score_grid", "score_grid_host", "pointwise_loglik", "psis_loo",
                 "simulate_table", "simulate_tournament", "posterior_predictive", "dynamic_forecast",
-                "pointwise_loglik_gameweeks", "posterior_predictive_gameweeks"):
+                "pointwise_loglik_gameweeks", "posterior_predictive_gameweeks", "market_draws", "row_quantiles"):
         from . import problem
         return getattr(problem, name)
     if name in ("DixonColesMatchPredictor", "ExtendedDixonColesMatchPredictor", "NeutralDixonColesMatchPredictor",

@@ -103,6 +103,17 @@ class PpcOutput(C.Structure):
     ]
 
 
+MARKET_MAX_LINES = 16  # BPLX_MARKET_MAX_LINES
+QUANTILE_MAX_LEVELS = 8  # BPLX_QUANTILE_MAX_LEVELS
+
+
+class MarketLines(C.Structure):
+    _fields_ = [
+        ("num_total_lines", C.c_int32), ("num_margin_lines", C.c_int32),
+        ("total_lines", C.c_double * MARKET_MAX_LINES), ("margin_lines", C.c_double * MARKET_MAX_LINES),
+    ]
+
+
 PSIS_MAX_TAIL = 16384  # BPLX_PSIS_MAX_TAIL
 SIM_MAX_TEAMS = 64  # BPLX_SIM_MAX_TEAMS
 SIM_MAX_KEY_FIXTURES, SIM_MAX_EVENTS = 64, 64  # BPLX_SIM_MAX_KEY_FIXTURES, BPLX_SIM_MAX_EVENTS
@@ -235,6 +246,14 @@ def declare(lib):
                                                         i, C.c_ulonglong, C.c_longlong, C.POINTER(PpcOutput), vp, sz,
                                                         vp]
     lib.bplx_posterior_predictive_gameweeks.restype = i
+    lib.bplx_market_draws_workspace_bytes.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), i,
+                                                      C.POINTER(MarketLines)]
+    lib.bplx_market_draws_workspace_bytes.restype = sz
+    lib.bplx_market_draws.argtypes = [C.POINTER(Samples), C.POINTER(Fixtures), i, C.POINTER(MarketLines), vp, sz, vp,
+                                      vp, vp, sz, vp]
+    lib.bplx_market_draws.restype = i
+    lib.bplx_row_quantiles.argtypes = [vp, i, i, sz, vp, i, vp, vp, vp, vp]
+    lib.bplx_row_quantiles.restype = i
     lib.bplx_reload_env.argtypes = []
     lib.bplx_reload_env.restype = None
     lib.bplx_last_error.argtypes = []

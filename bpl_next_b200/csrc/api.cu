@@ -14,6 +14,7 @@
 #include "plan.h"
 #include "problem.h"
 #include "loo.h"
+#include "markets.h"
 #include "ppc.h"
 #include "score_grid.h"
 #include "simulate.h"
@@ -1592,6 +1593,78 @@ int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks
   pp.scores = out->scores;
   pp.invalid = out->invalid;
   return launch_ppc_gameweeks(pp, st);
+}
+
+// ---- forecast uncertainty: per-draw markets and row quantiles ----------------------------------------------------
+static size_t market_plan_for(const bplx_samples* s, const bplx_fixtures* f, int max_goals, MarketParams* mp,
+                              const char** err) {
+  bind_samples(s, f, &mp->gp);
+  mp->gp.g = max_goals + 1;
+  return market_plan(mp, err);
+}
+
+size_t bplx_market_draws_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, int max_goals,
+                                         const bplx_market_lines* lines) {
+  if (!s || !f || !lines || max_goals < 1 || max_goals > 63 || s->num_samples <= 0 || s->num_teams <= 0 ||
+      f->num_fixtures <= 0)
+    return 0;
+  MarketParams mp{};
+  if (market_rows(lines, max_goals, &mp) != BPLX_OK) return 0;
+  return market_plan_for(s, f, max_goals, &mp, nullptr);
+}
+
+int bplx_market_draws(const bplx_samples* s, const bplx_fixtures* f, int max_goals, const bplx_market_lines* lines,
+                      float* draws, size_t ld, double* stats, int* invalid, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  int rc = check_sample_args(s, f, "markets");
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "markets: max_goals must be in [1, 63] (got %d)",
+               max_goals);
+  BPLX_REQUIRE(stats && invalid, BPLX_E_INVALID, "markets: stats and invalid must not be NULL");
+  BPLX_REQUIRE(!draws || ld >= (size_t)s->num_samples, BPLX_E_INVALID, "markets: ld (%zu) < num_samples (%d)", ld,
+               s->num_samples);
+  MarketParams mp{};
+  rc = market_rows(lines, max_goals, &mp);
+  if (rc != BPLX_OK) return rc;
+  const char* perr = nullptr;
+  const size_t need = market_plan_for(s, f, max_goals, &mp, &perr);
+  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "markets: unsupported shape");
+  rc = check_workspace(workspace, workspace_bytes, need);
+  if (rc != BPLX_OK) return rc;
+  mp.gp.table = static_cast<float*>(workspace);
+  mp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + table_layout(&mp.gp));
+  mp.draws = draws;
+  mp.ld = ld;
+  mp.stats = stats;
+  mp.invalid = invalid;
+  return launch_market_draws(mp, static_cast<cudaStream_t>(stream));
+}
+
+int bplx_row_quantiles(const float* rows, int num_rows, int num_samples, size_t ld, const double* levels, int nq,
+                       const double* odds, double* quantiles, long long* exceed, void* stream) {
+  BPLX_REQUIRE(rows != nullptr, BPLX_E_INVALID, "row quantiles: rows is NULL");
+  BPLX_REQUIRE(num_rows > 0 && num_samples > 0, BPLX_E_INVALID,
+               "row quantiles: num_rows and num_samples must be positive (got %d, %d)", num_rows, num_samples);
+  BPLX_REQUIRE(ld >= (size_t)num_samples, BPLX_E_INVALID, "row quantiles: ld (%zu) < num_samples (%d)", ld, num_samples);
+  BPLX_REQUIRE(nq >= 0 && nq <= BPLX_QUANTILE_MAX_LEVELS, BPLX_E_INVALID, "row quantiles: 0 .. %d levels (got %d)",
+               BPLX_QUANTILE_MAX_LEVELS, nq);
+  BPLX_REQUIRE(nq == 0 || (levels && quantiles), BPLX_E_INVALID, "row quantiles: levels and quantiles must not be NULL");
+  BPLX_REQUIRE(!odds || exceed, BPLX_E_INVALID, "row quantiles: odds given without exceed");
+  QuantileParams qp{};
+  for (int l = 0; l < nq; l++) {
+    BPLX_REQUIRE(levels[l] >= 0.0 && levels[l] <= 1.0, BPLX_E_INVALID, "row quantiles: level %g is outside [0, 1]",
+                 levels[l]);
+    qp.level[l] = levels[l];
+  }
+  qp.rows = rows;
+  qp.ld = ld;
+  qp.R = num_rows;
+  qp.S = num_samples;
+  qp.nq = nq;
+  qp.odds = odds;
+  qp.quantiles = quantiles;
+  qp.exceed = odds ? exceed : nullptr;
+  return launch_market_quantiles(qp, static_cast<cudaStream_t>(stream));
 }
 
 void bplx_reload_env(void) {

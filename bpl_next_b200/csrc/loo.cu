@@ -22,6 +22,7 @@
 //              (4) bitonic sort of the tail, generalised-Pareto fit, smoothing and the two log-sum-exps in float64.
 //              The row is read four times; after the first pass it is served from L2 (one row per CTA).
 #include "loo.h"
+#include "radix_select.cuh"
 
 #include <float.h>
 #include <math.h>
@@ -243,17 +244,13 @@ int launch_pointwise_segmented(PointwiseParams& pp, int ngw, cudaStream_t stream
 // ---- PSIS kernel -----------------------------------------------------------------------------------------------------
 namespace {
 
+using radix::f2key;
+using radix::hist_add;
+using radix::key2f;
+using radix::kBins;
 constexpr int kPsisWarps = kPsisThreads / 32;
-constexpr int kBins = 2048;             // radix digits of 11, 11 and 10 bits
 constexpr int kMaxCand = 32 + 30 + 128;  // GPD candidates: 30 + floor(sqrt(n)), n <= kPsisTailMax
 constexpr double kLogTiny = -708.3964185322641;  // log(DBL_MIN), ArviZ's cutoffmin
-
-// order-preserving keys: ascending key <=> ascending float
-__device__ __forceinline__ uint32_t f2key(float v) {
-  const uint32_t u = __float_as_uint(v);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(uint32_t k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
 
 struct PsisShared {
   double red[kPsisWarps + 1];
@@ -283,63 +280,6 @@ __device__ double block_sum(double v, PsisShared& sh) {
   return r;
 }
 
-// the bin of hist[0, nb) that holds the element of 1-based rank sh.rank; sh.rank becomes the rank inside that bin
-__device__ void find_bin(const uint32_t* hist, int nb, PsisShared& sh) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int per = nb / kPsisThreads;
-  uint32_t local = 0;
-  for (int b = 0; b < per; b++) local += hist[tid * per + b];
-  uint32_t incl = local;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += t;
-  }
-  if (lane == 31) sh.wsum[warp] = incl;
-  __syncthreads();
-  uint32_t before = 0;
-  for (int w = 0; w < warp; w++) before += sh.wsum[w];
-  const uint32_t excl = before + incl - local;
-  const uint32_t r = sh.rank;
-  __syncthreads();
-  if (r > excl && r <= excl + local) {
-    uint32_t c = excl;
-    for (int b = 0; b < per; b++) {
-      const uint32_t hb = hist[tid * per + b];
-      if (r <= c + hb) {
-        sh.bin = tid * per + b;
-        sh.rank = r - c;
-        break;
-      }
-      c += hb;
-    }
-  }
-  __syncthreads();
-}
-
-// hist[bin] += 1, one shared-memory atomic per distinct bin of the warp (the log-likelihoods of a match crowd into a
-// few top-bit bins: plain atomics would serialise on them)
-__device__ __forceinline__ void hist_add(uint32_t* hist, uint32_t bin) {
-  const uint32_t peers = __match_any_sync(__activemask(), bin);
-  if ((threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&hist[bin], (uint32_t)__popc(peers));
-}
-
-// fn(value) for every entry of the row; four independent loads in flight per thread
-template <class Fn>
-__device__ __forceinline__ void for_row(const float* __restrict__ row, int S, Fn&& fn) {
-  for (int i0 = threadIdx.x; i0 < S; i0 += 4 * kPsisThreads) {
-    float v[4];
-#pragma unroll
-    for (int u = 0; u < 4; u++) {
-      const int i = i0 + u * kPsisThreads;
-      v[u] = i < S ? __ldg(row + i) : 0.0f;
-    }
-#pragma unroll
-    for (int u = 0; u < 4; u++)
-      if (i0 + u * kPsisThreads < S) fn(v[u]);
-  }
-}
-
 }  // namespace
 
 __global__ void __launch_bounds__(kPsisThreads) psis_kernel(const __grid_constant__ PsisParams pp) {
@@ -359,7 +299,7 @@ __global__ void __launch_bounds__(kPsisThreads) psis_kernel(const __grid_constan
   // (1) min ll (= -max x), non-finite entries, histogram of the top 11 key bits
   float mn = INFINITY;
   int bad = 0;
-  for_row(row, S, [&](float v) {
+  radix::for_row<kPsisThreads>(row, S, [&](float v) {
     bad |= !isfinite(v);
     mn = fminf(mn, v);
     hist_add(hist, f2key(v) >> 21);
@@ -383,25 +323,25 @@ __global__ void __launch_bounds__(kPsisThreads) psis_kernel(const __grid_constan
   if (pp.Mt + 1 <= S) {
     if (tid == 0) sh.rank = (uint32_t)pp.Mt + 1;
     __syncthreads();
-    find_bin(hist, kBins, sh);
+    radix::find_bins<kPsisThreads, 1>(hist, kBins, 1u, &sh.rank, &sh.bin, sh.wsum);
     uint32_t prefix = sh.bin << 21;
     for (int i = tid; i < kBins; i += kPsisThreads) hist[i] = 0;
     __syncthreads();
-    for_row(row, S, [&](float v) {
+    radix::for_row<kPsisThreads>(row, S, [&](float v) {
       const uint32_t k = f2key(v);
       if ((k >> 21) == (prefix >> 21)) hist_add(hist, (k >> 10) & 2047u);
     });
     __syncthreads();
-    find_bin(hist, kBins, sh);
+    radix::find_bins<kPsisThreads, 1>(hist, kBins, 1u, &sh.rank, &sh.bin, sh.wsum);
     prefix |= sh.bin << 10;
     for (int i = tid; i < kBins; i += kPsisThreads) hist[i] = 0;
     __syncthreads();
-    for_row(row, S, [&](float v) {
+    radix::for_row<kPsisThreads>(row, S, [&](float v) {
       const uint32_t k = f2key(v);
       if ((k >> 10) == (prefix >> 10)) hist_add(hist, k & 1023u);
     });
     __syncthreads();
-    find_bin(hist, 1024, sh);
+    radix::find_bins<kPsisThreads, 1>(hist, 1024, 1u, &sh.rank, &sh.bin, sh.wsum);
     prefix |= sh.bin;
     x_cut = fmax(-(double)key2f(prefix) - xmax, kLogTiny);
   }
@@ -410,7 +350,7 @@ __global__ void __launch_bounds__(kPsisThreads) psis_kernel(const __grid_constan
   // (3) body sums (x <= x_cut) and the tail gather.  For the body, lw + ll = x + ll is -xmax up to rounding: the sum of
   // exp(x + ll + xmax) takes 1 + d + d^2/2 for the tiny d instead of a float64 exp
   double b1 = 0.0, b2 = 0.0;
-  for_row(row, S, [&](float v) {
+  radix::for_row<kPsisThreads>(row, S, [&](float v) {
     const double x = -(double)v - xmax;
     if (x > x_cut) {
       const uint32_t pos = atomicAdd(&sh.cnt, 1u);

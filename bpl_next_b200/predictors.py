@@ -33,6 +33,78 @@ LOO_MATRIX_BYTES = 4 << 30
 # device memory for the raw outputs of simulate_table / simulate_tournament(return_simulations=True) (positions, scores,
 # knockout entrants, scores and winners): larger runs are processed in ranges of posterior draws
 SIM_OUTPUT_BYTES = 1 << 30
+# device memory for the [fixtures x markets, draws] matrix of predict_proba_posterior(): larger fixture sets are
+# processed in ranges
+MARKET_MATRIX_BYTES = 4 << 30
+_RATE_ROWS = ("home_rate", "away_rate")
+
+
+def _half_lines(lines, lo: float, hi: float, what: str) -> list:
+    """Validated half-integer lines in [lo, hi] (no pushes), at most ``_abi.MARKET_MAX_LINES``, no repeats."""
+    from . import _abi
+
+    out = []
+    for x in lines:
+        v = float(x) if np.isscalar(x) and not isinstance(x, (bool, np.bool_, str)) else np.nan
+        if not np.isfinite(v) or (2.0 * v) % 2.0 != 1.0:
+            raise ValueError(f"{what} line {x!r} is not a half-integer (integer and quarter lines are not supported)")
+        if not lo <= v <= hi:
+            raise ValueError(f"{what} line {v:g} is outside [{lo:g}, {hi:g}] for this max_goals")
+        if v in out:
+            raise ValueError(f"{what} line {v:g} is given twice")
+        out.append(v)
+    if len(out) > _abi.MARKET_MAX_LINES:
+        raise ValueError(f"at most {_abi.MARKET_MAX_LINES} {what} lines (got {len(out)})")
+    return out
+
+
+def _market_args(total_lines, margin_lines, quantiles, odds, max_goals: int, F: int):
+    """Validated lines, levels and odds of ``predict_proba_posterior`` -> (total lines, margin lines, levels, row
+    names, odds [F, K] float64 with 0 where a row has none, the names of the rows with odds)."""
+    from . import _abi
+    from .problem import market_names
+
+    G = int(max_goals)
+    if not 1 <= G <= 63:
+        raise ValueError(f"max_goals must be in [1, 63] (got {max_goals})")
+    tl = _half_lines(total_lines, 0.5, 2 * G - 0.5, "total")
+    ml = _half_lines(margin_lines, -G + 0.5, G - 0.5, "margin")
+    lv = np.asarray(quantiles, dtype=np.float64).ravel()
+    if len(lv) > _abi.QUANTILE_MAX_LEVELS:
+        raise ValueError(f"at most {_abi.QUANTILE_MAX_LEVELS} quantile levels (got {len(lv)})")
+    if not (np.isfinite(lv) & (lv >= 0.0) & (lv <= 1.0)).all():
+        raise ValueError(f"quantile levels must lie in [0, 1] (got {list(lv)})")
+    names = market_names(tl, ml)
+    om = np.zeros((F, len(names)), np.float64)
+    priced = []
+    for name, o in (odds or {}).items():
+        if name in _RATE_ROWS:
+            raise ValueError(f"{name} is an expected number of goals: it takes no odds")
+        if name not in names:
+            raise ValueError(f"odds for {name!r}, which is not a row of this call (rows: {names})")
+        o = np.asarray(o, dtype=np.float64)
+        if o.ndim > 1 or (o.ndim == 1 and len(o) != F):
+            raise ValueError(f"odds for {name} must be a scalar or one value per fixture ({F})")
+        if not (np.isfinite(o) & (o > 1.0)).all():
+            raise ValueError(f"odds for {name} must be finite decimal odds > 1")
+        om[:, names.index(name)] = o
+        priced.append(name)
+    return tl, ml, lv, names, om, priced
+
+
+def _market_result(names, priced, lv, om, S: int, max_goals: int, stats, quant, exceed, draws) -> Dict[str, Any]:
+    """The dict ``predict_proba_posterior`` returns, from the per-fixture arrays of ``_market_posterior``."""
+    res: Dict[str, Any] = {}
+    for k, name in enumerate(names):
+        row = {"mean": stats[:, k, 0], "sd": stats[:, k, 1], "quantiles": quant[:, k, :]}
+        if name in priced:
+            row["edge_proba"] = exceed[:, k] / S
+            row["expected_value"] = stats[:, k, 0] * om[:, k] - 1.0
+        res[name] = row
+    res.update(markets=list(names), quantile_levels=np.asarray(lv, np.float64), num_draws=S, max_goals=int(max_goals))
+    if draws is not None:
+        res["draws"] = draws
+    return res
 
 
 def _str_to_list(*args):
@@ -294,6 +366,81 @@ class _BplxPredictor:
 
     def _extras_from_args(self, args, kw):
         return kw
+
+    # ---- forecast uncertainty: the posterior distribution of market probabilities --------------------------------
+    @staticmethod
+    def _market_posterior(model, samples, fx, max_goals, tl, ml, lv, om, return_draws):
+        """Per-draw markets of the fixtures ``fx`` (host index arrays) under the host posterior arrays ``samples``, in
+        ranges of fixtures within ``MARKET_MATRIX_BYTES``: (stats [F, K, 2], quantiles [F, K, Q], exceed [F, K] int64,
+        draws [F, K, S] or None).  Raises when a draw had a non-finite rate."""
+        from .problem import market_draws, row_quantiles
+
+        ds = {k: torch.from_numpy(np.ascontiguousarray(v, dtype=np.float32)).cuda() for k, v in samples.items()
+              if v is not None}
+        dfx = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in fx.items()}
+        F, K, S, Q = len(fx["home_team"]), om.shape[1], int(ds["attack"].shape[0]), len(lv)
+        per = max(1, min(F, MARKET_MATRIX_BYTES // (4 * S * K)))
+        buf = torch.empty((per * K, S), dtype=torch.float32, device="cuda")
+        dodds = torch.from_numpy(np.ascontiguousarray(om.reshape(-1))).cuda()
+        stats, quant = np.empty((F, K, 2)), np.empty((F, K, Q))
+        exceed = np.zeros((F, K), np.int64)
+        draws = np.empty((F, K, S), np.float32) if return_draws else None
+        invalid, ws = 0, None
+        for lo in range(0, F, per):
+            hi = min(F, lo + per)
+            mat, st, inv = market_draws(model, ds, {k: v[lo:hi] for k, v in dfx.items()}, max_goals, tl, ml, draws=buf,
+                                        workspace=ws)
+            q, e = row_quantiles(mat, lv, dodds[lo * K:hi * K])
+            invalid += int(inv.item())
+            stats[lo:hi] = st.cpu().numpy().reshape(hi - lo, K, 2)
+            quant[lo:hi] = q.cpu().numpy().reshape(hi - lo, K, Q)
+            exceed[lo:hi] = e.cpu().numpy().reshape(hi - lo, K)
+            if return_draws:
+                draws[lo:hi] = mat.cpu().numpy().reshape(hi - lo, K, S)
+        if invalid:
+            raise ValueError(f"{invalid} of {S * F} (draw, fixture) pairs have a non-finite scoring rate: check the "
+                             "posterior draws")
+        return stats, quant, exceed, draws
+
+    def _predict_proba_posterior(self, home_team, away_team, total_lines, margin_lines, quantiles, odds, max_goals,
+                                 return_draws, **kw):
+        fx = self._fixture_arrays(home_team, away_team, kw)
+        tl, ml, lv, names, om, priced = _market_args(total_lines, margin_lines, quantiles, odds, max_goals,
+                                                     len(fx["home_team"]))
+        samples = self._samples()
+        stats, quant, exceed, draws = self._market_posterior(self.model, samples, fx, max_goals, tl, ml, lv, om,
+                                                             return_draws)
+        return _market_result(names, priced, lv, om, int(np.shape(samples["attack"])[0]), max_goals, stats, quant,
+                              exceed, draws)
+
+    def predict_proba_posterior(self, home_team, away_team, total_lines=(1.5, 2.5, 3.5), margin_lines=(-1.5, 1.5),
+                                quantiles=(0.05, 0.5, 0.95), odds=None, max_goals: int = MAX_GOALS,
+                                return_draws: bool = False) -> Dict[str, Any]:
+        """Forecast uncertainty: the posterior distribution, over the S draws, of a fixture's market probabilities.
+
+        For draw s the grid is ``P_s(i, j) = tau(i, j) Pois(i; lh_s) Pois(j; la_s)`` for ``0 <= i, j <= max_goals``,
+        with the rates of ``predict_*`` (neutral venues and confederations included, no clip), ``c = corr_coef_s`` and
+        tau clamped at 0 on the four low cells ((0,0) ``1 - c lh la``, (0,1) ``1 + c lh``, (1,0) ``1 + c la``, (1,1)
+        ``1 - c``).  The grid is NOT normalised: these are the cells ``predict_score_grid_proba`` averages, so each
+        row's ``mean`` is what the averaged grid gives (``predict_outcome_proba`` for the outcome rows).  Rows per
+        fixture, in this order (``markets``): ``home_win``, ``draw``, ``away_win`` (i > j, i = j, i < j);
+        ``both_teams_score`` (i >= 1 and j >= 1); ``home_rate``, ``away_rate`` (the rates themselves: expected goals,
+        not truncated); per total line L ``total_over_L`` (i + j > L) and ``total_under_L`` (i + j < L); per margin
+        line h ``home_margin_over_h`` (i - j > h) and ``home_margin_under_h`` (i - j < h).  Lines are half-integers
+        (no pushes): total lines in [0.5, 2 max_goals - 0.5], margin lines in [-max_goals + 0.5, max_goals - 0.5], at
+        most 16 of each.  Over and under do not sum to 1 in a draw: the mass beyond ``max_goals`` is dropped, as
+        ``predict_score_grid_proba`` drops it.
+
+        Per row: ``mean`` and ``sd`` (divisor S) from float64 sums, ``quantiles [F, Q]`` at ``quantiles`` (numpy's
+        ``method="linear"`` on the row's S float32 values, exact order statistics).  ``odds`` maps a row name to
+        decimal odds (a scalar or one per fixture; finite, > 1; not the rate rows): the row then also has
+        ``edge_proba``, the share of draws with ``p_s * odds > 1`` (in how much of the posterior the bet is worth
+        taking), and ``expected_value = mean * odds - 1``.  Also returned: ``markets``, ``quantile_levels``,
+        ``num_draws``, ``max_goals``, and with ``return_draws`` the per-draw values ``draws [F, K, S]``.  The fixtures
+        run in ranges within ``MARKET_MATRIX_BYTES`` of device memory; the results do not depend on the range size.
+        Raises if a draw has a non-finite rate."""
+        return self._predict_proba_posterior(home_team, away_team, total_lines, margin_lines, quantiles, odds,
+                                             max_goals, return_draws)
 
     # ---- model comparison: pointwise log-likelihood, WAIC, PSIS-LOO, held-out log score ------------------------
     # ll[s, m] = log Pois(yh; lh) + log Pois(ya; la) + log tau(yh, ya; lh, la, corr_coef_s), with the rates of the predict
@@ -894,6 +1041,13 @@ class NeutralDixonColesMatchPredictor(_BplxPredictor):
     def predict_score_n_proba(self, n, team, opponent, home: bool = True, neutral_venue: int = 0, max_goals: int = MAX_GOALS):
         return self._n_proba(n, team, opponent, home, max_goals, True, neutral_venue=neutral_venue)
 
+    def predict_proba_posterior(self, home_team, away_team, neutral_venue, total_lines=(1.5, 2.5, 3.5),
+                                margin_lines=(-1.5, 1.5), quantiles=(0.05, 0.5, 0.95), odds=None,
+                                max_goals: int = MAX_GOALS, return_draws: bool = False) -> Dict[str, Any]:
+        """The base class's ``predict_proba_posterior`` with ``neutral_venue`` as in ``predict_outcome_proba``."""
+        return self._predict_proba_posterior(home_team, away_team, total_lines, margin_lines, quantiles, odds,
+                                             max_goals, return_draws, neutral_venue=neutral_venue)
+
     def sample_score(self, home_team, away_team, neutral_venue, num_samples: int = 1, random_state: Optional[int] = None,
                      max_goals: int = MAX_GOALS):
         return self._sample_score(home_team, away_team, num_samples, random_state, max_goals, neutral_venue=neutral_venue)
@@ -953,6 +1107,14 @@ class NeutralDixonColesMatchPredictorWC(NeutralDixonColesMatchPredictor):
                               max_goals: int = MAX_GOALS):
         return _BplxPredictor.predict_outcome_proba(self, home_team, away_team, max_goals=max_goals, knockout=knockout,
                                                     home_conf=home_conf, away_conf=away_conf, neutral_venue=neutral_venue)
+
+    def predict_proba_posterior(self, home_team, away_team, home_conf, away_conf, neutral_venue,
+                                total_lines=(1.5, 2.5, 3.5), margin_lines=(-1.5, 1.5), quantiles=(0.05, 0.5, 0.95),
+                                odds=None, max_goals: int = MAX_GOALS, return_draws: bool = False) -> Dict[str, Any]:
+        """The base class's ``predict_proba_posterior`` with the fixture arguments of ``predict_outcome_proba``."""
+        return self._predict_proba_posterior(home_team, away_team, total_lines, margin_lines, quantiles, odds,
+                                             max_goals, return_draws, home_conf=home_conf, away_conf=away_conf,
+                                             neutral_venue=neutral_venue)
 
     def sample_score(self, home_team, away_team, home_conf, away_conf, neutral_venue, num_samples: int = 1,
                      random_state: Optional[int] = None, max_goals: int = MAX_GOALS):
@@ -1165,6 +1327,30 @@ class DynamicNeutralDixonColesMatchPredictor(_BplxPredictor):
         return _BplxPredictor.predict_score_proba(self, home_team, away_team, home_goals, away_goals,
                                                   neutral_venue=neutral_venue, gameweek=gameweek,
                                                   forecast_seed=random_state)
+
+    def predict_proba_posterior(self, home_team, away_team, neutral_venue, total_lines=(1.5, 2.5, 3.5),
+                                margin_lines=(-1.5, 1.5), quantiles=(0.05, 0.5, 0.95), odds=None,
+                                max_goals: int = MAX_GOALS, return_draws: bool = False, gameweek=None,
+                                random_state: int = 0) -> Dict[str, Any]:
+        """NEUTRAL's ``predict_proba_posterior`` at ``gameweek`` (scalar or per fixture; default G - 1), forecast
+        gameweeks under ``random_state``: the fixtures are grouped by gameweek, each group on that gameweek's draws, so
+        every fixture's result is the bits of ``at_gameweek(g, random_state).predict_proba_posterior(...)``."""
+        self._require_predictive()
+        fx = self._fixture_arrays(home_team, away_team, {"neutral_venue": neutral_venue})
+        F = len(fx["home_team"])
+        gw = self._fixture_gameweeks(gameweek, F)
+        tl, ml, lv, names, om, priced = _market_args(total_lines, margin_lines, quantiles, odds, max_goals, F)
+        S, K = len(self.corr_coef), len(names)
+        stats, quant, exceed = np.empty((F, K, 2)), np.empty((F, K, len(lv))), np.zeros((F, K), np.int64)
+        draws = np.empty((F, K, S), np.float32) if return_draws else None
+        for gv, smp in self._slabs(np.unique(gw), int(random_state)).items():
+            idx = np.flatnonzero(gw == gv)
+            part = self._market_posterior("neutral", smp, {k: v[idx] for k, v in fx.items()}, max_goals, tl, ml, lv,
+                                          om[idx], return_draws)
+            stats[idx], quant[idx], exceed[idx] = part[:3]
+            if return_draws:
+                draws[idx] = part[3]
+        return _market_result(names, priced, lv, om, S, max_goals, stats, quant, exceed, draws)
 
     def predict_score_n_proba(self, n, team, opponent, home: bool = True, neutral_venue: int = 0,
                               max_goals: int = MAX_GOALS, gameweek=None, random_state: int = 0):

@@ -1,6 +1,7 @@
 """Python handles over the C ABI: ``Problem`` (log-density + gradient), ``score_grid``, ``pointwise_loglik``,
-``psis_loo``, ``simulate_table``, ``simulate_tournament`` and ``posterior_predictive``; for the dynamic model's
-gameweeks ``dynamic_forecast``, ``pointwise_loglik_gameweeks`` and ``posterior_predictive_gameweeks``.
+``psis_loo``, ``simulate_table``, ``simulate_tournament``, ``posterior_predictive``, ``market_draws`` and
+``row_quantiles``; for the dynamic model's gameweeks ``dynamic_forecast``, ``pointwise_loglik_gameweeks`` and
+``posterior_predictive_gameweeks``.
 
 torch is used only for device memory and streams; every number comes from ``libbplx.so``.
 """
@@ -307,6 +308,85 @@ def psis_loo(loglik: torch.Tensor, r_eff: float = 1.0, stream=None):
     _abi.check(lib.bplx_psis_loo(_dptr(loglik), M, S, ld, C.c_double(r_eff), _dptr(elpd), _dptr(khat), None, 0,
                                  _stream_ptr(stream)))
     return elpd, khat
+
+
+def market_names(total_lines=(), margin_lines=()):
+    """Names of the rows ``market_draws`` computes per fixture, in its order."""
+    names = ["home_win", "draw", "away_win", "both_teams_score", "home_rate", "away_rate"]
+    for x in total_lines:
+        names += [f"total_over_{float(x):g}", f"total_under_{float(x):g}"]
+    for x in margin_lines:
+        names += [f"home_margin_over_{float(x):g}", f"home_margin_under_{float(x):g}"]
+    return names
+
+
+def _market_lines(total_lines, margin_lines):
+    ln = _abi.MarketLines()
+    ln.num_total_lines, ln.num_margin_lines = len(total_lines), len(margin_lines)
+    if max(ln.num_total_lines, ln.num_margin_lines) > _abi.MARKET_MAX_LINES:
+        raise ValueError(f"at most {_abi.MARKET_MAX_LINES} lines of each kind")
+    for i, x in enumerate(total_lines):
+        ln.total_lines[i] = float(x)
+    for i, x in enumerate(margin_lines):
+        ln.margin_lines[i] = float(x)
+    return ln
+
+
+def market_draws(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor], max_goals: int,
+                 total_lines=(), margin_lines=(), want_matrix: bool = True, draws: Optional[torch.Tensor] = None,
+                 workspace=None, stream=None):
+    """Device path of ``bplx_market_draws``: per posterior draw and fixture, the K rows of ``market_names(total_lines,
+    margin_lines)`` read off the draw's own (unnormalised) score grid up to ``max_goals`` (include/bplx.h gives the
+    definitions).  ``samples`` / ``fixtures`` as for ``score_grid``.  Returns ``(draws, stats, invalid)``: ``draws`` the
+    row-major ``[F K, S]`` float32 matrix (row ``f K + r``; a view of the ``[F K, ld]`` buffer when one is passed in) or
+    None when ``want_matrix`` is false, ``stats [F K, 2]`` float64 (mean and sd over the draws, the same bits with or
+    without the matrix and whichever fixtures share the call), ``invalid`` (int32 ``[1]``: (draw, fixture) pairs with a
+    non-finite rate)."""
+    lib = _abi.lib()
+    keep = []
+    ptr = _device_ptr_fn(keep)
+    _check_inputs(samples, fixtures)
+    s = _samples_struct(model, samples, ptr)
+    f = _fixtures_struct(fixtures, ptr)
+    ln = _market_lines(total_lines, margin_lines)
+    F, S, K = f.num_fixtures, s.num_samples, 6 + 2 * len(total_lines) + 2 * len(margin_lines)
+    dev = samples["attack"].device
+    need = int(lib.bplx_market_draws_workspace_bytes(C.byref(s), C.byref(f), int(max_goals), C.byref(ln)))
+    workspace = _workspace(workspace, need, dev)
+    ld = 0
+    if want_matrix:
+        if draws is None:
+            draws = torch.empty((F * K, S), dtype=torch.float32, device=dev)
+        assert draws.dtype == torch.float32 and draws.shape[0] >= F * K and draws.stride(1) == 1
+        ld = int(draws.stride(0)) if F * K > 1 else max(S, int(draws.shape[1]))
+    stats = torch.empty((F * K, 2), dtype=torch.float64, device=dev)
+    invalid = torch.empty(1, dtype=torch.int32, device=dev)
+    _abi.check(lib.bplx_market_draws(C.byref(s), C.byref(f), int(max_goals), C.byref(ln),
+                                     _dptr(draws) if want_matrix else None, ld, _dptr(stats), _dptr(invalid),
+                                     _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    return (draws[:F * K, :S] if want_matrix else None), stats, invalid
+
+
+def row_quantiles(rows: torch.Tensor, levels=(), odds: Optional[torch.Tensor] = None, stream=None):
+    """Device path of ``bplx_row_quantiles`` over the ``[R, S]`` float32 matrix ``rows`` (unit inner stride; the row
+    pitch is passed as the leading dimension): ``quantiles [R, len(levels)]`` float64, numpy's ``method="linear"`` on
+    each row's values with exact order statistics, and with ``odds`` (float64 ``[R]`` on the device; <= 0 = none)
+    ``exceed [R]`` int64, the number of values v with ``v * odds > 1`` in float64 (else None)."""
+    assert rows.is_cuda and rows.dtype == torch.float32 and rows.dim() == 2
+    assert rows.stride(1) == 1 or rows.shape[1] == 1
+    lib = _abi.lib()
+    R, S = int(rows.shape[0]), int(rows.shape[1])
+    ld = int(rows.stride(0)) if R > 1 else S
+    lv = np.ascontiguousarray(levels, dtype=np.float64).ravel()
+    quantiles = torch.empty((R, len(lv)), dtype=torch.float64, device=rows.device)
+    exceed = None
+    if odds is not None:
+        assert odds.is_cuda and odds.dtype == torch.float64 and odds.is_contiguous() and odds.numel() == R
+        exceed = torch.empty(R, dtype=torch.int64, device=rows.device)
+    _abi.check(lib.bplx_row_quantiles(_dptr(rows), R, S, ld, lv.ctypes.data if len(lv) else None, len(lv),
+                                      _dptr(odds), _dptr(quantiles) if len(lv) else None, _dptr(exceed),
+                                      _stream_ptr(stream)))
+    return quantiles, exceed
 
 
 _TABLE_ARRAYS = ("start_points", "start_goals_for", "start_goals_against")

@@ -756,6 +756,64 @@ int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks
                                         long long first_draw, const bplx_ppc_output* out, void* workspace,
                                         size_t workspace_bytes, void* stream);
 
+/* ---- forecast uncertainty: per-draw market probabilities and their posterior quantiles ----------------------- */
+/*
+ * Definitions (the same in oracle/markets.py and the predictor docstring).  For posterior draw s and fixture f the rates
+ * lambda_h, lambda_a are the predict path's (bplx_score_grid: neutral venues and confederations included, no clip),
+ * c = corr_coef[s], G = max_goals, and the draw's grid is
+ *     P_s(i, j) = tau(i, j) e^-lambda_h lambda_h^i / i! e^-lambda_a lambda_a^j / j!,   0 <= i, j <= G,
+ * with tau clamped at 0 on the four low cells: (0,0) 1 - c lambda_h lambda_a, (0,1) 1 + c lambda_h, (1,0) 1 + c lambda_a,
+ * (1,1) 1 - c (as in the score sampler of bplx_simulate_table).  The grid is NOT normalised: these are the cells
+ * bplx_score_grid averages, so the mean over the draws of each row below is what the averaged grid gives.
+ *
+ * The K = 6 + 2 num_total_lines + 2 num_margin_lines rows of one fixture, in this order:
+ *   home_win, draw, away_win        sums over i > j, i = j, i < j
+ *   both_teams_score                sum over i >= 1 and j >= 1
+ *   home_rate, away_rate            lambda_h and lambda_a themselves (expected goals, not truncated at G)
+ *   per total line L                total_over_L (i + j > L), total_under_L (i + j < L)
+ *   per margin line h               home_margin_over_h (i - j > h), home_margin_under_h (i - j < h)
+ * Lines are half-integers (no cell sits on a line: no pushes): total lines in [0.5, 2G - 0.5], margin lines in
+ * [-G + 0.5, G - 0.5], at most BPLX_MARKET_MAX_LINES of each kind.  Over and under of a line do not sum to 1 in a draw:
+ * the mass beyond max_goals is dropped, as the averaged grid drops it.
+ */
+#define BPLX_MARKET_MAX_LINES 16
+#define BPLX_QUANTILE_MAX_LEVELS 8
+typedef struct {
+  int32_t num_total_lines;                      /* 0 .. BPLX_MARKET_MAX_LINES */
+  int32_t num_margin_lines;                     /* 0 .. BPLX_MARKET_MAX_LINES */
+  double total_lines[BPLX_MARKET_MAX_LINES];    /* the first num_total_lines are used */
+  double margin_lines[BPLX_MARKET_MAX_LINES];   /* the first num_margin_lines are used */
+} bplx_market_lines;
+
+size_t bplx_market_draws_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, int max_goals,
+                                         const bplx_market_lines* lines);
+/*
+ * draws[(f K + r) ld + s] (float32, device, row-major [F K, ld], ld >= S; may be NULL: statistics only) = row r of
+ * fixture f in draw s.  stats[(f K + r) 2 + 0, 1] (float64, device) = the mean and the standard deviation (divisor S)
+ * of the row over the draws, from float64 sums of the float32 values.  The draws are cut into splits planned from S
+ * alone and combined in a fixed order: a row's statistics are the same bits whichever fixtures share the call, and
+ * whether draws is NULL or not.  invalid (device int [1], overwritten) counts the (draw, fixture) pairs with a
+ * non-finite rate; their probability rows are NaN.  Asynchronous, no allocation.  Refusals: DYNAMIC (pass one
+ * gameweek's NEUTRAL samples): BPLX_E_UNSUPPORTED; max_goals outside 1..63, a line that is not a half-integer in its
+ * range, more than BPLX_MARKET_MAX_LINES lines of a kind, NULL stats or invalid, ld < S: BPLX_E_INVALID.
+ */
+int bplx_market_draws(const bplx_samples* s, const bplx_fixtures* f, int max_goals, const bplx_market_lines* lines,
+                      float* draws, size_t ld, double* stats, int* invalid, void* workspace, size_t workspace_bytes,
+                      void* stream);
+
+/*
+ * Per row of a row-major float32 matrix rows [num_rows, ld] (device, S values per row, ld >= S):
+ *   quantiles[r nq + l] (float64, device) = numpy.quantile(row as float64, levels[l], method="linear"): with the
+ *     sorted values x_(0) <= ... <= x_(S-1), h = (S - 1) levels[l] and k = floor(h), x_(k) + (h - k)(x_(k+1) - x_(k))
+ *     (numpy's two-sided form of the interpolation; x_(S-1) when k = S - 1).  Order statistics are exact (radix select).
+ *   exceed[r] (device) = the number of values v of the row with (double)v * odds[r] > 1; rows with odds[r] <= 0 get 0.
+ * levels: HOST array of nq values in [0, 1], 0 <= nq <= BPLX_QUANTILE_MAX_LEVELS (quantiles may be NULL when nq = 0).
+ * odds: device [num_rows] or NULL (exceed may then be NULL).  Rows of any length; the row is read three times whatever
+ * nq.  Rows with NaN entries give unspecified quantiles.  Asynchronous, no allocation.  Refusals: BPLX_E_INVALID.
+ */
+int bplx_row_quantiles(const float* rows, int num_rows, int num_samples, size_t ld, const double* levels, int nq,
+                       const double* odds, double* quantiles, long long* exceed, void* stream);
+
 /* ---- misc --------------------------------------------------------------------------------- */
 /* ---- predict over sample shards: the sum of the partial grids over the ranks, over peer memory ------------- */
 /*

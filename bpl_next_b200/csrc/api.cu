@@ -579,11 +579,56 @@ static int check_sample_args(const bplx_samples* s, const bplx_fixtures* f, cons
   return BPLX_OK;
 }
 
-static int check_grid_args(const bplx_samples* s, const bplx_fixtures* f, int max_goals) {
-  const int rc = check_sample_args(s, f, "score grid");
-  if (rc != BPLX_OK) return rc;
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "max_goals must be in [1, 63] (got %d)", max_goals);
+// the argument groups the posterior-draw consumers share (`what` prefixes the message)
+static int check_max_goals(int max_goals, const char* what) {
+  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
+               max_goals);
   return BPLX_OK;
+}
+
+static int check_points(int points_win, int points_draw, const char* what) {
+  BPLX_REQUIRE(points_win >= 1 && points_draw >= 0 && points_draw <= points_win, BPLX_E_INVALID,
+               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
+               points_win, points_draw);
+  return BPLX_OK;
+}
+
+// draws first_draw .. + S - 1, sims_per_draw each: simulation indices fit 63 bits, fewer than 2^31 of them per call
+static int check_draw_range(int S, int sims_per_draw, long long first_draw, bool per_gameweek, const char* what) {
+  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
+  BPLX_REQUIRE(first_draw >= 0 && first_draw + S <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
+               "%s: first_draw must be >= 0 and (first_draw + %s) * sims_per_draw must fit 63 bits", what,
+               per_gameweek ? "S" : "num_samples");
+  BPLX_REQUIRE((long long)S * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
+               "%s: %s * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges", what,
+               per_gameweek ? "draws" : "num_samples", (long long)S * sims_per_draw);
+  return BPLX_OK;
+}
+
+static int check_observed(const bplx_observations* obs, const char* what) {
+  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
+               what);
+  return BPLX_OK;
+}
+
+// what a size call needs before it plans (else it returns 0): S, T and F positive, F = 0 when `allow_no_fixtures`
+static bool plannable(const bplx_samples* s, const bplx_fixtures* f, bool allow_no_fixtures = false) {
+  return s && f && s->num_samples > 0 && s->num_teams > 0 && f->num_fixtures >= (allow_no_fixtures ? 0 : 1);
+}
+
+// Where each region of a consumer's workspace starts (bytes) and the total, 0 for an unsupported shape.  A consumer's
+// plan function fills it for its size call and its launch alike.
+struct WsPlan {
+  size_t table = 0;  // the bytes of the [S][row_floats] exponential table at 0: where the consumer's first region starts
+  size_t total = 0;
+  size_t seg = 0;  // CTA descriptors: pointwise log-likelihood over gameweeks
+  size_t played = 0, pair_beg = 0, pair_fix = 0;  // head-to-head ranking: played matrix, pair offsets, pair fixtures
+};
+
+static int check_grid_args(const bplx_samples* s, const bplx_fixtures* f, int max_goals, const char* what) {
+  const int rc = check_sample_args(s, f, what);
+  if (rc != BPLX_OK) return rc;
+  return check_max_goals(max_goals, what);
 }
 
 // the shape (model, S, T, Cf, F) and the sample / fixture arrays of gp; with F = 0 the fixture arrays may be NULL
@@ -615,16 +660,16 @@ static int check_workspace(const void* workspace, size_t workspace_bytes, size_t
   return BPLX_OK;
 }
 
-static size_t grid_plan(const bplx_samples* s, const bplx_fixtures* f, int max_goals, GridParams* gp, const char** err) {
+static WsPlan grid_plan(const bplx_samples* s, const bplx_fixtures* f, int max_goals, GridParams* gp, const char** err) {
   bind_samples(s, f, gp);
   gp->g = max_goals + 1;
-  return score_grid_plan(gp, err);
+  return {table_layout(gp), score_grid_plan(gp, err)};
 }
 
 size_t bplx_score_grid_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, int max_goals) {
-  if (!s || !f || max_goals < 1 || s->num_samples <= 0 || s->num_teams <= 0 || f->num_fixtures <= 0) return 0;
+  if (max_goals < 1 || !plannable(s, f)) return 0;
   GridParams gp{};
-  return grid_plan(s, f, max_goals, &gp, nullptr);
+  return grid_plan(s, f, max_goals, &gp, nullptr).total;
 }
 
 int bplx_score_grid(const bplx_samples* s, const bplx_fixtures* f, int max_goals, float scale, float* grid,
@@ -634,18 +679,18 @@ int bplx_score_grid(const bplx_samples* s, const bplx_fixtures* f, int max_goals
 
 int bplx_score_grid_ex(const bplx_samples* s, const bplx_fixtures* f, int max_goals, float scale, float* grid,
                        float* outcome, void* workspace, size_t workspace_bytes, void* stream, unsigned flags) {
-  int rc = check_grid_args(s, f, max_goals);
+  int rc = check_grid_args(s, f, max_goals, "score grid");
   if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(grid != nullptr, BPLX_E_INVALID, "grid is NULL");
   GridParams gp{};
   const char* perr = nullptr;
-  const size_t need = grid_plan(s, f, max_goals, &gp, &perr);
-  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "score grid: unsupported shape");
+  const WsPlan w = grid_plan(s, f, max_goals, &gp, &perr);
+  BPLX_REQUIRE(w.total > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "score grid: unsupported shape");
   gp.scale = scale;
-  rc = check_workspace(workspace, workspace_bytes, need);
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   gp.table = static_cast<float*>(workspace);
-  gp.partial = reinterpret_cast<float*>(static_cast<unsigned char*>(workspace) + table_layout(&gp));
+  gp.partial = reinterpret_cast<float*>(static_cast<unsigned char*>(workspace) + w.table);
   gp.grid = grid;
   gp.outcome = outcome;
   gp.reuse_tables = (flags & BPLX_GRID_REUSE_TABLES) ? 1 : 0;
@@ -654,7 +699,7 @@ int bplx_score_grid_ex(const bplx_samples* s, const bplx_fixtures* f, int max_go
 
 int bplx_score_grid_host(const bplx_samples* s, const bplx_fixtures* f, int max_goals, float scale, float* grid,
                          float* outcome) {
-  int rc = check_grid_args(s, f, max_goals);
+  int rc = check_grid_args(s, f, max_goals, "score grid");
   if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(grid != nullptr, BPLX_E_INVALID, "grid is NULL");
   const size_t S = s->num_samples, T = s->num_teams, F = f->num_fixtures, g = max_goals + 1;
@@ -736,15 +781,15 @@ int bplx_score_grid_host(const bplx_samples* s, const bplx_fixtures* f, int max_
 }
 
 // ---- pointwise log-likelihood and PSIS-LOO -----------------------------------------------------------------------
-static size_t pointwise_plan_for(const bplx_samples* s, const bplx_observations* o, PointwiseParams* pp, const char** err) {
+static WsPlan pointwise_plan_for(const bplx_samples* s, const bplx_observations* o, PointwiseParams* pp, const char** err) {
   bind_samples(s, &o->fixtures, &pp->gp);
-  return pointwise_plan(pp, err);
+  return {table_layout(&pp->gp), pointwise_plan(pp, err)};
 }
 
 size_t bplx_pointwise_loglik_workspace_bytes(const bplx_samples* s, const bplx_observations* obs) {
-  if (!s || !obs || s->num_samples <= 0 || s->num_teams <= 0 || obs->fixtures.num_fixtures <= 0) return 0;
+  if (!obs || !plannable(s, &obs->fixtures)) return 0;
   PointwiseParams pp{};
-  return pointwise_plan_for(s, obs, &pp, nullptr);
+  return pointwise_plan_for(s, obs, &pp, nullptr).total;
 }
 
 int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, float* loglik, size_t ld, double* stats,
@@ -752,19 +797,19 @@ int bplx_pointwise_loglik(const bplx_samples* s, const bplx_observations* obs, f
   BPLX_REQUIRE(obs != nullptr, BPLX_E_INVALID, "observations is NULL");
   int rc = check_sample_args(s, &obs->fixtures, "pointwise log-likelihood");
   if (rc != BPLX_OK) return rc;
-  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID,
-               "pointwise log-likelihood: home_goals and away_goals must not be NULL");
+  rc = check_observed(obs, "pointwise log-likelihood");
+  if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(stats != nullptr, BPLX_E_INVALID, "pointwise log-likelihood: stats is NULL");
   BPLX_REQUIRE(!loglik || ld >= (size_t)s->num_samples, BPLX_E_INVALID,
                "pointwise log-likelihood: ld (%zu) < num_samples (%d)", ld, s->num_samples);
   PointwiseParams pp{};
   const char* perr = nullptr;
-  const size_t need = pointwise_plan_for(s, obs, &pp, &perr);
-  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
-  rc = check_workspace(workspace, workspace_bytes, need);
+  const WsPlan w = pointwise_plan_for(s, obs, &pp, &perr);
+  BPLX_REQUIRE(w.total > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   pp.gp.table = static_cast<float*>(workspace);
-  pp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + table_layout(&pp.gp));
+  pp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + w.table);
   pp.hg = obs->home_goals;
   pp.ag = obs->away_goals;
   pp.ll = loglik;
@@ -799,20 +844,37 @@ int bplx_psis_loo(const float* loglik, int num_matches, int num_samples, size_t 
 }
 
 // ---- season / group-stage simulation --------------------------------------------------------------------------
-// the workspace of a simulation is the [S][row_floats] exponential table
-static size_t simulate_plan_for(const bplx_samples* s, const bplx_fixtures* f, SimParams* sp) {
+static bool head_to_head(const bplx_ranking* r) { return r && r->rule == BPLX_RANK_HEAD_TO_HEAD; }
+
+static size_t alloc_bytes(const bplx_bracket* b) {
+  return b->best_alloc ? ((size_t)b->best_count << b->num_groups) : 0;
+}
+
+// workspace of a simulation: the table | a tournament's allocation table | head-to-head: the played matrix [NT][NT]
+// int2, the pair offsets [NT NT + 1] and the pair fixture list [F]; binds the samples and fixtures of *sp.  Total 0: a
+// ranking no size call can size (not a BPLX_RANK_* rule, or head-to-head over a table the kernel does not take).
+static WsPlan simulate_plan(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t, const bplx_bracket* b,
+                            const bplx_ranking* r, SimParams* sp) {
   bind_samples(s, f, &sp->gp);
-  return table_layout(&sp->gp);
+  WsPlan w{table_layout(&sp->gp)};
+  w.played = w.total = w.table + (b ? align256(alloc_bytes(b)) : 0);
+  if (r && r->rule != BPLX_RANK_GOAL_DIFF && r->rule != BPLX_RANK_HEAD_TO_HEAD) return {};
+  if (head_to_head(r)) {
+    if (t->num_slots < 1 || t->num_slots > BPLX_SIM_MAX_TEAMS) return {};
+    const size_t nn = (size_t)t->num_slots * t->num_slots;
+    w.pair_beg = w.played + align256(nn * 8);
+    w.pair_fix = w.pair_beg + align256((nn + 1) * 4);
+    w.total = w.pair_fix + align256((size_t)(f->num_fixtures > 0 ? f->num_fixtures : 1) * 4);
+  }
+  return w;
 }
 
 size_t bplx_simulate_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t) {
-  if (!s || !f || !t || s->num_samples <= 0 || s->num_teams <= 0 || f->num_fixtures <= 0) return 0;
-  SimParams sp{};
-  return simulate_plan_for(s, f, &sp);
+  return bplx_simulate_table_ex_workspace_bytes(s, f, t, nullptr);
 }
 
 // validates the arguments bplx_simulate_table and bplx_simulate_tournament share and fills *sp (its samples, fixtures
-// and workspace aside: simulate_plan_for binds those)
+// and workspace aside: simulate_plan binds those)
 static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
                           const uint8_t* away_slot, const bplx_table* t, int max_goals, int sims_per_draw,
                           unsigned long long seed, long long first_draw, unsigned long long* position_counts,
@@ -828,21 +890,16 @@ static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const u
   BPLX_REQUIRE(t->num_positions >= 1 && t->num_positions <= t->num_slots && t->num_points_bins >= 1, BPLX_E_INVALID,
                "%s: num_positions must be in [1, num_slots] and num_points_bins >= 1 (got %d, %d)", what,
                t->num_positions, t->num_points_bins);
-  BPLX_REQUIRE(t->points_win >= 1 && t->points_draw >= 0 && t->points_draw <= t->points_win, BPLX_E_INVALID,
-               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
-               t->points_win, t->points_draw);
+  rc = check_points(t->points_win, t->points_draw, what);
+  if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(t->start_points && t->start_goals_for && t->start_goals_against, BPLX_E_INVALID,
                "%s: start_points, start_goals_for and start_goals_against must not be NULL", what);
   BPLX_REQUIRE((home_slot && away_slot) || f->num_fixtures == 0, BPLX_E_INVALID,
                "%s: home_slot and away_slot must not be NULL", what);
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
-               max_goals);
-  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
-  BPLX_REQUIRE(first_draw >= 0 && first_draw + s->num_samples <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
-               "%s: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits", what);
-  BPLX_REQUIRE((long long)s->num_samples * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
-               "%s: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
-               what, (long long)s->num_samples * sims_per_draw);
+  rc = check_max_goals(max_goals, what);
+  if (rc != BPLX_OK) return rc;
+  rc = check_draw_range(s->num_samples, sims_per_draw, first_draw, false, what);
+  if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(position_counts && points_counts && invalid, BPLX_E_INVALID,
                "%s: position_counts, points_counts and invalid must not be NULL", what);
   SimParams& sp = *out;
@@ -871,16 +928,6 @@ static int simulate_setup(const bplx_samples* s, const bplx_fixtures* f, const u
 }
 
 // ---- ranking rules --------------------------------------------------------------------------------------------
-static bool head_to_head(const bplx_ranking* r) { return r && r->rule == BPLX_RANK_HEAD_TO_HEAD; }
-
-// workspace bytes the ranking adds after `base` (256-aligned): head-to-head keeps the played matrix [NT][NT] int2, the
-// pair offsets [NT NT + 1] and the pair fixture list [F]
-static size_t ranking_bytes(const bplx_ranking* r, int NT, int F) {
-  if (!head_to_head(r)) return 0;
-  const size_t nn = (size_t)NT * NT;
-  return (nn * 8 + 255) / 256 * 256 + ((nn + 1) * 4 + 255) / 256 * 256 + ((size_t)(F > 0 ? F : 1) * 4 + 255) / 256 * 256;
-}
-
 static int check_ranking(const bplx_ranking* r, int NT, const char* what) {
   if (!r) return BPLX_OK;
   BPLX_REQUIRE(r->rule == BPLX_RANK_GOAL_DIFF || r->rule == BPLX_RANK_HEAD_TO_HEAD, BPLX_E_INVALID,
@@ -893,28 +940,26 @@ static int check_ranking(const bplx_ranking* r, int NT, const char* what) {
   return BPLX_OK;
 }
 
-// fills the head-to-head fields of *sp from the workspace region at `base` (the played matrix is copied there)
-static int bind_ranking(const bplx_ranking* r, void* workspace, size_t base, SimParams* sp, cudaStream_t stream) {
+// fills the head-to-head fields of *sp from the plan's regions (the played matrix is copied there)
+static int bind_ranking(const bplx_ranking* r, void* workspace, const WsPlan& w, SimParams* sp, cudaStream_t stream) {
   sp->rule = r ? r->rule : BPLX_RANK_GOAL_DIFF;
   if (!head_to_head(r)) return BPLX_OK;
-  const size_t nn = (size_t)sp->NT * sp->NT;
-  unsigned char* p = static_cast<unsigned char*>(workspace) + base;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
   if (r->played_h2h) {
-    BPLX_CUDA(cudaMemcpyAsync(p, r->played_h2h, nn * 8, cudaMemcpyHostToDevice, stream));
-    sp->h2h_played = reinterpret_cast<const int2*>(p);
+    BPLX_CUDA(cudaMemcpyAsync(ws + w.played, r->played_h2h, (size_t)sp->NT * sp->NT * 8, cudaMemcpyHostToDevice,
+                              stream));
+    sp->h2h_played = reinterpret_cast<const int2*>(ws + w.played);
   }
-  p += (nn * 8 + 255) / 256 * 256;
-  sp->pair_beg = reinterpret_cast<int*>(p);
-  sp->pair_fix = reinterpret_cast<int*>(p + ((nn + 1) * 4 + 255) / 256 * 256);
+  sp->pair_beg = reinterpret_cast<int*>(ws + w.pair_beg);
+  sp->pair_fix = reinterpret_cast<int*>(ws + w.pair_fix);
   return BPLX_OK;
 }
 
 size_t bplx_simulate_table_ex_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
                                               const bplx_ranking* r) {
-  const size_t base = bplx_simulate_workspace_bytes(s, f, t);
-  if (!base || (r && r->rule != BPLX_RANK_GOAL_DIFF && r->rule != BPLX_RANK_HEAD_TO_HEAD)) return 0;
-  if (t->num_slots < 1 || t->num_slots > BPLX_SIM_MAX_TEAMS) return head_to_head(r) ? 0 : base;
-  return base + ranking_bytes(r, t->num_slots, f->num_fixtures);
+  if (!t || !plannable(s, f)) return 0;
+  SimParams sp{};
+  return simulate_plan(s, f, t, nullptr, r, &sp).total;
 }
 
 int bplx_simulate_table(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot, const uint8_t* away_slot,
@@ -997,27 +1042,19 @@ int bplx_simulate_table_conditional(const bplx_samples* s, const bplx_fixtures* 
                           &sp.cd);
     if (rc != BPLX_OK) return rc;
   }
-  const size_t table = simulate_plan_for(s, f, &sp);
-  rc = check_workspace(workspace, workspace_bytes, table + ranking_bytes(r, t->num_slots, f->num_fixtures));
+  const WsPlan w = simulate_plan(s, f, t, nullptr, r, &sp);
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
-  rc = bind_ranking(r, workspace, table, &sp, static_cast<cudaStream_t>(stream));
+  rc = bind_ranking(r, workspace, w, &sp, static_cast<cudaStream_t>(stream));
   if (rc != BPLX_OK) return rc;
   return launch_simulate(sp, static_cast<cudaStream_t>(stream));
 }
 
 // ---- tournament simulation -----------------------------------------------------------------------------------
-static size_t alloc_bytes(const bplx_bracket* b) {
-  return b->best_alloc ? ((size_t)b->best_count << b->num_groups) : 0;
-}
-
 size_t bplx_simulate_tournament_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, const bplx_table* t,
                                                 const bplx_bracket* b) {
-  if (!s || !f || !t || !b || s->num_samples <= 0 || s->num_teams <= 0 || f->num_fixtures < 0) return 0;
-  if (b->num_groups < 0 || b->num_groups > BPLX_SIM_MAX_TEAMS || b->best_count < 0) return 0;
-  if (b->best_alloc && b->num_groups > BPLX_KO_MAX_ALLOC_GROUPS) return 0;
-  SimParams sp{};
-  return simulate_plan_for(s, f, &sp) + (alloc_bytes(b) + 255) / 256 * 256;
+  return bplx_simulate_tournament_ranked_workspace_bytes(s, f, t, b, nullptr);
 }
 
 // the bracket checks the kernel relies on; fills sp->ko
@@ -1126,10 +1163,11 @@ static int check_bracket(const bplx_bracket* b, const uint8_t* tie_format, const
 size_t bplx_simulate_tournament_ranked_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f,
                                                        const bplx_table* t, const bplx_bracket* b,
                                                        const bplx_ranking* r) {
-  const size_t base = bplx_simulate_tournament_workspace_bytes(s, f, t, b);
-  if (!base || (r && r->rule != BPLX_RANK_GOAL_DIFF && r->rule != BPLX_RANK_HEAD_TO_HEAD)) return 0;
-  if (t->num_slots < 1 || t->num_slots > BPLX_SIM_MAX_TEAMS) return head_to_head(r) ? 0 : base;
-  return base + ranking_bytes(r, t->num_slots, f->num_fixtures);
+  if (!t || !b || !plannable(s, f, true)) return 0;
+  if (b->num_groups < 0 || b->num_groups > BPLX_SIM_MAX_TEAMS || b->best_count < 0) return 0;
+  if (b->best_alloc && b->num_groups > BPLX_KO_MAX_ALLOC_GROUPS) return 0;
+  SimParams sp{};
+  return simulate_plan(s, f, t, b, r, &sp).total;
 }
 
 int bplx_simulate_tournament_ex(const bplx_samples* s, const bplx_fixtures* f, const uint8_t* home_slot,
@@ -1174,10 +1212,10 @@ int bplx_simulate_tournament_paired(const bplx_samples* s, const bplx_fixtures* 
   BPLX_REQUIRE(reach_counts && win_counts, BPLX_E_INVALID, "tournament: reach_counts and win_counts must not be NULL");
   rc = check_ranking(r, t->num_slots, "tournament");
   if (rc != BPLX_OK) return rc;
-  const size_t table = simulate_plan_for(s, f, &sp), alloc = (alloc_bytes(b) + 255) / 256 * 256;
-  rc = check_workspace(workspace, workspace_bytes, table + alloc + ranking_bytes(r, t->num_slots, f->num_fixtures));
+  const WsPlan w = simulate_plan(s, f, t, b, r, &sp);
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
-  rc = bind_ranking(r, workspace, table + alloc, &sp, static_cast<cudaStream_t>(stream));
+  rc = bind_ranking(r, workspace, w, &sp, static_cast<cudaStream_t>(stream));
   if (rc != BPLX_OK) return rc;
   sp.gp.table = static_cast<float*>(workspace);
   sp.ko.reach = reach_counts;
@@ -1188,7 +1226,7 @@ int bplx_simulate_tournament_paired(const bplx_samples* s, const bplx_fixtures* 
   sp.ko.winners = ko_winners;
   sp.ko.extra = ko_extra;
   if (b->best_alloc) {
-    uint8_t* const dst = static_cast<uint8_t*>(workspace) + table;
+    uint8_t* const dst = static_cast<uint8_t*>(workspace) + w.table;
     BPLX_CUDA(cudaMemcpyAsync(dst, b->best_alloc, alloc_bytes(b), cudaMemcpyHostToDevice,
                               static_cast<cudaStream_t>(stream)));
     sp.ko.alloc = dst;
@@ -1340,12 +1378,56 @@ int bplx_simulate_tournament_ranked(const bplx_samples* s, const bplx_fixtures* 
 }
 
 // ---- posterior predictive checks ------------------------------------------------------------------------------
-// the workspace is the [S][row_floats] exponential table, as for a simulation
+// workspace of a predictive check: the table (all G' S rows over gameweeks) | over gameweeks, the matches' gameweeks [M]
+static WsPlan ppc_plan(const bplx_samples* s, const bplx_observations* obs, bool gameweeks, GridParams* gp) {
+  bind_samples(s, &obs->fixtures, gp);
+  const size_t table = table_layout(gp);
+  return {table, table + (gameweeks ? (size_t)obs->fixtures.num_fixtures * sizeof(int32_t) : 0)};
+}
+
 size_t bplx_posterior_predictive_workspace_bytes(const bplx_samples* s, const bplx_observations* obs) {
-  if (!s || !obs || s->num_samples <= 0 || s->num_teams <= 0 || obs->fixtures.num_fixtures <= 0) return 0;
+  if (!obs || !plannable(s, &obs->fixtures)) return 0;
   GridParams gp{};
-  bind_samples(s, &obs->fixtures, &gp);
-  return table_layout(&gp);
+  return ppc_plan(s, obs, false, &gp).total;
+}
+
+// checks what both predictive checks take after samples (and gameweeks) into *pp; S: the call's draws (per gameweek)
+static int ppc_setup(const bplx_observations* obs, int S, bool per_gameweek, int max_goals, int score_bins,
+                     int points_win, int points_draw, int sims_per_draw, unsigned long long seed, long long first_draw,
+                     const bplx_ppc_output* out, const char* what, PpcParams* pp) {
+  int rc = check_observed(obs, what);
+  if (rc != BPLX_OK) return rc;
+  rc = check_max_goals(max_goals, what);
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(score_bins >= 2 && score_bins <= 16, BPLX_E_INVALID, "%s: score_bins must be in [2, 16] (got %d)", what,
+               score_bins);
+  rc = check_points(points_win, points_draw, what);
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE((long long)std::max(points_win, max_goals) * obs->fixtures.num_fixtures <= INT_MAX, BPLX_E_INVALID,
+               "%s: max(points_win, max_goals) * num_matches must be below 2^31 (a team count could overflow)", what);
+  rc = check_draw_range(S, sims_per_draw, first_draw, per_gameweek, what);
+  if (rc != BPLX_OK) return rc;
+  BPLX_REQUIRE(out->score_counts && out->outcome_counts && out->goals && out->total_goals_sq && out->team_points &&
+                   out->team_goals_for && out->team_goals_against && out->invalid,
+               BPLX_E_INVALID, "%s: every output but scores must be given", what);
+  pp->G = max_goals;
+  pp->B = score_bins;
+  pp->R = sims_per_draw;
+  pp->pw = points_win;
+  pp->pd = points_draw;
+  pp->seed = seed;
+  pp->first_draw = first_draw;
+  pp->N = S * sims_per_draw;
+  pp->score_counts = out->score_counts;
+  pp->outcome_counts = out->outcome_counts;
+  pp->goals = reinterpret_cast<long long*>(out->goals);
+  pp->total_goals_sq = reinterpret_cast<long long*>(out->total_goals_sq);
+  pp->team_points = out->team_points;
+  pp->team_goals_for = out->team_goals_for;
+  pp->team_goals_against = out->team_goals_against;
+  pp->scores = out->scores;
+  pp->invalid = out->invalid;
+  return BPLX_OK;
 }
 
 int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* obs, int max_goals, int score_bins,
@@ -1356,49 +1438,13 @@ int bplx_posterior_predictive(const bplx_samples* s, const bplx_observations* ob
   BPLX_REQUIRE(obs != nullptr && out != nullptr, BPLX_E_INVALID, "%s: observations / out is NULL", what);
   int rc = check_sample_args(s, &obs->fixtures, what);
   if (rc != BPLX_OK) return rc;
-  const int M = obs->fixtures.num_fixtures;
-  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
-               what);
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
-               max_goals);
-  BPLX_REQUIRE(score_bins >= 2 && score_bins <= 16, BPLX_E_INVALID, "%s: score_bins must be in [2, 16] (got %d)", what,
-               score_bins);
-  BPLX_REQUIRE(points_win >= 1 && points_draw >= 0 && points_draw <= points_win, BPLX_E_INVALID,
-               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
-               points_win, points_draw);
-  BPLX_REQUIRE((long long)std::max(points_win, max_goals) * M <= INT_MAX, BPLX_E_INVALID,
-               "%s: max(points_win, max_goals) * num_matches must be below 2^31 (a team count could overflow)", what);
-  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
-  BPLX_REQUIRE(first_draw >= 0 && first_draw + s->num_samples <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
-               "%s: first_draw must be >= 0 and (first_draw + num_samples) * sims_per_draw must fit 63 bits", what);
-  BPLX_REQUIRE((long long)s->num_samples * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
-               "%s: num_samples * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges",
-               what, (long long)s->num_samples * sims_per_draw);
-  BPLX_REQUIRE(out->score_counts && out->outcome_counts && out->goals && out->total_goals_sq && out->team_points &&
-                   out->team_goals_for && out->team_goals_against && out->invalid,
-               BPLX_E_INVALID, "%s: every output but scores must be given", what);
   PpcParams pp{};
-  bind_samples(s, &obs->fixtures, &pp.gp);
-  rc = check_workspace(workspace, workspace_bytes, table_layout(&pp.gp));
+  rc = ppc_setup(obs, s->num_samples, false, max_goals, score_bins, points_win, points_draw, sims_per_draw, seed,
+                 first_draw, out, what, &pp);
+  if (rc != BPLX_OK) return rc;
+  rc = check_workspace(workspace, workspace_bytes, ppc_plan(s, obs, false, &pp.gp).total);
   if (rc != BPLX_OK) return rc;
   pp.gp.table = static_cast<float*>(workspace);
-  pp.G = max_goals;
-  pp.B = score_bins;
-  pp.R = sims_per_draw;
-  pp.pw = points_win;
-  pp.pd = points_draw;
-  pp.seed = seed;
-  pp.first_draw = first_draw;
-  pp.N = s->num_samples * sims_per_draw;
-  pp.score_counts = out->score_counts;
-  pp.outcome_counts = out->outcome_counts;
-  pp.goals = reinterpret_cast<long long*>(out->goals);
-  pp.total_goals_sq = reinterpret_cast<long long*>(out->total_goals_sq);
-  pp.team_points = out->team_points;
-  pp.team_goals_for = out->team_goals_for;
-  pp.team_goals_against = out->team_goals_against;
-  pp.scores = out->scores;
-  pp.invalid = out->invalid;
   return launch_ppc(pp, static_cast<cudaStream_t>(stream));
 }
 
@@ -1453,27 +1499,24 @@ static int check_gameweeks(const bplx_samples* s, int ngw, const bplx_observatio
 
 // workspace of the segmented log-likelihood: [G' S] table rows | partial stats [nsplit][M][4] | CTA descriptors (at most
 // one per gameweek plus one per kPwThreads matches)
-static size_t pointwise_gw_plan(const bplx_samples* s, int ngw, const bplx_observations* o, PointwiseParams* pp,
-                                const char** err, size_t* off_partial, size_t* off_seg) {
+static WsPlan pointwise_gw_plan(const bplx_samples* s, int ngw, const bplx_observations* o, PointwiseParams* pp,
+                                const char** err) {
   bind_samples(s, &o->fixtures, &pp->gp);
   pp->gp.S = s->num_samples / ngw;
-  if (pointwise_plan(pp, err) == 0) return 0;
+  if (pointwise_plan(pp, err) == 0) return {};
   GridParams all = pp->gp;
   all.S = s->num_samples;
-  *off_partial = table_layout(&all);
-  *off_seg = align256(*off_partial + (size_t)pp->gp.nsplit * pp->gp.F * 4 * sizeof(double));
+  const size_t table = table_layout(&all);
+  const size_t seg = align256(table + (size_t)pp->gp.nsplit * pp->gp.F * 4 * sizeof(double));
   const size_t max_seg = (size_t)(pp->gp.F + kPwThreads - 1) / kPwThreads + ngw;
-  return *off_seg + max_seg * sizeof(int4);
+  return {table, seg + max_seg * sizeof(int4), seg};
 }
 
 size_t bplx_pointwise_loglik_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
                                                        const bplx_observations* obs) {
-  if (!s || !obs || num_gameweeks < 1 || s->num_samples <= 0 || s->num_samples % num_gameweeks || s->num_teams <= 0 ||
-      obs->fixtures.num_fixtures <= 0)
-    return 0;
+  if (!obs || !plannable(s, &obs->fixtures) || num_gameweeks < 1 || s->num_samples % num_gameweeks) return 0;
   PointwiseParams pp{};
-  size_t a, b;
-  return pointwise_gw_plan(s, num_gameweeks, obs, &pp, nullptr, &a, &b);
+  return pointwise_gw_plan(s, num_gameweeks, obs, &pp, nullptr).total;
 }
 
 int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
@@ -1486,16 +1529,15 @@ int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, co
   rc = check_gameweeks(s, num_gameweeks, obs, gameweek, true, what);
   if (rc != BPLX_OK) return rc;
   const int S = s->num_samples / num_gameweeks, M = obs->fixtures.num_fixtures;
-  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
-               what);
+  rc = check_observed(obs, what);
+  if (rc != BPLX_OK) return rc;
   BPLX_REQUIRE(stats != nullptr, BPLX_E_INVALID, "%s: stats is NULL", what);
   BPLX_REQUIRE(!loglik || ld >= (size_t)S, BPLX_E_INVALID, "%s: ld (%zu) < draws per gameweek (%d)", what, ld, S);
   PointwiseParams pp{};
   const char* perr = nullptr;
-  size_t off_partial = 0, off_seg = 0;
-  const size_t need = pointwise_gw_plan(s, num_gameweeks, obs, &pp, &perr, &off_partial, &off_seg);
-  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
-  rc = check_workspace(workspace, workspace_bytes, need);
+  const WsPlan w = pointwise_gw_plan(s, num_gameweeks, obs, &pp, &perr);
+  BPLX_REQUIRE(w.total > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "pointwise log-likelihood: unsupported shape");
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   // one descriptor per (gameweek, run of up to kPwThreads of its matches): CTAs are cut at gameweek boundaries
   std::vector<int4> seg;
@@ -1507,10 +1549,10 @@ int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, co
   }
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  BPLX_CUDA(cudaMemcpyAsync(ws + off_seg, seg.data(), seg.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+  BPLX_CUDA(cudaMemcpyAsync(ws + w.seg, seg.data(), seg.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
   pp.gp.table = reinterpret_cast<float*>(ws);
-  pp.partial = reinterpret_cast<double*>(ws + off_partial);
-  pp.seg = reinterpret_cast<const int4*>(ws + off_seg);
+  pp.partial = reinterpret_cast<double*>(ws + w.table);
+  pp.seg = reinterpret_cast<const int4*>(ws + w.seg);
   pp.nseg = (int)seg.size();
   pp.hg = obs->home_goals;
   pp.ag = obs->away_goals;
@@ -1520,15 +1562,11 @@ int bplx_pointwise_loglik_gameweeks(const bplx_samples* s, int num_gameweeks, co
   return launch_pointwise_segmented(pp, num_gameweeks, st);
 }
 
-// workspace of the multi-gameweek predictive check: [G' S] table rows | the matches' gameweeks [M]
 size_t bplx_posterior_predictive_gameweeks_workspace_bytes(const bplx_samples* s, int num_gameweeks,
                                                            const bplx_observations* obs) {
-  if (!s || !obs || num_gameweeks < 1 || s->num_samples <= 0 || s->num_samples % num_gameweeks || s->num_teams <= 0 ||
-      obs->fixtures.num_fixtures <= 0)
-    return 0;
+  if (!obs || !plannable(s, &obs->fixtures) || num_gameweeks < 1 || s->num_samples % num_gameweeks) return 0;
   GridParams gp{};
-  bind_samples(s, &obs->fixtures, &gp);
-  return table_layout(&gp) + (size_t)obs->fixtures.num_fixtures * sizeof(int32_t);
+  return ppc_plan(s, obs, true, &gp).total;
 }
 
 int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks, const bplx_observations* obs,
@@ -1542,84 +1580,45 @@ int bplx_posterior_predictive_gameweeks(const bplx_samples* s, int num_gameweeks
   if (rc != BPLX_OK) return rc;
   rc = check_gameweeks(s, num_gameweeks, obs, gameweek, false, what);
   if (rc != BPLX_OK) return rc;
-  const int S = s->num_samples / num_gameweeks, M = obs->fixtures.num_fixtures;
-  BPLX_REQUIRE(obs->home_goals && obs->away_goals, BPLX_E_INVALID, "%s: home_goals and away_goals must not be NULL",
-               what);
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "%s: max_goals must be in [1, 63] (got %d)", what,
-               max_goals);
-  BPLX_REQUIRE(score_bins >= 2 && score_bins <= 16, BPLX_E_INVALID, "%s: score_bins must be in [2, 16] (got %d)", what,
-               score_bins);
-  BPLX_REQUIRE(points_win >= 1 && points_draw >= 0 && points_draw <= points_win, BPLX_E_INVALID,
-               "%s: points must satisfy 0 <= points_draw <= points_win, points_win >= 1 (got %d, %d)", what,
-               points_win, points_draw);
-  BPLX_REQUIRE((long long)std::max(points_win, max_goals) * M <= INT_MAX, BPLX_E_INVALID,
-               "%s: max(points_win, max_goals) * num_matches must be below 2^31 (a team count could overflow)", what);
-  BPLX_REQUIRE(sims_per_draw >= 1, BPLX_E_INVALID, "%s: sims_per_draw must be >= 1 (got %d)", what, sims_per_draw);
-  BPLX_REQUIRE(first_draw >= 0 && first_draw + S <= LLONG_MAX / sims_per_draw, BPLX_E_INVALID,
-               "%s: first_draw must be >= 0 and (first_draw + S) * sims_per_draw must fit 63 bits", what);
-  BPLX_REQUIRE((long long)S * sims_per_draw <= INT_MAX, BPLX_E_UNSUPPORTED,
-               "%s: draws * sims_per_draw must be below 2^31 per call (got %lld): cut the draws into ranges", what,
-               (long long)S * sims_per_draw);
-  BPLX_REQUIRE(out->score_counts && out->outcome_counts && out->goals && out->total_goals_sq && out->team_points &&
-                   out->team_goals_for && out->team_goals_against && out->invalid,
-               BPLX_E_INVALID, "%s: every output but scores must be given", what);
+  const int S = s->num_samples / num_gameweeks;
   PpcParams pp{};
-  bind_samples(s, &obs->fixtures, &pp.gp);
-  const size_t off_gw = table_layout(&pp.gp);
-  rc = check_workspace(workspace, workspace_bytes, off_gw + (size_t)M * sizeof(int32_t));
+  rc = ppc_setup(obs, S, true, max_goals, score_bins, points_win, points_draw, sims_per_draw, seed, first_draw, out,
+                 what, &pp);
+  if (rc != BPLX_OK) return rc;
+  const WsPlan w = ppc_plan(s, obs, true, &pp.gp);
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  BPLX_CUDA(cudaMemcpyAsync(ws + off_gw, gameweek, (size_t)M * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  BPLX_CUDA(cudaMemcpyAsync(ws + w.table, gameweek, w.total - w.table, cudaMemcpyHostToDevice, st));
   pp.gp.S = S;
   pp.gp.table = reinterpret_cast<float*>(ws);
-  pp.gw = reinterpret_cast<const int32_t*>(ws + off_gw);
+  pp.gw = reinterpret_cast<const int32_t*>(ws + w.table);
   pp.ngw = num_gameweeks;
-  pp.G = max_goals;
-  pp.B = score_bins;
-  pp.R = sims_per_draw;
-  pp.pw = points_win;
-  pp.pd = points_draw;
-  pp.seed = seed;
-  pp.first_draw = first_draw;
-  pp.N = S * sims_per_draw;
-  pp.score_counts = out->score_counts;
-  pp.outcome_counts = out->outcome_counts;
-  pp.goals = reinterpret_cast<long long*>(out->goals);
-  pp.total_goals_sq = reinterpret_cast<long long*>(out->total_goals_sq);
-  pp.team_points = out->team_points;
-  pp.team_goals_for = out->team_goals_for;
-  pp.team_goals_against = out->team_goals_against;
-  pp.scores = out->scores;
-  pp.invalid = out->invalid;
   return launch_ppc_gameweeks(pp, st);
 }
 
 // ---- forecast uncertainty: per-draw markets and row quantiles ----------------------------------------------------
-static size_t market_plan_for(const bplx_samples* s, const bplx_fixtures* f, int max_goals, MarketParams* mp,
+static WsPlan market_plan_for(const bplx_samples* s, const bplx_fixtures* f, int max_goals, MarketParams* mp,
                               const char** err) {
   bind_samples(s, f, &mp->gp);
   mp->gp.g = max_goals + 1;
-  return market_plan(mp, err);
+  return {table_layout(&mp->gp), market_plan(mp, err)};
 }
 
 size_t bplx_market_draws_workspace_bytes(const bplx_samples* s, const bplx_fixtures* f, int max_goals,
                                          const bplx_market_lines* lines) {
-  if (!s || !f || !lines || max_goals < 1 || max_goals > 63 || s->num_samples <= 0 || s->num_teams <= 0 ||
-      f->num_fixtures <= 0)
-    return 0;
+  if (!lines || max_goals < 1 || max_goals > 63 || !plannable(s, f)) return 0;
   MarketParams mp{};
   if (market_rows(lines, max_goals, &mp) != BPLX_OK) return 0;
-  return market_plan_for(s, f, max_goals, &mp, nullptr);
+  return market_plan_for(s, f, max_goals, &mp, nullptr).total;
 }
 
 int bplx_market_draws(const bplx_samples* s, const bplx_fixtures* f, int max_goals, const bplx_market_lines* lines,
                       float* draws, size_t ld, double* stats, int* invalid, void* workspace, size_t workspace_bytes,
                       void* stream) {
-  int rc = check_sample_args(s, f, "markets");
+  int rc = check_grid_args(s, f, max_goals, "markets");
   if (rc != BPLX_OK) return rc;
-  BPLX_REQUIRE(max_goals >= 1 && max_goals <= 63, BPLX_E_INVALID, "markets: max_goals must be in [1, 63] (got %d)",
-               max_goals);
   BPLX_REQUIRE(stats && invalid, BPLX_E_INVALID, "markets: stats and invalid must not be NULL");
   BPLX_REQUIRE(!draws || ld >= (size_t)s->num_samples, BPLX_E_INVALID, "markets: ld (%zu) < num_samples (%d)", ld,
                s->num_samples);
@@ -1627,12 +1626,12 @@ int bplx_market_draws(const bplx_samples* s, const bplx_fixtures* f, int max_goa
   rc = market_rows(lines, max_goals, &mp);
   if (rc != BPLX_OK) return rc;
   const char* perr = nullptr;
-  const size_t need = market_plan_for(s, f, max_goals, &mp, &perr);
-  BPLX_REQUIRE(need > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "markets: unsupported shape");
-  rc = check_workspace(workspace, workspace_bytes, need);
+  const WsPlan w = market_plan_for(s, f, max_goals, &mp, &perr);
+  BPLX_REQUIRE(w.total > 0, BPLX_E_UNSUPPORTED, "%s", perr ? perr : "markets: unsupported shape");
+  rc = check_workspace(workspace, workspace_bytes, w.total);
   if (rc != BPLX_OK) return rc;
   mp.gp.table = static_cast<float*>(workspace);
-  mp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + table_layout(&mp.gp));
+  mp.partial = reinterpret_cast<double*>(static_cast<unsigned char*>(workspace) + w.table);
   mp.draws = draws;
   mp.ld = ld;
   mp.stats = stats;

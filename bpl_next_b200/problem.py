@@ -201,6 +201,40 @@ def _workspace(workspace, need: int, device):
     return workspace
 
 
+def _observations_struct(observations: dict, ptr):
+    o = _abi.Observations()
+    o.fixtures = _fixtures_struct(observations, ptr)
+    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    return o
+
+
+def _output_matrix(buf: Optional[torch.Tensor], rows: int, S: int, device, want: bool):
+    """``(matrix, ld)``: the ``[rows, ld]`` float32 output (``buf``, else a new ``[rows, S]`` one) or ``(None, 0)``."""
+    if not want:
+        return None, 0
+    if buf is None:
+        buf = torch.empty((rows, S), dtype=torch.float32, device=device)
+    assert buf.dtype == torch.float32 and buf.shape[0] >= rows and buf.stride(1) == 1
+    return buf, int(buf.stride(0)) if rows > 1 else max(S, int(buf.shape[1]))
+
+
+def _ppc_outputs(N: int, M: int, T: int, B: int, device, want_scores: bool):
+    """Outputs of a predictive check (N replicates, M matches, T teams, B score bins) and their ``_abi.PpcOutput``."""
+    i32, i64 = dict(dtype=torch.int32, device=device), dict(dtype=torch.int64, device=device)
+    shapes = {"score_counts": ((N, B, B), i32), "outcome_counts": ((N, 3), i32), "goals": ((N, 2), i64),
+              "total_goals_sq": ((N,), i64), "team_points": ((N, T), i32), "team_goals_for": ((N, T), i32),
+              "team_goals_against": ((N, T), i32)}
+    res = {k: torch.empty(shp, **kw) for k, (shp, kw) in shapes.items()}
+    res["invalid"] = torch.empty(1, **i64)
+    res["scores"] = torch.empty((N, M, 2), dtype=torch.uint8, device=device) if want_scores else None
+    return res, _abi.PpcOutput(**{k: _dptr(v) for k, v in res.items()})
+
+
+def _seed(seed: int) -> int:
+    """The 64-bit seed the C ABI takes (``unsigned long long``) of a Python int."""
+    return int(seed) & 0xFFFFFFFFFFFFFFFF
+
+
 def score_grid_workspace_bytes(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[str, torch.Tensor],
                                max_goals: int) -> int:
     """Bytes of device workspace ``score_grid`` needs for these shapes (``bplx_score_grid_workspace_bytes``)."""
@@ -273,21 +307,14 @@ def pointwise_loglik(model: str, samples: Dict[str, torch.Tensor], observations:
     ptr = _device_ptr_fn(keep)
     _check_inputs(samples, observations, ("home_goals", "away_goals"))
     s = _samples_struct(model, samples, ptr)
-    o = _abi.Observations()
-    o.fixtures = _fixtures_struct(observations, ptr)
-    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    o = _observations_struct(observations, ptr)
     M, S = o.fixtures.num_fixtures, s.num_samples
     dev = samples["attack"].device
     workspace = _workspace(workspace, int(lib.bplx_pointwise_loglik_workspace_bytes(C.byref(s), C.byref(o))), dev)
-    ld = 0
-    if want_matrix:
-        if loglik is None:
-            loglik = torch.empty((M, S), dtype=torch.float32, device=dev)
-        assert loglik.dtype == torch.float32 and loglik.shape[0] >= M and loglik.stride(1) == 1
-        ld = int(loglik.stride(0)) if M > 1 else max(S, int(loglik.shape[1]))
+    loglik, ld = _output_matrix(loglik, M, S, dev, want_matrix)
     stats = torch.empty((M, 4), dtype=torch.float64, device=dev)
-    _abi.check(lib.bplx_pointwise_loglik(C.byref(s), C.byref(o), _dptr(loglik) if want_matrix else None, ld,
-                                         _dptr(stats), _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    _abi.check(lib.bplx_pointwise_loglik(C.byref(s), C.byref(o), _dptr(loglik), ld, _dptr(stats), _dptr(workspace),
+                                         workspace.numel(), _stream_ptr(stream)))
     return (loglik[:M, :S] if want_matrix else None), stats
 
 
@@ -353,17 +380,12 @@ def market_draws(model: str, samples: Dict[str, torch.Tensor], fixtures: Dict[st
     dev = samples["attack"].device
     need = int(lib.bplx_market_draws_workspace_bytes(C.byref(s), C.byref(f), int(max_goals), C.byref(ln)))
     workspace = _workspace(workspace, need, dev)
-    ld = 0
-    if want_matrix:
-        if draws is None:
-            draws = torch.empty((F * K, S), dtype=torch.float32, device=dev)
-        assert draws.dtype == torch.float32 and draws.shape[0] >= F * K and draws.stride(1) == 1
-        ld = int(draws.stride(0)) if F * K > 1 else max(S, int(draws.shape[1]))
+    draws, ld = _output_matrix(draws, F * K, S, dev, want_matrix)
     stats = torch.empty((F * K, 2), dtype=torch.float64, device=dev)
     invalid = torch.empty(1, dtype=torch.int32, device=dev)
-    _abi.check(lib.bplx_market_draws(C.byref(s), C.byref(f), int(max_goals), C.byref(ln),
-                                     _dptr(draws) if want_matrix else None, ld, _dptr(stats), _dptr(invalid),
-                                     _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    _abi.check(lib.bplx_market_draws(C.byref(s), C.byref(f), int(max_goals), C.byref(ln), _dptr(draws), ld,
+                                     _dptr(stats), _dptr(invalid), _dptr(workspace), workspace.numel(),
+                                     _stream_ptr(stream)))
     return (draws[:F * K, :S] if want_matrix else None), stats, invalid
 
 
@@ -653,7 +675,7 @@ def _simulate(model, samples, fixtures, table, bracket, max_goals, sims_per_draw
             run, args = lib.bplx_simulate_tournament_paired, args + (None if r is None else C.byref(r), C.byref(pg))
         elif r is not None:
             run, args = lib.bplx_simulate_tournament_ranked, args + (C.byref(r),)
-    _abi.check(run(*args, int(max_goals), int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
+    _abi.check(run(*args, int(max_goals), int(sims_per_draw), _seed(seed), int(first_draw),
                    *outputs, _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
     return out
 
@@ -684,25 +706,16 @@ def posterior_predictive(model: str, samples: Dict[str, torch.Tensor], observati
     ptr = _device_ptr_fn(keep)
     _check_inputs(samples, observations, ("home_goals", "away_goals"))
     s = _samples_struct(model, samples, ptr)
-    o = _abi.Observations()
-    o.fixtures = _fixtures_struct(observations, ptr)
-    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
-    M, S, T, B = o.fixtures.num_fixtures, s.num_samples, s.num_teams, int(score_bins)
-    N = S * int(sims_per_draw)
+    o = _observations_struct(observations, ptr)
+    B = int(score_bins)
     dev = samples["attack"].device
     workspace = _workspace(workspace, int(lib.bplx_posterior_predictive_workspace_bytes(C.byref(s), C.byref(o))), dev)
-    i32, i64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.int64, device=dev)
-    shapes = {"score_counts": ((N, B, B), i32), "outcome_counts": ((N, 3), i32), "goals": ((N, 2), i64),
-              "total_goals_sq": ((N,), i64), "team_points": ((N, T), i32), "team_goals_for": ((N, T), i32),
-              "team_goals_against": ((N, T), i32)}
-    res = {k: torch.empty(shp, **kw) for k, (shp, kw) in shapes.items()}
-    res["invalid"] = torch.empty(1, **i64)
-    res["scores"] = torch.empty((N, M, 2), dtype=torch.uint8, device=dev) if want_scores else None
-    out = _abi.PpcOutput(**{k: _dptr(v) for k, v in res.items()})
+    res, out = _ppc_outputs(s.num_samples * int(sims_per_draw), o.fixtures.num_fixtures, s.num_teams, B, dev,
+                            want_scores)
     pw, pd = (int(x) for x in points)
     _abi.check(lib.bplx_posterior_predictive(C.byref(s), C.byref(o), int(max_goals), B, pw, pd, int(sims_per_draw),
-                                             int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw), C.byref(out),
-                                             _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+                                             _seed(seed), int(first_draw), C.byref(out), _dptr(workspace),
+                                             workspace.numel(), _stream_ptr(stream)))
     return res
 
 
@@ -722,8 +735,8 @@ def dynamic_forecast(attack_last: torch.Tensor, defence_last: torch.Tensor, hori
     S, T = int(attack_last.shape[0]), int(attack_last.shape[1])
     out = {k: torch.empty((int(horizon), S, T), dtype=torch.float32, device=attack_last.device) for k in _FORECAST_SITES}
     _abi.check(lib.bplx_dynamic_forecast(_dptr(attack_last), _dptr(defence_last), S, T, int(horizon),
-                                         int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
-                                         *(_dptr(out[k]) for k in _FORECAST_SITES), _stream_ptr(stream)))
+                                         _seed(seed), int(first_draw), *(_dptr(out[k]) for k in _FORECAST_SITES),
+                                         _stream_ptr(stream)))
     return out
 
 
@@ -744,9 +757,7 @@ def take_rows(v: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
 def _gw_observations(samples, observations, gameweek, keep):
     ptr = _device_ptr_fn(keep)
     _check_inputs(samples, observations, ("home_goals", "away_goals"))
-    o = _abi.Observations()
-    o.fixtures = _fixtures_struct(observations, ptr)
-    o.home_goals, o.away_goals = ptr(observations["home_goals"]), ptr(observations["away_goals"])
+    o = _observations_struct(observations, ptr)
     gw = np.ascontiguousarray(gameweek, dtype=np.int32)
     keep.append(gw)
     return o, gw
@@ -776,16 +787,11 @@ def pointwise_loglik_gameweeks(model: str, samples: Dict[str, torch.Tensor], obs
     dev = samples["attack"].device
     workspace = _workspace(workspace, int(lib.bplx_pointwise_loglik_gameweeks_workspace_bytes(C.byref(s), G,
                                                                                               C.byref(o))), dev)
-    ld = 0
-    if want_matrix:
-        if loglik is None:
-            loglik = torch.empty((M, S), dtype=torch.float32, device=dev)
-        assert loglik.dtype == torch.float32 and loglik.shape[0] >= M and loglik.stride(1) == 1
-        ld = int(loglik.stride(0)) if M > 1 else max(S, int(loglik.shape[1]))
+    loglik, ld = _output_matrix(loglik, M, S, dev, want_matrix)
     stats = torch.empty((M, 4), dtype=torch.float64, device=dev)
-    _abi.check(lib.bplx_pointwise_loglik_gameweeks(C.byref(s), G, C.byref(o), gw32.ctypes.data,
-                                                   _dptr(loglik) if want_matrix else None, ld, _dptr(stats),
-                                                   _dptr(workspace), workspace.numel(), _stream_ptr(stream)))
+    _abi.check(lib.bplx_pointwise_loglik_gameweeks(C.byref(s), G, C.byref(o), gw32.ctypes.data, _dptr(loglik), ld,
+                                                   _dptr(stats), _dptr(workspace), workspace.numel(),
+                                                   _stream_ptr(stream)))
     ll = loglik[:M, :S] if want_matrix else None
     if not grouped:
         inv = torch.from_numpy(np.argsort(order, kind="stable")).to(dev)
@@ -808,22 +814,14 @@ def posterior_predictive_gameweeks(model: str, samples: Dict[str, torch.Tensor],
     keep = []
     s = _samples_struct(model, flat, _device_ptr_fn(keep))
     o, gw32 = _gw_observations(flat, observations, gameweek, keep)
-    M, T, B = o.fixtures.num_fixtures, s.num_teams, int(score_bins)
-    N = S * int(sims_per_draw)
+    B = int(score_bins)
     dev = samples["attack"].device
     workspace = _workspace(workspace, int(lib.bplx_posterior_predictive_gameweeks_workspace_bytes(C.byref(s), G,
                                                                                                   C.byref(o))), dev)
-    i32, i64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.int64, device=dev)
-    shapes = {"score_counts": ((N, B, B), i32), "outcome_counts": ((N, 3), i32), "goals": ((N, 2), i64),
-              "total_goals_sq": ((N,), i64), "team_points": ((N, T), i32), "team_goals_for": ((N, T), i32),
-              "team_goals_against": ((N, T), i32)}
-    res = {k: torch.empty(shp, **kw) for k, (shp, kw) in shapes.items()}
-    res["invalid"] = torch.empty(1, **i64)
-    res["scores"] = torch.empty((N, M, 2), dtype=torch.uint8, device=dev) if want_scores else None
-    out = _abi.PpcOutput(**{k: _dptr(v) for k, v in res.items()})
+    res, out = _ppc_outputs(S * int(sims_per_draw), o.fixtures.num_fixtures, s.num_teams, B, dev, want_scores)
     pw, pd = (int(x) for x in points)
     _abi.check(lib.bplx_posterior_predictive_gameweeks(C.byref(s), G, C.byref(o), gw32.ctypes.data, int(max_goals), B,
-                                                       pw, pd, int(sims_per_draw), int(seed) & 0xFFFFFFFFFFFFFFFF,
-                                                       int(first_draw), C.byref(out), _dptr(workspace),
-                                                       workspace.numel(), _stream_ptr(stream)))
+                                                       pw, pd, int(sims_per_draw), _seed(seed), int(first_draw),
+                                                       C.byref(out), _dptr(workspace), workspace.numel(),
+                                                       _stream_ptr(stream)))
     return res
